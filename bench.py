@@ -3,6 +3,7 @@
 
   python bench.py [--gpus N --steps K --warmup W]            our arm: native sm_100a hot path
   python bench.py --impl reference [...]                     the reference algorithm on the host CPU cores (oracle port)
+  python bench.py --dump-outputs DIR [...]                   also write what the last timed step computed to DIR/*.npy
 
 A "step" is one pass of the hot path over one synthetic batch of `--batch` faces per GPU (config 2 of BASELINE.json:
 bf16, batch 128, 16x16 -> 128x128 with parsing-map and landmark priors): bicubic 8x upsample of the uint8 LR faces,
@@ -130,8 +131,8 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    # bounded sample: every step is batch 4 (about 1-3 s of CPU work); at most 12 timed steps whatever --steps says
-    value, cores, sec, kind, what = cpu_reference_step_rate(max(1, min(args.steps, 12)), max(1, min(args.warmup, 2)))
+    # every step is batch 4 (about 1-3 s of CPU work)
+    value, cores, sec, kind, what = cpu_reference_step_rate(args.steps, args.warmup)
     line = {"impl": "reference", "metric": METRIC, "value": value, "unit": "images/s", "n_gpus": args.gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": sec * 1e3, "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -351,6 +352,26 @@ def verify_dp(torch, dist, world, rank, dev, per_rank=4, size=128):
     return {"rel_err_allreduced_vs_single_gpu": rel, "cosine": cos, "images": n, "ranks": world, "pass": bool(rel < 1e-3)}
 
 
+OUTPUT_SAMPLE = 1 << 18     # elements kept of each forward output: the dump stays under 64 MB (params + grads are ~56 MB)
+
+
+def dump_outputs(out_dir, trainer, losses, batch):
+    """Writes what the last step computed as float32 DIR/<name>.npy, so that two builds can be compared output for output:
+    the losses step() returned (total, L_sr, L_coarse, L_lm, L_ce), the flat parameter arena after the RMSprop update and
+    the gradient arena it applied, and - when one chunk holds the whole batch (the default), so that the trainer still
+    has them - the four forward outputs, each as the same seeded sample of OUTPUT_SAMPLE elements (flat index order)."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"losses": losses, "params": trainer.flat_p, "grads": trainer.flat_g}
+    if trainer.outs is not None and trainer.outs[0].shape[0] == batch:
+        for name, t in zip(("coarse", "sr", "landmark", "parsing"), trainer.outs):
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), min(OUTPUT_SAMPLE, t.numel()), replace=False))
+            arrays["out_" + name] = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -434,6 +455,8 @@ def run_ours(args):
 
     ms, launches, clocks, last = timed(step_resident, args.steps, args.warmup)
     loss_val = float(last[0].item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, trainer, last, B)
     ms_e2e, _, _, _ = timed(step_e2e, max(2, args.steps // 2), 1)
     value = world * B * args.steps / (ms * 1e-3)
     e2e = world * B * max(2, args.steps // 2) / (ms_e2e * 1e-3)
@@ -506,7 +529,13 @@ def main():
                                                            "gradient of the concatenated batch")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the matcher / KD-step secondary measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the losses, parameters, gradients and "
+                                                          "a fixed sample of the forward outputs of the last step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the native path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

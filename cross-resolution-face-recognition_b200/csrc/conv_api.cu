@@ -293,12 +293,12 @@ extern "C" int crfr_conv_wgrad(int engine, const crfr_conv_desc* d, const void* 
       CRFR_TRY(crfr_tc_wgrad(d, x, dy, dw, ws, ws_bytes, st));
     } else if (!d->transposed) {
       CRFR_TRY(crfr_direct_wgrad(d->n, d->h, d->w, d->oh, d->ow, d->k, d->stride, d->pad, dy, d->out_ld, d->cout, x,
-                                 d->in_ld, d->cin, dw, st));
+                                 d->in_ld, d->cin, dw, ws, ws_bytes, st));
     } else {
       CRFR_TRY(crfr_direct_wgrad(d->n, d->oh, d->ow, d->h, d->w, d->k, d->stride, d->pad, x, d->in_ld, d->cin, dy,
-                                 d->out_ld, d->cout, dw, st));
+                                 d->out_ld, d->cout, dw, ws, ws_bytes, st));
     }
   }
-  if (dbias) CRFR_TRY(crfr_colsum(dy, d->out_ld, d->cout, (long long)d->n * d->oh * d->ow, dbias, st));
+  if (dbias) CRFR_TRY(crfr_colsum(dy, d->out_ld, d->cout, (long long)d->n * d->oh * d->ow, dbias, ws, ws_bytes, st));
   return CRFR_OK;
 }

@@ -157,8 +157,9 @@ gather_up_kernel(Geo g, const bf16* __restrict__ small, int small_ld, const bf16
   store_result<COG>(acc, r0, R, pix, y, y_ld, y_nchw, n, by * g.bw + bx, g.bh * g.bw);
 }
 
-// G[(a*B + b)*T + tap] += sum_p small[p][a] * big[p*stride - pad + tap][b]
-// grid: (pixel chunks, taps, pair blocks); each thread owns up to MAXP (a, 4 consecutive b) pairs.
+// G[chunk][(a*B + b)*T + tap] = sum over the chunk's pixels p of small[p][a] * big[p*stride - pad + tap][b]
+// grid: (pixel chunks, taps, pair blocks); each thread owns up to MAXP (a, 4 consecutive b) pairs.  Every chunk stores its own
+// slice; sum_chunks_kernel adds the slices in chunk order (no float atomics: the same bits on every run).
 constexpr int kWgThreads = 256;
 constexpr int kMaxPairs = 4;
 __global__ void __launch_bounds__(kWgThreads)
@@ -181,6 +182,7 @@ wgrad_kernel(Geo g, const bf16* __restrict__ small, int small_ld, int A, const b
     for (int e = 0; e < 4; ++e) acc[m][e] = 0.f;
   }
   const long long npix = (long long)g.n * g.sh * g.sw;
+  G += (long long)blockIdx.x * A * B * T;
   const long long p0 = (long long)blockIdx.x * chunk_pix;
   const long long p1 = min(npix, p0 + (long long)chunk_pix);
   for (long long p = p0; p < p1; ++p) {
@@ -208,14 +210,14 @@ wgrad_kernel(Geo g, const bf16* __restrict__ small, int small_ld, int A, const b
     if (live[m]) {
 #pragma unroll
       for (int e = 0; e < 4; ++e)
-        if (pb[m] + e < B) atomicAdd(&G[((long long)pa[m] * B + pb[m] + e) * T + tap], acc[m][e]);
+        if (pb[m] + e < B) G[((long long)pa[m] * B + pb[m] + e) * T + tap] = acc[m][e];
     }
   }
 }
 
-// out[c] += sum over pixels of t[pix][c]
+// part[chunk][c] = sum over the chunk's pixels of t[pix][c]
 __global__ void __launch_bounds__(256)
-colsum_kernel(const bf16* __restrict__ t, int ld, int c_total, long long npix, int chunk_pix, float* __restrict__ out) {
+colsum_kernel(const bf16* __restrict__ t, int ld, int c_total, long long npix, int chunk_pix, float* __restrict__ part) {
   extern __shared__ float sm[];  // [lanes][c]
   // blockIdx.y selects a block of up to 256 channels
   const int coff = blockIdx.y * 256;
@@ -231,8 +233,30 @@ colsum_kernel(const bf16* __restrict__ t, int ld, int c_total, long long npix, i
   if (threadIdx.x < c) {
     float s = 0.f;
     for (int l = 0; l < lanes; ++l) s += sm[l * c + threadIdx.x];
-    atomicAdd(&out[coff + threadIdx.x], s);
+    part[(long long)blockIdx.x * c_total + coff + threadIdx.x] = s;
   }
+}
+
+// out[i] += sum over the chunks of part[chunk][i], in chunk order
+__global__ void sum_chunks_kernel(const float* __restrict__ part, int chunks, long long n, float* __restrict__ out) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  float s = out[i];
+  for (int k = 0; k < chunks; ++k) s += part[k * n + i];
+  out[i] = s;
+}
+
+// as many chunks of the pixel range as `want` asks for and the workspace holds `slice` floats each (at least one)
+long long fit_chunks(long long want, long long slice, size_t ws_bytes) {
+  const long long fit = (long long)(ws_bytes / (sizeof(float) * (size_t)slice));
+  return want < fit ? want : (fit > 1 ? fit : 1);
+}
+
+int sum_chunks(const float* part, long long chunks, long long n, float* out, cudaStream_t st) {
+  sum_chunks_kernel<<<crfr_cdiv(n, 256), 256, 0, st>>>(part, (int)chunks, n, out);
+  CRFR_COUNT_LAUNCH();
+  CRFR_LAUNCH_CHECK();
+  return CRFR_OK;
 }
 
 template <typename K>
@@ -276,7 +300,8 @@ int crfr_direct_gather(int down, int n, int bh, int bw, int sh, int sw, int k, i
 }
 
 int crfr_direct_wgrad(int n, int bh, int bw, int sh, int sw, int k, int stride, int pad, const void* small,
-                      int small_ld, int A, const void* big, int big_ld, int B, float* G, cudaStream_t st) {
+                      int small_ld, int A, const void* big, int big_ld, int B, float* G, void* ws, size_t ws_bytes,
+                      cudaStream_t st) {
   if ((big_ld & 3) != 0) {
     crfr_set_error("direct wgrad: big-side ld %d must be a multiple of 4", big_ld);
     return CRFR_EUNSUPPORTED;
@@ -290,26 +315,32 @@ int crfr_direct_wgrad(int n, int bh, int bw, int sh, int sw, int k, int stride, 
   long long want = (148LL * 16) / ((long long)T * pair_blocks) + 1;
   long long chunks = npix / 256 < 1 ? 1 : npix / 256;
   if (chunks > want) chunks = want;
+  const long long slice = (long long)A * B * T;
+  CRFR_CHECK_ARG(ws && ws_bytes >= sizeof(float) * (size_t)slice, "direct wgrad: workspace %zu < %zu", ws_bytes,
+                 sizeof(float) * (size_t)slice);
+  chunks = fit_chunks(chunks, slice, ws_bytes);
   int chunk_pix = (int)((npix + chunks - 1) / chunks);
   chunks = (npix + chunk_pix - 1) / chunk_pix;
   wgrad_kernel<<<dim3((unsigned)chunks, T, pair_blocks), kWgThreads, 0, st>>>(g, (const bf16*)small, small_ld, A,
                                                                                (const bf16*)big, big_ld, B,
-                                                                               chunk_pix, G);
+                                                                               chunk_pix, (float*)ws);
   CRFR_COUNT_LAUNCH();
   CRFR_LAUNCH_CHECK();
-  return CRFR_OK;
+  return sum_chunks((const float*)ws, chunks, slice, G, st);
 }
 
-int crfr_colsum(const void* t, int ld, int c, long long npix, float* out, cudaStream_t st) {
+int crfr_colsum(const void* t, int ld, int c, long long npix, float* out, void* ws, size_t ws_bytes, cudaStream_t st) {
+  CRFR_CHECK_ARG(ws && ws_bytes >= sizeof(float) * (size_t)c, "colsum: workspace %zu < %zu", ws_bytes, sizeof(float) * (size_t)c);
   long long chunks = npix / 512 < 1 ? 1 : npix / 512;
   if (chunks > 148 * 4) chunks = 148 * 4;
+  chunks = fit_chunks(chunks, c, ws_bytes);
   int chunk_pix = (int)((npix + chunks - 1) / chunks);
   chunks = (npix + chunk_pix - 1) / chunk_pix;
   const int cb = c < 256 ? c : 256;
   const int lanes = 256 / cb > 0 ? 256 / cb : 1;
   colsum_kernel<<<dim3((unsigned)chunks, (unsigned)((c + 255) / 256)), 256, sizeof(float) * lanes * cb, st>>>(
-      (const bf16*)t, ld, c, npix, chunk_pix, out);
+      (const bf16*)t, ld, c, npix, chunk_pix, (float*)ws);
   CRFR_COUNT_LAUNCH();
   CRFR_LAUNCH_CHECK();
-  return CRFR_OK;
+  return sum_chunks((const float*)ws, chunks, c, out, st);
 }

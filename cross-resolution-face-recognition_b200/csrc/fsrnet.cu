@@ -383,7 +383,7 @@ struct Net {
   void prologue(int B, int S) {
     for (int i = 0; i < CRFR_FSRNET_NPARAMS; ++i) packed_fwd[i] = packed_bwd[i] = nullptr;
     // shared scratch: norm partials / wgrad accumulators of the largest layer
-    scratch_bytes = crfr_norm_ws_bytes(B, S * S, 128) + sizeof(float) * 9 * 192 * 128 + 4096;
+    scratch_bytes = crfr_norm_ws_bytes(B, S * S, 128) + sizeof(float) * 9 * 192 * 128 + 4096 + crfr_tc_wgrad_part_bytes();
     {  // the lowered edge layers (lowered_conv.cu) stage their im2col / partial-product buffers here
       const crfr_conv_desc shapes[5] = {
           {B, S, S, 64, 64, 3, 1, 1, S, S, 64, 64, 0},          // residual stacks (row-streaming kernels' scratch)
@@ -691,11 +691,14 @@ struct Net {
           if (run()) {
             check(cudaMemsetAsync(G, 0, sizeof(float) * 128 * kHeadsPad, st) == cudaSuccess ? CRFR_OK : CRFR_ECUDA);
             TcWgrad wg{x.p, x.n, x.h, x.w, 128, x.ld, d_heads, kHeadsPad, kHeadsPad, 0, G};
+            const size_t part_off = (sizeof(float) * 128 * kHeadsPad + 255) & ~(size_t)255;
+            wg.part = (float*)((uint8_t*)scratch + part_off);
+            wg.part_bytes = scratch_bytes - part_off;
             check(crfr_tc_wgrad_raw(wg, st));
             heads_unpack_kernel<<<crfr_cdiv(108 * 128, 256), 256, 0, st>>>(G, grad(P_FC_W), grad(P_FCL_W));
             CRFR_COUNT_LAUNCH();
-            if (grad(P_FC_B)) check(crfr_colsum(d_heads, kHeadsPad, 11, npix, grad(P_FC_B), st));
-            if (grad(P_FCL_B)) check(crfr_colsum(d_heads + 11, kHeadsPad, 97, npix, grad(P_FCL_B), st));
+            if (grad(P_FC_B)) check(crfr_colsum(d_heads, kHeadsPad, 11, npix, grad(P_FC_B), scratch, scratch_bytes, st));
+            if (grad(P_FCL_B)) check(crfr_colsum(d_heads + 11, kHeadsPad, 97, npix, grad(P_FCL_B), scratch, scratch_bytes, st));
             check(cudaMemsetAsync(wt, 0, (size_t)128 * kHeadsPad * sizeof(bf16), st) == cudaSuccess ? CRFR_OK : CRFR_ECUDA);
             check(crfr_pack_weight_cols(params[P_FC_W], wt, 128, 11, kHeadsPad, 0, st));
             check(crfr_pack_weight_cols(params[P_FCL_W], wt, 128, 97, kHeadsPad, 11, st));
@@ -715,7 +718,8 @@ struct Net {
           if (is_coarse && has_grad(op.out)) {
             if (run() && grad(op.b_idx))
               for (const Slot& sl : slots[op.out.id])
-                check(crfr_colsum(sl.p, sl.ld, 3, (long long)op.cd.n * op.cd.h * op.cd.w, grad(op.b_idx), st));
+                check(crfr_colsum(sl.p, sl.ld, 3, (long long)op.cd.n * op.cd.h * op.cd.w, grad(op.b_idx), scratch, scratch_bytes,
+                                 st));
             if (g) add_slot(op.out, g, 4);
             squash(op.out, 1);
             g = slots[op.out.id][0].p;

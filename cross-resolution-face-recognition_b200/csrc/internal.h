@@ -108,8 +108,9 @@ int crfr_direct_gather(int down, int n, int bh, int bw, int sh, int sw, int k, i
                        int src_ld, const void* w, int R, int s_pad, const float* bias, void* y, int y_ld,
                        float* y_nchw, cudaStream_t st);
 int crfr_direct_wgrad(int n, int bh, int bw, int sh, int sw, int k, int stride, int pad, const void* small,
-                      int small_ld, int A, const void* big, int big_ld, int B, float* G, cudaStream_t st);
-int crfr_colsum(const void* t, int ld, int c, long long npix, float* out, cudaStream_t st);
+                      int small_ld, int A, const void* big, int big_ld, int B, float* G, void* ws, size_t ws_bytes, cudaStream_t st);
+// out[c] += sum over pixels of t[pix][c]; per-chunk partials in ws (at least c floats), summed in a fixed order
+int crfr_colsum(const void* t, int ld, int c, long long npix, float* out, void* ws, size_t ws_bytes, cudaStream_t st);
 
 // tc_conv.cu: generic tcgen05 launchers used by the lowered (im2col) edge layers
 struct TcGemm {           // out[pixel][n] = bias[n] + sum_{tap,k} src[pixel + sign*(tap - pad)][k] * w[tap][n][k]
@@ -127,13 +128,18 @@ struct TcGemm {           // out[pixel][n] = bias[n] + sum_{tap,k} src[pixel + s
   int stat_batch = 0;
 };
 int crfr_tc_gemm(const TcGemm& g, cudaStream_t st);
-struct TcWgrad {          // G[tap][ci][co] += sum_pixel x[pixel + tap - 1][ci] * dy[pixel][co]   (fp32, caller zeroes G)
+struct TcWgrad {          // G[tap][ci][co] = sum_pixel x[pixel + tap - 1][ci] * dy[pixel][co]   (fp32, G is overwritten)
   const void* x; int n, h, w, cin, x_ld;
   const void* dy; int cout, dy_ld;
   int taps3x3;            // 1: 3x3 pad 1 (9 taps), 0: single tap
   float* G;
+  // per-split partial sums, added into G in a fixed order (no float atomics): the pixel dimension is split only as far
+  // as this buffer holds; crfr_tc_wgrad_part_bytes() bytes always suffice for the full split
+  float* part = nullptr;
+  size_t part_bytes = 0;
 };
 int crfr_tc_wgrad_raw(const TcWgrad& g, cudaStream_t st);
+size_t crfr_tc_wgrad_part_bytes();
 
 // tc_conv.cu (tcgen05 engine).  op: 0 = forward, 1 = dgrad, 2 = wgrad
 int crfr_tc_supported(int op, int h, int w, int cin, int cout, int k, int stride, int pad);

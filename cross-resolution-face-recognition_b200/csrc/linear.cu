@@ -96,6 +96,6 @@ extern "C" int crfr_linear_bwd(const void* x, const void* dy, int batch, int hw,
     CRFR_COUNT_LAUNCH();
     CRFR_LAUNCH_CHECK();
   }
-  if (dbias) CRFR_TRY(crfr_colsum(dy, out, out, batch, dbias, st));
+  if (dbias) CRFR_TRY(crfr_colsum(dy, out, out, batch, dbias, ws, ws_bytes, st));
   return CRFR_OK;
 }

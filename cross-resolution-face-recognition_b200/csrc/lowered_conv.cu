@@ -460,6 +460,11 @@ struct Arena {
     off = a + bytes;
     return base + a;
   }
+  void rest(float** p, size_t* bytes) {   // everything not taken yet (the wgrad's partial sums)
+    const size_t a = (off + 1023) & ~(size_t)1023;
+    *p = a < cap ? (float*)(base + a) : nullptr;
+    *bytes = a < cap ? cap - a : 0;
+  }
 };
 
 #define TAKE(ptr, type, arena, bytes)                                              \
@@ -531,7 +536,7 @@ size_t crfr_lowered_ws_bytes(const crfr_conv_desc* d) {
     default: return 0;
   }
   if (r == 1 || r == 3 || r == 5) b += stat_partial_bytes(d) + 1024;
-  return b + 16 * 1024;
+  return b + 16 * 1024 + crfr_tc_wgrad_part_bytes() + 1024;   // + the wgrad's per-split partial sums
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -717,6 +722,7 @@ int crfr_lowered_wgrad(const crfr_conv_desc* d, const void* x, const void* dy, f
     CRFR_TRY(launch_im2col_small((const bf16*)x, d->n, d->h, d->w, d->oh, d->ow, d->k, d->stride, d->pad, 1, P, kp, st));
     CRFR_CUDA(cudaMemsetAsync(G, 0, (size_t)kp * d->cout * 4, st));
     TcWgrad g{P, d->n, d->oh, d->ow, kp, kp, dy, d->cout, d->out_ld, 0, G};
+    A.rest(&g.part, &g.part_bytes);
     CRFR_TRY(crfr_tc_wgrad_raw(g, st));
     LAUNCH(unpack_lowered_kernel, (long long)d->cout * 3 * T, st, G, d->cout, dw, d->cout, 3, T, 0);
     return CRFR_OK;
@@ -730,6 +736,7 @@ int crfr_lowered_wgrad(const crfr_conv_desc* d, const void* x, const void* dy, f
            d->stride, d->pad, P, opix * T * (d->cin / 8));
     CRFR_CUDA(cudaMemsetAsync(G, 0, (size_t)kc * d->cout * 4, st));
     TcWgrad g{P, d->n, d->oh, d->ow, kc, kc, dy, d->cout, d->out_ld, 0, G};
+    A.rest(&g.part, &g.part_bytes);
     CRFR_TRY(crfr_tc_wgrad_raw(g, st));
     LAUNCH(unpack_lowered_kernel, (long long)d->cout * d->cin * T, st, G, d->cout, dw, d->cout, d->cin, T, 0);
     return CRFR_OK;
@@ -741,6 +748,7 @@ int crfr_lowered_wgrad(const crfr_conv_desc* d, const void* x, const void* dy, f
     CRFR_TRY(launch_im2col_small((const bf16*)dy, d->n, d->h, d->w, d->h, d->w, 3, 1, 1, -1, R, 64, st));
     CRFR_CUDA(cudaMemsetAsync(G, 0, (size_t)64 * 64 * 4, st));
     TcWgrad g{x, d->n, d->h, d->w, 64, d->in_ld, R, 64, 64, 0, G};
+    A.rest(&g.part, &g.part_bytes);
     CRFR_TRY(crfr_tc_wgrad_raw(g, st));
     LAUNCH(unpack_lowered_kernel, (long long)3 * 64 * T, st, G, 64, dw, 3, 64, T, 1);
     return CRFR_OK;
@@ -752,6 +760,7 @@ int crfr_lowered_wgrad(const crfr_conv_desc* d, const void* x, const void* dy, f
     LAUNCH(deconv_shuffle_kernel, opix * 8, st, (bf16*)const_cast<void*>(dy), d->out_ld, All, d->h, d->w, 1, opix * 8);
     CRFR_CUDA(cudaMemsetAsync(G, 0, (size_t)9 * 64 * 1024 * 4, st));
     TcWgrad g{x, d->n, d->h, d->w, 64, d->in_ld, All, 1024, 1024, 1, G};
+    A.rest(&g.part, &g.part_bytes);
     CRFR_TRY(crfr_tc_wgrad_raw(g, st));
     LAUNCH(deconv_subpixel_unpack_kernel, 64 * 64 * 49, st, G, dw);
     return CRFR_OK;

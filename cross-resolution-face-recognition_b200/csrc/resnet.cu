@@ -473,7 +473,7 @@ struct Net {
               CRFR_COUNT_LAUNCH();
               check_cuda(cudaGetLastError());
             }
-            if (grad(op.b_idx)) check(crfr_colsum(dy.p, dy.ld, kEmb, B, grad(op.b_idx), st));
+            if (grad(op.b_idx)) check(crfr_colsum(dy.p, dy.ld, kEmb, B, grad(op.b_idx), scratch, scratch_bytes, st));
           }
           add_slot(a, da, K / (a.h * a.w));
           break;

@@ -11,7 +11,8 @@
 //   dgrad is the same kernel on dY with flipped tap offsets and [tap][cin][cout] weights.
 // Wgrad: D[(kx,ci)][co] = sum_pixels X[p + tap][ci] * dY[p][co]: both operands are MN-major views of the same
 //   NHWC tiles (pixels are the K dimension); two kx taps are stacked in M=128 through the leading-byte-offset of
-//   the smem descriptor; fp32 partial results are reduced into a [tap][cin][cout] scratch with vector atomics.
+//   the smem descriptor; each pixel split stores its fp32 partial result to its own [tap][cin][cout] slice and one
+//   pass sums the slices in split order (no float atomics: the weight gradient is the same bits on every run).
 //
 // ref: the nn.Conv2d sites of model/FSRnet.py (:79,85,110,114,351,387,411,432) that carry 99 % of the FLOPs.
 #include <cudaTypedefs.h>
@@ -411,7 +412,7 @@ struct WgradParams {
   int bw, bh, bn, tiles_x, tiles_y, total_tiles;
   int cin, cout;   // cout = all dY channels; a CTA handles columns [ntile * N, +N)
   int rows;        // pixels per tile (bw*bh*bn <= 128); rows beyond it are kept zero in shared memory
-  float* G;        // [taps][cin][cout] fp32, pre-zeroed
+  float* G;        // [gridDim.x][taps][cin][cout] fp32: one slice per split, every element stored once
 };
 
 constexpr int kTile16K = 128 * 128;
@@ -434,8 +435,8 @@ struct WgCfg {
   static constexpr int kSmemBytes = kStages * kStageBytes + 1024 + 256;
 };
 
-__device__ __forceinline__ void red_add_v4(float* addr, float a, float b, float c, float d) {
-  asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(addr), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
+__device__ __forceinline__ void st_v4(float* addr, float a, float b, float c, float d) {
+  asm volatile("st.global.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(addr), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
 }
 
 template <int N, int TAPS, bool H>
@@ -475,6 +476,7 @@ tc_wgrad_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
 
   // TAPS == 3: blockIdx.y = ky (H: kx) + 3 * column tile;  TAPS == 1: blockIdx.y = column tile of dY
   const int ky = TAPS == 3 ? blockIdx.y % 3 : 0, kc = blockIdx.z;
+  float* const G = p.G + (long long)blockIdx.x * (TAPS == 3 ? 9 : 1) * p.cin * p.cout;   // this split's slice
   const int ncol0 = (TAPS == 3 ? blockIdx.y / 3 : blockIdx.y) * N;
   const uint32_t stage_tx = H ? (uint32_t)((p.bh + 2) * p.bw + Cfg::kDyTiles * p.rows) * 128u
                               : (uint32_t)(TAPS + Cfg::kDyTiles) * (uint32_t)p.rows * 128u;
@@ -564,11 +566,10 @@ tc_wgrad_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
         tmem_ld_wait();
         const int a = c0 / 64;
         const int tap = H ? a * 3 + ky : ky * 3 + a;
-        float* dst = p.G + ((long long)tap * p.cin + kc * 64 + (c0 & 63)) * p.cout + ncol0 + co;
+        float* dst = G + ((long long)tap * p.cin + kc * 64 + (c0 & 63)) * p.cout + ncol0 + co;
         if (live) {
 #pragma unroll
-          for (int j = 0; j < 32; ++j)
-            asm volatile("red.global.add.f32 [%0], %1;" ::"l"(dst + (long long)j * p.cout), "f"(__uint_as_float(v[j])) : "memory");
+          for (int j = 0; j < 32; ++j) dst[(long long)j * p.cout] = __uint_as_float(v[j]);
         }
       }
     } else
@@ -577,7 +578,7 @@ tc_wgrad_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
       const int kx = half == 0 ? (r >> 6) : 2;                          // (H: this is the tap's ky, and `ky` its kx)
       const bool live = TAPS == 3 ? (half == 0 || r < 64) : (r < 64);   // warp-uniform (32-row granularity)
       const int tap = TAPS == 3 ? (H ? kx * 3 + ky : ky * 3 + kx) : 0;
-      float* dst = p.G + ((long long)tap * p.cin + ci) * p.cout + ncol0;
+      float* dst = G + ((long long)tap * p.cin + ci) * p.cout + ncol0;
 #pragma unroll
       for (int c0 = 0; c0 < N; c0 += 32) {
         uint32_t v[32];
@@ -586,8 +587,8 @@ tc_wgrad_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
         if (live) {
 #pragma unroll
           for (int j = 0; j < 32; j += 4)
-            red_add_v4(dst + c0 + j, __uint_as_float(v[j]), __uint_as_float(v[j + 1]), __uint_as_float(v[j + 2]),
-                       __uint_as_float(v[j + 3]));
+            st_v4(dst + c0 + j, __uint_as_float(v[j]), __uint_as_float(v[j + 1]), __uint_as_float(v[j + 2]),
+                  __uint_as_float(v[j + 3]));
         }
       }
     }
@@ -598,6 +599,18 @@ tc_wgrad_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
     tc_fence_after();
     tmem_dealloc<Cfg::kTmemCols>(tmem);
   }
+}
+
+// G[i] = sum of the `splits` partial slices in split order (a fixed order: the same bits on every run)
+__global__ void wgrad_split_sum_kernel(const float4* __restrict__ part, int splits, long long slice4, float4* __restrict__ G) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= slice4) return;
+  float4 s = part[i];
+  for (int k = 1; k < splits; ++k) {
+    const float4 v = part[k * slice4 + i];
+    s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
+  }
+  G[i] = s;
 }
 
 // dW[co][ci][t] += G[t][ci][co]
@@ -718,6 +731,26 @@ int crfr_tc_gemm(const TcGemm& g, cudaStream_t st) {
   return CRFR_EUNSUPPORTED;
 }
 
+namespace {
+int launch_wgrad_any(const TcWgrad& g, const Tiling& t, const CUtensorMap& tmX, const CUtensorMap& tmDY, const WgradParams& p,
+                     int splits, cudaStream_t st) {
+  if (g.taps3x3) {
+    if (t.bn == 1 && (t.bh + 2) * t.bw <= 256 && (g.cout == 64 || g.cout % 128 == 0)) {
+      CUtensorMap tmXh;   // the X box with its two halo rows
+      CRFR_TRY(make_act_map(&tmXh, g.x, g.n, g.h, g.w, g.cin, g.x_ld, t.bw, t.bh + 2, 1));
+      if (g.cout == 64) return launch_wgrad<64, 3, true>(tmXh, tmDY, p, splits, st);
+      return launch_wgrad<128, 3, true>(tmXh, tmDY, p, splits, st);
+    }
+    if (g.cout == 64) return launch_wgrad<64, 3>(tmX, tmDY, p, splits, st);
+    if (g.cout % 128 == 0) return launch_wgrad<128, 3>(tmX, tmDY, p, splits, st);
+    crfr_set_error("tc_wgrad: 3x3 needs cout 64 or a multiple of 128, got %d", g.cout);
+    return CRFR_EUNSUPPORTED;
+  }
+  if (g.cout % 128 == 0) return launch_wgrad<128, 1>(tmX, tmDY, p, splits, st);
+  return launch_wgrad<64, 1>(tmX, tmDY, p, splits, st);
+}
+}  // namespace
+
 int crfr_tc_wgrad_raw(const TcWgrad& g, cudaStream_t st) {
   CRFR_CHECK_ARG(((uintptr_t)g.x & 15) == 0 && ((uintptr_t)g.dy & 15) == 0 && (g.x_ld & 7) == 0 && (g.dy_ld & 7) == 0,
                  "tc_wgrad: pointers must be 16B aligned and ld a multiple of 8");
@@ -734,7 +767,7 @@ int crfr_tc_wgrad_raw(const TcWgrad& g, cudaStream_t st) {
   p.n = g.n; p.h = g.h; p.w = g.w;
   p.bw = t.bw; p.bh = t.bh; p.bn = t.bn; p.tiles_x = t.tiles_x; p.tiles_y = t.tiles_y;
   p.total_tiles = t.tiles_x * t.tiles_y * t.tiles_n;
-  p.cin = g.cin; p.cout = g.cout; p.G = g.G;
+  p.cin = g.cin; p.cout = g.cout;
   p.rows = t.rows;
   const int tile_n = (g.cout % 128 == 0) ? 128 : 64;
   const int ctas_per_split = (g.taps3x3 ? 3 : 1) * (g.cout / tile_n) * (g.cin / 64);
@@ -745,20 +778,24 @@ int crfr_tc_wgrad_raw(const TcWgrad& g, cudaStream_t st) {
   if (splits < 1) splits = ctas_per_split <= sms ? sms / ctas_per_split : 1;
   if (splits > p.total_tiles) splits = p.total_tiles;
   if (splits < 1) splits = 1;
-  if (g.taps3x3) {
-    if (t.bn == 1 && (t.bh + 2) * t.bw <= 256 && (g.cout == 64 || g.cout % 128 == 0)) {
-      CUtensorMap tmXh;   // the X box with its two halo rows
-      CRFR_TRY(make_act_map(&tmXh, g.x, g.n, g.h, g.w, g.cin, g.x_ld, t.bw, t.bh + 2, 1));
-      if (g.cout == 64) return launch_wgrad<64, 3, true>(tmXh, tmDY, p, splits, st);
-      return launch_wgrad<128, 3, true>(tmXh, tmDY, p, splits, st);
-    }
-    if (g.cout == 64) return launch_wgrad<64, 3>(tmX, tmDY, p, splits, st);
-    if (g.cout % 128 == 0) return launch_wgrad<128, 3>(tmX, tmDY, p, splits, st);
-    crfr_set_error("tc_wgrad: 3x3 needs cout 64 or a multiple of 128, got %d", g.cout);
-    return CRFR_EUNSUPPORTED;
+  // several splits store their partials into g.part and are summed into G afterwards; as many as fit (one: straight into G)
+  const long long slice = (long long)(g.taps3x3 ? 9 : 1) * g.cin * g.cout;
+  const long long fit = g.part ? (long long)(g.part_bytes / (sizeof(float) * (size_t)slice)) : 0;
+  if (splits > fit) splits = fit > 1 ? (int)fit : 1;
+  CRFR_CHECK_ARG(splits == 1 || ((uintptr_t)g.part & 15) == 0, "tc_wgrad: partial buffer must be 16B aligned");
+  p.G = splits > 1 ? g.part : g.G;
+  CRFR_TRY(launch_wgrad_any(g, t, tmX, tmDY, p, splits, st));
+  if (splits > 1) {
+    wgrad_split_sum_kernel<<<crfr_cdiv(slice / 4, 256), 256, 0, st>>>((const float4*)g.part, splits, slice / 4, (float4*)g.G);
+    CRFR_COUNT_LAUNCH();
+    CRFR_LAUNCH_CHECK();
   }
-  if (tile_n == 128) return launch_wgrad<128, 1>(tmX, tmDY, p, splits, st);
-  return launch_wgrad<64, 1>(tmX, tmDY, p, splits, st);
+  return CRFR_OK;
+}
+
+size_t crfr_tc_wgrad_part_bytes() {
+  // splits x slice <= 2 * SMs x (3 tap rows x 64 cin x 128 cout per CTA) floats whatever the shape (see crfr_tc_wgrad_raw)
+  return sizeof(float) * (size_t)2 * conv_sm_count() * 3 * 64 * 128 + 256;
 }
 
 int crfr_tc_supported(int op, int h, int w, int cin, int cout, int k, int stride, int pad) {
@@ -774,7 +811,8 @@ int crfr_tc_supported(int op, int h, int w, int cin, int cout, int k, int stride
 }
 
 size_t crfr_tc_workspace_bytes(const crfr_conv_desc* d) {
-  size_t wg = sizeof(float) * (size_t)d->k * d->k * d->cin * d->cout + 256;  // wgrad scratch
+  // wgrad: the [tap][cin][cout] result + the per-split partial sums
+  size_t wg = sizeof(float) * (size_t)d->k * d->k * d->cin * d->cout + 256 + crfr_tc_wgrad_part_bytes();
   {   // statistics partials of the fused epilogue: [n][tiles per image x 4][2][cout]
     Tiling t;
     if (make_tiling(d->n, d->oh, d->ow, &t)) {
@@ -840,6 +878,9 @@ int crfr_tc_wgrad(const crfr_conv_desc* d, const void* x, const void* dy, float*
   TcWgrad g;
   g.x = x; g.n = d->n; g.h = d->h; g.w = d->w; g.cin = d->cin; g.x_ld = d->in_ld;
   g.dy = dy; g.cout = d->cout; g.dy_ld = d->out_ld; g.taps3x3 = 1; g.G = (float*)ws;
+  const size_t part_off = (need + 255) & ~(size_t)255;
+  g.part = ws_bytes > part_off ? (float*)((uint8_t*)ws + part_off) : nullptr;
+  g.part_bytes = ws_bytes > part_off ? ws_bytes - part_off : 0;
   CRFR_TRY(crfr_tc_wgrad_raw(g, st));
   long long total = (long long)d->cout * d->cin * 9;
   wgrad_unpack_kernel<<<crfr_cdiv(total, 256), 256, 0, st>>>((const float*)ws, dw, d->cin, d->cout, 9);

@@ -19,6 +19,7 @@ from oracle import ref_loader as R           # noqa: E402
 from oracle import resnet_oracle as RO       # noqa: E402
 
 OUT = os.path.join(os.path.dirname(HERE), "tests", "golden")
+GRAD_SAMPLE = 8192          # elements stored of each large full-gradient tensor in fsrnet_small.npz
 
 
 def ref_fsrnet(seed):
@@ -77,7 +78,12 @@ def golden_fsrnet():
             for k in ("_coarse_sr_network.residual.0.conv1.weight", "_fine_sr_decoder.deconv.weight",
                       "_prior_estimation_network.hg.hg.0.0.0.conv1.weight", "_fine_sr_encoder.conv_input.weight",
                       "_fine_sr_decoder.conv_out.weight", "_prior_estimation_network.fc_landmark.weight"):
-                d["grad:" + k] = dict(net.named_parameters())[k].grad.numpy()
+                a = dict(net.named_parameters())[k].grad.numpy()
+                if a.size > 2 * GRAD_SAMPLE:      # keeps the fixture under 1 MB: a seeded sample plus its flat indices
+                    idx = np.sort(np.random.default_rng(0).choice(a.size, GRAD_SAMPLE, replace=False))
+                    a = a.reshape(-1)[idx]
+                    d["gidx:" + k] = idx.astype(np.int32)
+                d["grad:" + k] = a
         else:
             d.update(out_mean=outs[1].mean().item(), out_std=outs[1].std().item(), coarse_mean=outs[0].mean().item())
         np.savez_compressed(os.path.join(OUT, "fsrnet_%s.npz" % tag), **d)

@@ -55,6 +55,8 @@ def test_fsrnet_forward_backward_small(golden_dir):
         if k.startswith("grad:") and k[5:] not in FO.FSRNET_NULL_GRAD:
             ref = torch.from_numpy(g[k])
             got = gd[k[5:]]
+            if "gidx:" + k[5:] in g.files:          # large gradients are stored as a fixed sample of their elements
+                got = got.reshape(-1)[torch.from_numpy(g["gidx:" + k[5:]]).long()]
             assert ((got - ref).norm() / (ref.norm() + 1e-30)).item() < 2e-2, k
 
 
