@@ -124,6 +124,9 @@ SIGNATURES = {
     "crfr_kd_train_step": (ci, [ci, vp, vp, vp, vp, vp, vp, vp, vp, C.POINTER(KdIO), vp, vp, csz, vp]),
     "crfr_ir50_workspace_bytes": (csz, [ci, ci]),
     "crfr_ir50_forward": (ci, [ci, vp, vp, C.POINTER(ResnetIO), vp, csz, vp]),
+    "crfr_ir50_grad_workspace_bytes": (csz, [ci, ci]),
+    "crfr_ir50_tape": (ci, [ci, ci, C.POINTER(TapeEntry), ci]),
+    "crfr_ir50_backward": (ci, [ci, vp, vp, C.POINTER(ResnetIO), vp, vp, vp, vp, csz, vp]),
     "crfr_resnet34_backward": (ci, [ci, vp, vp, C.POINTER(ResnetIO), vp, vp, vp, csz, vp]),
 }
 

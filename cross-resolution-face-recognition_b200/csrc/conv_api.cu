@@ -33,7 +33,7 @@ const OptDef kOpts[CRFR_OPT_COUNT] = {
     {"norm_bwd_impl", "CRFR_NORM_BWD", 1},    {"norm_fwd_stream", "CRFR_NORM_FWD_STREAM", 1},
     {"rowwgrad_pair", "CRFR_ROWWGRAD_PAIR", 1}, {"fuse_norm_bwd", "CRFR_FUSE_NORM_BWD", 1},
     {"fuse_norm_fwd", "CRFR_FUSE_NORM_FWD", 0}, {"pdl", "CRFR_PDL", 0}, {"tc_t2", "CRFR_TC_T2", 1}, {"bn_fused_stats", "CRFR_BN_FUSED_STATS", 1}, {"matcher_cluster", "CRFR_MATCHER_CLUSTER", 1},
-    {"pair_debug", "CRFR_PAIR_DEBUG", 0}};
+    {"pair_debug", "CRFR_PAIR_DEBUG", 0}, {"ir50_stem_tc", "CRFR_IR50_STEM_TC", 1}};
 std::atomic<int> g_opt[CRFR_OPT_COUNT];
 std::atomic<int> g_opt_init{0};
 void opts_init() {

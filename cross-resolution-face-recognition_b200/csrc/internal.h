@@ -11,7 +11,7 @@
 
 // ---- process-wide tuning switches (conv_api.cu).  Every setting computes the same results; they exist for A/B
 // measurements and debugging.  Defaults come from the environment (CRFR_ROWCONV, CRFR_ROWCONV_PAIR, CRFR_PAIR_SWAP,
-// CRFR_WGRAD_STREAM, CRFR_NORM_BWD=regs|stream, CRFR_NORM_FWD_STREAM) once; crfr_set_option overrides atomically.
+// CRFR_WGRAD_STREAM, CRFR_NORM_BWD=regs|stream, CRFR_NORM_FWD_STREAM, ...) once; crfr_set_option overrides atomically.
 enum {
   CRFR_OPT_ROWCONV = 0,      // row-streaming kernels for 64 -> 64 convolutions at width 128 (else the tile engine)
   CRFR_OPT_ROWCONV_PAIR,     // cta_group::2 form of the row-streaming forward / dgrad kernel (even image counts)
@@ -28,6 +28,7 @@ enum {
   CRFR_OPT_MATCHER_CLUSTER,  // cosine_topk: gallery blocks multicast inside clusters of two CTAs
   CRFR_OPT_PAIR_DEBUG,       // ablation bits for tools/pair_diag.py (results are WRONG when set): 1 no loads, 2 no MMAs,
                              // 4 no pack / store / statistics, 8 no store, 16 no statistics
+  CRFR_OPT_IR50_STEM_TC,     // IR_50 input gradient: stem dgrad on the tcgen05 GEMM (else the direct kernel)
   CRFR_OPT_COUNT
 };
 int crfr_opt(int id);
@@ -53,13 +54,17 @@ struct CUtensorMap_st;
 int crfr_tmap_encode_bf16(CUtensorMap_st* m, const void* ptr, int rank, const unsigned long long* dims,
                           const unsigned long long* strides_bytes, const unsigned int* box, const char* what);
 
-// layout.cu: dst[t][r][s] (bf16, s padded to s_pad) = src[r * rs + s * ss + t] for a list of jobs, 64 per launch
+// layout.cu: dst[t][r][s] (bf16, s padded to s_pad) = src[r * rs + s * ss + t] (* rscale[r]) (* sscale[s]) for a list of
+// jobs, 64 per launch.  The optional fp32 scales fold a per-channel factor (an eval-mode BatchNorm's gamma * rstd) into the
+// weights before the one rounding to bf16.
 #define CRFR_PACK_BATCH 64
 struct crfr_pack_job {
   const float* src; void* dst;
   int T, R, S, s_pad;
   long long rs, ss;
   int block0, reserved;   // filled by the launcher
+  const float* rscale = nullptr;
+  const float* sscale = nullptr;
 };
 struct crfr_pack_batch {
   crfr_pack_job job[CRFR_PACK_BATCH];
@@ -165,6 +170,10 @@ int crfr_lowered_dgrad(const crfr_conv_desc* d, const void* dy, const void* w_pa
                        size_t ws_bytes, cudaStream_t st);
 int crfr_lowered_wgrad(const crfr_conv_desc* d, const void* x, const void* dy, float* dw, void* ws, size_t ws_bytes,
                        cudaStream_t st);
+// dgrad of recipe 1's shape (3-channel input, 3x3 s1) on the tcgen05 GEMM; crfr_conv_dgrad keeps the direct kernel there
+size_t crfr_lowered_dgrad_cin3_ws_bytes(const crfr_conv_desc* d);
+int crfr_lowered_dgrad_cin3(const crfr_conv_desc* d, const void* dy, const void* w_packed_t, void* dx, void* ws,
+                            size_t ws_bytes, cudaStream_t st);
 
 // rowconv.cu: persistent row-streaming kernel for 3x3 64->64 convolutions at width 128
 int crfr_rowconv_supported(int h, int w, int cin, int cout, int k, int stride, int pad);

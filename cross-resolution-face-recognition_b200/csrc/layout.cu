@@ -97,7 +97,12 @@ __global__ void pack_weight_batch_kernel(const __grid_constant__ crfr_pack_batch
   const int s = (int)(i % J.s_pad);
   const long long q = i / J.s_pad;
   const int r = (int)(q % J.R), t = (int)(q / J.R);
-  const float v = (s < J.S) ? J.src[r * J.rs + s * J.ss + t] : 0.f;
+  float v = 0.f;
+  if (s < J.S) {
+    v = J.src[r * J.rs + s * J.ss + t];
+    if (J.rscale) v *= J.rscale[r];
+    if (J.sscale) v *= J.sscale[s];
+  }
   reinterpret_cast<bf16*>(J.dst)[i] = __float2bfloat16_rn(v);
 }
 

@@ -267,7 +267,7 @@ col2im3_s1_kernel(const float* __restrict__ src, int h, int w, int sgn, const fl
                   float* __restrict__ y_nchw, bf16* __restrict__ y, int y_ld) {
   constexpr int TH = 8, TW = 32, SH = TH + 2, SW = TW + 2, LD = 33;
   __shared__ float tile[SH * SW * LD];
-  const int tiles_x = w / TW, tiles_y = h / TH;
+  const int tiles_x = (w + TW - 1) / TW, tiles_y = h / TH;   // a last partial column tile when w % 32 != 0
   int b = blockIdx.x;
   const int tx0 = (b % tiles_x) * TW;
   b /= tiles_x;
@@ -296,6 +296,7 @@ col2im3_s1_kernel(const float* __restrict__ src, int h, int w, int sgn, const fl
       for (int c = 0; c < 3; ++c) acc[c] += t[c];
     }
   const int Y = ty0 + ly, X = tx0 + lx;
+  if (X >= w) return;
   if (y_nchw)
 #pragma unroll
     for (int c = 0; c < 3; ++c) y_nchw[((n * 3 + c) * h + Y) * w + X] = acc[c];
@@ -704,6 +705,34 @@ int crfr_lowered_dgrad(const crfr_conv_desc* d, const void* dy, const void* w_pa
   }
   crfr_set_error("lowered dgrad: no recipe for this shape");
   return CRFR_EUNSUPPORTED;
+}
+
+// dgrad of recipe 1's shape (3x3 s1 p1, 3 -> cout channels), a 3x3 cout -> 3 convolution of dY: recipe 2's forward GEMM
+// with the transposed pack [tap][ci(3)][cout] as its weight rows (tap*3 + ci), then the col2im over the taps in the
+// opposite direction.  dX[q][ci] = sum_tap Q[q + (pad - tap)][tap*3 + ci],  Q[p][tap*3 + ci] = sum_co dY[p][co] W[co][ci][tap]
+size_t crfr_lowered_dgrad_cin3_ws_bytes(const crfr_conv_desc* d) {
+  return (size_t)d->n * d->h * d->w * 32 * 4 + (size_t)32 * 64 * 2 + 4096;
+}
+
+int crfr_lowered_dgrad_cin3(const crfr_conv_desc* d, const void* dy, const void* w_packed_t, void* dx, void* ws,
+                            size_t ws_bytes, cudaStream_t st) {
+  if (crfr_lowered_recipe(d) != 1 || d->cout != 64 || d->out_ld != 64 || d->h % 8) {
+    crfr_set_error("lowered dgrad (3-channel input): unsupported shape");
+    return CRFR_EUNSUPPORTED;
+  }
+  Arena A{(uint8_t*)ws, ws_bytes, 0};
+  const long long pix = (long long)d->n * d->h * d->w;
+  TAKE(Q, float, A, (size_t)pix * 32 * 4);
+  TAKE(Wq, bf16, A, (size_t)32 * 64 * 2);
+  CRFR_CUDA(cudaMemsetAsync(Wq, 0, (size_t)32 * 64 * 2, st));
+  CRFR_CUDA(cudaMemcpyAsync(Wq, w_packed_t, (size_t)27 * 64 * 2, cudaMemcpyDeviceToDevice, st));
+  TcGemm g{dy, d->n, d->h, d->w, 64, d->out_ld, Wq, 1, 0, 1, 32, 32, Q, 32, 1, nullptr};
+  CRFR_TRY(crfr_tc_gemm(g, st));
+  col2im3_s1_kernel<<<(unsigned)(d->n * (d->h / 8) * ((d->w + 31) / 32)), 256, 0, st>>>(Q, d->h, d->w, 1, nullptr, nullptr,
+                                                                                       (bf16*)dx, d->in_ld);
+  CRFR_COUNT_LAUNCH();
+  CRFR_LAUNCH_CHECK();
+  return CRFR_OK;
 }
 
 // ---------------------------------------------------------------------------------------------------------

@@ -8,8 +8,10 @@
 // head as a tcgen05 GEMM over the NHWC-flattened feature (weights re-ordered from the reference's NCHW flatten), and
 // BatchNorm1d on the embedding.
 //
-// The frozen IR_50 teacher (DISTILLATION/model/model_irse.py) is a second, forward-only program over the same ops:
-// BN -> conv3x3 -> PReLU -> conv3x3(stride) -> BN, plus a MaxPool2d(1, stride) / conv1x1+BN shortcut, 24 blocks.
+// The frozen IR_50 teacher (DISTILLATION/model/model_irse.py) is a second program over the same ops:
+// BN -> conv3x3 -> PReLU -> conv3x3(stride) -> BN, plus a MaxPool2d(1, stride) / conv1x1+BN shortcut, 24 blocks.  Its
+// backward (backward_ir50) is the gradient with respect to the input image only: eval-mode BatchNorm couples no images,
+// so it is a per-sample linear map of dgrads, per-channel scales and PReLU masks.
 //
 // ref: model/resnet.py:18-47 (BasicBlock), :152-225 (ResNet.__init__/_make_layer/forward), :231-236 (ResNet_34);
 //      DISTILLATION/model/model_irse.py:49-66 (bottleneck_IR), :103-110 (get_blocks(50)), :129-172 (Backbone).
@@ -31,12 +33,12 @@ struct Slot {
   bf16* p;
   int ld;
 };
-enum OpKind { OP_CONV, OP_BN, OP_LINEAR };
+enum OpKind { OP_CONV, OP_BN, OP_LINEAR, OP_PRELU, OP_SUB2 };
 struct Op {
   OpKind kind;
   Tensor a, b, out;
   crfr_conv_desc cd;
-  int w_idx = -1, b_idx = -1, g_idx = -1, beta_idx = -1;
+  int w_idx = -1, b_idx = -1, g_idx = -1, beta_idx = -1, alpha_idx = -1;
   int cin_pad = 0;
   float* stats = nullptr;
   bool relu = false, has_res = false, x_needs_grad = true;
@@ -44,16 +46,21 @@ struct Op {
 
 constexpr int kFeat = 512, kEmb = 512;
 
-// W [o][c*HW + hw] (fp32, reference flatten order) -> Wp [o][hw*C + c] and WpT [hw*C + c][o] (bf16)
+// W [o][c*HW + hw] (fp32, reference flatten order) -> Wp [o][hw*C + c] and WpT [hw*C + c][o] (bf16); the optional fp32
+// scales o_scale[o] and c_scale[c] multiply the weight before its rounding (BatchNorm scales folded into the input gradient)
 __global__ void linear_pack_kernel(const float* __restrict__ w, bf16* __restrict__ wp, bf16* __restrict__ wpt, int O,
-                                   int C, int HW) {
+                                   int C, int HW, const float* __restrict__ o_scale = nullptr,
+                                   const float* __restrict__ c_scale = nullptr) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const long long K = (long long)C * HW;
   if (i >= (long long)O * K) return;
   const int o = (int)(i / K);
   const long long k = i - (long long)o * K;       // hw*C + c
   const int hw = (int)(k / C), c = (int)(k - (long long)hw * C);
-  const bf16 v = __float2bfloat16_rn(w[(long long)o * K + (long long)c * HW + hw]);
+  float f = w[(long long)o * K + (long long)c * HW + hw];
+  if (o_scale) f *= o_scale[o];
+  if (c_scale) f *= c_scale[c];
+  const bf16 v = __float2bfloat16_rn(f);
   if (wp) wp[i] = v;
   if (wpt) wpt[k * O + o] = v;
 }
@@ -93,6 +100,73 @@ __global__ void identity_stats_kernel(float* __restrict__ stats, int c) {
   }
 }
 
+// s[c] = gamma[c] * rstd[c]: the scale of an eval-mode BatchNorm (stats [c][2] = (mean, rstd))
+__global__ void bn_scale_kernel(const float* __restrict__ stats, const float* __restrict__ gamma, int c,
+                                float* __restrict__ s) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < c) s[i] = gamma[i] * stats[2 * i + 1];
+}
+
+// Element-wise input-gradient pass of the IR_50 backward (eval-mode BatchNorm and / or PReLU, plus a second gradient):
+//   out[p][c] = s[c] * act'(s[c] * y[p][c] + t[c]) * g[p][c] (+ add)
+// with s = gamma * rstd, t = beta - mean * s computed as the forward's normalise kernel does (no stats: s = 1, t = 0),
+// act' = 1 where z > 0 and alpha[c] elsewhere (no alpha: identity; no y: act' = 1, the pass is a plain sum).
+// add_mode 1 adds add[p][c]; 2 adds the gradient of a stride-2 pixel subsampling (MaxPool2d(1, 2)), i.e. add at the
+// half-resolution pixel for the even pixels and nothing elsewhere - a gather, so no atomics.  One thread per 8 channels
+// of a pixel (16-byte loads and store), fp32 arithmetic, one rounding.  out may alias g (each element is read, then
+// written, by the same thread).
+__global__ void __launch_bounds__(256)
+ir50_bwd_ew_kernel(const bf16* g, int g_ld, const bf16* __restrict__ y, int y_ld, const float* __restrict__ stats,
+                   const float* __restrict__ gamma, const float* __restrict__ beta, const float* __restrict__ alpha,
+                   const bf16* __restrict__ add, int add_ld, int add_mode, bf16* out, int out_ld, int h, int w, int groups,
+                   long long total) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= total) return;
+  const int cg = (int)(i % groups);
+  const long long p = i / groups;
+  float v[8];
+  unpack8(*reinterpret_cast<const bf16x8*>(g + p * g_ld + cg * 8), v);
+  if (y) {
+    float f[8];
+    unpack8(*reinterpret_cast<const bf16x8*>(y + p * y_ld + cg * 8), f);
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      const int ch = cg * 8 + j;
+      float sc = 1.f, sh = 0.f;
+      if (stats) {
+        sc = gamma[ch] * stats[2 * ch + 1];
+        sh = beta[ch] - stats[2 * ch] * sc;
+      }
+      const float z = fmaf(f[j], sc, sh);
+      v[j] *= (alpha && !(z > 0.f)) ? sc * alpha[ch] : sc;
+    }
+  }
+  if (add_mode == 1) {
+    float a[8];
+    unpack8(*reinterpret_cast<const bf16x8*>(add + p * add_ld + cg * 8), a);
+#pragma unroll
+    for (int j = 0; j < 8; ++j) v[j] += a[j];
+  } else if (add_mode == 2) {
+    const int x = (int)(p % w);
+    const long long q = p / w;
+    const int yy = (int)(q % h);
+    const long long n = q / h;
+    if (((x | yy) & 1) == 0) {
+      const long long ps = (n * (h / 2) + yy / 2) * (w / 2) + x / 2;
+      float a[8];
+      unpack8(*reinterpret_cast<const bf16x8*>(add + ps * add_ld + cg * 8), a);
+#pragma unroll
+      for (int j = 0; j < 8; ++j) v[j] += a[j];
+    }
+  }
+  *reinterpret_cast<bf16x8*>(out + p * out_ld + cg * 8) = pack8(v);
+}
+
+// tape indices of one bottleneck_IR unit of the IR_50 program (-1: absent)
+struct IrUnit {
+  int sc_conv = -1, sc_bn = -1, sub = -1, bn0, conv1, prelu, conv2, bn4;
+};
+
 struct Net {
   int engine;
   const float* const* params;
@@ -116,6 +190,8 @@ struct Net {
   bf16* wp = nullptr;    // packed linear weights (forward)
   bf16* wpt = nullptr;   // transposed (backward)
   int pcur = 0, bncur = 0;
+  std::vector<IrUnit> ir_units;               // IR_50: the 24 units, and the stem / head ops, as tape indices
+  int ir_stem_conv = -1, ir_stem_bn = -1, ir_head_bn0 = -1, ir_head_lin = -1, ir_head_bn1 = -1;
 
   void* alloc(size_t bytes) {
     size_t a = (off + 1023) & ~(size_t)1023;
@@ -206,7 +282,8 @@ struct Net {
     }
     Op op;
     op.kind = OP_BN;
-    op.a = y; op.out = out; op.stats = stats; op.g_idx = g_idx; op.beta_idx = g_idx + 1; op.relu = relu != 0;
+    op.a = y; op.out = out; op.stats = stats; op.g_idx = g_idx; op.beta_idx = g_idx + 1; op.alpha_idx = alpha_idx;
+    op.relu = relu != 0;
     op.has_res = res != nullptr;
     if (res) op.b = *res;
     tape.push_back(op);
@@ -305,12 +382,17 @@ struct Net {
     to_nchw(emb, io->emb);
   }
 
-  // ---- IR_50 (forward only, eval-mode BatchNorm) ----
+  // ---- IR_50 (eval-mode BatchNorm) ----
+  int last() const { return (int)tape.size() - 1; }
   Tensor prelu(const Tensor& y, int alpha_idx, float* ident) {   // plain PReLU pass
     Tensor out = new_tensor(y.n, y.h, y.w, y.c);
     if (run())
       check(crfr_norm_act_fwd(y.p, y.ld, ident, nullptr, nullptr, params[alpha_idx], 0, nullptr, 8, out.p, out.ld, 1,
                               y.n * y.h * y.w, y.c, st));
+    Op op;
+    op.kind = OP_PRELU;
+    op.a = y; op.out = out; op.alpha_idx = alpha_idx;
+    tape.push_back(op);
     return out;
   }
   Tensor subsample2(const Tensor& x) {
@@ -321,6 +403,10 @@ struct Net {
       CRFR_COUNT_LAUNCH();
       check_cuda(cudaGetLastError());
     }
+    Op op;
+    op.kind = OP_SUB2;
+    op.a = x; op.out = out;
+    tape.push_back(op);
     return out;
   }
 
@@ -339,6 +425,8 @@ struct Net {
     Tensor x4 = new_tensor(B, S, S, 3);
     if (run()) check(crfr_nchw_f32_to_nhwc_bf16(io->x, x4.p, B, 3, S, S, 4, 4, st));
     Tensor a = bn(conv(x4, 0, 64, 3, 1, 1, false), 1, 0, nullptr, 3, 0);     // input_layer: conv, BN, PReLU
+    ir_stem_conv = last() - 1; ir_stem_bn = last();
+    ir_units.clear();
     int p = 10, bi = 3;
     const int units[4] = {3, 4, 14, 3}, depth[4] = {64, 128, 256, 512};
     int in_ch = 64;
@@ -346,17 +434,25 @@ struct Net {
       for (int u = 0; u < units[l]; ++u) {   // bottleneck_IR, model_irse.py:49-66
         const int stride = u == 0 ? 2 : 1, d = depth[l];
         const bool conv_sc = in_ch != d;
+        IrUnit un;
         Tensor sc = a;
         if (conv_sc) {
           sc = bn(conv(a, p, d, 1, stride, 0, false), p + 1, 0, nullptr, -1, bi);
+          un.sc_conv = last() - 1; un.sc_bn = last();
           p += 3; bi += 1;
         } else if (stride == 2) {
           sc = subsample2(a);
+          un.sub = last();
         }
         Tensor r = bn(a, p, 0, nullptr, -1, bi);                       // res_layer.0
+        un.bn0 = last();
         r = prelu(conv(r, p + 2, d, 3, 1, 1, false), p + 3, ident);    // res_layer.1, .2
+        un.conv1 = last() - 1; un.prelu = last();
         r = conv(r, p + 4, d, 3, stride, 1, false);                    // res_layer.3
+        un.conv2 = last();
         a = bn(r, p + 5, 0, &sc, -1, bi + 1);                          // res_layer.4 + shortcut
+        un.bn4 = last();
+        ir_units.push_back(un);
         p += 7; bi += 2;
         in_ch = d;
         if (u == units[l] - 1) {   // stage output: 64@56^2, 128@28^2, 256@14^2, 512@7^2 - the shapes of ResNet_34's x1..x4,
@@ -365,8 +461,11 @@ struct Net {
         }
       }
     Tensor o = bn(a, 4, 0, nullptr, -1, 1);                            // output_layer.0 (Dropout: identity in eval)
+    ir_head_bn0 = last();
     Tensor y = linear(o, 6);                                           // output_layer.3
+    ir_head_lin = last();
     emb = bn(y, 8, 0, nullptr, -1, 2);                                 // output_layer.4 (BatchNorm1d)
+    ir_head_bn1 = last();
     to_nchw(emb, io->emb);
   }
 
@@ -386,6 +485,148 @@ struct Net {
       if (b > m) m = b;
     }
     return m + 4096;
+  }
+
+  // ---- IR_50 input gradient (after a forward_ir50 over the same arena; parameters stay frozen) ----
+  Tensor map_like(const Tensor& t) { return Tensor{(bf16*)alloc((size_t)t.n * t.h * t.w * t.ld * sizeof(bf16)), t.n, t.h, t.w, t.c, t.ld}; }
+  float* bn_scale(const Op& b) {
+    float* s = (float*)alloc((size_t)b.a.c * sizeof(float));
+    if (run()) {
+      bn_scale_kernel<<<crfr_cdiv(b.a.c, 128), 128, 0, st>>>(b.stats, params[b.g_idx], b.a.c, s);
+      CRFR_COUNT_LAUNCH();
+      check_cuda(cudaGetLastError());
+    }
+    return s;
+  }
+  // transposed pack [tap][cin][cout] of a convolution, with the optional folded scales (rscale: cin, sscale: cout)
+  bf16* dgrad_pack(const Op& cv, const float* rscale, const float* sscale, std::vector<crfr_pack_job>& jobs) {
+    const crfr_conv_desc& d = cv.cd;
+    const int T = d.k * d.k;
+    bf16* wt = (bf16*)alloc((size_t)T * d.cin * d.cout * sizeof(bf16));
+    crfr_pack_job j{params ? params[cv.w_idx] : nullptr, wt, T, d.cin, d.cout, d.cout, T, (long long)d.cin * T, 0, 0, rscale, sscale};
+    jobs.push_back(j);
+    return wt;
+  }
+  void dgrad(const Op& cv, const Slot& dy, const bf16* wt, const Tensor& dx, bool stem = false) {
+    crfr_conv_desc d = cv.cd;
+    d.out_ld = dy.ld;
+    d.in_ld = dx.ld;
+    if (!run()) return;
+    if (stem && engine != CRFR_ENGINE_DIRECT && crfr_opt(CRFR_OPT_IR50_STEM_TC) && crfr_lowered_recipe(&d) == 1 &&
+        d.cout == 64 && d.h % 8 == 0)
+      check(crfr_lowered_dgrad_cin3(&d, dy.p, wt, dx.p, scratch, scratch_bytes, st));
+    else
+      check(crfr_conv_dgrad(engine, &d, dy.p, wt, d.cout, dx.p, scratch, scratch_bytes, st));
+  }
+  // out = s * act'(z) * g (+ add): see ir50_bwd_ew_kernel; bn (may be null) supplies stats / gamma / beta
+  void ew(const Slot& g, const Tensor& y, const Op* bn, int alpha_idx, const Slot* add, int add_mode, const Tensor& out) {
+    if (!run()) return;
+    const float* alpha = alpha_idx >= 0 ? params[alpha_idx] : nullptr;
+    const long long total = (long long)out.n * out.h * out.w * (out.c / 8);
+    ir50_bwd_ew_kernel<<<crfr_cdiv(total, 256), 256, 0, st>>>(
+        g.p, g.ld, y.p, y.ld, bn ? bn->stats : nullptr, bn ? params[bn->g_idx] : nullptr,
+        bn ? params[bn->beta_idx] : nullptr, alpha, add ? add->p : nullptr, add ? add->ld : 8, add_mode, out.p, out.ld,
+        out.h, out.w, out.c / 8, total);
+    CRFR_COUNT_LAUNCH();
+    check_cuda(cudaGetLastError());
+  }
+
+  // Per unit, from the unit's output gradient g: res_layer.4's scale is folded into res_layer.3's dgrad weights and
+  // res_layer.0's into res_layer.1's, the shortcut BatchNorm's into its 1x1 convolution, output_layer.0's and the
+  // BatchNorm1d's into the transposed linear weights; what remains element-wise (PReLU masks, the stem's BatchNorm +
+  // PReLU, the gradient sum at each unit's input) is ir50_bwd_ew_kernel.
+  void backward_ir50(const float* d_emb, const float* const* d_feat, float* dx) {
+    const int B = io->batch;
+    size_t need = crfr_lowered_dgrad_cin3_ws_bytes(&tape[ir_stem_conv].cd);
+    for (const Op& op : tape)
+      if (op.kind == OP_CONV) {
+        const size_t b = crfr_conv_workspace_bytes(&op.cd);
+        if (b > need) need = b;
+      }
+    if (need > scratch_bytes) {   // the forward's scratch is reused where it is large enough
+      scratch_bytes = need;
+      scratch = alloc(need);
+    }
+    // folded scales and weight packs, all issued before the walk (one batched pack launch)
+    std::vector<crfr_pack_job> jobs;
+    std::vector<bf16*> w1(ir_units.size()), w2(ir_units.size()), wsc(ir_units.size(), nullptr);
+    for (size_t u = 0; u < ir_units.size(); ++u) {
+      const IrUnit& U = ir_units[u];
+      w2[u] = dgrad_pack(tape[U.conv2], nullptr, bn_scale(tape[U.bn4]), jobs);
+      w1[u] = dgrad_pack(tape[U.conv1], bn_scale(tape[U.bn0]), nullptr, jobs);
+      if (U.sc_conv >= 0) wsc[u] = dgrad_pack(tape[U.sc_conv], nullptr, bn_scale(tape[U.sc_bn]), jobs);
+    }
+    bf16* w0 = dgrad_pack(tape[ir_stem_conv], nullptr, nullptr, jobs);
+    const Op& lin = tape[ir_head_lin];
+    const Tensor& a4 = tape[ir_head_bn0].a;
+    const int K = a4.h * a4.w * a4.c;
+    bf16* wlt = nullptr;
+    if (d_emb) {
+      const float* s_o0 = bn_scale(tape[ir_head_bn0]);
+      const float* s_emb = bn_scale(tape[ir_head_bn1]);
+      wlt = (bf16*)alloc((size_t)kEmb * K * sizeof(bf16));
+      if (run()) {
+        const long long total = (long long)kEmb * K;
+        linear_pack_kernel<<<crfr_cdiv(total, 256), 256, 0, st>>>(params[lin.w_idx], nullptr, wlt, kEmb, a4.c,
+                                                                  a4.h * a4.w, s_emb, s_o0);
+        CRFR_COUNT_LAUNCH();
+        check_cuda(cudaGetLastError());
+      }
+    }
+    if (run()) check(crfr_pack_weight_batch(jobs.data(), (int)jobs.size(), st));
+
+    // head: d a4 = s_o0 * W^T (s_emb * d_emb)
+    if (d_emb) {
+      seed_grad(emb, d_emb);
+      const Slot de = slots[emb.id][0];
+      Tensor da = map_like(a4);
+      if (run()) {
+        TcGemm g{de.p, B, 1, 1, kEmb, de.ld, wlt, 1, 0, 1, K, 0, da.p, K, 0, nullptr};
+        check(crfr_tc_gemm(g, st));
+      }
+      add_slot(a4, da.p, da.ld);
+    }
+    for (int l = 0; l < 4; ++l) seed_grad(feat[l], d_feat ? d_feat[l] : nullptr);
+
+    for (int u = (int)ir_units.size() - 1; u >= 0 && ok(); --u) {
+      const IrUnit& U = ir_units[u];
+      const Op& b4 = tape[U.bn4];
+      const Op& pr = tape[U.prelu];
+      const Tensor& in = tape[U.bn0].a;
+      if (!has_grad(b4.out)) continue;
+      squash(b4.out, 1);
+      const Slot g = slots[b4.out.id][0];
+      Tensor d_r2 = map_like(pr.out);
+      dgrad(tape[U.conv2], g, w2[u], d_r2);                               // res_layer.4 + .3
+      const Slot s_r2{d_r2.p, d_r2.ld};
+      ew(s_r2, pr.a, nullptr, pr.alpha_idx, nullptr, 0, d_r2);     // res_layer.2, in place
+      Tensor d_in = map_like(in);
+      dgrad(tape[U.conv1], s_r2, w1[u], d_in);                            // res_layer.1 + .0
+      const Slot s_in{d_in.p, d_in.ld};
+      if (U.sc_conv >= 0) {                                                // conv1x1 + BN shortcut
+        Tensor d_sc = map_like(in);
+        dgrad(tape[U.sc_conv], g, wsc[u], d_sc);
+        const Slot s_sc{d_sc.p, d_sc.ld};
+        ew(s_in, Tensor{}, nullptr, -1, &s_sc, 1, d_in);
+      } else {                                                             // identity / MaxPool2d(1, 2)
+        ew(s_in, Tensor{}, nullptr, -1, &g, U.sub >= 0 ? 2 : 1, d_in);
+      }
+      add_slot(in, d_in.p, d_in.ld);
+    }
+
+    // stem: BatchNorm + PReLU, then the dgrad of the 3 -> 64 convolution into the 4-channel input
+    const Op& sb = tape[ir_stem_bn];
+    const Op& s0 = tape[ir_stem_conv];
+    if (!has_grad(sb.out)) {
+      if (run()) check_cuda(cudaMemsetAsync(dx, 0, sizeof(float) * (size_t)B * 3 * io->size * io->size, st));
+      return;
+    }
+    squash(sb.out, 1);
+    Tensor dy0 = map_like(sb.a);
+    ew(slots[sb.out.id][0], sb.a, &sb, sb.alpha_idx, nullptr, 0, dy0);
+    Tensor dx4 = map_like(s0.a);
+    dgrad(s0, Slot{dy0.p, dy0.ld}, w0, dx4, true);
+    if (run()) check(crfr_nhwc_bf16_to_nchw_f32(dx4.p, dx, B, 3, dx4.h, dx4.w, dx4.ld, st));
   }
 
   // ---- backward ----
@@ -518,19 +759,15 @@ extern "C" size_t crfr_resnet34_workspace_bytes(int batch, int size, int trainin
 // entry per recorded op in program order - kind 0 convolution, 1 BatchNorm (+ residual) (+ ReLU), 7 linear head; out_off /
 // in_off / stats_off are bytes from the workspace base.  The parity tests read the stored bf16 activations through this
 // table and replay them into the CPU oracle (teacher-forced forward / backward checks, tests/test_resnet_forced_gpu.py).
-extern "C" int crfr_resnet34_tape(int batch, int size, int training, crfr_tape_entry* entries, int max_entries) {
-  if (batch <= 0 || size != 112) return -1;
-  crfr_resnet_io io = {};
-  io.batch = batch; io.size = size; io.training = training; io.momentum = 0.1f; io.eps = 1e-5f;
-  Net net;
-  init_net(net, CRFR_ENGINE_AUTO, nullptr, nullptr, nullptr, &io, nullptr, ~(size_t)0 >> 2, nullptr, false);
-  net.forward();
+namespace {
+// kinds: 0 convolution, 1 BatchNorm (+ residual) (+ ReLU / PReLU), 7 linear head, 8 PReLU pass, 9 stride-2 subsampling
+int fill_tape(const Net& net, crfr_tape_entry* entries, int max_entries) {
   const int count = (int)net.tape.size();
   for (int i = 0; i < count && i < max_entries && entries; ++i) {
     const Op& op = net.tape[i];
     crfr_tape_entry& e = entries[i];
     const Tensor& t = op.out;
-    e.kind = op.kind == OP_CONV ? 0 : (op.kind == OP_BN ? 1 : 7);
+    e.kind = op.kind == OP_CONV ? 0 : op.kind == OP_BN ? 1 : op.kind == OP_LINEAR ? 7 : op.kind == OP_PRELU ? 8 : 9;
     e.n = t.n; e.h = t.h; e.w = t.w; e.c = t.c; e.ld = t.ld;
     e.out_off = t.p ? (long long)((uint8_t*)t.p - (uint8_t*)nullptr) : -1;
     e.in_off = op.a.p ? (long long)((uint8_t*)op.a.p - (uint8_t*)nullptr) : -1;
@@ -539,6 +776,29 @@ extern "C" int crfr_resnet34_tape(int batch, int size, int training, crfr_tape_e
     e.has_res = op.has_res ? 1 : 0;
   }
   return count;
+}
+}  // namespace
+
+extern "C" int crfr_resnet34_tape(int batch, int size, int training, crfr_tape_entry* entries, int max_entries) {
+  if (batch <= 0 || size != 112) return -1;
+  crfr_resnet_io io = {};
+  io.batch = batch; io.size = size; io.training = training; io.momentum = 0.1f; io.eps = 1e-5f;
+  Net net;
+  init_net(net, CRFR_ENGINE_AUTO, nullptr, nullptr, nullptr, &io, nullptr, ~(size_t)0 >> 2, nullptr, false);
+  net.forward();
+  return fill_tape(net, entries, max_entries);
+}
+
+// The same table for the IR_50 program (eval mode): every stored tensor of crfr_ir50_forward in program order, for the
+// teacher-forced parity test of its input gradient (tests/test_ir50_grad_gpu.py).
+extern "C" int crfr_ir50_tape(int batch, int size, crfr_tape_entry* entries, int max_entries) {
+  if (batch <= 0 || size != 112) return -1;
+  crfr_resnet_io io = {};
+  io.batch = batch; io.size = size; io.training = 0; io.momentum = 0.1f; io.eps = 1e-5f;
+  Net net;
+  init_net(net, CRFR_ENGINE_AUTO, nullptr, nullptr, nullptr, &io, nullptr, ~(size_t)0 >> 2, nullptr, false);
+  net.forward_ir50();
+  return fill_tape(net, entries, max_entries);
 }
 
 extern "C" int crfr_resnet34_forward(int engine, const float* const* host_params, void* const* host_buffers,
@@ -703,6 +963,40 @@ extern "C" int crfr_ir50_forward(int engine, const float* const* host_params, vo
   Net net;
   init_net(net, engine, host_params, nullptr, host_buffers, io, ws, ws_bytes, (cudaStream_t)stream, true);
   net.forward_ir50();
+  return net.err;
+}
+
+// forward arena of crfr_ir50_workspace_bytes (same layout), then the input-gradient buffers
+extern "C" size_t crfr_ir50_grad_workspace_bytes(int batch, int size) {
+  if (batch <= 0 || size != 112) return 0;
+  crfr_resnet_io io = {};
+  io.batch = batch; io.size = size; io.training = 0; io.momentum = 0.1f; io.eps = 1e-5f;
+  static float dummy = 0.f;   // non-null marker so that the dry run sizes every optional buffer
+  const float* feats[4] = {&dummy, &dummy, &dummy, &dummy};
+  Net net;
+  init_net(net, CRFR_ENGINE_AUTO, nullptr, nullptr, nullptr, &io, nullptr, ~(size_t)0 >> 2, nullptr, false);
+  net.forward_ir50();
+  net.backward_ir50(&dummy, feats, &dummy);
+  return net.off + 65536;
+}
+
+extern "C" int crfr_ir50_backward(int engine, const float* const* host_params, void* const* host_buffers,
+                                  const crfr_resnet_io* io, const float* d_emb, const float* const* d_feat, float* dx,
+                                  void* ws, size_t ws_bytes, void* stream) {
+  CRFR_TRY(check_io(io, "ir50_backward"));
+  CRFR_CHECK_ARG(host_params && dx && ws, "ir50_backward: null pointer");
+  CRFR_CHECK_ARG(!io->training, "ir50_backward: the forward must have run in eval mode");
+  const size_t need = crfr_ir50_grad_workspace_bytes(io->batch, io->size);
+  if (ws_bytes < need) {
+    crfr_set_error("ir50_backward: workspace %zu < %zu (crfr_ir50_grad_workspace_bytes)", ws_bytes, need);
+    return CRFR_EWORKSPACE;
+  }
+  Net net;
+  init_net(net, engine, host_params, nullptr, host_buffers, io, ws, ws_bytes, (cudaStream_t)stream, false);
+  net.forward_ir50();   // dry run: rebuild the tape and the saved-activation offsets
+  if (!net.ok()) return net.err;
+  net.exec = true;
+  net.backward_ir50(d_emb, d_feat, dx);
   return net.err;
 }
 

@@ -1,4 +1,4 @@
-"""Drop-in IR_50 teacher backed by the native sm_100a network program (forward only).
+"""Drop-in IR_50 teacher backed by the native sm_100a network program (forward, and the gradient w.r.t. the input).
 
 Mirror of the reference's DISTILLATION/model/model_irse.py for the configuration distill_main.py:14,201 uses
 (``IR_50([112, 112])``): same class names (``Backbone``, ``bottleneck_IR``, ``Flatten``, ``l2_norm``, ``get_blocks``),
@@ -9,12 +9,24 @@ teacher checkpoint loads) and construction + initialisation order.  The torch la
 The teacher is frozen and evaluated in ``eval()`` mode by the reference (distill_main.py:43, 112-114); only that mode
 is native: train-mode Dropout (model_irse.py:144) is stochastic and has no parity definition, so ``forward`` in
 training mode raises.  The SE variants and the 100/152-layer variants are not on the hot path.
+
+When ``x.requires_grad`` (and grad mode is on), ``forward`` / ``forward_features`` are differentiable with respect to
+``x`` through ``crfr_ir50_backward``, so that IR_50 can drive an identity or perceptual loss on a super-resolved face
+(SUPER_RESOLUTION/train_FHN.py:255-265)::
+
+    sr = fsrnet(x)[1][:, :, 8:120, 8:120]
+    f_sr, f_hr = ir50.forward_features(sr), ir50.forward_features(hr)
+    loss = pixel_loss + sum(F.mse_loss(a, b) for a, b in zip(f_sr, f_hr))
+    loss.backward()          # reaches fsrnet's parameters through IR_50
+
+IR_50's own parameters stay frozen: they never receive a ``.grad``, even with ``requires_grad=True``.
 """
 import ctypes as C
 from collections import namedtuple
 
 import torch
 import torch.nn as nn
+from torch.autograd.function import once_differentiable
 from torch.nn import BatchNorm1d, BatchNorm2d, Conv2d, Dropout, Linear, MaxPool2d, Module, PReLU, Sequential
 
 from .. import _lib as L
@@ -111,7 +123,7 @@ class Backbone(Module):
                 if m.bias is not None:
                     m.bias.data.zero_()
 
-    def _run(self, x, want_features):
+    def _check(self, x):
         if not self._native:
             raise NotImplementedError("only IR_50([112, 112]) has a native network program")
         if self.training:
@@ -121,7 +133,9 @@ class Backbone(Module):
             raise RuntimeError("crfr_b200 IR_50 needs a CUDA tensor: the hot path has no CPU fallback")
         if x.dim() != 4 or tuple(x.shape[1:]) != (3, 112, 112):
             raise ValueError("expected [B,3,112,112], got %s" % (tuple(x.shape),))
-        x = x.contiguous().float()
+
+    def _launch(self, x, want_features, ws=None):
+        """crfr_ir50_forward into ``ws`` (default: the shared workspace) -> (emb, feats, tables, io)."""
         b = x.shape[0]
         emb = torch.empty((b, 512), dtype=torch.float32, device=x.device)
         feats = [torch.empty((b, c, s, s), dtype=torch.float32, device=x.device)
@@ -134,12 +148,22 @@ class Backbone(Module):
         for i, f in enumerate(feats):
             io.feat[i] = f.data_ptr()
         io.training, io.momentum, io.eps = 0, 0.1, 1e-5
-        ws = ops.workspace(L.lib().crfr_ir50_workspace_bytes(b, 112))
+        if ws is None:
+            ws = ops.workspace(L.lib().crfr_ir50_workspace_bytes(b, 112))
         L.call("crfr_ir50_forward", self.engine, ptab.arr, btab.arr, C.byref(io), ws.data_ptr(), ws.numel(), ops.stream())
+        return emb, feats, (ptab, btab), io
+
+    def _run(self, x, want_features):
+        self._check(x)
+        if torch.is_grad_enabled() and x.requires_grad:
+            outs = _IR50InputGrad.apply(self, want_features, x)
+            return outs[0], list(outs[1:])
+        emb, feats, _, _ = self._launch(x.contiguous().float(), want_features)
         return emb, feats
 
     def forward(self, x):
-        """ref: model_irse.py:167-172: the embedding only."""
+        """ref: model_irse.py:167-172: the embedding only.  Differentiable with respect to ``x`` when
+        ``x.requires_grad``; the parameters never receive a gradient."""
         return self._run(x, False)[0]
 
     def forward_features(self, x):
@@ -148,6 +172,38 @@ class Backbone(Module):
         (perceptual features, SUPER_RESOLUTION/train_FHN.py:255-265)."""
         emb, feats = self._run(x, True)
         return (emb,) + tuple(feats)
+
+
+class _IR50InputGrad(torch.autograd.Function):
+    """IR_50 forward whose backward is the native input gradient (``crfr_ir50_backward``).  The forward runs in a private
+    workspace that keeps the saved activations for the backward; the parameters are constants of this function."""
+
+    @staticmethod
+    def forward(ctx, net, want_features, x):
+        x = x.detach().contiguous().float()
+        ws = torch.empty(L.lib().crfr_ir50_grad_workspace_bytes(x.shape[0], 112), dtype=torch.uint8, device=x.device)
+        emb, feats, tables, io = net._launch(x, want_features, ws)
+        ctx.set_materialize_grads(False)
+        ctx.saved = (net.engine, tables, io, ws, x)   # x: io.x points at it
+        return (emb,) + tuple(feats)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, d_emb, *d_feats):
+        engine, (ptab, btab), io, ws, x = ctx.saved
+        keep = []
+
+        def ptr(g):
+            if g is None:
+                return None
+            g = g.contiguous().float()
+            keep.append(g)
+            return g.data_ptr()
+        dfeat = (C.c_void_p * 4)(*([ptr(g) for g in d_feats] + [None] * (4 - len(d_feats))))
+        dx = torch.empty_like(x)
+        L.call("crfr_ir50_backward", engine, ptab.arr, btab.arr, C.byref(io), ptr(d_emb), dfeat, dx.data_ptr(),
+               ws.data_ptr(), ws.numel(), ops.stream())
+        return None, None, dx
 
 
 def IR_50(input_size):

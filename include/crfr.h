@@ -49,7 +49,9 @@ unsigned long long crfr_launch_count(void);
  *   "fuse_norm_bwd": crfr_conv_dgrad_norm_bwd as 0 = dgrad + crfr_norm_act_bwd, 1 = first pass of the normalisation
  *                    backward inside the dgrad epilogue where the row-streaming pair kernel runs (default).
  *   "norm_fwd_stream": crfr_norm_act_fwd as 0 = register-staged kernel, 1 = persistent TMA-fed kernel (default where the
- *                    views are TMA-addressable); identical results bit for bit. */
+ *                    views are TMA-addressable); identical results bit for bit.
+ *   "ir50_stem_tc":  crfr_ir50_backward, dgrad of the 3 -> 64 stem convolution as 1 = im2col-free tcgen05 GEMM + col2im
+ *                    (default), 0 = the direct CUDA-core kernel; equal up to the order of the fp32 sums. */
 int crfr_set_option(const char* name, int value);
 /* debugging aid (tools/pair_diag.py): cycle counters of the last rowconv pair-kernel launch made with option
  * "pair_debug" bit 32; 16 counters per cluster */
@@ -390,7 +392,7 @@ int crfr_kd_train_step(int engine, const float* const* teacher_params, void* con
                        float* const* assistant_grads, const crfr_kd_io* io, float* losses, void* ws, size_t ws_bytes,
                        void* stream);
 
-/* ---------------------------------------------------------------- IR_50 teacher (forward only) -------------- */
+/* ---------------------------------------------------------------- IR_50 teacher ----------------------------- */
 #define CRFR_IR50_NPARAMS 187 /* named_parameters() order of DISTILLATION/model/model_irse.py:IR_50 */
 #define CRFR_IR50_NBN 54      /* BatchNorm layers in module order (input_layer, output_layer, body) */
 /* ref: Backbone.forward model_irse.py:167-172 in eval mode (the frozen teacher of distill_main.py:43,201): returns the
@@ -399,6 +401,21 @@ int crfr_kd_train_step(int engine, const float* const* teacher_params, void* con
 size_t crfr_ir50_workspace_bytes(int batch, int size);
 int crfr_ir50_forward(int engine, const float* const* host_params, void* const* host_buffers,
                       const crfr_resnet_io* io, void* ws, size_t ws_bytes, void* stream);
+/* ref: autograd through Backbone.forward model_irse.py:167-172 in eval mode, with respect to the input image only (an
+ * identity / perceptual loss on the features of a super-resolved face, SUPER_RESOLUTION/train_FHN.py:255-265).
+ * crfr_ir50_grad_workspace_bytes: the forward arena (the same layout as crfr_ir50_workspace_bytes) plus the backward
+ * buffers.  crfr_ir50_backward: ws holds a crfr_ir50_forward of the same io over a workspace of at least that size;
+ * d_emb [B,512] and d_feat[k] (the shapes of io->feat[k]) are fp32 upstream gradients, any of them NULL; dx [B,3,112,112]
+ * fp32 is overwritten.  No parameter gradient is computed.  The saved forward is not modified: repeated calls give the
+ * same bits. */
+size_t crfr_ir50_grad_workspace_bytes(int batch, int size);
+/* Layout of the stored forward tensors of crfr_ir50_forward (dry run), as crfr_resnet34_tape: kind 0 convolution,
+ * 1 BatchNorm (+ residual) (+ PReLU at the stem), 7 linear head, 8 PReLU pass, 9 stride-2 subsampling (MaxPool2d(1, 2)).
+ * For teacher-forced parity tests. */
+int crfr_ir50_tape(int batch, int size, crfr_tape_entry* entries, int max_entries);
+int crfr_ir50_backward(int engine, const float* const* host_params, void* const* host_buffers,
+                       const crfr_resnet_io* io, const float* d_emb, const float* const* d_feat, float* dx, void* ws,
+                       size_t ws_bytes, void* stream);
 
 #ifdef __cplusplus
 }

@@ -1,0 +1,172 @@
+"""Throughput of IR_50([112, 112]) forward and forward + input gradient (crfr_ir50_backward) at the KD batch size.
+
+Usage: python tools/bench_ir50_grad.py [--batch 256] [--iters 20] [--warmup 3]
+
+Times, with CUDA events after warm-up and in one process:
+  * forward only (no grad: the shared-workspace path) and forward + input gradient (autograd path, all five outputs seeded),
+    reported as images/s and GFLOP/s with the FLOPs counted from the layer shapes below;
+  * the backward alone, with the stem's dgrad on the tcgen05 GEMM (option "ir50_stem_tc" = 1) and on the direct kernel
+    (= 0), alternated; their difference is the difference of the two stem paths;
+  * the direct stem dgrad by itself (crfr_conv_dgrad on the stem's shape);
+  * each stem path's own kernels inside the backward, from torch.profiler in a separate pass: the device time of the
+    kernels (and copies) between the last element-wise backward kernel and the final NHWC -> NCHW conversion of dx.
+Prints the device name and power limit, then one JSON line.  Writes nothing.
+"""
+import argparse
+import ctypes as C
+import json
+import os
+import subprocess
+import sys
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+
+
+def ir50_flops_per_image():
+    """(forward FLOPs, input-gradient FLOPs) per 112x112 image: 2 * MACs of every convolution and of the linear head.
+    The input gradient runs one dgrad of the same size per convolution and per linear layer (element-wise passes not
+    counted)."""
+    from oracle.resnet_oracle import ir50_block_specs
+    macs, s = 112 * 112 * 64 * 3 * 9, 112      # stem 3x3 3 -> 64
+    for cin, d, stride in ir50_block_specs():
+        so = s // stride
+        macs += s * s * d * cin * 9             # res_layer.1: 3x3 s1 at the input resolution
+        macs += so * so * d * d * 9             # res_layer.3: 3x3, stride
+        if cin != d:
+            macs += so * so * d * cin           # shortcut 1x1 s2
+        s = so
+    macs += 512 * 7 * 7 * 512                   # output_layer.3
+    return 2.0 * macs, 2.0 * macs
+
+
+def kernel_name(sig):
+    """'void (anonymous namespace)::foo<3>(float const*, ...)' -> 'foo'"""
+    return sig.replace("(anonymous namespace)::", "").replace("void ", "").split("(")[0].split("<")[0].strip()
+
+
+def gpu_info():
+    try:
+        out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True,
+                             text=True, timeout=30).stdout.strip().splitlines()
+        name, power = [v.strip() for v in out[0].split(",")]
+        return name, power
+    except Exception as e:   # the numbers are still reported, with the reason the card could not be read
+        import torch
+        return torch.cuda.get_device_name(), "unknown (%s)" % type(e).__name__
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--batch", type=int, default=256)
+    ap.add_argument("--iters", type=int, default=20)
+    ap.add_argument("--warmup", type=int, default=3)
+    args = ap.parse_args()
+    import torch
+    if not torch.cuda.is_available():
+        raise SystemExit("bench_ir50_grad: needs a CUDA device")
+    from crfr_b200 import _lib as L
+    from crfr_b200 import ops
+    from crfr_b200.model.model_irse import IR_50
+    from oracle import resnet_oracle as RO
+
+    B = args.batch
+    net = IR_50([112, 112])
+    net.load_state_dict(RO.randomize_bn_everywhere(RO.build_ir50_state_dict(91), 191))
+    net = net.cuda().eval()
+    g = torch.Generator().manual_seed(1)
+    x = torch.randn(B, 3, 112, 112, generator=g).cuda()
+    seeds = [t.cuda() for t in (torch.randn(B, 512, generator=g), torch.randn(B, 64, 56, 56, generator=g),
+                                torch.randn(B, 128, 28, 28, generator=g), torch.randn(B, 256, 14, 14, generator=g),
+                                torch.randn(B, 512, 7, 7, generator=g))]
+    lib = L.lib()
+
+    def timed(fn, iters):
+        for _ in range(args.warmup):
+            fn()
+        torch.cuda.synchronize()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        for _ in range(iters):
+            fn()
+        e1.record()
+        torch.cuda.synchronize()
+        return e0.elapsed_time(e1) / iters
+
+    def fwd():
+        with torch.no_grad():
+            net.forward_features(x)
+
+    xg = x.clone().requires_grad_(True)
+
+    def fwd_bwd():
+        outs = net.forward_features(xg)
+        torch.autograd.grad(outs, xg, seeds)
+
+    t_fwd = timed(fwd, args.iters)
+    t_fb = timed(fwd_bwd, args.iters)
+
+    # backward alone on one saved forward, both stem paths alternated
+    outs = net.forward_features(xg)
+    t_bwd = {1: [], 0: []}
+    for _ in range(3):
+        for opt in (1, 0):
+            L.call("crfr_set_option", b"ir50_stem_tc", opt)
+            t_bwd[opt].append(timed(lambda: torch.autograd.grad(outs, xg, seeds, retain_graph=True), args.iters))
+    L.call("crfr_set_option", b"ir50_stem_tc", 1)
+
+    # direct stem dgrad alone: dX [B,112,112,4] <- dY [B,112,112,64]
+    d = L.ConvDesc(B, 112, 112, 3, 64, 3, 1, 1, 112, 112, 4, 64, 0)
+    dy = torch.randn(B, 112, 112, 64, generator=g).to(torch.bfloat16).cuda()
+    dxs = torch.empty(B, 112, 112, 4, dtype=torch.bfloat16, device="cuda")
+    wt = torch.empty(9 * 3 * 64, dtype=torch.bfloat16, device="cuda")
+    w = net.input_layer[0].weight.detach()
+    L.call("crfr_pack_weight", w.data_ptr(), wt.data_ptr(), 9, 3, 64, 64, 9, 27, 1, ops.stream())
+    wsb = lib.crfr_conv_workspace_bytes(C.byref(d))
+    ws = torch.empty(max(wsb, 1), dtype=torch.uint8, device="cuda")
+    t_stem_direct = timed(lambda: L.call("crfr_conv_dgrad", L.ENGINE_AUTO, C.byref(d), dy.data_ptr(), wt.data_ptr(), 64,
+                                         dxs.data_ptr(), ws.data_ptr(), wsb, ops.stream()), args.iters)
+
+    # each stem path's kernels alone, profiled in their own pass (the profiler slows the host, not the kernels)
+    def stem_kernels_ms(opt):
+        from torch.profiler import ProfilerActivity, profile
+        L.call("crfr_set_option", b"ir50_stem_tc", opt)
+        torch.autograd.grad(outs, xg, seeds, retain_graph=True)
+        torch.cuda.synchronize()
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            torch.autograd.grad(outs, xg, seeds, retain_graph=True)
+            torch.cuda.synchronize()
+        L.call("crfr_set_option", b"ir50_stem_tc", 1)
+        ev = sorted((e for e in prof.events() if e.device_type == torch.autograd.DeviceType.CUDA),
+                    key=lambda e: e.time_range.start)
+        last_ew = max(i for i, e in enumerate(ev) if "ir50_bwd_ew_kernel" in e.name)
+        last_cvt = max(i for i, e in enumerate(ev) if "nhwc_to_nchw_kernel" in e.name)
+        stem = ev[last_ew + 1:last_cvt]
+        return sum(e.time_range.elapsed_us() for e in stem) / 1e3, sorted({kernel_name(e.name) for e in stem})
+
+    stem_tc_ms, stem_tc_kernels = stem_kernels_ms(1)
+    stem_direct_ms, stem_direct_kernels = stem_kernels_ms(0)
+
+    f_fwd, f_bwd = ir50_flops_per_image()
+    name, power = gpu_info()
+    best = {k: min(v) for k, v in t_bwd.items()}
+    res = {
+        "device": name, "power_limit": power, "batch": B, "iters": args.iters,
+        "gflop_per_image_fwd": round(f_fwd / 1e9, 3), "gflop_per_image_dgrad": round(f_bwd / 1e9, 3),
+        "fwd_ms": round(t_fwd, 3), "fwd_images_per_s": round(B / t_fwd * 1e3, 1),
+        "fwd_tflops": round(B * f_fwd / t_fwd / 1e9, 1),
+        "fwd_grad_ms": round(t_fb, 3), "fwd_grad_images_per_s": round(B / t_fb * 1e3, 1),
+        "fwd_grad_tflops": round(B * (f_fwd + f_bwd) / t_fb / 1e9, 1),
+        "bwd_ms_stem_tc": round(best[1], 3), "bwd_ms_stem_direct": round(best[0], 3),
+        "bwd_ms_all": {k: [round(v, 3) for v in vs] for k, vs in t_bwd.items()},
+        "bwd_over_fwd": round(best[1] / t_fwd, 2),
+        "stem_dgrad_direct_ms": round(t_stem_direct, 3),
+        "stem_dgrad_in_bwd_ms": {"tcgen05": round(stem_tc_ms, 3), "direct": round(stem_direct_ms, 3)},
+        "stem_dgrad_kernels": {"tcgen05": stem_tc_kernels, "direct": stem_direct_kernels},
+    }
+    print("device: %s, power limit: %s" % (name, power))
+    print(json.dumps(res))
+
+
+if __name__ == "__main__":
+    main()
