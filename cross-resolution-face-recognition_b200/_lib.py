@@ -43,7 +43,7 @@ class ResnetIO(C.Structure):
 
 class KdIO(C.Structure):
     _fields_ = [("batch", ci), ("size", ci), ("x", vp), ("momentum", cf), ("eps", cf), ("assistant_grad_to_student", ci),
-                ("x_lr", vp), ("teacher_ir50", ci), ("events", vp * 2)]
+                ("x_lr", vp), ("teacher_ir50", ci), ("events", vp * 2), ("teacher_ir_layers", ci), ("teacher_ir_se", ci)]
 
 
 RESNET34_NPARAMS, RESNET34_NBN = 114, 38
@@ -128,6 +128,13 @@ SIGNATURES = {
     "crfr_ir50_tape": (ci, [ci, ci, C.POINTER(TapeEntry), ci]),
     "crfr_ir50_backward": (ci, [ci, vp, vp, C.POINTER(ResnetIO), vp, vp, vp, vp, csz, vp]),
     "crfr_resnet34_backward": (ci, [ci, vp, vp, C.POINTER(ResnetIO), vp, vp, vp, csz, vp]),
+    "crfr_kd_workspace_bytes_ir": (csz, [ci, ci, ci, ci]),
+    "crfr_irnet_sizes": (ci, [ci, ci, C.POINTER(ci), C.POINTER(ci)]),
+    "crfr_irnet_workspace_bytes": (csz, [ci, ci, ci, ci]),
+    "crfr_irnet_forward": (ci, [ci, ci, ci, vp, vp, C.POINTER(ResnetIO), vp, csz, vp]),
+    "crfr_irnet_grad_workspace_bytes": (csz, [ci, ci, ci, ci]),
+    "crfr_irnet_tape": (ci, [ci, ci, ci, ci, C.POINTER(TapeEntry), ci]),
+    "crfr_irnet_backward": (ci, [ci, ci, ci, vp, vp, C.POINTER(ResnetIO), vp, vp, vp, vp, csz, vp]),
 }
 
 _lib = None
@@ -156,3 +163,10 @@ def check(rc, what=""):
 
 def call(name, *args):
     check(getattr(lib(), name)(*args), name)
+
+
+def irnet_sizes(num_layers, se):
+    """(named_parameters count, BatchNorm count) of the IR variant (num_layers, se) (crfr_irnet_sizes)."""
+    n_params, n_bn = ci(), ci()
+    call("crfr_irnet_sizes", num_layers, int(se), C.byref(n_params), C.byref(n_bn))
+    return n_params.value, n_bn.value

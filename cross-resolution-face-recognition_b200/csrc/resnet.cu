@@ -8,13 +8,15 @@
 // head as a tcgen05 GEMM over the NHWC-flattened feature (weights re-ordered from the reference's NCHW flatten), and
 // BatchNorm1d on the embedding.
 //
-// The frozen IR_50 teacher (DISTILLATION/model/model_irse.py) is a second program over the same ops:
-// BN -> conv3x3 -> PReLU -> conv3x3(stride) -> BN, plus a MaxPool2d(1, stride) / conv1x1+BN shortcut, 24 blocks.  Its
-// backward (backward_ir50) is the gradient with respect to the input image only: eval-mode BatchNorm couples no images,
-// so it is a per-sample linear map of dgrads, per-channel scales and PReLU masks.
+// The frozen IR teachers (DISTILLATION/model/model_irse.py: IR_50 / 101 / 152 and IR_SE_50 / 101 / 152) are a second
+// program over the same ops: BN -> conv3x3 -> PReLU -> conv3x3(stride) -> BN [-> SEModule], plus a MaxPool2d(1, stride) /
+// conv1x1+BN shortcut, 24 / 49 / 50 blocks.  Its backward (backward_ir) is the gradient with respect to the input image
+// only: eval-mode BatchNorm couples no images, so it is a per-sample linear map of dgrads, per-channel scales, PReLU masks
+// and, with SE, the per-image excitation and its squeeze path.
 //
 // ref: model/resnet.py:18-47 (BasicBlock), :152-225 (ResNet.__init__/_make_layer/forward), :231-236 (ResNet_34);
-//      DISTILLATION/model/model_irse.py:49-66 (bottleneck_IR), :103-110 (get_blocks(50)), :129-172 (Backbone).
+//      DISTILLATION/model/model_irse.py:49-66 (bottleneck_IR), SEModule and bottleneck_IR_SE, :101-126 (get_blocks),
+//      :129-172 (Backbone).
 #include <vector>
 
 #include "common.cuh"
@@ -33,16 +35,27 @@ struct Slot {
   bf16* p;
   int ld;
 };
-enum OpKind { OP_CONV, OP_BN, OP_LINEAR, OP_PRELU, OP_SUB2 };
+enum OpKind { OP_CONV, OP_BN, OP_LINEAR, OP_PRELU, OP_SUB2, OP_SE };
 struct Op {
   OpKind kind;
   Tensor a, b, out;
   crfr_conv_desc cd;
   int w_idx = -1, b_idx = -1, g_idx = -1, beta_idx = -1, alpha_idx = -1;
   int cin_pad = 0;
-  float* stats = nullptr;
+  float* stats = nullptr;   // OP_SE: the excitation e [n][c]
+  float* bn_stats = nullptr, *squeeze = nullptr;   // OP_SE: res_layer.4's (mean, rstd) [c][2], mean_hw(y) [n][c][2]
   bool relu = false, has_res = false, x_needs_grad = true;
 };
+
+// IR / IR-SE variants (DISTILLATION/model/model_irse.py:101-126): units per stage
+bool ir_units_of(int num_layers, int units[4]) {
+  static const int t50[4] = {3, 4, 14, 3}, t100[4] = {3, 13, 30, 3}, t152[4] = {3, 8, 36, 3};
+  const int* t = num_layers == 50 ? t50 : num_layers == 100 ? t100 : num_layers == 152 ? t152 : nullptr;
+  if (!t) return false;
+  for (int l = 0; l < 4; ++l) units[l] = t[l];
+  return true;
+}
+constexpr int kSeReduction = 16;   // SEModule(depth, 16): hidden widths 4, 8, 16, 32
 
 constexpr int kFeat = 512, kEmb = 512;
 
@@ -107,25 +120,40 @@ __global__ void bn_scale_kernel(const float* __restrict__ stats, const float* __
   if (i < c) s[i] = gamma[i] * stats[2 * i + 1];
 }
 
+// 8 consecutive fp32 values (32-byte aligned) as two 16-byte loads
+__device__ __forceinline__ void load8f(const float* __restrict__ p, float* v) {
+  const float4 a = *reinterpret_cast<const float4*>(p), b = *reinterpret_cast<const float4*>(p + 4);
+  v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
+}
+
 // Element-wise input-gradient pass of the IR_50 backward (eval-mode BatchNorm and / or PReLU, plus a second gradient):
 //   out[p][c] = s[c] * act'(s[c] * y[p][c] + t[c]) * g[p][c] (+ add)
 // with s = gamma * rstd, t = beta - mean * s computed as the forward's normalise kernel does (no stats: s = 1, t = 0),
 // act' = 1 where z > 0 and alpha[c] elsewhere (no alpha: identity; no y: act' = 1, the pass is a plain sum).
 // add_mode 1 adds add[p][c]; 2 adds the gradient of a stride-2 pixel subsampling (MaxPool2d(1, 2)), i.e. add at the
-// half-resolution pixel for the even pixels and nothing elsewhere - a gather, so no atomics.  One thread per 8 channels
-// of a pixel (16-byte loads and store), fp32 arithmetic, one rounding.  out may alias g (each element is read, then
-// written, by the same thread).
+// half-resolution pixel for the even pixels and nothing elsewhere - a gather, so no atomics.  With nscale (the SE unit's
+// residual branch) the first factor is per (image, channel) instead: v = nscale[n][c] * g + nshift[n][c].  One thread per
+// 8 channels of a pixel (16-byte loads and store), fp32 arithmetic, one rounding.  out may alias g (each element is read,
+// then written, by the same thread).
 __global__ void __launch_bounds__(256)
 ir50_bwd_ew_kernel(const bf16* g, int g_ld, const bf16* __restrict__ y, int y_ld, const float* __restrict__ stats,
                    const float* __restrict__ gamma, const float* __restrict__ beta, const float* __restrict__ alpha,
                    const bf16* __restrict__ add, int add_ld, int add_mode, bf16* out, int out_ld, int h, int w, int groups,
-                   long long total) {
+                   long long total, const float* __restrict__ nscale = nullptr, const float* __restrict__ nshift = nullptr) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= total) return;
   const int cg = (int)(i % groups);
   const long long p = i / groups;
   float v[8];
   unpack8(*reinterpret_cast<const bf16x8*>(g + p * g_ld + cg * 8), v);
+  if (nscale) {
+    const long long nc = (p / ((long long)h * w)) * groups * 8 + cg * 8;
+    float a[8], b[8];
+    load8f(nscale + nc, a);
+    load8f(nshift + nc, b);
+#pragma unroll
+    for (int j = 0; j < 8; ++j) v[j] = fmaf(a[j], v[j], b[j]);
+  }
   if (y) {
     float f[8];
     unpack8(*reinterpret_cast<const bf16x8*>(y + p * y_ld + cg * 8), f);
@@ -162,9 +190,161 @@ ir50_bwd_ew_kernel(const bf16* g, int g_ld, const bf16* __restrict__ y, int y_ld
   *reinterpret_cast<bf16x8*>(out + p * out_ld + cg * 8) = pack8(v);
 }
 
-// tape indices of one bottleneck_IR unit of the IR_50 program (-1: absent)
+// ---- squeeze-excitation unit (SEModule(depth, 16), model_irse.py: x * sigmoid(fc2(relu(fc1(mean_hw(x)))))) ----
+// The SE input is r = s * y + t, res_layer.4's eval-mode BatchNorm of the res_layer.3 output y (s = gamma * rstd,
+// t = beta - mean * s), so its squeeze is s * mean_hw(y) + t: it comes from the InstanceNorm statistics of the stored y.
+
+// pooled[c] = s_c * mean_hw(y)[n][c] + t_c into shared memory, then the hidden pre-activation pre[j] = W1[j][:] . pooled
+// (one warp per hidden unit, lanes over channels, shuffle reduction: a fixed order, shared by the forward and backward
+// so both see the same ReLU mask)
+__device__ __forceinline__ void se_hidden(const float* __restrict__ sq, const float* __restrict__ bnst,
+                                          const float* __restrict__ gamma, const float* __restrict__ beta,
+                                          const float* __restrict__ w1, int n, int C, int Hd, float* pooled, float* pre) {
+  for (int c = threadIdx.x; c < C; c += blockDim.x) {
+    const float s = gamma[c] * bnst[2 * c + 1];
+    pooled[c] = fmaf(sq[2 * ((long long)n * C + c)], s, beta[c] - bnst[2 * c] * s);
+  }
+  __syncthreads();
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
+  for (int j = warp; j < Hd; j += nwarps) {
+    float acc = 0.f;
+    for (int c = lane; c < C; c += 32) acc = fmaf(w1[(long long)j * C + c], pooled[c], acc);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+    if (lane == 0) pre[j] = acc;
+  }
+  __syncthreads();
+}
+
+// Excitation, one CTA per image: e[n][c] = sigmoid(W2[c][:] . relu(pre)), fp32 (W1 [Hd][C], W2 [C][Hd]: the reference's
+// [out][in][1][1] layouts); also the unit output's per-(image, channel) affine map e * BN_4: ea = e * s_c, eb = e * t_c
+__global__ void __launch_bounds__(256)
+se_excite_kernel(const float* __restrict__ sq, const float* __restrict__ bnst, const float* __restrict__ gamma,
+                 const float* __restrict__ beta, const float* __restrict__ w1, const float* __restrict__ w2, int C, int Hd,
+                 float* __restrict__ e, float* __restrict__ ea, float* __restrict__ eb) {
+  __shared__ float pooled[512], pre[32];
+  const int n = blockIdx.x;
+  se_hidden(sq, bnst, gamma, beta, w1, n, C, Hd, pooled, pre);
+  for (int c = threadIdx.x; c < C; c += blockDim.x) {
+    float acc = 0.f;
+    for (int j = 0; j < Hd; ++j) acc = fmaf(w2[(long long)c * Hd + j], fmaxf(pre[j], 0.f), acc);
+    const float ex = 1.f / (1.f + expf(-acc)), s = gamma[c] * bnst[2 * c + 1];
+    e[(long long)n * C + c] = ex;
+    ea[(long long)n * C + c] = ex * s;
+    eb[(long long)n * C + c] = ex * (beta[c] - bnst[2 * c] * s);
+  }
+}
+
+// Unit output with SE: out = res + ea[n][c] * y + eb[n][c] (= res + e * (s_c * y + t_c)), fp32, one rounding (replaces the
+// BatchNorm + residual pass; same traffic).  One thread per 8 channels of a pixel, 16-byte loads throughout.
+__global__ void __launch_bounds__(256)
+se_apply_kernel(const bf16* __restrict__ y, int y_ld, const float* __restrict__ ea, const float* __restrict__ eb,
+                const bf16* __restrict__ res, int res_ld, bf16* __restrict__ out, int out_ld, int hw, int groups,
+                long long total) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= total) return;
+  const int cg = (int)(i % groups);
+  const long long p = i / groups;
+  const long long nc = (p / hw) * groups * 8 + cg * 8;
+  float f[8], r[8], a[8], b[8];
+  unpack8(*reinterpret_cast<const bf16x8*>(y + p * y_ld + cg * 8), f);
+  unpack8(*reinterpret_cast<const bf16x8*>(res + p * res_ld + cg * 8), r);
+  load8f(ea + nc, a);
+  load8f(eb + nc, b);
+#pragma unroll
+  for (int j = 0; j < 8; ++j) r[j] += fmaf(a[j], f[j], b[j]);
+  *reinterpret_cast<bf16x8*>(out + p * out_ld + cg * 8) = pack8(r);
+}
+
+// Pixel chunks of the SE backward reduction: a function of the image size only, so that the order of the fp32 sums (and
+// the bits) do not depend on the batch
+__host__ __device__ inline int se_chunks(int hw) { return (hw + 255) / 256; }
+
+// First pass of the SE backward: per (image, pixel chunk) the sums (sum g * y, sum g) over the chunk's pixels of every
+// channel -> part[n][chunk][2][C].  Thread = (channel group of 8, pixel lane); the lanes are combined in shared memory in
+// a fixed order (no atomics).
+__global__ void __launch_bounds__(256)
+se_bwd_reduce_kernel(const bf16* __restrict__ g, int g_ld, const bf16* __restrict__ y, int y_ld, int hw, int C,
+                     float* __restrict__ part) {
+  __shared__ float red[2 * 2048];
+  const int n = blockIdx.y, chunk = blockIdx.x, chunks = gridDim.x;
+  const int groups = C / 8, lanes = blockDim.x / groups;
+  const int cg = threadIdx.x % groups, lane = threadIdx.x / groups;
+  const int p0 = (int)((long long)hw * chunk / chunks), p1 = (int)((long long)hw * (chunk + 1) / chunks);
+  float sgy[8], sg[8];
+#pragma unroll
+  for (int j = 0; j < 8; ++j) sgy[j] = sg[j] = 0.f;
+  if (lane < lanes) {
+    for (int p = p0 + lane; p < p1; p += lanes) {
+      const long long pix = (long long)n * hw + p;
+      float a[8], b[8];
+      unpack8(*reinterpret_cast<const bf16x8*>(g + pix * g_ld + cg * 8), a);
+      unpack8(*reinterpret_cast<const bf16x8*>(y + pix * y_ld + cg * 8), b);
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {
+        sgy[j] = fmaf(a[j], b[j], sgy[j]);
+        sg[j] += a[j];
+      }
+    }
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      red[(lane * 2 + 0) * C + cg * 8 + j] = sgy[j];
+      red[(lane * 2 + 1) * C + cg * 8 + j] = sg[j];
+    }
+  }
+  __syncthreads();
+  for (int k = threadIdx.x; k < 2 * C; k += blockDim.x) {
+    const int which = k / C, c = k - which * C;
+    float acc = 0.f;
+    for (int l = 0; l < lanes; ++l) acc += red[(l * 2 + which) * C + c];
+    part[(((long long)n * chunks + chunk) * 2 + which) * C + c] = acc;
+  }
+}
+
+// Tail of the SE backward, one CTA per image: de[c] = s_c * sum(g*y) + t_c * sum(g) (= sum_hw g * r), u = de * e (1 - e),
+// dh = W2^T u masked by relu', dpool = W1^T dh; shift[n][c] = dpool[c] / hw, the part of dr that every pixel shares
+// (dr = e * g + shift, see ir50_bwd_ew_kernel).
+__global__ void __launch_bounds__(256)
+se_bwd_tail_kernel(const float* __restrict__ part, int chunks, const float* __restrict__ sq, const float* __restrict__ bnst,
+                   const float* __restrict__ gamma, const float* __restrict__ beta, const float* __restrict__ w1,
+                   const float* __restrict__ w2, const float* __restrict__ e, int C, int Hd, int hw,
+                   float* __restrict__ shift) {
+  __shared__ float pooled[512], u[512], pre[32], dh[32];
+  const int n = blockIdx.x;
+  for (int c = threadIdx.x; c < C; c += blockDim.x) {
+    float sgy = 0.f, sg = 0.f;
+    for (int k = 0; k < chunks; ++k) {
+      sgy += part[(((long long)n * chunks + k) * 2 + 0) * C + c];
+      sg += part[(((long long)n * chunks + k) * 2 + 1) * C + c];
+    }
+    const float s = gamma[c] * bnst[2 * c + 1];
+    const float de = fmaf(s, sgy, (beta[c] - bnst[2 * c] * s) * sg);
+    const float ec = e[(long long)n * C + c];
+    u[c] = de * ec * (1.f - ec);
+  }
+  se_hidden(sq, bnst, gamma, beta, w1, n, C, Hd, pooled, pre);   // (its first __syncthreads also publishes u)
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
+  for (int j = warp; j < Hd; j += nwarps) {
+    float acc = 0.f;
+    for (int c = lane; c < C; c += 32) acc = fmaf(w2[(long long)c * Hd + j], u[c], acc);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+    if (lane == 0) dh[j] = pre[j] > 0.f ? acc : 0.f;
+  }
+  __syncthreads();
+  const float inv = 1.f / (float)hw;
+  for (int c = threadIdx.x; c < C; c += blockDim.x) {
+    float acc = 0.f;
+    for (int j = 0; j < Hd; ++j) acc = fmaf(w1[(long long)j * C + c], dh[j], acc);
+    shift[(long long)n * C + c] = acc * inv;
+  }
+}
+
+// tape indices of one bottleneck_IR / bottleneck_IR_SE unit of the IR program (-1: absent); bn4 is the SE apply op
+// (OP_SE) in an SE unit
 struct IrUnit {
   int sc_conv = -1, sc_bn = -1, sub = -1, bn0, conv1, prelu, conv2, bn4;
+  int fc1 = -1;   // SE units: parameter index of res_layer.5.fc1 (fc2 follows)
 };
 
 struct Net {
@@ -190,8 +370,9 @@ struct Net {
   bf16* wp = nullptr;    // packed linear weights (forward)
   bf16* wpt = nullptr;   // transposed (backward)
   int pcur = 0, bncur = 0;
-  std::vector<IrUnit> ir_units;               // IR_50: the 24 units, and the stem / head ops, as tape indices
+  std::vector<IrUnit> ir_units;               // IR program: the units, and the stem / head ops, as tape indices
   int ir_stem_conv = -1, ir_stem_bn = -1, ir_head_bn0 = -1, ir_head_lin = -1, ir_head_bn1 = -1;
+  int ir_layers = 50, ir_se = 0;              // IR program variant: 50 / 100 / 152 layers, bottleneck_IR(_SE)
 
   void* alloc(size_t bytes) {
     size_t a = (off + 1023) & ~(size_t)1023;
@@ -228,7 +409,9 @@ struct Net {
   float* grad(int idx) { return (grads && idx >= 0) ? grads[idx] : nullptr; }
 
   // ---- forward ops ----
-  Tensor conv(const Tensor& x, int w_idx, int cout, int k, int stride, int pad, bool x_needs_grad) {
+  // inst_stats: also the per-(image, channel) (mean, rstd) [n][cout][2] of the stored output (the SE unit's squeeze)
+  Tensor conv(const Tensor& x, int w_idx, int cout, int k, int stride, int pad, bool x_needs_grad,
+              float* inst_stats = nullptr) {
     Op op;
     op.kind = OP_CONV;
     crfr_conv_desc& d = op.cd;
@@ -250,7 +433,7 @@ struct Net {
       if (bn_stats)
         check(crfr_conv_fwd_bnstats(engine, &d, x.p, wpk, op.cin_pad, y.p, bn_stats, io->eps, scratch, scratch_bytes, st));
       else
-        check(crfr_conv_fwd(engine, &d, x.p, wpk, op.cin_pad, nullptr, y.p, nullptr, nullptr, io->eps, scratch,
+        check(crfr_conv_fwd(engine, &d, x.p, wpk, op.cin_pad, nullptr, y.p, nullptr, inst_stats, io->eps, scratch,
                             scratch_bytes, st));
     }
     op.a = x; op.out = y; op.w_idx = w_idx; op.x_needs_grad = x_needs_grad;
@@ -409,13 +592,57 @@ struct Net {
     tape.push_back(op);
     return out;
   }
+  // res_layer.4 (eval-mode BatchNorm, parameters g_idx, g_idx + 1) + res_layer.5 (SEModule, fc1 / fc2 at fc1_idx,
+  // fc1_idx + 1) + the shortcut res; sq: the squeeze statistics of y from its convolution
+  Tensor se_unit_out(const Tensor& y, int g_idx, int bn_index, int fc1_idx, const Tensor& res, float* sq) {
+    Tensor out = new_tensor(y.n, y.h, y.w, y.c);
+    float* stats = (float*)alloc((size_t)y.c * 2 * sizeof(float));
+    float* e = (float*)alloc((size_t)y.n * y.c * sizeof(float));
+    float* ea = (float*)alloc((size_t)y.n * y.c * sizeof(float));
+    float* eb = (float*)alloc((size_t)y.n * y.c * sizeof(float));
+    if (run()) {
+      check(crfr_bn_running_to_stats((const float*)buffers[3 * bn_index], (const float*)buffers[3 * bn_index + 1], y.c,
+                                     io->eps, stats, st));
+      se_excite_kernel<<<y.n, 256, 0, st>>>(sq, stats, params[g_idx], params[g_idx + 1], params[fc1_idx],
+                                            params[fc1_idx + 1], y.c, y.c / kSeReduction, e, ea, eb);
+      CRFR_COUNT_LAUNCH();
+      check_cuda(cudaGetLastError());
+      const long long total = (long long)y.n * y.h * y.w * (y.c / 8);
+      se_apply_kernel<<<crfr_cdiv(total, 256), 256, 0, st>>>(y.p, y.ld, ea, eb, res.p, res.ld, out.p, out.ld, y.h * y.w,
+                                                             y.c / 8, total);
+      CRFR_COUNT_LAUNCH();
+      check_cuda(cudaGetLastError());
+    }
+    Op op;
+    op.kind = OP_SE;
+    op.a = y; op.b = res; op.out = out; op.has_res = true;
+    op.stats = e; op.bn_stats = stats; op.squeeze = sq;
+    op.g_idx = g_idx; op.beta_idx = g_idx + 1; op.w_idx = fc1_idx;
+    tape.push_back(op);
+    return out;
+  }
 
-  // parameter order (named_parameters): input_layer (4), output_layer (6), body blocks (7, or 10 with a conv shortcut);
-  // BatchNorm order (named_buffers): input_layer.1, output_layer.0, output_layer.4, then per block
-  // [shortcut_layer.1], res_layer.0, res_layer.4
-  void forward_ir50() {
+  // parameter order (named_parameters): input_layer (4), output_layer (6), body blocks (7, or 10 with a conv shortcut,
+  // + 2 with SE: res_layer.5.fc1 / fc2); BatchNorm order (named_buffers): input_layer.1, output_layer.0, output_layer.4,
+  // then per block [shortcut_layer.1], res_layer.0, res_layer.4.  The variant is (ir_layers, ir_se); IR_50 is (50, 0).
+  void forward_ir() {
     const int B = io->batch, S = io->size;
     scratch_bytes = scratch_need_ir50(B, S);
+    if (ir_se) {   // the squeeze statistics of res_layer.3 may take a separate per-image pass (crfr_norm_stats)
+      const int q = S / 2;
+      const crfr_conv_desc shapes[] = {
+          {B, S, S, 64, 64, 3, 2, 1, q, q, 64, 64, 0},
+          {B, q, q, 64, 64, 3, 1, 1, q, q, 64, 64, 0},
+          {B, q, q, 128, 128, 3, 2, 1, q / 2, q / 2, 128, 128, 0},
+          {B, q / 2, q / 2, 128, 128, 3, 1, 1, q / 2, q / 2, 128, 128, 0},
+          {B, q / 2, q / 2, 256, 256, 3, 2, 1, q / 4, q / 4, 256, 256, 0},
+          {B, q / 4, q / 4, 256, 256, 3, 1, 1, q / 4, q / 4, 256, 256, 0},
+          {B, q / 4, q / 4, 512, 512, 3, 2, 1, q / 8, q / 8, 512, 512, 0}};
+      for (const crfr_conv_desc& d : shapes) {
+        const size_t b = crfr_conv_workspace_bytes(&d) + 4096;
+        if (b > scratch_bytes) scratch_bytes = b;
+      }
+    }
     scratch = alloc(scratch_bytes);
     float* ident = (float*)alloc(512 * 2 * sizeof(float));
     if (run()) {
@@ -428,10 +655,12 @@ struct Net {
     ir_stem_conv = last() - 1; ir_stem_bn = last();
     ir_units.clear();
     int p = 10, bi = 3;
-    const int units[4] = {3, 4, 14, 3}, depth[4] = {64, 128, 256, 512};
+    int units[4];
+    ir_units_of(ir_layers, units);
+    const int depth[4] = {64, 128, 256, 512};
     int in_ch = 64;
     for (int l = 0; l < 4; ++l)
-      for (int u = 0; u < units[l]; ++u) {   // bottleneck_IR, model_irse.py:49-66
+      for (int u = 0; u < units[l]; ++u) {   // bottleneck_IR(_SE), model_irse.py:49-66
         const int stride = u == 0 ? 2 : 1, d = depth[l];
         const bool conv_sc = in_ch != d;
         IrUnit un;
@@ -448,15 +677,21 @@ struct Net {
         un.bn0 = last();
         r = prelu(conv(r, p + 2, d, 3, 1, 1, false), p + 3, ident);    // res_layer.1, .2
         un.conv1 = last() - 1; un.prelu = last();
-        r = conv(r, p + 4, d, 3, stride, 1, false);                    // res_layer.3
+        float* sq = ir_se ? (float*)alloc((size_t)B * d * 2 * sizeof(float)) : nullptr;
+        r = conv(r, p + 4, d, 3, stride, 1, false, sq);                // res_layer.3 (+ the SE squeeze)
         un.conv2 = last();
-        a = bn(r, p + 5, 0, &sc, -1, bi + 1);                          // res_layer.4 + shortcut
+        if (ir_se) {
+          a = se_unit_out(r, p + 5, bi + 1, p + 7, sc, sq);            // res_layer.4 + .5 (SE) + shortcut
+          un.fc1 = p + 7;
+        } else {
+          a = bn(r, p + 5, 0, &sc, -1, bi + 1);                        // res_layer.4 + shortcut
+        }
         un.bn4 = last();
         ir_units.push_back(un);
-        p += 7; bi += 2;
+        p += ir_se ? 9 : 7; bi += 2;
         in_ch = d;
         if (u == units[l] - 1) {   // stage output: 64@56^2, 128@28^2, 256@14^2, 512@7^2 - the shapes of ResNet_34's x1..x4,
-          feat[l] = a;             // i.e. the t_k of the residual-KD loss when IR_50 is the teacher (distill_main.py:59,68-69)
+          feat[l] = a;             // i.e. the t_k of the residual-KD loss when IR is the teacher (distill_main.py:59,68-69)
           to_nchw(a, io->feat[l]);
         }
       }
@@ -487,12 +722,13 @@ struct Net {
     return m + 4096;
   }
 
-  // ---- IR_50 input gradient (after a forward_ir50 over the same arena; parameters stay frozen) ----
+  // ---- IR input gradient (after a forward_ir over the same arena; parameters stay frozen) ----
   Tensor map_like(const Tensor& t) { return Tensor{(bf16*)alloc((size_t)t.n * t.h * t.w * t.ld * sizeof(bf16)), t.n, t.h, t.w, t.c, t.ld}; }
   float* bn_scale(const Op& b) {
     float* s = (float*)alloc((size_t)b.a.c * sizeof(float));
     if (run()) {
-      bn_scale_kernel<<<crfr_cdiv(b.a.c, 128), 128, 0, st>>>(b.stats, params[b.g_idx], b.a.c, s);
+      bn_scale_kernel<<<crfr_cdiv(b.a.c, 128), 128, 0, st>>>(b.kind == OP_SE ? b.bn_stats : b.stats, params[b.g_idx],
+                                                             b.a.c, s);
       CRFR_COUNT_LAUNCH();
       check_cuda(cudaGetLastError());
     }
@@ -518,24 +754,48 @@ struct Net {
     else
       check(crfr_conv_dgrad(engine, &d, dy.p, wt, d.cout, dx.p, scratch, scratch_bytes, st));
   }
-  // out = s * act'(z) * g (+ add): see ir50_bwd_ew_kernel; bn (may be null) supplies stats / gamma / beta
-  void ew(const Slot& g, const Tensor& y, const Op* bn, int alpha_idx, const Slot* add, int add_mode, const Tensor& out) {
+  // out = s * act'(z) * g (+ add): see ir50_bwd_ew_kernel; bn (may be null) supplies stats / gamma / beta; nscale /
+  // nshift: per-(image, channel) factor and shift instead (the SE unit)
+  void ew(const Slot& g, const Tensor& y, const Op* bn, int alpha_idx, const Slot* add, int add_mode, const Tensor& out,
+          const float* nscale = nullptr, const float* nshift = nullptr) {
     if (!run()) return;
     const float* alpha = alpha_idx >= 0 ? params[alpha_idx] : nullptr;
     const long long total = (long long)out.n * out.h * out.w * (out.c / 8);
     ir50_bwd_ew_kernel<<<crfr_cdiv(total, 256), 256, 0, st>>>(
         g.p, g.ld, y.p, y.ld, bn ? bn->stats : nullptr, bn ? params[bn->g_idx] : nullptr,
         bn ? params[bn->beta_idx] : nullptr, alpha, add ? add->p : nullptr, add ? add->ld : 8, add_mode, out.p, out.ld,
-        out.h, out.w, out.c / 8, total);
+        out.h, out.w, out.c / 8, total, nscale, nshift);
     CRFR_COUNT_LAUNCH();
     check_cuda(cudaGetLastError());
+  }
+
+  // SE unit: the gradient dr at the SE input r from the unit's output gradient g (dr = e * g + W1^T dh / hw, see
+  // se_bwd_tail_kernel) - a deterministic per-(image, channel) reduction, the tiny per-image tail, one element-wise pass
+  Tensor se_grad(const Op& se, const Slot& g) {
+    const Tensor& y = se.a;
+    const int hw = y.h * y.w, chunks = se_chunks(hw), hid = y.c / kSeReduction;
+    float* part = (float*)alloc((size_t)y.n * chunks * 2 * y.c * sizeof(float));
+    float* shift = (float*)alloc((size_t)y.n * y.c * sizeof(float));
+    Tensor dr = map_like(y);
+    if (run()) {
+      se_bwd_reduce_kernel<<<dim3(chunks, y.n), 256, 0, st>>>(g.p, g.ld, y.p, y.ld, hw, y.c, part);
+      CRFR_COUNT_LAUNCH();
+      check_cuda(cudaGetLastError());
+      se_bwd_tail_kernel<<<y.n, 256, 0, st>>>(part, chunks, se.squeeze, se.bn_stats, params[se.g_idx], params[se.beta_idx],
+                                              params[se.w_idx], params[se.w_idx + 1], se.stats, y.c, hid, hw, shift);
+      CRFR_COUNT_LAUNCH();
+      check_cuda(cudaGetLastError());
+    }
+    ew(g, Tensor{}, nullptr, -1, nullptr, 0, dr, se.stats, shift);
+    return dr;
   }
 
   // Per unit, from the unit's output gradient g: res_layer.4's scale is folded into res_layer.3's dgrad weights and
   // res_layer.0's into res_layer.1's, the shortcut BatchNorm's into its 1x1 convolution, output_layer.0's and the
   // BatchNorm1d's into the transposed linear weights; what remains element-wise (PReLU masks, the stem's BatchNorm +
-  // PReLU, the gradient sum at each unit's input) is ir50_bwd_ew_kernel.
-  void backward_ir50(const float* d_emb, const float* const* d_feat, float* dx) {
+  // PReLU, the gradient sum at each unit's input) is ir50_bwd_ew_kernel.  In an SE unit the per-(image, channel)
+  // excitation cannot be folded: se_grad turns g into the residual branch's gradient first.
+  void backward_ir(const float* d_emb, const float* const* d_feat, float* dx) {
     const int B = io->batch;
     size_t need = crfr_lowered_dgrad_cin3_ws_bytes(&tape[ir_stem_conv].cd);
     for (const Op& op : tape)
@@ -597,7 +857,12 @@ struct Net {
       squash(b4.out, 1);
       const Slot g = slots[b4.out.id][0];
       Tensor d_r2 = map_like(pr.out);
-      dgrad(tape[U.conv2], g, w2[u], d_r2);                               // res_layer.4 + .3
+      if (U.fc1 >= 0) {
+        const Tensor dr = se_grad(b4, g);                                  // res_layer.5
+        dgrad(tape[U.conv2], Slot{dr.p, dr.ld}, w2[u], d_r2);             // res_layer.4 + .3
+      } else {
+        dgrad(tape[U.conv2], g, w2[u], d_r2);                             // res_layer.4 + .3
+      }
       const Slot s_r2{d_r2.p, d_r2.ld};
       ew(s_r2, pr.a, nullptr, pr.alpha_idx, nullptr, 0, d_r2);     // res_layer.2, in place
       Tensor d_in = map_like(in);
@@ -760,14 +1025,16 @@ extern "C" size_t crfr_resnet34_workspace_bytes(int batch, int size, int trainin
 // in_off / stats_off are bytes from the workspace base.  The parity tests read the stored bf16 activations through this
 // table and replay them into the CPU oracle (teacher-forced forward / backward checks, tests/test_resnet_forced_gpu.py).
 namespace {
-// kinds: 0 convolution, 1 BatchNorm (+ residual) (+ ReLU / PReLU), 7 linear head, 8 PReLU pass, 9 stride-2 subsampling
+// kinds: 0 convolution, 1 BatchNorm (+ residual) (+ ReLU / PReLU), 7 linear head, 8 PReLU pass, 9 stride-2 subsampling,
+// 10 SE unit output (BatchNorm + excitation + residual; stats_off: the excitation e [n][c] fp32)
 int fill_tape(const Net& net, crfr_tape_entry* entries, int max_entries) {
   const int count = (int)net.tape.size();
   for (int i = 0; i < count && i < max_entries && entries; ++i) {
     const Op& op = net.tape[i];
     crfr_tape_entry& e = entries[i];
     const Tensor& t = op.out;
-    e.kind = op.kind == OP_CONV ? 0 : op.kind == OP_BN ? 1 : op.kind == OP_LINEAR ? 7 : op.kind == OP_PRELU ? 8 : 9;
+    e.kind = op.kind == OP_CONV ? 0 : op.kind == OP_BN ? 1 : op.kind == OP_LINEAR ? 7 : op.kind == OP_PRELU ? 8
+           : op.kind == OP_SUB2 ? 9 : 10;
     e.n = t.n; e.h = t.h; e.w = t.w; e.c = t.c; e.ld = t.ld;
     e.out_off = t.p ? (long long)((uint8_t*)t.p - (uint8_t*)nullptr) : -1;
     e.in_off = op.a.p ? (long long)((uint8_t*)op.a.p - (uint8_t*)nullptr) : -1;
@@ -789,16 +1056,52 @@ extern "C" int crfr_resnet34_tape(int batch, int size, int training, crfr_tape_e
   return fill_tape(net, entries, max_entries);
 }
 
-// The same table for the IR_50 program (eval mode): every stored tensor of crfr_ir50_forward in program order, for the
-// teacher-forced parity test of its input gradient (tests/test_ir50_grad_gpu.py).
-extern "C" int crfr_ir50_tape(int batch, int size, crfr_tape_entry* entries, int max_entries) {
-  if (batch <= 0 || size != 112) return -1;
-  crfr_resnet_io io = {};
+namespace {
+bool ir_variant_ok(int num_layers, int se) {
+  int units[4];
+  return ir_units_of(num_layers, units) && (se == 0 || se == 1);
+}
+int check_ir_variant(int num_layers, int se, const char* who) {
+  CRFR_CHECK_ARG(ir_variant_ok(num_layers, se), "%s: unsupported IR variant (num_layers %d, se %d): 50, 100 or 152 layers, "
+                 "se 0 or 1", who, num_layers, se);
+  return CRFR_OK;
+}
+// a dry run of the IR program's forward (and, with grad, of its input gradient) at (batch, 112): arena offsets and tape
+void ir_dry_run(Net& net, crfr_resnet_io& io, int num_layers, int se, int batch, int size, bool grad) {
+  io = {};
   io.batch = batch; io.size = size; io.training = 0; io.momentum = 0.1f; io.eps = 1e-5f;
-  Net net;
   init_net(net, CRFR_ENGINE_AUTO, nullptr, nullptr, nullptr, &io, nullptr, ~(size_t)0 >> 2, nullptr, false);
-  net.forward_ir50();
+  net.ir_layers = num_layers; net.ir_se = se;
+  net.forward_ir();
+  if (grad) {
+    static float dummy = 0.f;   // non-null marker so that the dry run sizes every optional buffer
+    const float* feats[4] = {&dummy, &dummy, &dummy, &dummy};
+    net.backward_ir(&dummy, feats, &dummy);
+  }
+}
+}  // namespace
+
+extern "C" int crfr_irnet_sizes(int num_layers, int se, int* n_params, int* n_bn) {
+  CRFR_TRY(check_ir_variant(num_layers, se, "irnet_sizes"));
+  int units[4];
+  ir_units_of(num_layers, units);
+  const int n = units[0] + units[1] + units[2] + units[3];
+  if (n_params) *n_params = 10 + n * (se ? 9 : 7) + 3 * 3;   // three units have a conv1x1 + BN shortcut
+  if (n_bn) *n_bn = 3 + 2 * n + 3;
+  return CRFR_OK;
+}
+
+// The same table for the IR programs (eval mode): every stored tensor of crfr_irnet_forward in program order, for the
+// teacher-forced parity tests of the input gradient (tests/test_ir50_grad_gpu.py, tests/test_irnet_gpu.py).
+extern "C" int crfr_irnet_tape(int num_layers, int se, int batch, int size, crfr_tape_entry* entries, int max_entries) {
+  if (!ir_variant_ok(num_layers, se) || batch <= 0 || size != 112) return -1;
+  crfr_resnet_io io;
+  Net net;
+  ir_dry_run(net, io, num_layers, se, batch, size, false);
   return fill_tape(net, entries, max_entries);
+}
+extern "C" int crfr_ir50_tape(int batch, int size, crfr_tape_entry* entries, int max_entries) {
+  return crfr_irnet_tape(50, 0, batch, size, entries, max_entries);
 }
 
 extern "C" int crfr_resnet34_forward(int engine, const float* const* host_params, void* const* host_buffers,
@@ -827,10 +1130,11 @@ __global__ void kd_total_kernel(const float* __restrict__ parts, float* __restri
 struct KdLayout {
   size_t teacher, train, scratch, total;
 };
-KdLayout kd_layout(int batch, int size, int teacher_ir50 = 0) {
+// ir_layers = 0: a ResNet_34 teacher, else the IR variant (ir_layers, ir_se)
+KdLayout kd_layout(int batch, int size, int ir_layers = 0, int ir_se = 0) {
   KdLayout l;
-  l.teacher = ((teacher_ir50 ? crfr_ir50_workspace_bytes(batch, size) : crfr_resnet34_workspace_bytes(batch, size, 0)) + 4095) &
-              ~(size_t)4095;
+  l.teacher = ((ir_layers ? crfr_irnet_workspace_bytes(ir_layers, ir_se, batch, size)
+                          : crfr_resnet34_workspace_bytes(batch, size, 0)) + 4095) & ~(size_t)4095;
   // + room for the second embedding-gradient slot of the student (L_s and L_a both reach s_emb)
   l.train = (crfr_resnet34_workspace_bytes(batch, size, 1) + (size_t)batch * kEmb * 2 + (4u << 20)) & ~(size_t)4095;
   l.scratch = 1 << 20;
@@ -846,7 +1150,11 @@ extern "C" size_t crfr_kd_workspace_bytes(int batch, int size) {
 }
 extern "C" size_t crfr_kd_workspace_bytes_ex(int batch, int size, int teacher_ir50) {
   if (batch <= 0 || size != 112) return 0;
-  return kd_layout(batch, size, teacher_ir50).total;
+  return kd_layout(batch, size, teacher_ir50 ? 50 : 0).total;
+}
+extern "C" size_t crfr_kd_workspace_bytes_ir(int batch, int size, int teacher_ir_layers, int teacher_ir_se) {
+  if (batch <= 0 || size != 112 || !ir_variant_ok(teacher_ir_layers, teacher_ir_se)) return 0;
+  return kd_layout(batch, size, teacher_ir_layers, teacher_ir_se).total;
 }
 
 extern "C" int crfr_kd_train_step(int engine, const float* const* teacher_params, void* const* teacher_buffers,
@@ -858,7 +1166,10 @@ extern "C" int crfr_kd_train_step(int engine, const float* const* teacher_params
   CRFR_CHECK_ARG(teacher_params && teacher_buffers && student_params && student_grads && assistant_params &&
                      assistant_grads && losses && ws,
                  "kd_train_step: null pointer");
-  const KdLayout lay = kd_layout(kio->batch, kio->size, kio->teacher_ir50);
+  const int t_layers = kio->teacher_ir50 ? (kio->teacher_ir_layers ? kio->teacher_ir_layers : 50) : 0;
+  const int t_se = kio->teacher_ir50 ? kio->teacher_ir_se : 0;
+  if (t_layers) CRFR_TRY(check_ir_variant(t_layers, t_se, "kd_train_step"));
+  const KdLayout lay = kd_layout(kio->batch, kio->size, t_layers, t_se);
   if (ws_bytes < lay.total) {
     crfr_set_error("kd_train_step: workspace %zu < %zu", ws_bytes, lay.total);
     return CRFR_EWORKSPACE;
@@ -876,8 +1187,12 @@ extern "C" int crfr_kd_train_step(int engine, const float* const* teacher_params
   io_train.training = 1;
   // The program of one step over three networks; real = false: dry run (arena offsets and weight-pack jobs only)
   auto program = [&](Net& T, Net& S, Net& A, bool real) -> int {
-    if (kio->teacher_ir50) T.forward_ir50();
-    else T.forward();
+    if (t_layers) {
+      T.ir_layers = t_layers; T.ir_se = t_se;
+      T.forward_ir();
+    } else {
+      T.forward();
+    }
     if (!T.ok()) return T.err;
     S.forward();
     if (!S.ok()) return S.err;
@@ -945,59 +1260,70 @@ extern "C" int crfr_kd_train_step(int engine, const float* const* teacher_params
   return program(T, S, A, true);
 }
 
-extern "C" size_t crfr_ir50_workspace_bytes(int batch, int size) {
-  if (batch <= 0 || size != 112) return 0;
-  crfr_resnet_io io = {};
-  io.batch = batch; io.size = size; io.training = 0; io.momentum = 0.1f; io.eps = 1e-5f;
+extern "C" size_t crfr_irnet_workspace_bytes(int num_layers, int se, int batch, int size) {
+  if (!ir_variant_ok(num_layers, se) || batch <= 0 || size != 112) return 0;
+  crfr_resnet_io io;
   Net net;
-  init_net(net, CRFR_ENGINE_AUTO, nullptr, nullptr, nullptr, &io, nullptr, ~(size_t)0 >> 2, nullptr, false);
-  net.forward_ir50();
+  ir_dry_run(net, io, num_layers, se, batch, size, false);
   return net.off + 65536;
 }
+extern "C" size_t crfr_ir50_workspace_bytes(int batch, int size) { return crfr_irnet_workspace_bytes(50, 0, batch, size); }
 
-extern "C" int crfr_ir50_forward(int engine, const float* const* host_params, void* const* host_buffers,
-                                 const crfr_resnet_io* io, void* ws, size_t ws_bytes, void* stream) {
-  CRFR_TRY(check_io(io, "ir50_forward"));
-  CRFR_CHECK_ARG(host_params && host_buffers && ws, "ir50_forward: null pointer");
-  CRFR_CHECK_ARG(!io->training, "ir50_forward: the teacher runs in eval mode only (train-mode Dropout is stochastic)");
+extern "C" int crfr_irnet_forward(int engine, int num_layers, int se, const float* const* host_params,
+                                  void* const* host_buffers, const crfr_resnet_io* io, void* ws, size_t ws_bytes,
+                                  void* stream) {
+  CRFR_TRY(check_ir_variant(num_layers, se, "irnet_forward"));
+  CRFR_TRY(check_io(io, "irnet_forward"));
+  CRFR_CHECK_ARG(host_params && host_buffers && ws, "irnet_forward: null pointer");
+  CRFR_CHECK_ARG(!io->training, "irnet_forward: the teacher runs in eval mode only (train-mode Dropout is stochastic)");
   Net net;
   init_net(net, engine, host_params, nullptr, host_buffers, io, ws, ws_bytes, (cudaStream_t)stream, true);
-  net.forward_ir50();
+  net.ir_layers = num_layers; net.ir_se = se;
+  net.forward_ir();
   return net.err;
 }
-
-// forward arena of crfr_ir50_workspace_bytes (same layout), then the input-gradient buffers
-extern "C" size_t crfr_ir50_grad_workspace_bytes(int batch, int size) {
-  if (batch <= 0 || size != 112) return 0;
-  crfr_resnet_io io = {};
-  io.batch = batch; io.size = size; io.training = 0; io.momentum = 0.1f; io.eps = 1e-5f;
-  static float dummy = 0.f;   // non-null marker so that the dry run sizes every optional buffer
-  const float* feats[4] = {&dummy, &dummy, &dummy, &dummy};
-  Net net;
-  init_net(net, CRFR_ENGINE_AUTO, nullptr, nullptr, nullptr, &io, nullptr, ~(size_t)0 >> 2, nullptr, false);
-  net.forward_ir50();
-  net.backward_ir50(&dummy, feats, &dummy);
-  return net.off + 65536;
+extern "C" int crfr_ir50_forward(int engine, const float* const* host_params, void* const* host_buffers,
+                                 const crfr_resnet_io* io, void* ws, size_t ws_bytes, void* stream) {
+  return crfr_irnet_forward(engine, 50, 0, host_params, host_buffers, io, ws, ws_bytes, stream);
 }
 
-extern "C" int crfr_ir50_backward(int engine, const float* const* host_params, void* const* host_buffers,
-                                  const crfr_resnet_io* io, const float* d_emb, const float* const* d_feat, float* dx,
-                                  void* ws, size_t ws_bytes, void* stream) {
-  CRFR_TRY(check_io(io, "ir50_backward"));
-  CRFR_CHECK_ARG(host_params && dx && ws, "ir50_backward: null pointer");
-  CRFR_CHECK_ARG(!io->training, "ir50_backward: the forward must have run in eval mode");
-  const size_t need = crfr_ir50_grad_workspace_bytes(io->batch, io->size);
+// forward arena of crfr_irnet_workspace_bytes (same layout), then the input-gradient buffers
+extern "C" size_t crfr_irnet_grad_workspace_bytes(int num_layers, int se, int batch, int size) {
+  if (!ir_variant_ok(num_layers, se) || batch <= 0 || size != 112) return 0;
+  crfr_resnet_io io;
+  Net net;
+  ir_dry_run(net, io, num_layers, se, batch, size, true);
+  return net.off + 65536;
+}
+extern "C" size_t crfr_ir50_grad_workspace_bytes(int batch, int size) {
+  return crfr_irnet_grad_workspace_bytes(50, 0, batch, size);
+}
+
+extern "C" int crfr_irnet_backward(int engine, int num_layers, int se, const float* const* host_params,
+                                   void* const* host_buffers, const crfr_resnet_io* io, const float* d_emb,
+                                   const float* const* d_feat, float* dx, void* ws, size_t ws_bytes, void* stream) {
+  CRFR_TRY(check_ir_variant(num_layers, se, "irnet_backward"));
+  CRFR_TRY(check_io(io, "irnet_backward"));
+  CRFR_CHECK_ARG(host_params && dx && ws, "irnet_backward: null pointer");
+  CRFR_CHECK_ARG(!io->training, "irnet_backward: the forward must have run in eval mode");
+  const size_t need = crfr_irnet_grad_workspace_bytes(num_layers, se, io->batch, io->size);
   if (ws_bytes < need) {
-    crfr_set_error("ir50_backward: workspace %zu < %zu (crfr_ir50_grad_workspace_bytes)", ws_bytes, need);
+    crfr_set_error("irnet_backward: workspace %zu < %zu (crfr_irnet_grad_workspace_bytes)", ws_bytes, need);
     return CRFR_EWORKSPACE;
   }
   Net net;
   init_net(net, engine, host_params, nullptr, host_buffers, io, ws, ws_bytes, (cudaStream_t)stream, false);
-  net.forward_ir50();   // dry run: rebuild the tape and the saved-activation offsets
+  net.ir_layers = num_layers; net.ir_se = se;
+  net.forward_ir();   // dry run: rebuild the tape and the saved-activation offsets
   if (!net.ok()) return net.err;
   net.exec = true;
-  net.backward_ir50(d_emb, d_feat, dx);
+  net.backward_ir(d_emb, d_feat, dx);
   return net.err;
+}
+extern "C" int crfr_ir50_backward(int engine, const float* const* host_params, void* const* host_buffers,
+                                  const crfr_resnet_io* io, const float* d_emb, const float* const* d_feat, float* dx,
+                                  void* ws, size_t ws_bytes, void* stream) {
+  return crfr_irnet_backward(engine, 50, 0, host_params, host_buffers, io, d_emb, d_feat, dx, ws, ws_bytes, stream);
 }
 
 extern "C" int crfr_resnet34_backward(int engine, const float* const* host_params, float* const* host_grads,

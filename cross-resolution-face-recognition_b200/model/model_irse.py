@@ -1,25 +1,27 @@
-"""Drop-in IR_50 teacher backed by the native sm_100a network program (forward, and the gradient w.r.t. the input).
+"""Drop-in IR / IR-SE teachers backed by the native sm_100a network program (forward, and the gradient w.r.t. the input).
 
-Mirror of the reference's DISTILLATION/model/model_irse.py for the configuration distill_main.py:14,201 uses
-(``IR_50([112, 112])``): same class names (``Backbone``, ``bottleneck_IR``, ``Flatten``, ``l2_norm``, ``get_blocks``),
-constructor arguments, sub-module / parameter / buffer names (identical ``state_dict`` keys, so the pretrained
-teacher checkpoint loads) and construction + initialisation order.  The torch layers are parameter containers only;
-``Backbone.forward`` runs ``crfr_ir50_forward``.
+Mirror of the reference's DISTILLATION/model/model_irse.py (face.evoLVe): the six constructors ``IR_50``, ``IR_101``,
+``IR_152``, ``IR_SE_50``, ``IR_SE_101`` and ``IR_SE_152`` (distill_main.py:14,201 uses ``IR_50([112, 112])``), with the
+same class names (``Backbone``, ``bottleneck_IR``, ``bottleneck_IR_SE``, ``SEModule``, ``Flatten``, ``l2_norm``,
+``get_blocks``), constructor arguments, sub-module / parameter / buffer names (identical ``state_dict`` keys, so the
+pretrained face.evoLVe checkpoints load) and construction + initialisation order.  The torch layers are parameter
+containers only; ``Backbone.forward`` runs ``crfr_irnet_forward`` for the variant (num_layers, mode).  Every variant is
+native at 112 x 112; 224 x 224 is not.
 
 The teacher is frozen and evaluated in ``eval()`` mode by the reference (distill_main.py:43, 112-114); only that mode
 is native: train-mode Dropout (model_irse.py:144) is stochastic and has no parity definition, so ``forward`` in
-training mode raises.  The SE variants and the 100/152-layer variants are not on the hot path.
+training mode raises.
 
 When ``x.requires_grad`` (and grad mode is on), ``forward`` / ``forward_features`` are differentiable with respect to
-``x`` through ``crfr_ir50_backward``, so that IR_50 can drive an identity or perceptual loss on a super-resolved face
-(SUPER_RESOLUTION/train_FHN.py:255-265)::
+``x`` through ``crfr_irnet_backward``, so that the teacher can drive an identity or perceptual loss on a super-resolved
+face (SUPER_RESOLUTION/train_FHN.py:255-265)::
 
     sr = fsrnet(x)[1][:, :, 8:120, 8:120]
     f_sr, f_hr = ir50.forward_features(sr), ir50.forward_features(hr)
     loss = pixel_loss + sum(F.mse_loss(a, b) for a, b in zip(f_sr, f_hr))
     loss.backward()          # reaches fsrnet's parameters through IR_50
 
-IR_50's own parameters stay frozen: they never receive a ``.grad``, even with ``requires_grad=True``.
+The teacher's own parameters stay frozen: they never receive a ``.grad``, even with ``requires_grad=True``.
 """
 import ctypes as C
 from collections import namedtuple
@@ -27,12 +29,14 @@ from collections import namedtuple
 import torch
 import torch.nn as nn
 from torch.autograd.function import once_differentiable
-from torch.nn import BatchNorm1d, BatchNorm2d, Conv2d, Dropout, Linear, MaxPool2d, Module, PReLU, Sequential
+from torch.nn import (AdaptiveAvgPool2d, BatchNorm1d, BatchNorm2d, Conv2d, Dropout, Linear, MaxPool2d, Module, PReLU, ReLU,
+                      Sequential, Sigmoid)
 
 from .. import _lib as L
 from .. import ops
 
-__all__ = ["Backbone", "IR_50", "bottleneck_IR", "Flatten", "l2_norm", "get_blocks"]
+__all__ = ["Backbone", "IR_50", "IR_101", "IR_152", "IR_SE_50", "IR_SE_101", "IR_SE_152", "bottleneck_IR",
+           "bottleneck_IR_SE", "SEModule", "Flatten", "l2_norm", "get_blocks"]
 
 
 class Flatten(Module):
@@ -61,6 +65,35 @@ class bottleneck_IR(Module):
         self.res_layer = Sequential(BatchNorm2d(in_channel),
                                     Conv2d(in_channel, depth, (3, 3), (1, 1), 1, bias=False), PReLU(depth),
                                     Conv2d(depth, depth, (3, 3), stride, 1, bias=False), BatchNorm2d(depth))
+
+
+class SEModule(Module):
+    """ref: model_irse.py SEModule: x * sigmoid(fc2(relu(fc1(avg_pool(x))))).  fc1 is xavier-initialised at construction
+    (and again by Backbone._initialize_weights), as the reference does: seeded construction draws the same numbers."""
+
+    def __init__(self, channels, reduction):
+        super().__init__()
+        self.avg_pool = AdaptiveAvgPool2d(1)
+        self.fc1 = Conv2d(channels, channels // reduction, kernel_size=1, padding=0, bias=False)
+        nn.init.xavier_uniform_(self.fc1.weight.data)
+        self.relu = ReLU(inplace=True)
+        self.fc2 = Conv2d(channels // reduction, channels, kernel_size=1, padding=0, bias=False)
+        self.sigmoid = Sigmoid()
+
+
+class bottleneck_IR_SE(Module):
+    """ref: model_irse.py bottleneck_IR_SE: bottleneck_IR whose residual ends in SEModule(depth, 16)."""
+
+    def __init__(self, in_channel, depth, stride):
+        super().__init__()
+        if in_channel == depth:
+            self.shortcut_layer = MaxPool2d(1, stride)
+        else:
+            self.shortcut_layer = Sequential(Conv2d(in_channel, depth, (1, 1), stride, bias=False), BatchNorm2d(depth))
+        self.res_layer = Sequential(BatchNorm2d(in_channel),
+                                    Conv2d(in_channel, depth, (3, 3), (1, 1), 1, bias=False), PReLU(depth),
+                                    Conv2d(depth, depth, (3, 3), stride, 1, bias=False), BatchNorm2d(depth),
+                                    SEModule(depth, 16))
 
 
 class Bottleneck(namedtuple("Block", ["in_channel", "depth", "stride"])):
@@ -93,20 +126,20 @@ class Backbone(Module):
         assert input_size[0] in [112, 224], "input_size should be [112, 112] or [224, 224]"
         assert num_layers in [50, 100, 152], "num_layers should be 50, 100 or 152"
         assert mode in ["ir", "ir_se"], "mode should be ir or ir_se"
-        if mode != "ir":
-            raise NotImplementedError("the squeeze-excitation variants are not part of the native hot path")
         blocks = get_blocks(num_layers)
+        unit_module = bottleneck_IR if mode == "ir" else bottleneck_IR_SE
         self.input_layer = Sequential(Conv2d(3, 64, (3, 3), 1, 1, bias=False), BatchNorm2d(64), PReLU(64))
         feat = 512 * 7 * 7 if input_size[0] == 112 else 512 * 14 * 14
         self.output_layer = Sequential(BatchNorm2d(512), Dropout(), Flatten(), Linear(feat, 512), BatchNorm1d(512))
         modules = []
         for block in blocks:
             for bottleneck in block:
-                modules.append(bottleneck_IR(bottleneck.in_channel, bottleneck.depth, bottleneck.stride))
+                modules.append(unit_module(bottleneck.in_channel, bottleneck.depth, bottleneck.stride))
         self.body = Sequential(*modules)
         self._initialize_weights()
         self.engine = L.ENGINE_AUTO
-        self._native = num_layers == 50 and input_size[0] == 112
+        self._variant = (num_layers, 1 if mode == "ir_se" else 0)   # (num_layers, se) of the crfr_irnet_* calls
+        self._native = input_size[0] == 112
 
     def _initialize_weights(self):
         """ref: model_irse.py:174-188."""
@@ -125,38 +158,40 @@ class Backbone(Module):
 
     def _check(self, x):
         if not self._native:
-            raise NotImplementedError("only IR_50([112, 112]) has a native network program")
+            raise NotImplementedError("only the 112 x 112 IR / IR_SE backbones have a native network program")
         if self.training:
-            raise RuntimeError("the native IR_50 is the frozen teacher: call .eval() first (train-mode Dropout is "
+            raise RuntimeError("the native IR backbone is the frozen teacher: call .eval() first (train-mode Dropout is "
                                "stochastic and has no parity definition)")
         if not x.is_cuda:
-            raise RuntimeError("crfr_b200 IR_50 needs a CUDA tensor: the hot path has no CPU fallback")
+            raise RuntimeError("crfr_b200 IR backbone needs a CUDA tensor: the hot path has no CPU fallback")
         if x.dim() != 4 or tuple(x.shape[1:]) != (3, 112, 112):
             raise ValueError("expected [B,3,112,112], got %s" % (tuple(x.shape),))
 
     def _launch(self, x, want_features, ws=None):
-        """crfr_ir50_forward into ``ws`` (default: the shared workspace) -> (emb, feats, tables, io)."""
+        """crfr_irnet_forward into ``ws`` (default: the shared workspace) -> (emb, feats, tables, io)."""
         b = x.shape[0]
         emb = torch.empty((b, 512), dtype=torch.float32, device=x.device)
         feats = [torch.empty((b, c, s, s), dtype=torch.float32, device=x.device)
                  for c, s in ((64, 56), (128, 28), (256, 14), (512, 7))] if want_features else []
         params = [p.detach() for _, p in self.named_parameters()]
         buffers = [t for _, t in self.named_buffers()]
-        ptab, btab = _Table(params, L.IR50_NPARAMS), _Table(buffers, 3 * L.IR50_NBN)
+        n_params, n_bn = L.irnet_sizes(*self._variant)
+        ptab, btab = _Table(params, n_params), _Table(buffers, 3 * n_bn)
         io = L.ResnetIO()
         io.batch, io.size, io.x, io.emb = b, 112, x.data_ptr(), emb.data_ptr()
         for i, f in enumerate(feats):
             io.feat[i] = f.data_ptr()
         io.training, io.momentum, io.eps = 0, 0.1, 1e-5
         if ws is None:
-            ws = ops.workspace(L.lib().crfr_ir50_workspace_bytes(b, 112))
-        L.call("crfr_ir50_forward", self.engine, ptab.arr, btab.arr, C.byref(io), ws.data_ptr(), ws.numel(), ops.stream())
+            ws = ops.workspace(L.lib().crfr_irnet_workspace_bytes(*self._variant, b, 112))
+        L.call("crfr_irnet_forward", self.engine, *self._variant, ptab.arr, btab.arr, C.byref(io), ws.data_ptr(), ws.numel(),
+               ops.stream())
         return emb, feats, (ptab, btab), io
 
     def _run(self, x, want_features):
         self._check(x)
         if torch.is_grad_enabled() and x.requires_grad:
-            outs = _IR50InputGrad.apply(self, want_features, x)
+            outs = _IRInputGrad.apply(self, want_features, x)
             return outs[0], list(outs[1:])
         emb, feats, _, _ = self._launch(x.contiguous().float(), want_features)
         return emb, feats
@@ -174,23 +209,24 @@ class Backbone(Module):
         return (emb,) + tuple(feats)
 
 
-class _IR50InputGrad(torch.autograd.Function):
-    """IR_50 forward whose backward is the native input gradient (``crfr_ir50_backward``).  The forward runs in a private
-    workspace that keeps the saved activations for the backward; the parameters are constants of this function."""
+class _IRInputGrad(torch.autograd.Function):
+    """IR / IR-SE forward whose backward is the native input gradient (``crfr_irnet_backward``).  The forward runs in a
+    private workspace that keeps the saved activations for the backward; the parameters are constants of this function."""
 
     @staticmethod
     def forward(ctx, net, want_features, x):
         x = x.detach().contiguous().float()
-        ws = torch.empty(L.lib().crfr_ir50_grad_workspace_bytes(x.shape[0], 112), dtype=torch.uint8, device=x.device)
+        ws = torch.empty(L.lib().crfr_irnet_grad_workspace_bytes(*net._variant, x.shape[0], 112), dtype=torch.uint8,
+                         device=x.device)
         emb, feats, tables, io = net._launch(x, want_features, ws)
         ctx.set_materialize_grads(False)
-        ctx.saved = (net.engine, tables, io, ws, x)   # x: io.x points at it
+        ctx.saved = (net.engine, net._variant, tables, io, ws, x)   # x: io.x points at it
         return (emb,) + tuple(feats)
 
     @staticmethod
     @once_differentiable
     def backward(ctx, d_emb, *d_feats):
-        engine, (ptab, btab), io, ws, x = ctx.saved
+        engine, variant, (ptab, btab), io, ws, x = ctx.saved
         keep = []
 
         def ptr(g):
@@ -201,7 +237,7 @@ class _IR50InputGrad(torch.autograd.Function):
             return g.data_ptr()
         dfeat = (C.c_void_p * 4)(*([ptr(g) for g in d_feats] + [None] * (4 - len(d_feats))))
         dx = torch.empty_like(x)
-        L.call("crfr_ir50_backward", engine, ptab.arr, btab.arr, C.byref(io), ptr(d_emb), dfeat, dx.data_ptr(),
+        L.call("crfr_irnet_backward", engine, *variant, ptab.arr, btab.arr, C.byref(io), ptr(d_emb), dfeat, dx.data_ptr(),
                ws.data_ptr(), ws.numel(), ops.stream())
         return None, None, dx
 
@@ -209,3 +245,28 @@ class _IR50InputGrad(torch.autograd.Function):
 def IR_50(input_size):
     """Constructs a ir-50 model (ref: model_irse.py:191-197)."""
     return Backbone(input_size, 50, "ir")
+
+
+def IR_101(input_size):
+    """Constructs a ir-101 model (ref: model_irse.py IR_101)."""
+    return Backbone(input_size, 100, "ir")
+
+
+def IR_152(input_size):
+    """Constructs a ir-152 model (ref: model_irse.py IR_152)."""
+    return Backbone(input_size, 152, "ir")
+
+
+def IR_SE_50(input_size):
+    """Constructs a ir_se-50 model (ref: model_irse.py IR_SE_50)."""
+    return Backbone(input_size, 50, "ir_se")
+
+
+def IR_SE_101(input_size):
+    """Constructs a ir_se-101 model (ref: model_irse.py IR_SE_101)."""
+    return Backbone(input_size, 100, "ir_se")
+
+
+def IR_SE_152(input_size):
+    """Constructs a ir_se-152 model (ref: model_irse.py IR_SE_152)."""
+    return Backbone(input_size, 152, "ir_se")

@@ -192,22 +192,32 @@ def _flat_grads(net):
 
 
 def _is_ir50(net):
+    """A native IR teacher: any of IR_50 / 101 / 152 and IR_SE_50 / 101 / 152 at 112 x 112."""
     from .model_irse import Backbone
     return isinstance(net, Backbone) and net._native
 
 
 def _teacher_tables(teacher):
+    """(params, buffers) tables of the teacher and its (num_layers, se) variant, or None for ResNet_34."""
     if _is_ir50(teacher):
         params = [p.detach() for _, p in teacher.named_parameters()]
         buffers = [t for _, t in teacher.named_buffers()]
-        return _TableOfPointers(params, L.IR50_NPARAMS), _TableOfPointers(buffers, 3 * L.IR50_NBN), 1
+        n_params, n_bn = L.irnet_sizes(*teacher._variant)
+        return _TableOfPointers(params, n_params), _TableOfPointers(buffers, 3 * n_bn), teacher._variant
     return (_TableOfPointers([p.detach() for p in teacher.ordered_parameters()], L.RESNET34_NPARAMS),
-            _TableOfPointers(teacher.ordered_buffers(), 3 * L.RESNET34_NBN), 0)
+            _TableOfPointers(teacher.ordered_buffers(), 3 * L.RESNET34_NBN), None)
+
+
+def kd_workspace_bytes(teacher, batch):
+    """Workspace of crfr_kd_train_step with this teacher (a native ResNet_34 or IR / IR-SE backbone)."""
+    if _is_ir50(teacher):
+        return L.lib().crfr_kd_workspace_bytes_ir(batch, 112, *teacher._variant)
+    return L.lib().crfr_kd_workspace_bytes_ex(batch, 112, 0)
 
 
 def check_kd_nets(teacher, student, assistant):
     if not ((isinstance(teacher, ResNet) and teacher._native) or _is_ir50(teacher)):
-        raise NotImplementedError("the KD teacher must be a native ResNet_34 or IR_50")
+        raise NotImplementedError("the KD teacher must be a native ResNet_34 or a 112 x 112 IR / IR_SE backbone")
     for net in (student, assistant):
         if not (isinstance(net, ResNet) and net._native):
             raise NotImplementedError("the KD student and assistant must be native ResNet_34 modules")
@@ -225,16 +235,18 @@ def kd_native_call(teacher, student, assistant, x_hr, x_lr, stabs, atabs, losses
                    events=None, ws=None):
     """crfr_kd_train_step on prepared tables: stabs / atabs = (params, buffers, grads) _TableOfPointers of the student and
     the assistant (gradients are ACCUMULATED into the grads tables)."""
-    tp, tb, is_ir50 = _teacher_tables(teacher)
+    tp, tb, variant = _teacher_tables(teacher)
     b = x_hr.shape[0]
     io = L.KdIO()
     io.batch, io.size, io.x = b, 112, x_hr.data_ptr()
     io.x_lr = None if x_lr is None else x_lr.data_ptr()
-    io.teacher_ir50 = is_ir50
+    if variant is not None:
+        io.teacher_ir50 = 1
+        io.teacher_ir_layers, io.teacher_ir_se = variant
     io.momentum, io.eps, io.assistant_grad_to_student = 0.1, 1e-5, int(bool(assistant_grad_to_student))
     for i, e in enumerate(events or ()):
         io.events[i] = e.cuda_event
-    need = L.lib().crfr_kd_workspace_bytes_ex(b, 112, is_ir50)
+    need = kd_workspace_bytes(teacher, b)
     if ws is None or ws.numel() < need:
         ws = ops.workspace(need)
     L.call("crfr_kd_train_step", student.engine, tp.arr, tb.arr, stabs[0].arr, stabs[1].arr, stabs[2].arr, atabs[0].arr,
@@ -247,8 +259,8 @@ def kd_train_step(teacher, student, assistant, x, x_lr=None, assistant_grad_to_s
     distill_main.py:63,68-70 on the bf16 features in place, and both backward passes.
 
     ``x`` is the HR batch the teacher sees; the student and the assistant see ``x_lr`` when given ("HR teacher / LR
-    student"), else ``x`` as well (what distill_main.py:59-61 does).  The teacher is a native ``ResNet_34`` or ``IR_50``
-    (whose four stage outputs are the t_k).
+    student"), else ``x`` as well (what distill_main.py:59-61 does).  The teacher is a native ``ResNet_34`` or one of the
+    IR / IR-SE backbones at 112 x 112 (``IR_50``, ``IR_SE_50``, ``IR_152``, ...: their four stage outputs are the t_k).
 
     Sets ``p.grad`` of the student to d(L_s [+ L_a])/dp and of the assistant to dL_a/dp (overwriting), and returns the
     device tensor ``(L_s, L_a)``.  Equivalent to ``(mse(s_emb, t_emb) + sum_k kd(t_k, s_k, a_k)).backward()`` through

@@ -357,8 +357,8 @@ class KDTrainer:
     """Data-parallel residual knowledge-distillation loop (the replacement for distill_main.py:42-74 with the optimisers
     of :222-225), one process per GPU.
 
-    Per step and per rank: ONE native call (crfr_kd_train_step) runs the frozen teacher (ResNet_34 or IR_50, eval), the
-    student and the assistant (ResNet_34, train: per-replica BatchNorm statistics, as the reference's single-device
+    Per step and per rank: ONE native call (crfr_kd_train_step) runs the frozen teacher (ResNet_34 or an IR / IR-SE
+    backbone, eval), the student and the assistant (ResNet_34, train: per-replica BatchNorm statistics, as the reference's single-device
     semantics) on this rank's share of the batch, the six MSE terms and both backward passes.  Student and assistant
     gradients live in one flat arena each = one all-reduce bucket each (136 MB fp32): the native call records an event
     when the student's gradients are final, its NCCL all-reduce is issued on a side stream behind that event and
@@ -416,7 +416,7 @@ class KDTrainer:
             self._static[0].copy_(x_hr)
             if x_lr is not None:
                 self._static[1].copy_(x_lr)
-            need = L.lib().crfr_kd_workspace_bytes_ex(x_hr.shape[0], 112, 1 if R._is_ir50(self.teacher) else 0)
+            need = R.kd_workspace_bytes(self.teacher, x_hr.shape[0])
             self._ws = torch.empty(need, dtype=torch.uint8, device=x_hr.device)     # private: the graph holds its address
             # eager warm-up (kernel attributes, helper streams) with the BatchNorm buffers restored afterwards, so that the
             # first replayed step is the first running-statistics update

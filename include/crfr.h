@@ -378,14 +378,19 @@ typedef struct crfr_kd_io {
   int assistant_grad_to_student; /* 1: keep the reference's un-detached t_k - s_k in L_a */
   const float* x_lr;             /* optional: the LR batch for the student and the assistant ("HR teacher / LR student");
                                     NULL: all three networks see x, as distill_main.py:59-61 feeds them */
-  int teacher_ir50;              /* 1: teacher_params / teacher_buffers are IR_50's tables (187 / 3 x 54), its four stage outputs
-                                    are the t_k (DISTILLATION/model/model_irse.py: 64@56^2, 128@28^2, 256@14^2, 512@7^2) */
+  int teacher_ir50;              /* 1: teacher_params / teacher_buffers are the tables of an IR teacher (IR_50: 187 / 3 x 54; the
+                                    variant is teacher_ir_layers / teacher_ir_se below), its four stage outputs are the t_k
+                                    (DISTILLATION/model/model_irse.py: 64@56^2, 128@28^2, 256@14^2, 512@7^2) */
   void* events[2];               /* optional cudaEvent_t handles recorded on `stream`: [0] student gradients final (the data-
                                     parallel loop starts their all-reduce behind it, overlapping the assistant's backward),
                                     [1] assistant gradients final */
+  int teacher_ir_layers;         /* read only when teacher_ir50 != 0: 50 (or 0), 100 or 152 */
+  int teacher_ir_se;             /* read only when teacher_ir50 != 0: 1 = the IR_SE variant (tables of crfr_irnet_sizes) */
 } crfr_kd_io;
 size_t crfr_kd_workspace_bytes(int batch, int size);
 size_t crfr_kd_workspace_bytes_ex(int batch, int size, int teacher_ir50);
+/* the workspace of crfr_kd_train_step with the IR teacher (teacher_ir_layers, teacher_ir_se); 0 for an unsupported variant */
+size_t crfr_kd_workspace_bytes_ir(int batch, int size, int teacher_ir_layers, int teacher_ir_se);
 int crfr_kd_train_step(int engine, const float* const* teacher_params, void* const* teacher_buffers,
                        const float* const* student_params, void* const* student_buffers, float* const* student_grads,
                        const float* const* assistant_params, void* const* assistant_buffers,
@@ -416,6 +421,25 @@ int crfr_ir50_tape(int batch, int size, crfr_tape_entry* entries, int max_entrie
 int crfr_ir50_backward(int engine, const float* const* host_params, void* const* host_buffers,
                        const crfr_resnet_io* io, const float* d_emb, const float* const* d_feat, float* dx, void* ws,
                        size_t ws_bytes, void* stream);
+
+/* ---------------------------------------------------------------- IR / IR-SE teachers ----------------------- */
+/* ref: IR_50 / IR_101 / IR_152 / IR_SE_50 / IR_SE_101 / IR_SE_152 and Backbone(input_size, num_layers, mode),
+ * DISTILLATION/model/model_irse.py:129-172 (get_blocks :101-126; mode "ir_se": bottleneck_IR_SE, whose res_layer ends in
+ * SEModule(depth, 16) = x * sigmoid(fc2(relu(fc1(mean_hw(x)))))), at 112 x 112 in eval mode.  The variant is
+ * (num_layers in {50, 100, 152}, se in {0, 1}); crfr_irnet_*(50, 0, ...) is crfr_ir50_* (same arena, launches and bits).
+ * Any other variant is rejected: the size queries return 0 (the tape -1), the calls an error code with a message.
+ * crfr_irnet_sizes: the number of named_parameters() and of BatchNorm layers (buffers: 3 per BatchNorm), host pointers,
+ * either may be NULL.  The other calls behave as their crfr_ir50_* counterparts; the tape adds kind 10, an SE unit's
+ * output (res_layer.4 BatchNorm x excitation + shortcut), whose stats_off is the excitation e [n][c] fp32. */
+int crfr_irnet_sizes(int num_layers, int se, int* n_params, int* n_bn);
+size_t crfr_irnet_workspace_bytes(int num_layers, int se, int batch, int size);
+int crfr_irnet_forward(int engine, int num_layers, int se, const float* const* host_params, void* const* host_buffers,
+                       const crfr_resnet_io* io, void* ws, size_t ws_bytes, void* stream);
+size_t crfr_irnet_grad_workspace_bytes(int num_layers, int se, int batch, int size);
+int crfr_irnet_tape(int num_layers, int se, int batch, int size, crfr_tape_entry* entries, int max_entries);
+int crfr_irnet_backward(int engine, int num_layers, int se, const float* const* host_params, void* const* host_buffers,
+                        const crfr_resnet_io* io, const float* d_emb, const float* const* d_feat, float* dx, void* ws,
+                        size_t ws_bytes, void* stream);
 
 #ifdef __cplusplus
 }
