@@ -55,7 +55,6 @@ SIGNATURES = {
     "crfr_version": (ci, []),
     "crfr_launch_count": (C.c_ulonglong, []),
     "crfr_set_option": (ci, [C.c_char_p, ci]),
-    "crfr_debug_pair_profile": (ci, [C.POINTER(cll), ci]),
     "crfr_conv_engine_supported": (ci, [ci] * 9),
     "crfr_nchw_f32_to_nhwc_bf16": (ci, [vp, vp, ci, ci, ci, ci, ci, ci, vp]),
     "crfr_nhwc_bf16_to_nchw_f32": (ci, [vp, vp, ci, ci, ci, ci, ci, vp]),
@@ -69,8 +68,6 @@ SIGNATURES = {
     "crfr_norm_act_fwd": (ci, [vp, ci, vp, vp, vp, vp, ci, vp, ci, vp, ci, ci, ci, ci, vp]),
     "crfr_norm_act_bwd": (ci, [vp, ci, vp, ci, vp, ci, vp, vp, vp, vp, ci, vp, ci, vp, ci, vp, ci, vp, vp, vp, ci, ci,
                                ci, vp, csz, vp]),
-    "crfr_norm_act_conv_fwd": (ci, [ci, C.POINTER(ConvDesc), vp, ci, vp, vp, vp, vp, ci, vp, ci, vp, ci, vp, ci, vp, vp, vp,
-                                    cf, vp, csz, vp]),
     "crfr_conv_dgrad_norm_bwd_workspace_bytes": (csz, [C.POINTER(ConvDesc)]),
     "crfr_conv_dgrad_norm_bwd": (ci, [ci, C.POINTER(ConvDesc), vp, vp, ci, vp, ci, vp, ci, vp, vp, vp, vp, ci, vp, ci, vp,
                                       ci, vp, ci, vp, vp, vp, vp, csz, vp]),

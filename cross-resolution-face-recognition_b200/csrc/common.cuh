@@ -51,40 +51,6 @@ extern unsigned long long g_crfr_launches;
 #define CRFR_COUNT_LAUNCH() (++g_crfr_launches)
 
 // ------------------------------------------------------------------------------------------------
-// programmatic dependent launch: a kernel launched through crfr_launch_pdl may become resident while the kernel before it
-// on the stream drains (its tail, the launch latency and this kernel's own prologue overlap); it must execute pdl_wait()
-// before it touches anything a predecessor wrote - griddepcontrol.wait returns once the preceding grid has completed and
-// its memory is visible - and calls pdl_trigger() early so that ITS successor may do the same.  Both are no-ops for a
-// kernel launched the ordinary way.  Option "pdl" (CRFR_PDL) switches the launch attribute; default 0: measured on B200 it changes nothing under CUDA-graph
-// replay (40.30 vs 40.36 ms per step) and -0.3 ms per step in eager mode.
-// ------------------------------------------------------------------------------------------------
-#ifdef __CUDACC__
-int crfr_pdl_enabled();
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-template <typename... KArgs, typename... Args>
-inline cudaError_t crfr_launch_pdl_if(bool allow, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem,
-                                      cudaStream_t st, Args... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid;
-  cfg.blockDim = block;
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = (allow && crfr_pdl_enabled()) ? 1 : 0;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
-}
-template <typename... KArgs, typename... Args>
-inline cudaError_t crfr_launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
-                                   Args... args) {
-  return crfr_launch_pdl_if(true, kernel, grid, block, smem, st, args...);
-}
-#endif
-
-// ------------------------------------------------------------------------------------------------
 // small device helpers
 // ------------------------------------------------------------------------------------------------
 #ifdef __CUDACC__

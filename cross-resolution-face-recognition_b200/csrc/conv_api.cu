@@ -28,12 +28,9 @@ extern "C" unsigned long long crfr_launch_count(void) { return g_crfr_launches; 
 namespace {
 struct OptDef { const char* name; const char* env; int dflt; };
 const OptDef kOpts[CRFR_OPT_COUNT] = {
-    {"rowconv", "CRFR_ROWCONV", 1},           {"rowconv_pair", "CRFR_ROWCONV_PAIR", 1},
-    {"pair_swap", "CRFR_PAIR_SWAP", 0},       {"wgrad_stream", "CRFR_WGRAD_STREAM", 1},
-    {"norm_bwd_impl", "CRFR_NORM_BWD", 1},    {"norm_fwd_stream", "CRFR_NORM_FWD_STREAM", 1},
-    {"rowwgrad_pair", "CRFR_ROWWGRAD_PAIR", 1}, {"fuse_norm_bwd", "CRFR_FUSE_NORM_BWD", 1},
-    {"fuse_norm_fwd", "CRFR_FUSE_NORM_FWD", 0}, {"pdl", "CRFR_PDL", 0}, {"tc_t2", "CRFR_TC_T2", 1}, {"bn_fused_stats", "CRFR_BN_FUSED_STATS", 1}, {"matcher_cluster", "CRFR_MATCHER_CLUSTER", 1},
-    {"pair_debug", "CRFR_PAIR_DEBUG", 0}, {"ir50_stem_tc", "CRFR_IR50_STEM_TC", 1}};
+    {"rowconv_pair", "CRFR_ROWCONV_PAIR", 1},   {"wgrad_stream", "CRFR_WGRAD_STREAM", 1},
+    {"norm_bwd_impl", "CRFR_NORM_BWD", 1},      {"norm_fwd_stream", "CRFR_NORM_FWD_STREAM", 1},
+    {"fuse_norm_bwd", "CRFR_FUSE_NORM_BWD", 1}};
 std::atomic<int> g_opt[CRFR_OPT_COUNT];
 std::atomic<int> g_opt_init{0};
 void opts_init() {
@@ -58,8 +55,6 @@ int crfr_opt(int id) {
   opts_init();
   return (id >= 0 && id < CRFR_OPT_COUNT) ? g_opt[id].load(std::memory_order_relaxed) : 0;
 }
-
-int crfr_pdl_enabled() { return crfr_opt(CRFR_OPT_PDL); }
 
 int crfr_sm_count() {
   int dev = 0;
@@ -163,7 +158,7 @@ extern "C" int crfr_conv_fwd(int engine, const crfr_conv_desc* d, const void* x,
 int crfr_conv_fwd_bnstats(int engine, const crfr_conv_desc* d, const void* x, const void* w_packed, int cin_pad, void* y,
                           float* bn_stats, float eps, void* ws, size_t ws_bytes, cudaStream_t st) {
   const long long count = (long long)d->n * d->oh * d->ow;
-  if (crfr_opt(CRFR_OPT_BN_FUSED_STATS) && engine != CRFR_ENGINE_DIRECT && !d->transposed && cin_pad == d->cin &&
+  if (engine != CRFR_ENGINE_DIRECT && !d->transposed && cin_pad == d->cin &&
       crfr_lowered_recipe(d) == 0 && crfr_tc_supported(0, d->h, d->w, d->cin, d->cout, d->k, d->stride, d->pad) &&
       count < (1ll << 31))
     return crfr_tc_conv(d, 0, x, w_packed, nullptr, y, bn_stats, eps, ws, ws_bytes, st, 1);
@@ -196,33 +191,10 @@ extern "C" int crfr_conv_dgrad(int engine, const crfr_conv_desc* d, const void* 
                             d->cin, cout_pad, nullptr, dx, d->in_ld, nullptr, st);
 }
 
-// ---- normalisation + activation (+ residual) + convolution forward as one operation -------------------------------
-extern "C" int crfr_norm_act_conv_fwd(int engine, const crfr_conv_desc* d, const void* y, int y_ld, const float* stats,
-                                      const float* gamma, const float* beta, const float* alpha, int relu, const void* res,
-                                      int res_ld, void* act, int act_ld, const void* w_packed, int cin_pad,
-                                      const float* bias, void* out, float* out_stats, float eps, void* ws, size_t ws_bytes,
-                                      void* stream) {
-  CRFR_TRY(check_desc(d, "norm_act_conv_fwd"));
-  CRFR_CHECK_ARG(y && stats && act && w_packed && out, "norm_act_conv_fwd: null pointer");
-  CRFR_CHECK_ARG(cin_pad >= d->cin && act_ld >= cin_pad && d->in_ld == act_ld && y_ld >= d->cin,
-                 "norm_act_conv_fwd: in_ld must be the ld of the activated map");
-  cudaStream_t st = (cudaStream_t)stream;
-  if (engine != CRFR_ENGINE_DIRECT && crfr_opt(CRFR_OPT_FUSE_NORM_FWD) && crfr_opt(CRFR_OPT_ROWCONV) &&
-      crfr_opt(CRFR_OPT_ROWCONV_PAIR) && !d->transposed && cin_pad == d->cin && crfr_lowered_recipe(d) == 0 &&
-      crfr_rowconv_supported(d->h, d->w, d->cin, d->cout, d->k, d->stride, d->pad) && crfr_rowconv_pair_supported(d->n, d->h)) {
-    crfr_rowconv_xform xf = {y, y_ld, res, res ? res_ld : 8, stats, gamma, beta, alpha, relu, act, act_ld};
-    return crfr_rowconv_pair(y, y_ld, d->n, d->h, w_packed, 0, bias, out, d->out_ld, out_stats, eps, ws, ws_bytes, st,
-                             nullptr, &xf);
-  }
-  CRFR_TRY(crfr_norm_act_fwd(y, y_ld, stats, gamma, beta, alpha, relu, res, res ? res_ld : 8, act, act_ld, d->n,
-                             d->h * d->w, d->cin, stream));
-  return crfr_conv_fwd(engine, d, act, w_packed, cin_pad, bias, out, nullptr, out_stats, eps, ws, ws_bytes, stream);
-}
-
 // ---- dgrad + backward of the normalisation that produced the convolution's input, as one operation ----------------
 static bool dgrad_norm_fusable(int engine, const crfr_conv_desc* d, int cout_pad) {
-  return engine != CRFR_ENGINE_DIRECT && crfr_opt(CRFR_OPT_FUSE_NORM_BWD) && crfr_opt(CRFR_OPT_ROWCONV) &&
-         crfr_opt(CRFR_OPT_ROWCONV_PAIR) && !d->transposed && cout_pad == d->cout && crfr_lowered_recipe(d) < 2 &&
+  return engine != CRFR_ENGINE_DIRECT && crfr_opt(CRFR_OPT_FUSE_NORM_BWD) && crfr_opt(CRFR_OPT_ROWCONV_PAIR) &&
+         !d->transposed && cout_pad == d->cout && crfr_lowered_recipe(d) < 2 &&
          crfr_rowconv_supported(d->h, d->w, d->cin, d->cout, d->k, d->stride, d->pad) &&
          crfr_rowconv_pair_supported(d->n, d->h);
 }

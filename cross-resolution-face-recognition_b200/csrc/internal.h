@@ -9,26 +9,16 @@
 #include <atomic>
 #endif
 
-// ---- process-wide tuning switches (conv_api.cu).  Every setting computes the same results; they exist for A/B
-// measurements and debugging.  Defaults come from the environment (CRFR_ROWCONV, CRFR_ROWCONV_PAIR, CRFR_PAIR_SWAP,
-// CRFR_WGRAD_STREAM, CRFR_NORM_BWD=regs|stream, CRFR_NORM_FWD_STREAM, ...) once; crfr_set_option overrides atomically.
+// ---- process-wide implementation switches (conv_api.cu).  Every setting computes equivalent results: each switch selects
+// a reference implementation that tests compare against, or a serial schedule for profiles.  Defaults come from the
+// environment (CRFR_ROWCONV_PAIR, CRFR_WGRAD_STREAM, CRFR_NORM_BWD=regs|stream, CRFR_NORM_FWD_STREAM, CRFR_FUSE_NORM_BWD)
+// once; crfr_set_option overrides atomically.
 enum {
-  CRFR_OPT_ROWCONV = 0,      // row-streaming kernels for 64 -> 64 convolutions at width 128 (else the tile engine)
-  CRFR_OPT_ROWCONV_PAIR,     // cta_group::2 form of the row-streaming forward / dgrad kernel (even image counts)
-  CRFR_OPT_PAIR_SWAP,        // debugging: which CTA of a pair holds the lower half of B
+  CRFR_OPT_ROWCONV_PAIR = 0, // cta_group::2 form of the row-streaming forward / dgrad kernel (even image counts)
   CRFR_OPT_WGRAD_STREAM,     // FSRNet backward: weight gradients on a helper stream
   CRFR_OPT_NORM_BWD_STREAM,  // TMA-fed normalisation backward (else register-staged)
   CRFR_OPT_NORM_FWD_STREAM,  // TMA-fed normalisation forward
-  CRFR_OPT_ROWWGRAD_PAIR,    // cta_group::2 form of the row-streaming weight gradient
   CRFR_OPT_FUSE_NORM_BWD,    // crfr_conv_dgrad_norm_bwd: first pass of the normalisation backward in the dgrad epilogue
-  CRFR_OPT_FUSE_NORM_FWD,    // crfr_norm_act_conv_fwd: normalise + activate inside the convolution's producer warps
-  CRFR_OPT_PDL,              // programmatic dependent launch of the persistent kernels (common.cuh)
-  CRFR_OPT_TC_T2,            // tile engine, N = 128: two pixel tiles per weight tile
-  CRFR_OPT_BN_FUSED_STATS,   // ResNet program: train-mode BatchNorm statistics from the tile engine's epilogue
-  CRFR_OPT_MATCHER_CLUSTER,  // cosine_topk: gallery blocks multicast inside clusters of two CTAs
-  CRFR_OPT_PAIR_DEBUG,       // ablation bits for tools/pair_diag.py (results are WRONG when set): 1 no loads, 2 no MMAs,
-                             // 4 no pack / store / statistics, 8 no store, 16 no statistics
-  CRFR_OPT_IR50_STEM_TC,     // IR_50 input gradient: stem dgrad on the tcgen05 GEMM (else the direct kernel)
   CRFR_OPT_COUNT
 };
 int crfr_opt(int id);
@@ -191,18 +181,10 @@ struct crfr_rowconv_fuse {
   const float* stats; const float* gamma; const float* beta; const float* alpha; int relu;
   float* partial;                 // out: [n][crfr_rowconv_pair_parts(n, h, !db && !res)][3][64]
 };
-// optional transform producer (forward only): the convolution's input is act(gamma * (y - mean) * rstd + beta (+ res)),
-// computed on the fly from the raw map y; out (nullable) also receives the activated map
-struct crfr_rowconv_xform {
-  const void* y; int y_ld;
-  const void* res; int res_ld;
-  const float* stats; const float* gamma; const float* beta; const float* alpha; int relu;
-  void* out; int out_ld;
-};
 int crfr_rowconv_pair_parts(int n, int h, int plain = 0);   // partial slots per image of the fused pass (plain: no db / res)
 int crfr_rowconv_pair(const void* src, int src_ld, int n, int h, const void* w_packed, int flip, const float* bias,
                       void* dst, int dst_ld, float* stats, float eps, void* ws, size_t ws_bytes, cudaStream_t st,
-                      const crfr_rowconv_fuse* fuse = nullptr, const crfr_rowconv_xform* xf = nullptr);
+                      const crfr_rowconv_fuse* fuse = nullptr);
 // rowwgrad.cu: persistent row-streaming weight gradient of the same shape (deterministic slab reduction)
 int crfr_rowwgrad_supported(int h, int w, int cin, int cout, int k, int stride, int pad);
 size_t crfr_rowwgrad_ws_bytes(int n, int h);

@@ -468,7 +468,7 @@ extern "C" int crfr_cosine_topk(int engine, const void* probes, const void* gall
     return CRFR_EWORKSPACE;
   }
   cudaStream_t st = (cudaStream_t)stream;
-  const bool cl = crfr_opt(CRFR_OPT_MATCHER_CLUSTER) != 0 && s.tiles >= 2;
+  const bool cl = s.tiles >= 2;
   CUtensorMap tmP, tmG;
   CRFR_TRY(make_rows_map(&tmP, probes, p, dim, 128));
   CRFR_TRY(make_rows_map(&tmG, gallery, g, dim, cl ? kGBlock / 2 : kGBlock));

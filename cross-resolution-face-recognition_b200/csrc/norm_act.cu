@@ -115,8 +115,6 @@ __global__ void __launch_bounds__(kThreads)
 stats_finalize_kernel(const float* __restrict__ partial, int chunks, int c, float inv_hw, float eps,
                       float* __restrict__ stats) {
   __shared__ float sm[2][kThreads];
-  pdl_trigger();
-  pdl_wait();
   const int n = blockIdx.x, ch = blockIdx.y * 8 + (threadIdx.x & 7), lane = threadIdx.x >> 3;
   const float* p = partial + (long long)n * chunks * 2 * c;
   float s = 0.f, q = 0.f;
@@ -281,8 +279,6 @@ __global__ void __launch_bounds__(kThreads)
 bwd_fold_kernel(const float* __restrict__ partial, int chunks, int c, float inv_hw, float* __restrict__ bstats,
                 float* __restrict__ tot) {
   __shared__ float sm[3][kThreads];
-  pdl_trigger();
-  pdl_wait();
   const int n = blockIdx.x, ch = blockIdx.y * 8 + (threadIdx.x & 7), lane = threadIdx.x >> 3;
   const float* p = partial + (long long)n * chunks * 3 * c;
   float s[3] = {0.f, 0.f, 0.f};
@@ -425,7 +421,7 @@ size_t crfr_norm_ws_bytes(int n, int hw, int c) {
 // Finalise (mean, rstd) from partials laid out [n][chunks][2][c]; shared with the conv epilogue statistics.
 int crfr_norm_finalize(const float* partial, int n, int chunks, int hw, int c, float eps, float* stats,
                        cudaStream_t st) {
-  CRFR_CUDA(crfr_launch_pdl(stats_finalize_kernel, dim3(n, c / 8), dim3(kThreads), 0, st, partial, chunks, c, 1.f / (float)hw, eps, stats));
+  stats_finalize_kernel<<<dim3(n, c / 8), kThreads, 0, st>>>(partial, chunks, c, 1.f / (float)hw, eps, stats);
   CRFR_COUNT_LAUNCH();
   CRFR_LAUNCH_CHECK();
   return CRFR_OK;
@@ -553,7 +549,7 @@ int crfr_norm_bwd_finish(const float* partial, int chunks, const void* dsrc, int
   // statistic group over the whole batch (BatchNorm: hundreds of slots) the fold stays a kernel of its own
   const bool fold_inside = use_stream && chunks <= 16;
   if (!fold_inside) {
-    CRFR_CUDA(crfr_launch_pdl(bwd_fold_kernel, dim3(n, c / 8), dim3(kThreads), 0, st, partial, chunks, c, 1.f / (float)hw, bstats, tot));
+    bwd_fold_kernel<<<dim3(n, c / 8), kThreads, 0, st>>>(partial, chunks, c, 1.f / (float)hw, bstats, tot);
     CRFR_COUNT_LAUNCH();
     CRFR_LAUNCH_CHECK();
   }

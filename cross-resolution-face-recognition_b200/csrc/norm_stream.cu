@@ -136,8 +136,6 @@ __device__ __forceinline__ Setup setup(const StreamArgs& a, uint8_t* smem_raw) {
     fence_barrier_init();
   }
   __syncthreads();
-  pdl_trigger();
-  pdl_wait();   // everything below reads what earlier kernels wrote (maps through TMA, statistics, partial sums)
   return u;
 }
 
@@ -579,7 +577,7 @@ int crfr_norm_bwd_reduce_stream(const void* da, int da_ld, const void* db, int d
   a.out = (bf16*)dz; a.out_ld = dz_ld;
   a.partial = partial;
   CRFR_TRY(set_attrs());
-  CRFR_CUDA(crfr_launch_pdl(norm_bwd_reduce_stream_kernel, dim3(grid_for(npix, c)), dim3(kThreads), kSmemBytes, st, maps, a));
+  norm_bwd_reduce_stream_kernel<<<grid_for(npix, c), kThreads, kSmemBytes, st>>>(maps, a);
   CRFR_COUNT_LAUNCH();
   CRFR_LAUNCH_CHECK();
   return CRFR_OK;
@@ -610,7 +608,7 @@ int crfr_norm_bwd_apply_stream(const void* dsrc, int dsrc_ld, int recompute, con
   a.out = (bf16*)dy; a.out_ld = dy_ld;
   a.dgamma = dgamma; a.dbeta = dbeta; a.dalpha = dalpha;
   CRFR_TRY(set_attrs());
-  CRFR_CUDA(crfr_launch_pdl(norm_bwd_apply_stream_kernel, dim3(grid_for(npix, c)), dim3(kThreads), kSmemBytes, st, maps, a));
+  norm_bwd_apply_stream_kernel<<<grid_for(npix, c), kThreads, kSmemBytes, st>>>(maps, a);
   CRFR_COUNT_LAUNCH();
   CRFR_LAUNCH_CHECK();
   return CRFR_OK;
@@ -637,7 +635,7 @@ int crfr_norm_fwd_stream(const void* y, int y_ld, const float* stats, const floa
   a.stats = stats; a.gamma = gamma; a.beta = beta; a.alpha = alpha;
   a.out = (bf16*)out; a.out_ld = out_ld;
   CRFR_TRY(set_attrs());
-  CRFR_CUDA(crfr_launch_pdl(norm_fwd_stream_kernel, dim3(grid_for(npix, c)), dim3(kThreads), kSmemBytes, st, maps, a));
+  norm_fwd_stream_kernel<<<grid_for(npix, c), kThreads, kSmemBytes, st>>>(maps, a);
   CRFR_COUNT_LAUNCH();
   CRFR_LAUNCH_CHECK();
   return CRFR_OK;

@@ -748,8 +748,7 @@ struct Net {
     d.out_ld = dy.ld;
     d.in_ld = dx.ld;
     if (!run()) return;
-    if (stem && engine != CRFR_ENGINE_DIRECT && crfr_opt(CRFR_OPT_IR50_STEM_TC) && crfr_lowered_recipe(&d) == 1 &&
-        d.cout == 64 && d.h % 8 == 0)
+    if (stem && engine != CRFR_ENGINE_DIRECT && crfr_lowered_recipe(&d) == 1 && d.cout == 64 && d.h % 8 == 0)
       check(crfr_lowered_dgrad_cin3(&d, dy.p, wt, dx.p, scratch, scratch_bytes, st));
     else
       check(crfr_conv_dgrad(engine, &d, dy.p, wt, d.cout, dx.p, scratch, scratch_bytes, st));

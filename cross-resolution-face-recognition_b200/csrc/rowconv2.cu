@@ -53,23 +53,17 @@ constexpr int kWeightBytes = 3 * kKxBytes;
 //   FUSE = 1: 3 groups of 4 warps; warp q owns 32 pixels x 64 channels: 152 registers for the extra maps and sums
 // Group g takes the output rows with orow % kGroups == g.
 // Kernel variants V: 0 = plain, 1 = fused dgrad epilogue (FUSE above; 3 = the same for a normalisation without residual and
-// without a second gradient, whose epilogue fits the 16-warp half-row layout), 2 = forward with a TRANSFORM producer: 8 warps read
-// the raw map the preceding normalisation would have read, apply out = act(gamma * (y - mean) * rstd + beta (+ res)) in
-// registers and write the activated row straight into the shared-memory ring (and, optionally, to global memory for the
-// weight gradient): the separate normalisation pass over 2-3 maps disappears.  Whole-row epilogue, 2 groups.
+// without a second gradient, whose epilogue fits the 16-warp half-row layout).
 template <int V>
 struct Cfg {
   static constexpr int kGroups = V == 1 ? 3 : 2;
-  static constexpr int kRowWarps = (V == 0 || V == 3) ? 8 : 4;        // warps that share one output row
-  static constexpr int kXformWarps = V == 2 ? 8 : 0;                  // two teams of 4, alternate input rows
+  static constexpr int kRowWarps = V == 1 ? 4 : 8;                    // warps that share one output row
   static constexpr int kEpiThreads = 32 * kRowWarps * kGroups;
-  static constexpr int kThreads = 128 + kEpiThreads + 32 * kXformWarps;   // 640 / 512 / 640
-  // the CTA's register pool is what the launch allocates; the epilogue's share once the other warpgroups keep theirs
+  static constexpr int kThreads = 128 + kEpiThreads;                  // V = 0, 1, 3: 640 / 512 / 640
+  // the CTA's register pool is what the launch allocates; the epilogue's share once warpgroup 0 keeps its own
   static constexpr int kRegsLaunch = (65536 / kThreads) & ~7;
   static constexpr int kRegsLean = V == 1 ? 56 : 64;
-  static constexpr int kRegsXform = 96;
-  static constexpr int kRegsEpi =
-      ((kThreads * kRegsLaunch - 128 * kRegsLean - 32 * kXformWarps * kRegsXform) / kEpiThreads) & ~7;
+  static constexpr int kRegsEpi = ((kThreads * kRegsLaunch - 128 * kRegsLean) / kEpiThreads) & ~7;
 };
 constexpr int kMaxGroups = 3;
 constexpr int kAccSlots = 8;
@@ -83,8 +77,6 @@ struct PairParams {
   int n, h;              // images (even), rows per image
   int total_rows;        // (n / 2) * h: rows of the flattened (image pair, row) space
   int flip;              // 1: dgrad
-  int swap_halves;       // debugging aid: rank 0 holds the upper half of B
-  int dbg;               // ablation bits (CRFR_OPT_PAIR_DEBUG), 0 in production
   const float* bias;
   float* partial;        // InstanceNorm partials [n][parts][2][64] or nullptr
   int parts;
@@ -98,12 +90,6 @@ struct PairParams {
   const bf16* fres; int fres_ld;      // nullable
   const float* fstats; const float* fgamma; const float* fbeta; const float* falpha; int frelu;
   float* partial3;                    // [n][parts][3][64]: sum dz, sum dz * xhat, sum D * min(z, 0)
-  // V = 2 (forward only): the input rows are produced by transform warps from the raw map of the preceding normalisation,
-  // in = act(gamma * (xy - mean) * rstd + beta (+ xres)); xout (nullable): the activated rows also go to global memory
-  const bf16* xy; int xy_ld;
-  const bf16* xres; int xres_ld;
-  const float* xstats; const float* xgamma; const float* xbeta; const float* xalpha; int xrelu;
-  bf16* xout; int xout_ld;
 };
 
 // first row (of the 320 per kx) of the half that belongs to the sub-range (first tap j0, cnt taps) of the stacked B
@@ -114,15 +100,6 @@ __host__ __device__ __forceinline__ int case_row(int j0, int cnt) {
 __device__ __forceinline__ int first_cluster_of_row(long long x, int R, int G) {
   return (int)(((x + 1) * G + R - 1) / R) - 1;
 }
-
-// cycle counters for tools/pair_diag.py (compiled in with -DCRFR_PAIR_PROF=1 only: they cost the epilogue ~12 registers;
-// written when the debug option has bit 32): per cluster
-// [0] MMA warp total, [1] wait acc_empty, [2] wait full, [3] wait peer_full, [4] issue + commits,
-// [5] epilogue group 0 total, [6] its wait acc_full, [7] its tcgen05.ld / st / arrive, [8] its pack + store, [9] its statistics
-#ifndef CRFR_PAIR_PROF
-#define CRFR_PAIR_PROF 0
-#endif
-__device__ long long g_pair_prof[74 * 16];
 
 // input rows (with the halo rows of every segment) of a cluster's range, in load order
 struct RowWalk {
@@ -269,8 +246,6 @@ __device__ __forceinline__ void epilogue_half(const PairParams& p, const EpiCtx&
 #pragma unroll
   for (int k = 0; k < 4; ++k) sc[k] = sh[k] = al[k] = ad[k] = make_float2(0.f, 0.f);
   const bool f_act = FP && (p.frelu || p.falpha != nullptr);
-  const bool prof = CRFR_PAIR_PROF && (p.dbg & 32) != 0 && rank == 0 && ew == 0;
-  long long e_wait = 0, e_tmem = 0, e_pack = 0, e_stat = 0, e_start = clock64(), t0 = 0;
   int orow = 0;
   int gbase = 0;              // input rows of the previous segments
   long long r = cx.r_begin;
@@ -303,9 +278,7 @@ __device__ __forceinline__ void epilogue_half(const PairParams& p, const EpiCtx&
       const long long pix0 = ((long long)n * p.h + y) * kW + (q * 32 + pg * 4);
       if (FP && hf == 0)   // pull the lines of y this row reads into L2 while the warp waits for the MMAs
         asm volatile("prefetch.global.L2 [%0];" ::"l"(p.fy + (((long long)n * p.h + y) * kW + (q * 32 + lane)) * p.fy_ld));
-      if (prof) t0 = clock64();
       mbar_wait(&cx.done[g & (kDone - 1)], (g / kDone) & 1);
-      if (prof) { const long long t1 = clock64(); e_wait += t1 - t0; t0 = t1; }
       tc_fence_after();
       const uint32_t tcol = tmem + ((uint32_t)(q * 32) << 16) + slot * kC + hf * 32;
       uint32_t v[32];
@@ -316,8 +289,6 @@ __device__ __forceinline__ void epilogue_half(const PairParams& p, const EpiCtx&
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive_cluster(remote_acc_empty0 + 8u * (uint32_t)slot);
-      if (prof) { const long long t1 = clock64(); e_tmem += t1 - t0; t0 = t1; }
-      if (p.dbg & 4) continue;
       // + bias, round to bf16: w[4 c .. 4 c + 3] = chunk c (channels 32 hf + 8 c .. + 7) of this lane's pixel
       uint32_t w[16];
 #pragma unroll
@@ -372,14 +343,11 @@ __device__ __forceinline__ void epilogue_half(const PairParams& p, const EpiCtx&
           }
         }
       }
-      if (!(p.dbg & 8)) {
-        bf16* line = p.dst + pix0 * p.dst_ld + ch0;
+      bf16* line = p.dst + pix0 * p.dst_ld + ch0;
 #pragma unroll
-        for (int i = 0; i < 4; ++i)
-          *reinterpret_cast<uint4*>(line + (long long)i * p.dst_ld) = make_uint4(w[4 * i], w[4 * i + 1], w[4 * i + 2], w[4 * i + 3]);
-      }
-      if (prof) { const long long t1 = clock64(); e_pack += t1 - t0; t0 = t1; }
-      if (!FP && p.partial && !(p.dbg & 16)) {
+      for (int i = 0; i < 4; ++i)
+        *reinterpret_cast<uint4*>(line + (long long)i * p.dst_ld) = make_uint4(w[4 * i], w[4 * i + 1], w[4 * i + 2], w[4 * i + 3]);
+      if (!FP && p.partial) {
         // per-channel sums of the stored (rounded) values: this lane's 8 channels over its 4 pixels, packed fp32x2
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
@@ -391,7 +359,6 @@ __device__ __forceinline__ void epilogue_half(const PairParams& p, const EpiCtx&
           }
         }
       }
-      if (prof) e_stat += clock64() - t0;
     }
     if (FP || p.partial) {
       // end of this CTA's rows of image n: fold the group's pixel lanes in fixed order (8 lanes by shuffle, the 4
@@ -449,20 +416,14 @@ __device__ __forceinline__ void epilogue_half(const PairParams& p, const EpiCtx&
     gbase += iy1 - iy0 + 1;
     r += seg;
   }
-  if (prof && lane == 0) {
-    long long* o = g_pair_prof + cid * 16;
-    o[5] = clock64() - e_start; o[6] = e_wait; o[7] = e_tmem; o[8] = e_pack; o[9] = e_stat;
-  }
 }
 
 // FUSE = 1 (dgrad): the first pass of the normalisation backward on the rounded dgrad output, exactly as norm_stream.cu's
 // reduce pass: D = dgrad (+ db); z = sc * y + sh (+ res); z <= 0: ad += D * z, D *= al; dz = bf16(D) is stored in place of
 // the dgrad output; as += dz; aq += dz * y.  3 groups of 4 warps; warp q owns 32 pixels x 64 channels.
-template <int V>
 __device__ __forceinline__ void epilogue_row(const PairParams& p, const EpiCtx& cx) {
-  constexpr int kGroups = Cfg<V>::kGroups;
-  constexpr bool FUSED = V == 1;            // else: bias, plain store, InstanceNorm statistics of the stored values
-  constexpr int NQ = FUSED ? 3 : 2;
+  constexpr int kGroups = Cfg<1>::kGroups;
+  constexpr int NQ = 3;
   const int warp = cx.warp, lane = cx.lane;
   const uint32_t tmem = cx.tmem;
   const int ew = warp - 4, gi = ew >> 2;
@@ -473,9 +434,8 @@ __device__ __forceinline__ void epilogue_row(const PairParams& p, const EpiCtx& 
   const int bar_stat = 1 + gi;
   float* sSt = cx.sStat + gi * 768;         // [4 warps][NQ][64]
   const uint32_t remote_acc_empty0 = map_to_rank(&cx.acc_empty[0], 0);
-  const bool f_act = FUSED && (p.frelu || p.falpha != nullptr);
-  const bool f_b = FUSED && p.fb != nullptr, f_res = f_act && p.fres != nullptr;
-  const bool has_bias = !FUSED && p.bias != nullptr;
+  const bool f_act = p.frelu || p.falpha != nullptr;
+  const bool f_b = p.fb != nullptr, f_res = f_act && p.fres != nullptr;
   // coefficients of this lane's 8 channels for the current image (z = sc * y + sh, slope al for z <= 0); sums
   float2 sc[4], sh[4], al[4], as[4], aq[4], ad[4];
 #pragma unroll
@@ -490,7 +450,6 @@ __device__ __forceinline__ void epilogue_row(const PairParams& p, const EpiCtx& 
     const int n = 2 * pr + (int)cx.rank;
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
-      if (!FUSED) break;
       float t[6];
 #pragma unroll
       for (int e = 0; e < 2; ++e) {
@@ -510,11 +469,10 @@ __device__ __forceinline__ void epilogue_row(const PairParams& p, const EpiCtx& 
       const int g = gbase + (min(y + 1, iy1) - iy0);       // the input row whose MMAs complete this output row
       // element offset of this lane's 8 pixels of the row (pixel q * 32 + pg * 8 + i), before the per-map ld
       const long long pix0 = ((long long)n * p.h + y) * kW + (q * 32 + pg * 8);
-      if (FUSED) {   // pull the lines the fused pass reads into L2 while this warp waits for the MMAs (lane cg: pixel cg of its 8)
-        asm volatile("prefetch.global.L2 [%0];" ::"l"(p.fy + (pix0 + cg) * p.fy_ld));
-        if (f_b) asm volatile("prefetch.global.L2 [%0];" ::"l"(p.fb + (pix0 + cg) * p.fb_ld));
-        if (f_res) asm volatile("prefetch.global.L2 [%0];" ::"l"(p.fres + (pix0 + cg) * p.fres_ld));
-      }
+      // pull the lines the fused pass reads into L2 while this warp waits for the MMAs (lane cg: pixel cg of its 8)
+      asm volatile("prefetch.global.L2 [%0];" ::"l"(p.fy + (pix0 + cg) * p.fy_ld));
+      if (f_b) asm volatile("prefetch.global.L2 [%0];" ::"l"(p.fb + (pix0 + cg) * p.fb_ld));
+      if (f_res) asm volatile("prefetch.global.L2 [%0];" ::"l"(p.fres + (pix0 + cg) * p.fres_ld));
       mbar_wait(&cx.done[g & (kDone - 1)], (g / kDone) & 1);
       tc_fence_after();
       // two halves of 32 accumulator columns, each packed to bf16 before the next is read (bounds the live registers):
@@ -526,8 +484,7 @@ __device__ __forceinline__ void epilogue_row(const PairParams& p, const EpiCtx& 
         tmem_ld_wait();
 #pragma unroll
         for (int k = 0; k < 16; ++k) {
-          const __nv_bfloat162 lo = __floats2bfloat162_rn(__uint_as_float(v[2 * k]) + (has_bias ? cx.sBias[2 * k] : 0.f),
-                                                          __uint_as_float(v[2 * k + 1]) + (has_bias ? cx.sBias[2 * k + 1] : 0.f));
+          const __nv_bfloat162 lo = __floats2bfloat162_rn(__uint_as_float(v[2 * k]), __uint_as_float(v[2 * k + 1]));
           w[k] = *reinterpret_cast<const uint32_t*>(&lo);
         }
         tmem_ld32(tmem + ((uint32_t)(q * 32) << 16) + slot * kC + 32, v);
@@ -540,8 +497,7 @@ __device__ __forceinline__ void epilogue_row(const PairParams& p, const EpiCtx& 
         if (lane == 0) mbar_arrive_cluster(remote_acc_empty0 + 8u * (uint32_t)slot);
 #pragma unroll
         for (int k = 0; k < 16; ++k) {
-          const __nv_bfloat162 hi = __floats2bfloat162_rn(__uint_as_float(v[2 * k]) + (has_bias ? cx.sBias[32 + 2 * k] : 0.f),
-                                                          __uint_as_float(v[2 * k + 1]) + (has_bias ? cx.sBias[33 + 2 * k] : 0.f));
+          const __nv_bfloat162 hi = __floats2bfloat162_rn(__uint_as_float(v[2 * k]), __uint_as_float(v[2 * k + 1]));
           w[16 + k] = *reinterpret_cast<const uint32_t*>(&hi);
         }
       }
@@ -565,7 +521,6 @@ __device__ __forceinline__ void epilogue_row(const PairParams& p, const EpiCtx& 
       const bf16* bp = p.fb + pix0 * p.fb_ld + cg * 8;
       const bf16* rp = p.fres + pix0 * p.fres_ld + cg * 8;
       bf16* line = p.dst + pix0 * p.dst_ld + cg * 8;
-      if (FUSED) {
 #pragma unroll
       for (int h2 = 0; h2 < 4; ++h2) {   // four quarters of 2 pixels: bounds the registers of the maps in flight
         uint4 Yv[2], Bv[2], Rv[2];
@@ -585,11 +540,11 @@ __device__ __forceinline__ void epilogue_row(const PairParams& p, const EpiCtx& 
 #pragma unroll
           for (int k = 0; k < 4; ++k) {
             float2 gd = bf2(w[4 * i + k]);
-            if (f_b) gd = __fadd2_rn(gd, bf2(k == 0 ? Bv[i4].x : (k == 1 ? Bv[i4].y : (k == 2 ? Bv[i4].z : Bv[i4].w))));
-            const float2 f = bf2(k == 0 ? Yv[i4].x : (k == 1 ? Yv[i4].y : (k == 2 ? Yv[i4].z : Yv[i4].w)));
+            if (f_b) gd = __fadd2_rn(gd, bf2(uw(Bv[i4], k)));
+            const float2 f = bf2(uw(Yv[i4], k));
             if (f_act) {
               float2 z = __ffma2_rn(f, sc[k], sh[k]);
-              if (f_res) z = __fadd2_rn(z, bf2(k == 0 ? Rv[i4].x : (k == 1 ? Rv[i4].y : (k == 2 ? Rv[i4].z : Rv[i4].w))));
+              if (f_res) z = __fadd2_rn(z, bf2(uw(Rv[i4], k)));
               if (!(z.x > 0.f)) { ad[k].x = fmaf(gd.x, z.x, ad[k].x); gd.x *= al[k].x; }
               if (!(z.y > 0.f)) { ad[k].y = fmaf(gd.y, z.y, ad[k].y); gd.y *= al[k].y; }
             }
@@ -603,178 +558,52 @@ __device__ __forceinline__ void epilogue_row(const PairParams& p, const EpiCtx& 
           *reinterpret_cast<uint4*>(line + (long long)i * p.dst_ld) = make_uint4(w[4 * i], w[4 * i + 1], w[4 * i + 2], w[4 * i + 3]);
         }
       }
-      } else {
-#pragma unroll
-        for (int i = 0; i < 8; ++i)
-          *reinterpret_cast<uint4*>(line + (long long)i * p.dst_ld) = make_uint4(w[4 * i], w[4 * i + 1], w[4 * i + 2], w[4 * i + 3]);
-        if (p.partial) {
-          // per-channel sums of the stored (rounded) values: this lane's 8 channels over its 8 pixels, packed fp32x2
-#pragma unroll
-          for (int i = 0; i < 8; ++i) {
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-              const float2 f = bf2(w[4 * i + k]);
-              as[k] = __fadd2_rn(as[k], f);
-              aq[k] = __ffma2_rn(f, f, aq[k]);
-            }
-          }
-        }
-      }
     }
-    if (FUSED || p.partial) {
-      // end of this CTA's rows of image n: fold the group's pixel lanes in fixed order (4 lanes by shuffle, the 4 warps
-      // through shared memory) and publish the group's partial in its own slot - also when it is all zero
+    // end of this CTA's rows of image n: fold the group's pixel lanes in fixed order (4 lanes by shuffle, the 4 warps
+    // through shared memory) and publish the group's partial in its own slot - also when it is all zero
 #pragma unroll
-      for (int o = 8; o <= 16; o <<= 1) {
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-          as[k].x += __shfl_xor_sync(0xffffffffu, as[k].x, o);  as[k].y += __shfl_xor_sync(0xffffffffu, as[k].y, o);
-          aq[k].x += __shfl_xor_sync(0xffffffffu, aq[k].x, o);  aq[k].y += __shfl_xor_sync(0xffffffffu, aq[k].y, o);
-          if (FUSED) { ad[k].x += __shfl_xor_sync(0xffffffffu, ad[k].x, o);  ad[k].y += __shfl_xor_sync(0xffffffffu, ad[k].y, o); }
-        }
-      }
-      named_bar_sync(bar_stat, 128);   // previous use of the scratch is over
-      if (lane < 8) {
-        float* d0 = sSt + ((ew & 3) * NQ + 0) * kC + cg * 8;
-        float* d1 = sSt + ((ew & 3) * NQ + 1) * kC + cg * 8;
-        float* d2 = sSt + ((ew & 3) * NQ + 2) * kC + cg * 8;
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-          d0[2 * k] = as[k].x; d0[2 * k + 1] = as[k].y;
-          d1[2 * k] = aq[k].x; d1[2 * k + 1] = aq[k].y;
-          if (FUSED) { d2[2 * k] = ad[k].x; d2[2 * k + 1] = ad[k].y; }
-        }
-      }
-      named_bar_sync(bar_stat, 128);
-      const int b0 = first_cluster_of_row((long long)pr * p.h, p.total_rows, cx.ncl);
-      const int part = cx.cid - b0;
-      if (!FUSED) {
-        float* dst2 = p.partial + ((long long)n * p.parts + kGroups * part + gi) * 2 * kC;
-        dst2[et] = (sSt[et] + sSt[128 + et]) + (sSt[256 + et] + sSt[384 + et]);
-        if (y0 + seg == p.h && gi == 0)   // last cluster of this image: the unused slots must read as zero
-          for (int z = kGroups * (part + 1); z < p.parts; ++z) p.partial[((long long)n * p.parts + z) * 2 * kC + et] = 0.f;
-      }
-      float* dst = p.partial3 + ((long long)n * p.parts + kGroups * part + gi) * 3 * kC;
-      if (FUSED && et < kC) {
-        float t[3];
-#pragma unroll
-        for (int j = 0; j < 3; ++j)
-          t[j] = (sSt[j * kC + et] + sSt[(3 + j) * kC + et]) + (sSt[(6 + j) * kC + et] + sSt[(9 + j) * kC + et]);
-        // centre and scale: sum(dz * xhat) = rstd * (sum(dz * y) - mean * sum(dz))
-        const float mu = p.fstats[2 * (n * kC + et)], rs = p.fstats[2 * (n * kC + et) + 1];
-        dst[et] = t[0];
-        dst[kC + et] = (t[1] - mu * t[0]) * rs;
-        dst[2 * kC + et] = t[2];
-      }
-      if (FUSED && y0 + seg == p.h && gi == 0)   // last cluster of this image: the unused slots must read as zero
-        for (int z = kGroups * (part + 1); z < p.parts; ++z)
-          for (int j = et; j < 3 * kC; j += 128) p.partial3[((long long)n * p.parts + z) * 3 * kC + j] = 0.f;
-#pragma unroll
-      for (int k = 0; k < 4; ++k) as[k] = aq[k] = ad[k] = make_float2(0.f, 0.f);
-    }
-    gbase += iy1 - iy0 + 1;
-    r += seg;
-  }
-}
-
-
-// V = 2: the transform producer.  Two teams of 4 warps take alternate input rows; thread tt of a team owns the 16-byte chunk
-// cg = tt % 8 (channels 8 cg .. 8 cg + 7: its coefficients stay in registers) of pixels tt / 8 + 16 j.  A row is read with
-// ld.global (L2-resident: every thread pulls one 128-byte line of the row kXfAhead rows ahead into L2), normalised and
-// activated in registers and stored with st.shared.v4 exactly where the TMA box load of the plain kernel puts it
-// (SWIZZLE_128B: chunk index xor (row & 7); row 0 and row 129 of a slot are the zero halo, written once at start); then
-// fence.proxy.async (the tensor core reads through the async proxy) and one arrival per warp on the slot's barrier.
-constexpr int kXfAhead = 8;   // even: a team prefetches the rows it will transform itself
-__device__ __forceinline__ void sts128(uint32_t addr, const uint4& v) {
-  asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-}
-__device__ __forceinline__ void xform_produce(const PairParams& p, uint8_t* sRing, uint64_t* full, uint64_t* done,
-                                              long long r_begin, long long r_end, uint32_t rank, int tw, int lane) {
-  const int team = tw >> 2, tt = (tw & 3) * 32 + lane;
-  const int cg = tt & 7, px0 = tt >> 3;
-  const bool act = p.xrelu || p.xalpha != nullptr, has_res = p.xres != nullptr, side = p.xout != nullptr;
-  // byte offset of this thread's chunk of pixel px0 inside a slot (+ 2048 per 16 pixels: the swizzle phase repeats)
-  const uint32_t soff = (uint32_t)((px0 + 1) * 128 + ((cg ^ ((px0 + 1) & 7)) << 4));
-  float2 sc[4], sh[4], al[4];
-#pragma unroll
-  for (int k = 0; k < 4; ++k) sc[k] = sh[k] = al[k] = make_float2(0.f, 0.f);
-  int cur = -1;
-  RowWalk ld(r_begin, r_end, p.h);
-  // L2 prefetch cursor over the OUTPUT rows of the range (the input rows are the same rows +- 1), kXfAhead rows ahead
-  int ppr = (int)(r_begin / p.h), py = (int)(r_begin % p.h), pleft = (int)(r_end - r_begin);
-#define CRFR_XF_PREFETCH_STEP(mine)                                                                        \
-  if (pleft > 0) {                                                                                         \
-    if (mine) {                                                                                            \
-      const long long pl = ((long long)(2 * ppr + (int)rank) * p.h + py) * kW + tt;                        \
-      asm volatile("prefetch.global.L2 [%0];" ::"l"(p.xy + pl * p.xy_ld));                                 \
-      if (has_res) asm volatile("prefetch.global.L2 [%0];" ::"l"(p.xres + pl * p.xres_ld));                \
-    }                                                                                                      \
-    if (++py == p.h) { py = 0; ++ppr; }                                                                    \
-    --pleft;                                                                                               \
-  }
-#pragma unroll 1
-  for (int g = 0; g < kXfAhead; ++g) { CRFR_XF_PREFETCH_STEP((g & 1) == team) }
-#pragma unroll 1
-  for (int g = 0; ld.valid; ++g, ld.next()) {
-    CRFR_XF_PREFETCH_STEP((g & 1) == team)
-    if ((g & 1) != team) continue;
-    const int s = g % kSlots;
-    const int n = 2 * ld.pr + (int)rank;
-    if (n != cur) {
-      cur = n;
+    for (int o = 8; o <= 16; o <<= 1) {
 #pragma unroll
       for (int k = 0; k < 4; ++k) {
-        float t[6];
-#pragma unroll
-        for (int e = 0; e < 2; ++e) {
-          const int ch = cg * 8 + 2 * k + e;
-          const float mu = p.xstats[2 * (n * kC + ch)], rs = p.xstats[2 * (n * kC + ch) + 1];
-          t[e] = (p.xgamma ? p.xgamma[ch] : 1.f) * rs;
-          t[2 + e] = (p.xbeta ? p.xbeta[ch] : 0.f) - mu * t[e];
-          t[4 + e] = p.xrelu ? 0.f : (p.xalpha ? p.xalpha[ch] : 1.f);
-        }
-        sc[k] = make_float2(t[0], t[1]);
-        sh[k] = make_float2(t[2], t[3]);
-        al[k] = make_float2(t[4], t[5]);
+        as[k].x += __shfl_xor_sync(0xffffffffu, as[k].x, o);  as[k].y += __shfl_xor_sync(0xffffffffu, as[k].y, o);
+        aq[k].x += __shfl_xor_sync(0xffffffffu, aq[k].x, o);  aq[k].y += __shfl_xor_sync(0xffffffffu, aq[k].y, o);
+        ad[k].x += __shfl_xor_sync(0xffffffffu, ad[k].x, o);  ad[k].y += __shfl_xor_sync(0xffffffffu, ad[k].y, o);
       }
     }
-    const long long rowpix = ((long long)n * p.h + ld.iy) * kW + px0;
-    const bf16* src = p.xy + rowpix * p.xy_ld + cg * 8;
-    const bf16* rsrc = p.xres + rowpix * p.xres_ld + cg * 8;
-    bf16* osrc = p.xout + rowpix * p.xout_ld + cg * 8;
-    const uint32_t sbase = smem_u32(sRing + s * kSlotBytes) + soff;
+    named_bar_sync(bar_stat, 128);   // previous use of the scratch is over
+    if (lane < 8) {
+      float* d0 = sSt + ((ew & 3) * NQ + 0) * kC + cg * 8;
+      float* d1 = sSt + ((ew & 3) * NQ + 1) * kC + cg * 8;
+      float* d2 = sSt + ((ew & 3) * NQ + 2) * kC + cg * 8;
 #pragma unroll
-    for (int hh = 0; hh < 2; ++hh) {
-      uint4 Y[4], R[4];
-#pragma unroll
-      for (int j = 0; j < 4; ++j) Y[j] = ldg_stream(src + (long long)(16 * (4 * hh + j)) * p.xy_ld);
-      if (has_res) {
-#pragma unroll
-        for (int j = 0; j < 4; ++j) R[j] = ldg_stream(rsrc + (long long)(16 * (4 * hh + j)) * p.xres_ld);
-      }
-      if (hh == 0 && g >= kSlots) mbar_wait(&done[(g - kSlots) % kDone], ((g - kSlots) / kDone) & 1);   // slot consumed
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        uint4 O;
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-          float2 z = __ffma2_rn(bf2(uw(Y[j], k)), sc[k], sh[k]);
-          if (has_res) z = __fadd2_rn(z, bf2(uw(R[j], k)));
-          if (act) {
-            if (!(z.x > 0.f)) z.x *= al[k].x;
-            if (!(z.y > 0.f)) z.y *= al[k].y;
-          }
-          const __nv_bfloat162 pb = __floats2bfloat162_rn(z.x, z.y);
-          const uint32_t wv = *reinterpret_cast<const uint32_t*>(&pb);
-          if (k == 0) O.x = wv; else if (k == 1) O.y = wv; else if (k == 2) O.z = wv; else O.w = wv;
-        }
-        sts128(sbase + (uint32_t)((4 * hh + j) * 2048), O);
-        if (side) *reinterpret_cast<uint4*>(osrc + (long long)(16 * (4 * hh + j)) * p.xout_ld) = O;
+      for (int k = 0; k < 4; ++k) {
+        d0[2 * k] = as[k].x; d0[2 * k + 1] = as[k].y;
+        d1[2 * k] = aq[k].x; d1[2 * k + 1] = aq[k].y;
+        d2[2 * k] = ad[k].x; d2[2 * k + 1] = ad[k].y;
       }
     }
-    fence_proxy_async();
-    __syncwarp();
-    if (lane == 0) mbar_arrive(&full[s]);
+    named_bar_sync(bar_stat, 128);
+    const int b0 = first_cluster_of_row((long long)pr * p.h, p.total_rows, cx.ncl);
+    const int part = cx.cid - b0;
+    float* dst = p.partial3 + ((long long)n * p.parts + kGroups * part + gi) * 3 * kC;
+    if (et < kC) {
+      float t[3];
+#pragma unroll
+      for (int j = 0; j < 3; ++j)
+        t[j] = (sSt[j * kC + et] + sSt[(3 + j) * kC + et]) + (sSt[(6 + j) * kC + et] + sSt[(9 + j) * kC + et]);
+      // centre and scale: sum(dz * xhat) = rstd * (sum(dz * y) - mean * sum(dz))
+      const float mu = p.fstats[2 * (n * kC + et)], rs = p.fstats[2 * (n * kC + et) + 1];
+      dst[et] = t[0];
+      dst[kC + et] = (t[1] - mu * t[0]) * rs;
+      dst[2 * kC + et] = t[2];
+    }
+    if (y0 + seg == p.h && gi == 0)   // last cluster of this image: the unused slots must read as zero
+      for (int z = kGroups * (part + 1); z < p.parts; ++z)
+        for (int j = et; j < 3 * kC; j += 128) p.partial3[((long long)n * p.parts + z) * 3 * kC + j] = 0.f;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) as[k] = aq[k] = ad[k] = make_float2(0.f, 0.f);
+    gbase += iy1 - iy0 + 1;
+    r += seg;
   }
 }
 
@@ -801,7 +630,7 @@ rowconv_pair_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_consta
   const int cid = blockIdx.x >> 1, ncl = gridDim.x >> 1;
   if (threadIdx.x == 0) {
     for (int s = 0; s < kSlots; ++s) {
-      mbar_init(&full[s], FUSE == 2 ? 4 : 1);
+      mbar_init(&full[s], 1);
       mbar_init(&peer_full[s], 1);
     }
     for (int b = 0; b < kDone; ++b) mbar_init(&done[b], 1);
@@ -813,13 +642,6 @@ rowconv_pair_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_consta
     prefetch_tmap(&tmW);
   }
   if (threadIdx.x >= 64 && threadIdx.x < 64 + kC) sBias[threadIdx.x - 64] = p.bias ? p.bias[threadIdx.x - 64] : 0.f;
-  if (FUSE == 2) {   // zero halo pixels (rows 0 and 129) of every ring slot: the transform producer never writes them
-    for (int i = threadIdx.x; i < kSlots * 2 * 32; i += Cfg<FUSE>::kThreads) {
-      const int s = i >> 6, row = ((i >> 5) & 1) ? 129 : 0, word = i & 31;
-      *reinterpret_cast<uint32_t*>(sRing + s * kSlotBytes + row * 128 + word * 4) = 0u;
-    }
-    fence_proxy_async();
-  }
   if (warp == 1) tmem_alloc_pair(tmem_slot);
   tc_fence_before();
   __syncthreads();
@@ -833,9 +655,6 @@ rowconv_pair_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_consta
   __syncthreads();
   cluster_sync_all();   // barriers initialised and TMEM zeroed in BOTH CTAs before any remote arrive / pair MMA
   tc_fence_after();
-  pdl_trigger();
-  pdl_wait();           // the prologue above overlapped the previous kernel's tail; from here on its output is read
-                        // (a launch with a bias, which the prologue stages, does not use the attribute)
 
   // contiguous range of flattened (image pair, row) rows for this cluster; this CTA works on image 2 * pair + rank.
   // (Computed after setmaxnreg in each branch: what is live across it is spilled to local memory and reloaded in the loops.)
@@ -848,7 +667,7 @@ rowconv_pair_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_consta
     const bool leader = elect_one();
     if (leader) {
       mbar_expect_tx(w_full, kWeightBytes);
-      const int hi = (int)(rank ^ (uint32_t)p.swap_halves);   // 0: lower half of the stacked rows, 1: upper half
+      const int hi = (int)rank;                        // 0: lower half of the stacked rows, 1: upper half
       for (int kx = 0; kx < 3; ++kx)
         for (int cnt = 1; cnt <= 3; ++cnt)
           for (int j0 = 0; j0 + cnt <= 3; ++j0) {
@@ -866,16 +685,12 @@ rowconv_pair_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_consta
     // this warp's lanes - made the kernel 3-6 us SLOWER once the issuing warp was no longer the bottleneck: the launch moves
     // 537 MB in ~120 us, i.e. the memory system is already at 4.4 TB/s of mixed read / write traffic.)
     RowWalk ld(r_begin, r_end, p.h);
-    for (int g = 0; FUSE != 2 && ld.valid; ++g, ld.next()) {
+    for (int g = 0; ld.valid; ++g, ld.next()) {
       const int s = g % kSlots;
       if (g >= kSlots) mbar_wait(&done[(g - kSlots) % kDone], ((g - kSlots) / kDone) & 1);   // row g - kSlots consumed
       if (leader) {
-        if (p.dbg & 1) {
-          mbar_arrive(&full[s]);
-        } else {
-          mbar_expect_tx(&full[s], kRowBytes);
-          tma_load_4d(sRing + s * kSlotBytes, &tmX, &full[s], 0, -1, ld.iy, 2 * ld.pr + (int)rank);
-        }
+        mbar_expect_tx(&full[s], kRowBytes);
+        tma_load_4d(sRing + s * kSlotBytes, &tmX, &full[s], 0, -1, ld.iy, 2 * ld.pr + (int)rank);
       }
     }
   } else if (warp == 1 && rank != 0) {
@@ -904,8 +719,6 @@ rowconv_pair_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_consta
                    idesc3 = make_idesc_bf16(256, 3 * kC, 0, 0);
     mbar_wait(w_full, 0);
     mbar_wait_cluster(peer_w_full, 0);
-    const bool prof = CRFR_PAIR_PROF && (p.dbg & 32) != 0;
-    long long c_acc = 0, c_full = 0, c_peer = 0, c_issue = 0, t_start = clock64(), t0 = 0;
     int sg = 0;                 // ring slot of the current input row, and its parity
     uint32_t sph = 0;
     int dg = 0;                 // done barrier of the current input row (g % kDone)
@@ -920,22 +733,18 @@ rowconv_pair_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_consta
         // output rows fed by this input row, clipped to the segment
         const int t_lo = max(iy - 1, y0), t_hi = min(iy + 1, y0 + seg - 1);
         const int o_lo = obase + (t_lo - y0), o_hi = obase + (t_hi - y0);
-        if (prof) t0 = clock64();
         while (o_touched <= o_hi) {   // first touch: both epilogues have drained (and zeroed) the slot
           mbar_wait_cluster(&acc_empty[o_touched & (kAccSlots - 1)], ((o_touched >> 3) & 1) ^ 1);
           ++o_touched;
         }
-        if (prof) { const long long t1 = clock64(); c_acc += t1 - t0; t0 = t1; }
         const int slot = o_lo & (kAccSlots - 1);
         const int cnt = o_hi - o_lo + 1;
         const int j0 = t_lo - (iy - 1);
         mbar_wait(&full[sg], sph);
-        if (prof) { const long long t1 = clock64(); c_full += t1 - t0; t0 = t1; }
         mbar_wait_cluster(&peer_full[sg], sph);
-        if (prof) { const long long t1 = clock64(); c_peer += t1 - t0; t0 = t1; }
         tc_fence_after();
         const uint32_t a_lo = ring_lo + (uint32_t)(sg * (kSlotBytes >> 4));
-        if (leader && !(p.dbg & 2)) {
+        if (leader) {
           if (slot + cnt <= kAccSlots) {
             issue_row(tmem + slot * kC, a_lo, w_lo + (uint32_t)(case_row(j0, cnt) * 8), desc_hi,
                       cnt == 3 ? idesc3 : (cnt == 2 ? idesc2 : idesc1));
@@ -949,35 +758,25 @@ rowconv_pair_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_consta
         __syncwarp();
         if (++sg == kSlots) { sg = 0; sph ^= 1; }
         dg = (dg + 1) & (kDone - 1);
-        if (prof) c_issue += clock64() - t0;
       }
       obase += seg;
       r += seg;
     }
-    if (prof && lane == 0) {
-      long long* o = g_pair_prof + cid * 16;
-      o[0] = clock64() - t_start; o[1] = c_acc; o[2] = c_full; o[3] = c_peer; o[4] = c_issue;
-    }
   }
-  } else if (FUSE == 2 && warp >= 4 + Cfg<FUSE>::kEpiThreads / 32) {
-    asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(Cfg<FUSE>::kRegsXform));
-    const long long r_begin = (long long)p.total_rows * cid / ncl;
-    const long long r_end = (long long)p.total_rows * (cid + 1) / ncl;
-    xform_produce(p, sRing, full, done, r_begin, r_end, rank, warp - 4 - Cfg<FUSE>::kEpiThreads / 32, lane);
   } else {
     asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(Cfg<FUSE>::kRegsEpi));
     const long long r_begin = (long long)p.total_rows * cid / ncl;
     const long long r_end = (long long)p.total_rows * (cid + 1) / ncl;
     const EpiCtx cx = {tmem, done, acc_empty, sStat, sBias, r_begin, r_end, cid, ncl, rank, warp, lane};
     if (FUSE == 0 || FUSE == 3) epilogue_half<FUSE == 3>(p, cx);
-    else epilogue_row<FUSE>(p, cx);
+    else epilogue_row(p, cx);
   }
   tc_fence_before();
   __syncthreads();
   cluster_sync_all();   // nobody frees TMEM or leaves while the peer may still issue MMAs / remote arrives
   if (warp == 1) {
     tc_fence_after();
-    tmem_dealloc_pair(tmem);
+    tmem_dealloc_pair(*tmem_slot);   // read again: a register held across the setmaxnreg above may be spilled
   }
 }
 
@@ -1013,7 +812,7 @@ int crfr_rowconv_pair_parts(int n, int h, int plain) {
 // first pass to fuse->partial ([n][crfr_rowconv_pair_parts(n, h)][3][64] floats, to be folded by bwd_fold_kernel).
 int crfr_rowconv_pair(const void* src, int src_ld, int n, int h, const void* w_packed, int flip, const float* bias,
                       void* dst, int dst_ld, float* stats, float eps, void* ws, size_t ws_bytes, cudaStream_t st,
-                      const crfr_rowconv_fuse* fuse, const crfr_rowconv_xform* xf) {
+                      const crfr_rowconv_fuse* fuse) {
   CRFR_CHECK_ARG(crfr_rowconv_pair_supported(n, h), "rowconv_pair: needs an even number of images");
   CRFR_CHECK_ARG(((uintptr_t)src & 15) == 0 && ((uintptr_t)dst & 15) == 0 && ((uintptr_t)w_packed & 15) == 0 &&
                      (src_ld & 7) == 0 && (dst_ld & 7) == 0,
@@ -1023,14 +822,6 @@ int crfr_rowconv_pair(const void* src, int src_ld, int n, int h, const void* w_p
     CRFR_CHECK_ARG(((uintptr_t)fuse->y & 15) == 0 && ((uintptr_t)fuse->db & 15) == 0 && ((uintptr_t)fuse->res & 15) == 0 &&
                        ((fuse->y_ld | fuse->db_ld | fuse->res_ld) & 7) == 0,
                    "rowconv_pair: fused maps must be 16B aligned and ld a multiple of 8");
-  }
-  if (xf) {   // transform producer: src is not read (the rows come from xf->y), the activation map describes xf->y instead
-    CRFR_CHECK_ARG(!flip && !fuse && xf->y && xf->stats, "rowconv_pair: transform producer needs forward, y, stats");
-    CRFR_CHECK_ARG(((uintptr_t)xf->y & 15) == 0 && ((uintptr_t)xf->res & 15) == 0 && ((uintptr_t)xf->out & 15) == 0 &&
-                       ((xf->y_ld | xf->res_ld | xf->out_ld) & 7) == 0,
-                   "rowconv_pair: transform maps must be 16B aligned and ld a multiple of 8");
-    src = xf->y;
-    src_ld = xf->y_ld;
   }
   CUtensorMap tmX, tmW;
   {
@@ -1045,15 +836,12 @@ int crfr_rowconv_pair(const void* src, int src_ld, int n, int h, const void* w_p
     unsigned int box[2] = {64, 32};
     CRFR_TRY(crfr_tmap_encode_bf16(&tmW, w_packed, 2, dims, strides, box, "weights"));
   }
-  static std::atomic<unsigned long long> attr0{0}, attr1{0}, attr2{0}, attr3{0};
+  static std::atomic<unsigned long long> attr0{0}, attr1{0}, attr3{0};
   CRFR_CUDA((cudaError_t)crfr_smem_attr(rowconv_pair_kernel<3>, kSmemBytes, attr3));
   CRFR_CUDA((cudaError_t)crfr_smem_attr(rowconv_pair_kernel<0>, kSmemBytes, attr0));
   CRFR_CUDA((cudaError_t)crfr_smem_attr(rowconv_pair_kernel<1>, kSmemBytes, attr1));
-  CRFR_CUDA((cudaError_t)crfr_smem_attr(rowconv_pair_kernel<2>, kSmemBytes, attr2));
   PairParams p = {};
   p.n = n; p.h = h; p.total_rows = (n / 2) * h; p.flip = flip;
-  p.swap_halves = crfr_opt(CRFR_OPT_PAIR_SWAP);
-  p.dbg = crfr_opt(CRFR_OPT_PAIR_DEBUG);
   p.bias = bias;
   p.partial = nullptr;
   p.parts = 0;
@@ -1077,29 +865,16 @@ int crfr_rowconv_pair(const void* src, int src_ld, int n, int h, const void* w_p
     p.partial3 = fuse->partial;
     if (!fuse->db && !fuse->res) {   // plain form: 16-warp half-row epilogue
       p.parts = parts_for(n / 2, h, Cfg<3>::kGroups);
-      CRFR_CUDA(crfr_launch_pdl(rowconv_pair_kernel<3>, dim3(2 * clusters_for(p.total_rows)), dim3(Cfg<3>::kThreads), kSmemBytes, st, tmX, tmW, p));
+      rowconv_pair_kernel<3><<<2 * clusters_for(p.total_rows), Cfg<3>::kThreads, kSmemBytes, st>>>(tmX, tmW, p);
     } else {
       p.parts = parts_for(n / 2, h, Cfg<1>::kGroups);
-      CRFR_CUDA(crfr_launch_pdl(rowconv_pair_kernel<1>, dim3(2 * clusters_for(p.total_rows)), dim3(Cfg<1>::kThreads), kSmemBytes, st, tmX, tmW, p));
+      rowconv_pair_kernel<1><<<2 * clusters_for(p.total_rows), Cfg<1>::kThreads, kSmemBytes, st>>>(tmX, tmW, p);
     }
-  } else if (xf) {
-    p.xy = (const bf16*)xf->y; p.xy_ld = xf->y_ld;
-    p.xres = (const bf16*)xf->res; p.xres_ld = xf->res_ld;
-    p.xstats = xf->stats; p.xgamma = xf->gamma; p.xbeta = xf->beta; p.xalpha = xf->alpha; p.xrelu = xf->relu;
-    p.xout = (bf16*)xf->out; p.xout_ld = xf->out_ld;
-    CRFR_CUDA(crfr_launch_pdl_if(bias == nullptr, rowconv_pair_kernel<2>, dim3(2 * clusters_for(p.total_rows)), dim3(Cfg<2>::kThreads), kSmemBytes, st, tmX, tmW, p));
   } else {
-    CRFR_CUDA(crfr_launch_pdl_if(bias == nullptr, rowconv_pair_kernel<0>, dim3(2 * clusters_for(p.total_rows)), dim3(Cfg<0>::kThreads), kSmemBytes, st, tmX, tmW, p));
+    rowconv_pair_kernel<0><<<2 * clusters_for(p.total_rows), Cfg<0>::kThreads, kSmemBytes, st>>>(tmX, tmW, p);
   }
   CRFR_COUNT_LAUNCH();
   CRFR_LAUNCH_CHECK();
   if (stats) CRFR_TRY(crfr_norm_finalize(p.partial, n, p.parts, h * kW, kC, eps, stats, st));
-  return CRFR_OK;
-}
-
-// debugging aid for tools/pair_diag.py: copies the cycle counters of the last profiled launch (option pair_debug bit 32)
-extern "C" int crfr_debug_pair_profile(long long* host_out, int count) {
-  CRFR_CHECK_ARG(host_out && count > 0 && count <= 74 * 16, "debug_pair_profile: bad argument");
-  CRFR_CUDA(cudaMemcpyFromSymbol(host_out, g_pair_prof, sizeof(long long) * (size_t)count));
   return CRFR_OK;
 }

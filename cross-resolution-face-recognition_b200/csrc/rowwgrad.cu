@@ -112,8 +112,6 @@ rowwgrad_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
-  pdl_trigger();
-  pdl_wait();   // (common.cuh) the prologue overlapped the previous kernel's tail; x / dy are read from here on
 
   // paired: ranges of whole row pairs (h even: an image boundary is a pair boundary too)
   const long long units = p.paired ? p.total_rows / 2 : p.total_rows;
@@ -357,8 +355,6 @@ rowwgrad_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
 __global__ void __launch_bounds__(256)
 slab_reduce_kernel(const float* __restrict__ slabs, int nslabs, float* __restrict__ dw) {
   __shared__ float part[4][64];
-  pdl_trigger();
-  pdl_wait();
   const int o = threadIdx.x & 63, grp = threadIdx.x >> 6;
   const int i = blockIdx.x * 64 + o;   // over [t][ci][co]
   float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
@@ -422,10 +418,10 @@ int crfr_rowwgrad(const void* x, int x_ld, const void* dy, int dy_ld, int n, int
   p.prefetch = kPrefetch;
   p.paired = (h & 1) ? 0 : 1;
   const int grid = grid_for(p.total_rows, h);
-  CRFR_CUDA(crfr_launch_pdl(rowwgrad_kernel, dim3(grid), dim3(kThreads), kSmemBytes, st, tmX, tmDY, p));
+  rowwgrad_kernel<<<grid, kThreads, kSmemBytes, st>>>(tmX, tmDY, p);
   CRFR_COUNT_LAUNCH();
   CRFR_LAUNCH_CHECK();
-  CRFR_CUDA(crfr_launch_pdl(slab_reduce_kernel, dim3(kSlabFloats / 64), dim3(256), 0, st, (const float*)ws, grid, dw));
+  slab_reduce_kernel<<<kSlabFloats / 64, 256, 0, st>>>((const float*)ws, grid, dw);
   CRFR_COUNT_LAUNCH();
   CRFR_LAUNCH_CHECK();
   return CRFR_OK;

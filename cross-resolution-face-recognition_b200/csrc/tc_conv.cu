@@ -721,7 +721,7 @@ int crfr_tc_gemm(const TcGemm& g, cudaStream_t st) {
       return launch_conv<64>(tmA, tmB, tmY, p, tiles, st);
     case 96: return launch_conv<96>(tmA, tmB, tmY, p, tiles, st);
     case 128:
-      if (crfr_opt(CRFR_OPT_TC_T2) && tiles >= 4 * conv_sm_count()) return launch_conv<128, 2>(tmA, tmB, tmY, p, tiles, st);
+      if (tiles >= 4 * conv_sm_count()) return launch_conv<128, 2>(tmA, tmB, tmY, p, tiles, st);
       return launch_conv<128>(tmA, tmB, tmY, p, tiles, st);
     case 192: return launch_conv<192>(tmA, tmB, tmY, p, tiles, st);
     case 224: return launch_conv<224>(tmA, tmB, tmY, p, tiles, st);
@@ -829,11 +829,9 @@ size_t crfr_tc_workspace_bytes(const crfr_conv_desc* d) {
   return wg;
 }
 
-static int rowconv_enabled() { return crfr_opt(CRFR_OPT_ROWCONV); }
-
 int crfr_tc_conv(const crfr_conv_desc* d, int dgrad, const void* src, const void* w_packed, const float* bias,
                  void* dst, float* stats, float eps, void* ws, size_t ws_bytes, cudaStream_t st, int batch_stats) {
-  if (!batch_stats && rowconv_enabled() && crfr_rowconv_supported(d->h, d->w, d->cin, d->cout, d->k, d->stride, d->pad)) {
+  if (!batch_stats && crfr_rowconv_supported(d->h, d->w, d->cin, d->cout, d->k, d->stride, d->pad)) {
     return crfr_rowconv(src, dgrad ? d->out_ld : d->in_ld, d->n, d->h, w_packed, dgrad, bias, dst,
                         dgrad ? d->in_ld : d->out_ld, dgrad ? nullptr : stats, eps, ws, ws_bytes, st);
   }
@@ -867,7 +865,7 @@ int crfr_tc_conv(const crfr_conv_desc* d, int dgrad, const void* src, const void
 
 int crfr_tc_wgrad(const crfr_conv_desc* d, const void* x, const void* dy, float* dw, void* ws, size_t ws_bytes,
                   cudaStream_t st) {
-  if (rowconv_enabled() && crfr_rowwgrad_supported(d->h, d->w, d->cin, d->cout, d->k, d->stride, d->pad))
+  if (crfr_rowwgrad_supported(d->h, d->w, d->cin, d->cout, d->k, d->stride, d->pad))
     return crfr_rowwgrad(x, d->in_ld, dy, d->out_ld, d->n, d->h, dw, ws, ws_bytes, st);
   const size_t need = sizeof(float) * (size_t)9 * d->cin * d->cout;
   if (!ws || ws_bytes < need) {

@@ -135,7 +135,7 @@ def conv_wgrad(x, dy, cin, cout, k, stride, pad, engine=L.ENGINE_AUTO, transpose
 
 
 def set_option(name, value):
-    """Implementation switch for A/B measurements and tests (crfr_set_option in include/crfr.h)."""
+    """Implementation switch for tests and profiles (crfr_set_option in include/crfr.h)."""
     L.call("crfr_set_option", name.encode(), int(value))
 
 
@@ -192,23 +192,6 @@ def norm_act_bwd(dout, y, stats, gamma=None, beta=None, alpha=None, relu=False, 
            ld, ptr(stats), ptr(gamma), ptr(beta), ptr(alpha), int(relu), ptr(res), 8 if res is None else res.shape[3],
            ptr(dz), c, ptr(dy), c, ptr(dg), ptr(db), ptr(da), nn_, hw, c, ptr(ws), ws.numel(), stream())
     return dz, dy, dg, db, da
-
-
-def norm_act_conv_fwd(y, stats, w_packed, cin, cout, k, stride, pad, gamma=None, beta=None, alpha=None, relu=False, res=None,
-                      bias=None, want_stats=True, engine=L.ENGINE_AUTO):
-    """act = norm_act_fwd(y, ...); out = conv_fwd(act) as one call (crfr_norm_act_conv_fwd).  Returns (act, out, out_stats)."""
-    _need_cuda(y, stats, w_packed)
-    n, h, w, ld = y.shape
-    oh, ow = (h + 2 * pad - k) // stride + 1, (w + 2 * pad - k) // stride + 1
-    d = L.ConvDesc(n, h, w, cin, cout, k, stride, pad, oh, ow, cin, cout, 0)
-    act = torch.empty((n, h, w, cin), dtype=torch.bfloat16, device=y.device)
-    out = torch.empty((n, oh, ow, cout), dtype=torch.bfloat16, device=y.device)
-    st = torch.empty((n, cout, 2), dtype=torch.float32, device=y.device) if want_stats else None
-    ws = workspace(L.lib().crfr_conv_workspace_bytes(C.byref(d)))
-    L.call("crfr_norm_act_conv_fwd", engine, C.byref(d), ptr(y), ld, ptr(stats), ptr(gamma), ptr(beta), ptr(alpha), int(relu),
-           ptr(res), 8 if res is None else res.shape[3], ptr(act), cin, ptr(w_packed), cin, ptr(bias), ptr(out), ptr(st),
-           1e-5, ptr(ws), ws.numel(), stream())
-    return act, out, st
 
 
 def conv_dgrad_norm_bwd(dout, w_packed_t, y, stats, cin, cout, k, stride, pad, gamma=None, beta=None, alpha=None,

@@ -33,29 +33,19 @@ const char* crfr_last_error(void);
 int crfr_version(void);
 /* number of kernel launches issued by this library in this process (bench.py reports it as gpu_launches) */
 unsigned long long crfr_launch_count(void);
-/* Implementation switches for A/B measurements and tests (results are equivalent either way):
+/* Implementation switches for tests and profiles (results are equivalent either way); any other name is CRFR_EINVAL:
+ *   "rowconv_pair":  3x3 64 -> 64 convolutions at width 128 (forward and dgrad) with an even image count as 1 = the
+ *                    cta_group::2 kernel that pairs two CTAs (default), 0 = the single-CTA kernel; identical bits.
+ *   "wgrad_stream":  FSRNet backward, weight gradients as 1 = on a helper stream behind each layer's dgrad (default),
+ *                    0 = serially on the caller's stream (for profiles whose kernel times add up).
  *   "norm_bwd_impl": crfr_norm_act_bwd as 0 = register-staged reduce + fold + apply kernels, 1 = persistent TMA-fed
  *                    reduce + fold + apply kernels (default where the views are TMA-addressable: channels a multiple
  *                    of 64, 16-byte aligned), -1 = default / environment CRFR_NORM_BWD=regs|stream.
- *   "bn_fused_stats": ResNet program, train-mode BatchNorm statistics of the 3x3 stride-1 layers as 1 = from the tile engine's
- *                    epilogue (default), 0 = a separate pass over the stored output.
- *   "matcher_cluster": crfr_cosine_topk as 1 = clusters of two CTAs that multicast the gallery blocks (default), 0 = single CTAs.
- *   "tc_t2": tile engine at N = 128 as 0 = one pixel tile per weight tile, 1 = two (default; fewer TMA requests).
- *   "pdl": programmatic dependent launch of the persistent kernels, 0 (default) / 1.
- *   "fuse_norm_fwd": crfr_norm_act_conv_fwd as 0 = crfr_norm_act_fwd + crfr_conv_fwd (default), 1 = normalisation inside
- *                    the convolution's producer warps where the row-streaming pair kernel runs (identical bits; measured
- *                    SLOWER on B200, 208 us against 193 us per 128-image layer: the SM's instruction issue slots, which the
- *                    epilogue already uses to 60 %, are what the element-wise pass is bound by wherever it runs).
- *   "fuse_norm_bwd": crfr_conv_dgrad_norm_bwd as 0 = dgrad + crfr_norm_act_bwd, 1 = first pass of the normalisation
- *                    backward inside the dgrad epilogue where the row-streaming pair kernel runs (default).
  *   "norm_fwd_stream": crfr_norm_act_fwd as 0 = register-staged kernel, 1 = persistent TMA-fed kernel (default where the
  *                    views are TMA-addressable); identical results bit for bit.
- *   "ir50_stem_tc":  crfr_ir50_backward, dgrad of the 3 -> 64 stem convolution as 1 = im2col-free tcgen05 GEMM + col2im
- *                    (default), 0 = the direct CUDA-core kernel; equal up to the order of the fp32 sums. */
+ *   "fuse_norm_bwd": crfr_conv_dgrad_norm_bwd as 0 = dgrad + crfr_norm_act_bwd, 1 = first pass of the normalisation
+ *                    backward inside the dgrad epilogue where the row-streaming pair kernel runs (default). */
 int crfr_set_option(const char* name, int value);
-/* debugging aid (tools/pair_diag.py): cycle counters of the last rowconv pair-kernel launch made with option
- * "pair_debug" bit 32; 16 counters per cluster */
-int crfr_debug_pair_profile(long long* host_out, int count);
 /* 1 if the engine can run the shape (h,w,cin,cout,k,stride,pad), else 0 */
 int crfr_conv_engine_supported(int engine, int op, int h, int w, int cin, int cout, int k, int stride, int pad);
 
@@ -116,18 +106,6 @@ int crfr_norm_act_bwd(const void* dout_a, int da_ld, const void* dout_b, int db_
                       const float* stats, const float* gamma, const float* beta, const float* alpha, int relu,
                       const void* res, int res_ld, void* dz, int dz_ld, void* dy, int dy_ld, float* dgamma,
                       float* dbeta, float* dalpha, int n, int hw, int c, void* ws, size_t ws_bytes, void* stream);
-
-/* Forward of "conv(act(norm(y) (+ res)))" as one operation (ref: in1 -> relu -> conv2 and in2 -> add -> relu_out -> next
- * conv1 of _Residual_Block, model/FSRnet.py:91-97): act = crfr_norm_act_fwd(y, stats, ...) and out = crfr_conv_fwd(act)
- * (+ the InstanceNorm statistics of out).  d->in_ld must equal act_ld.  For the row-streaming shapes (3x3 s1 64 -> 64 at
- * width 128, even image count) with option "fuse_norm_fwd" = 1 the convolution's producer warps read y (and res),
- * normalise and activate in registers and write the rows straight into the shared-memory operand ring - `act` is written
- * as a by-product (the weight gradient needs it) and the separate pass over 2-3 maps disappears; identical results bit for
- * bit.  Default (option 0, see crfr_set_option) and other shapes: the two calls.  ws >= crfr_conv_workspace_bytes(d). */
-int crfr_norm_act_conv_fwd(int engine, const crfr_conv_desc* d, const void* y, int y_ld, const float* stats,
-                           const float* gamma, const float* beta, const float* alpha, int relu, const void* res, int res_ld,
-                           void* act, int act_ld, const void* w_packed, int cin_pad, const float* bias, void* out,
-                           float* out_stats, float eps, void* ws, size_t ws_bytes, void* stream);
 
 /* Backward of "conv(act(norm(y) (+ res)))" across the convolution's input, as one operation (ref: the
  * InstanceNorm2d -> PReLU -> Conv2d and InstanceNorm2d -> add -> PReLU -> Conv2d chains of _Residual_Block,

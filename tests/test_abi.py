@@ -59,6 +59,16 @@ def test_error_convention(lib):
     assert lib.crfr_fsrnet_workspace_bytes(4, 100, 1) == 0          # size must be a multiple of 16
 
 
+def test_set_option_names(lib):
+    """crfr_set_option takes the five implementation switches at their defaults and rejects the retired ones by name."""
+    for name in ("rowconv_pair", "wgrad_stream", "norm_bwd_impl", "norm_fwd_stream", "fuse_norm_bwd"):
+        assert lib.crfr_set_option(name.encode(), 1) == 0, lib.crfr_last_error()
+    for name in ("rowconv", "pair_swap", "rowwgrad_pair", "fuse_norm_fwd", "pdl", "tc_t2", "bn_fused_stats",
+                 "matcher_cluster", "pair_debug", "ir50_stem_tc"):
+        assert lib.crfr_set_option(name.encode(), 0) == 1                # CRFR_EINVAL
+        assert ("'%s'" % name).encode() in lib.crfr_last_error()
+
+
 def test_bicubic_tables_match_oracle(lib):
     from crfr_b200 import ops
     from oracle import bicubic_oracle as BO

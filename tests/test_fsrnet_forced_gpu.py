@@ -202,7 +202,7 @@ def test_batch128_forward_layers_and_backward_linearity(cuda):
     print("B=128 backward vs 32 x B=4 on the same forward: worst %.2e (%s)" % worst)
 
 
-@pytest.mark.parametrize("option,value", [("fuse_norm_bwd", 0), ("norm_bwd_impl", 0), ("wgrad_stream", 0), ("pdl", 1)])
+@pytest.mark.parametrize("option,value", [("fuse_norm_bwd", 0), ("norm_bwd_impl", 0), ("wgrad_stream", 0)])
 def test_backward_implementation_switches_agree_at_128(cuda, option, value):
     """The backward-side implementation switches at the BASELINE resolution (B = 4, 128 x 128: the row-streaming kernels, the
     fused dgrad + normalisation-backward epilogue, the weight-gradient helper stream) leave the forward untouched - losses
@@ -215,7 +215,7 @@ def test_backward_implementation_switches_agree_at_128(cuda, option, value):
     st = _Step(net, x, (hr, hm, lbl.contiguous()))
     losses0, grads0 = st.train_step()
     outs0 = [o.clone() for o in st.outs]
-    default = {"fuse_norm_bwd": 1, "norm_bwd_impl": -1, "wgrad_stream": 1, "pdl": 0}[option]
+    default = {"fuse_norm_bwd": 1, "norm_bwd_impl": -1, "wgrad_stream": 1}[option]
     try:
         ops.set_option(option, value)
         losses1, grads1 = st.train_step()
@@ -231,9 +231,9 @@ def test_backward_implementation_switches_agree_at_128(cuda, option, value):
         errs.append((rel_err(a, b), k))
     errs.sort(reverse=True)
     print("%s=%d against the default: largest gradient differences %s" % (option, value, ["%.2e %s" % e for e in errs[:4]]))
-    # wgrad_stream / pdl only reorder launches: equal up to the float atomics of the 3-channel edge layers' weight gradient
+    # wgrad_stream only reorders launches: equal up to the float atomics of the 3-channel edge layers' weight gradient
     # (direct_conv.cu); the other two re-associate the fp32 sums of the normalisation backward: a few dy elements round
     # the other way, and the bf16 storage of the gradients below carries that like any other rounding noise (the bound of
     # the deep half of the network, GRAD_TOL_DEEP; measured worst 1.7e-2 on a PReLU slope of the coarse network)
     for e, k in errs:
-        assert e < (1e-5 if option in ("wgrad_stream", "pdl") else _tol(k, REASSOC_TOL_DEEP)), (k, e)
+        assert e < (1e-5 if option == "wgrad_stream" else _tol(k, REASSOC_TOL_DEEP)), (k, e)

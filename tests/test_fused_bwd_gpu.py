@@ -107,37 +107,3 @@ def test_fused_dgrad_norm_bwd_other_shapes_fall_back(cuda):
     o.backward(dout)
     assert rel_err(to_nchw(dy), yr.grad) < 2e-2 and rel_err(da, ar.grad) < 1e-2
 
-
-@pytest.mark.parametrize("n,h,res", [(2, 1, False), (2, 2, True), (6, 3, True), (40, 16, False), (8, 50, True),
-                                     (2, 128, False), (34, 128, True), (300, 1, True)])
-def test_fused_norm_act_conv_fwd(cuda, n, h, res):
-    """crfr_norm_act_conv_fwd: the transform producer of rowconv2.cu (option fuse_norm_fwd) normalises and activates the
-    raw rows on their way into the shared-memory operand ring.  Same arithmetic per element as crfr_norm_act_fwd and the
-    same MMA order as the plain kernel -> the activated map and the convolution output are identical BIT FOR BIT to the
-    two separate calls; the statistics differ only in fp32 summation order.  Both against fp32 PyTorch."""
-    from crfr_b200 import _lib as L, ops
-    y, r, _, wgt, _, gamma, beta, alpha = _case(n, h, res, False, 1300 + n + h)
-    g = torch.Generator().manual_seed(n)
-    bias = torch.randn(64, generator=g)
-    yg = nhwc_from(y)
-    stats = ops.norm_stats(yg)
-    wp = ops.pack_conv_weight(wgt.cuda())
-    rg = nhwc_from(r) if res else None
-    out = {}
-    try:
-        for mode in (0, 1):
-            ops.set_option("fuse_norm_fwd", mode)
-            out[mode] = ops.norm_act_conv_fwd(yg, stats, wp, 64, 64, 3, 1, 1, gamma.cuda(), beta.cuda(), alpha.cuda(), res=rg,
-                                              bias=bias.cuda(), engine=L.ENGINE_TCGEN05)
-            torch.cuda.synchronize()
-    finally:
-        ops.set_option("fuse_norm_fwd", 1)
-    assert torch.equal(out[0][0], out[1][0]), "activated map differs: %.3e" % rel_err(out[1][0].float(), out[0][0].float())
-    assert torch.equal(out[0][1], out[1][1]), "conv output differs: %.3e" % rel_err(out[1][1].float(), out[0][1].float())
-    assert rel_err(out[1][2], out[0][2]) < 1e-5
-    z = F.instance_norm(y, weight=gamma, bias=beta, eps=1e-5)
-    if res:
-        z = z + r
-    a_ref = F.prelu(z, alpha)
-    assert rel_err(to_nchw(out[1][0]), a_ref) < 5e-3
-    assert rel_err(to_nchw(out[1][1]), F.conv2d(bf16_round(a_ref), wgt, bias, 1, 1)) < 1e-2

@@ -43,6 +43,7 @@ DIRECT_SHAPES = [
     (256, 512, 1, 2, 0, 14),   # layer4.0.downsample.0
     (3, 64, 7, 4, 3, 48),      # stems at sizes whose pixel count is no multiple of the gather kernel's 64-pixel blocks
     (3, 64, 7, 2, 3, 50),
+    (3, 64, 3, 1, 1, 112),     # IR stem            (model/model_irse.py:131)
 ]
 
 

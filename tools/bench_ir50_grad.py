@@ -2,22 +2,17 @@
 
 Usage: python tools/bench_ir50_grad.py [--batch 256] [--iters 20] [--warmup 3] [--arch ir50]
 
---arch ir_se50 | ir101 | ir152 | ir_se101 | ir_se152 times the other IR / IR-SE teachers instead: forward and forward +
-input gradient (crfr_irnet_*), and for the SE variants the device time of each SE kernel in one forward + backward
-(torch.profiler, a separate pass) next to the bytes it moves.  The stem-path comparison below is IR_50's only.
+--arch ir_se50 | ir101 | ir152 | ir_se101 | ir_se152 times the other IR / IR-SE teachers instead (crfr_irnet_*).
 
 Times, with CUDA events after warm-up and in one process:
   * forward only (no grad: the shared-workspace path) and forward + input gradient (autograd path, all five outputs seeded),
     reported as images/s and GFLOP/s with the FLOPs counted from the layer shapes below;
-  * the backward alone, with the stem's dgrad on the tcgen05 GEMM (option "ir50_stem_tc" = 1) and on the direct kernel
-    (= 0), alternated; their difference is the difference of the two stem paths;
-  * the direct stem dgrad by itself (crfr_conv_dgrad on the stem's shape);
-  * each stem path's own kernels inside the backward, from torch.profiler in a separate pass: the device time of the
-    kernels (and copies) between the last element-wise backward kernel and the final NHWC -> NCHW conversion of dx.
+  * the backward alone, repeated on one saved forward;
+  * for the SE variants, the device time of each SE kernel in one forward + backward (torch.profiler, a separate pass) next
+    to the bytes it moves.
 Prints the device name and power limit, then one JSON line.  Writes nothing.
 """
 import argparse
-import ctypes as C
 import json
 import os
 import subprocess
@@ -109,8 +104,6 @@ def main():
     import torch
     if not torch.cuda.is_available():
         raise SystemExit("bench_ir50_grad: needs a CUDA device")
-    from crfr_b200 import _lib as L
-    from crfr_b200 import ops
     from crfr_b200.model import model_irse as M
     from oracle import resnet_oracle as RO
 
@@ -128,7 +121,6 @@ def main():
     seeds = [t.cuda() for t in (torch.randn(B, 512, generator=g), torch.randn(B, 64, 56, 56, generator=g),
                                 torch.randn(B, 128, 28, 28, generator=g), torch.randn(B, 256, 14, 14, generator=g),
                                 torch.randn(B, 512, 7, 7, generator=g))]
-    lib = L.lib()
 
     def timed(fn, iters):
         for _ in range(args.warmup):
@@ -154,84 +146,23 @@ def main():
 
     t_fwd = timed(fwd, args.iters)
     t_fb = timed(fwd_bwd, args.iters)
-    if args.arch != "ir50":
-        f_fwd, f_bwd = ir50_flops_per_image(num_layers)
-        name, power = gpu_info()
-        res = {
-            "arch": ctor, "device": name, "power_limit": power, "batch": B, "iters": args.iters,
-            "gflop_per_image_fwd": round(f_fwd / 1e9, 3), "gflop_per_image_dgrad": round(f_bwd / 1e9, 3),
-            "fwd_ms": round(t_fwd, 3), "fwd_images_per_s": round(B / t_fwd * 1e3, 1),
-            "fwd_tflops": round(B * f_fwd / t_fwd / 1e9, 1),
-            "fwd_grad_ms": round(t_fb, 3), "fwd_grad_images_per_s": round(B / t_fb * 1e3, 1),
-            "fwd_grad_tflops": round(B * (f_fwd + f_bwd) / t_fb / 1e9, 1),
-        }
-        if se:
-            res["se_kernels"] = se_kernel_profile(torch, fwd_bwd, B, num_layers)
-        print("device: %s, power limit: %s" % (name, power))
-        print(json.dumps(res))
-        return
-
-    # backward alone on one saved forward, both stem paths alternated
     outs = net.forward_features(xg)
-    t_bwd = {1: [], 0: []}
-    for _ in range(3):
-        for opt in (1, 0):
-            L.call("crfr_set_option", b"ir50_stem_tc", opt)
-            t_bwd[opt].append(timed(lambda: torch.autograd.grad(outs, xg, seeds, retain_graph=True), args.iters))
-    L.call("crfr_set_option", b"ir50_stem_tc", 1)
-
-    # direct stem dgrad alone: dX [B,112,112,4] <- dY [B,112,112,64]
-    d = L.ConvDesc(B, 112, 112, 3, 64, 3, 1, 1, 112, 112, 4, 64, 0)
-    dy = torch.randn(B, 112, 112, 64, generator=g).to(torch.bfloat16).cuda()
-    dxs = torch.empty(B, 112, 112, 4, dtype=torch.bfloat16, device="cuda")
-    wt = torch.empty(9 * 3 * 64, dtype=torch.bfloat16, device="cuda")
-    w = net.input_layer[0].weight.detach()
-    L.call("crfr_pack_weight", w.data_ptr(), wt.data_ptr(), 9, 3, 64, 64, 9, 27, 1, ops.stream())
-    wsb = lib.crfr_conv_workspace_bytes(C.byref(d))
-    ws = torch.empty(max(wsb, 1), dtype=torch.uint8, device="cuda")
-    t_stem_direct = timed(lambda: L.call("crfr_conv_dgrad", L.ENGINE_AUTO, C.byref(d), dy.data_ptr(), wt.data_ptr(), 64,
-                                         dxs.data_ptr(), ws.data_ptr(), wsb, ops.stream()), args.iters)
-
-    # each stem path's kernels alone, profiled in their own pass (the profiler slows the host, not the kernels)
-    def stem_kernels_ms(opt):
-        from torch.profiler import ProfilerActivity, profile
-        L.call("crfr_set_option", b"ir50_stem_tc", opt)
-        torch.autograd.grad(outs, xg, seeds, retain_graph=True)
-        torch.cuda.synchronize()
-        with profile(activities=[ProfilerActivity.CUDA]) as prof:
-            torch.autograd.grad(outs, xg, seeds, retain_graph=True)
-            torch.cuda.synchronize()
-        L.call("crfr_set_option", b"ir50_stem_tc", 1)
-        ev = sorted((e for e in prof.events() if e.device_type == torch.autograd.DeviceType.CUDA),
-                    key=lambda e: e.time_range.start)
-        last_ew = max(i for i, e in enumerate(ev) if "ir50_bwd_ew_kernel" in e.name)
-        last_cvt = max(i for i, e in enumerate(ev) if "nhwc_to_nchw_kernel" in e.name)
-        stem = ev[last_ew + 1:last_cvt]
-        return sum(e.time_range.elapsed_us() for e in stem) / 1e3, sorted({kernel_name(e.name) for e in stem})
-
-    stem_tc_ms, stem_tc_kernels = stem_kernels_ms(1)
-    stem_direct_ms, stem_direct_kernels = stem_kernels_ms(0)
-
-    f_fwd, f_bwd = ir50_flops_per_image()
+    t_bwd = timed(lambda: torch.autograd.grad(outs, xg, seeds, retain_graph=True), args.iters)
+    f_fwd, f_bwd = ir50_flops_per_image(num_layers)
     name, power = gpu_info()
-    best = {k: min(v) for k, v in t_bwd.items()}
     res = {
-        "device": name, "power_limit": power, "batch": B, "iters": args.iters,
+        "arch": ctor, "device": name, "power_limit": power, "batch": B, "iters": args.iters,
         "gflop_per_image_fwd": round(f_fwd / 1e9, 3), "gflop_per_image_dgrad": round(f_bwd / 1e9, 3),
         "fwd_ms": round(t_fwd, 3), "fwd_images_per_s": round(B / t_fwd * 1e3, 1),
         "fwd_tflops": round(B * f_fwd / t_fwd / 1e9, 1),
         "fwd_grad_ms": round(t_fb, 3), "fwd_grad_images_per_s": round(B / t_fb * 1e3, 1),
         "fwd_grad_tflops": round(B * (f_fwd + f_bwd) / t_fb / 1e9, 1),
-        "bwd_ms_stem_tc": round(best[1], 3), "bwd_ms_stem_direct": round(best[0], 3),
-        "bwd_ms_all": {k: [round(v, 3) for v in vs] for k, vs in t_bwd.items()},
-        "bwd_over_fwd": round(best[1] / t_fwd, 2),
-        "stem_dgrad_direct_ms": round(t_stem_direct, 3),
-        "stem_dgrad_in_bwd_ms": {"tcgen05": round(stem_tc_ms, 3), "direct": round(stem_direct_ms, 3)},
-        "stem_dgrad_kernels": {"tcgen05": stem_tc_kernels, "direct": stem_direct_kernels},
+        "bwd_ms": round(t_bwd, 3), "bwd_over_fwd": round(t_bwd / t_fwd, 2),
     }
+    if se:
+        res["se_kernels"] = se_kernel_profile(torch, fwd_bwd, B, num_layers)
     print("device: %s, power limit: %s" % (name, power))
     print(json.dumps(res))
-
 
 if __name__ == "__main__":
     main()
