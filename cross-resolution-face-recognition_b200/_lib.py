@@ -131,6 +131,7 @@ SIGNATURES = {
     "crfr_irnet_forward": (ci, [ci, ci, ci, vp, vp, C.POINTER(ResnetIO), vp, csz, vp]),
     "crfr_irnet_grad_workspace_bytes": (csz, [ci, ci, ci, ci]),
     "crfr_irnet_tape": (ci, [ci, ci, ci, ci, C.POINTER(TapeEntry), ci]),
+    "crfr_irnet_grad_tape": (ci, [ci, ci, ci, ci, ci, C.POINTER(TapeEntry), ci]),
     "crfr_irnet_backward": (ci, [ci, ci, ci, vp, vp, C.POINTER(ResnetIO), vp, vp, vp, vp, csz, vp]),
 }
 

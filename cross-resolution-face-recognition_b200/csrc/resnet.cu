@@ -373,6 +373,7 @@ struct Net {
   std::vector<IrUnit> ir_units;               // IR program: the units, and the stem / head ops, as tape indices
   int ir_stem_conv = -1, ir_stem_bn = -1, ir_head_bn0 = -1, ir_head_lin = -1, ir_head_bn1 = -1;
   int ir_layers = 50, ir_se = 0;              // IR program variant: 50 / 100 / 152 layers, bottleneck_IR(_SE)
+  std::vector<crfr_tape_entry>* grad_tape = nullptr;   // set: backward_ir lists its stored gradients here (kinds 11-16)
 
   void* alloc(size_t bytes) {
     size_t a = (off + 1023) & ~(size_t)1023;
@@ -768,9 +769,24 @@ struct Net {
     check_cuda(cudaGetLastError());
   }
 
+  // one entry of the gradient tape (crfr_irnet_grad_tape): the bf16 gradient at p (pixel stride ld) with respect to the
+  // stored forward tensor `of`, and an optional fp32 side result; offsets are bytes from the workspace base
+  void record_grad(int kind, int unit, const Tensor& of, const bf16* p, int ld, const float* stats = nullptr) {
+    if (!grad_tape) return;
+    crfr_tape_entry e;
+    e.kind = kind;
+    e.n = of.n; e.h = of.h; e.w = of.w; e.c = of.c; e.ld = ld;
+    e.out_off = (long long)((const uint8_t*)p - ws);
+    e.in_off = (long long)((const uint8_t*)of.p - ws);
+    e.stats_off = stats ? (long long)((const uint8_t*)stats - ws) : -1;
+    e.w_idx = unit;
+    e.has_res = 0;
+    grad_tape->push_back(e);
+  }
+
   // SE unit: the gradient dr at the SE input r from the unit's output gradient g (dr = e * g + W1^T dh / hw, see
   // se_bwd_tail_kernel) - a deterministic per-(image, channel) reduction, the tiny per-image tail, one element-wise pass
-  Tensor se_grad(const Op& se, const Slot& g) {
+  Tensor se_grad(const Op& se, const Slot& g, int unit) {
     const Tensor& y = se.a;
     const int hw = y.h * y.w, chunks = se_chunks(hw), hid = y.c / kSeReduction;
     float* part = (float*)alloc((size_t)y.n * chunks * 2 * y.c * sizeof(float));
@@ -786,6 +802,7 @@ struct Net {
       check_cuda(cudaGetLastError());
     }
     ew(g, Tensor{}, nullptr, -1, nullptr, 0, dr, se.stats, shift);
+    record_grad(13, unit, y, dr.p, dr.ld, shift);
     return dr;
   }
 
@@ -843,6 +860,7 @@ struct Net {
         TcGemm g{de.p, B, 1, 1, kEmb, de.ld, wlt, 1, 0, 1, K, 0, da.p, K, 0, nullptr};
         check(crfr_tc_gemm(g, st));
       }
+      record_grad(11, -1, a4, da.p, da.ld);
       add_slot(a4, da.p, da.ld);
     }
     for (int l = 0; l < 4; ++l) seed_grad(feat[l], d_feat ? d_feat[l] : nullptr);
@@ -855,15 +873,17 @@ struct Net {
       if (!has_grad(b4.out)) continue;
       squash(b4.out, 1);
       const Slot g = slots[b4.out.id][0];
+      record_grad(12, u, b4.out, g.p, g.ld);
       Tensor d_r2 = map_like(pr.out);
       if (U.fc1 >= 0) {
-        const Tensor dr = se_grad(b4, g);                                  // res_layer.5
+        const Tensor dr = se_grad(b4, g, u);                               // res_layer.5
         dgrad(tape[U.conv2], Slot{dr.p, dr.ld}, w2[u], d_r2);             // res_layer.4 + .3
       } else {
         dgrad(tape[U.conv2], g, w2[u], d_r2);                             // res_layer.4 + .3
       }
       const Slot s_r2{d_r2.p, d_r2.ld};
       ew(s_r2, pr.a, nullptr, pr.alpha_idx, nullptr, 0, d_r2);     // res_layer.2, in place
+      record_grad(14, u, pr.a, d_r2.p, d_r2.ld);
       Tensor d_in = map_like(in);
       dgrad(tape[U.conv1], s_r2, w1[u], d_in);                            // res_layer.1 + .0
       const Slot s_in{d_in.p, d_in.ld};
@@ -875,6 +895,7 @@ struct Net {
       } else {                                                             // identity / MaxPool2d(1, 2)
         ew(s_in, Tensor{}, nullptr, -1, &g, U.sub >= 0 ? 2 : 1, d_in);
       }
+      record_grad(15, u, in, d_in.p, d_in.ld);
       add_slot(in, d_in.p, d_in.ld);
     }
 
@@ -888,6 +909,7 @@ struct Net {
     squash(sb.out, 1);
     Tensor dy0 = map_like(sb.a);
     ew(slots[sb.out.id][0], sb.a, &sb, sb.alpha_idx, nullptr, 0, dy0);
+    record_grad(16, -1, sb.a, dy0.p, dy0.ld);
     Tensor dx4 = map_like(s0.a);
     dgrad(s0, Slot{dy0.p, dy0.ld}, w0, dx4, true);
     if (run()) check(crfr_nhwc_bf16_to_nchw_f32(dx4.p, dx, B, 3, dx4.h, dx4.w, dx4.ld, st));
@@ -1025,7 +1047,12 @@ extern "C" size_t crfr_resnet34_workspace_bytes(int batch, int size, int trainin
 // table and replay them into the CPU oracle (teacher-forced forward / backward checks, tests/test_resnet_forced_gpu.py).
 namespace {
 // kinds: 0 convolution, 1 BatchNorm (+ residual) (+ ReLU / PReLU), 7 linear head, 8 PReLU pass, 9 stride-2 subsampling,
-// 10 SE unit output (BatchNorm + excitation + residual; stats_off: the excitation e [n][c] fp32)
+// 10 SE unit output (BatchNorm + excitation + residual; stats_off: the excitation e [n][c] fp32).
+// Gradient tape of the IR backward (crfr_irnet_grad_tape; in_off: out_off of the stored forward tensor differentiated,
+// w_idx: the unit, -1 outside the body): 11 the head's input gradient (at output_layer.0's input), 12 a unit's summed
+// output gradient g, 13 an SE unit's dr at r = BN_4(y) (in_off: y; stats_off: shift [n][c] fp32 = dpool / hw), 14 the
+// gradient at res_layer.1's output (after the PReLU pass), 15 a unit's input gradient, 16 the stem's dy0 (at
+// input_layer.0's output)
 int fill_tape(const Net& net, crfr_tape_entry* entries, int max_entries) {
   const int count = (int)net.tape.size();
   for (int i = 0; i < count && i < max_entries && entries; ++i) {
@@ -1098,6 +1125,25 @@ extern "C" int crfr_irnet_tape(int num_layers, int se, int batch, int size, crfr
   Net net;
   ir_dry_run(net, io, num_layers, se, batch, size, false);
   return fill_tape(net, entries, max_entries);
+}
+// Where crfr_irnet_backward leaves each stored gradient: the dry run that the call performs (forward, then backward_ir
+// with exec false), recorded from inside backward_ir, so the offsets are those of the real call.  seed_mask: which upstream
+// gradients are given (1 = d_emb, 2 / 4 / 8 / 16 = d_feat[0..3]); the layout depends on it.
+extern "C" int crfr_irnet_grad_tape(int num_layers, int se, int batch, int size, int seed_mask, crfr_tape_entry* entries,
+                                    int max_entries) {
+  if (!ir_variant_ok(num_layers, se) || batch <= 0 || size != 112 || seed_mask <= 0 || seed_mask > 31) return -1;
+  crfr_resnet_io io;
+  Net net;
+  ir_dry_run(net, io, num_layers, se, batch, size, false);
+  std::vector<crfr_tape_entry> rec;
+  net.grad_tape = &rec;
+  static float dummy = 0.f;   // non-null marker of a given seed
+  const float* feats[4];
+  for (int l = 0; l < 4; ++l) feats[l] = (seed_mask >> (l + 1)) & 1 ? &dummy : nullptr;
+  net.backward_ir(seed_mask & 1 ? &dummy : nullptr, feats, &dummy);
+  const int count = (int)rec.size();
+  for (int i = 0; i < count && i < max_entries && entries; ++i) entries[i] = rec[i];
+  return count;
 }
 extern "C" int crfr_ir50_tape(int batch, int size, crfr_tape_entry* entries, int max_entries) {
   return crfr_irnet_tape(50, 0, batch, size, entries, max_entries);

@@ -415,6 +415,15 @@ int crfr_irnet_forward(int engine, int num_layers, int se, const float* const* h
                        const crfr_resnet_io* io, void* ws, size_t ws_bytes, void* stream);
 size_t crfr_irnet_grad_workspace_bytes(int num_layers, int se, int batch, int size);
 int crfr_irnet_tape(int num_layers, int se, int batch, int size, crfr_tape_entry* entries, int max_entries);
+/* Where crfr_irnet_backward leaves its stored bf16 gradients in the workspace (a dry run of that call), in backward order.
+ * seed_mask: the upstream gradients given (1 = d_emb, 2 / 4 / 8 / 16 = d_feat[0..3], at least one); the layout depends
+ * on it.  Kinds: 11 the head's input gradient, then per unit with a gradient 12 its summed output gradient g, 13 (SE) dr
+ * at the SE input BN_4(y) with stats_off the fp32 shift [n][c] = dpool / hw, 14 the gradient at res_layer.1's output,
+ * 15 its input gradient; last 16 the stem's gradient at input_layer.0's output.  in_off is the out_off of the
+ * crfr_irnet_tape entry whose tensor the gradient is of (for kind 13: the res_layer.3 output y); w_idx is the unit (-1
+ * for 11 and 16).  A kind-12 entry may share its buffer with the entry that produced it.  -1 on bad arguments. */
+int crfr_irnet_grad_tape(int num_layers, int se, int batch, int size, int seed_mask, crfr_tape_entry* entries,
+                         int max_entries);
 int crfr_irnet_backward(int engine, int num_layers, int se, const float* const* host_params, void* const* host_buffers,
                         const crfr_resnet_io* io, const float* d_emb, const float* const* d_feat, float* dx, void* ws,
                         size_t ws_bytes, void* stream);

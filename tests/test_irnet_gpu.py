@@ -72,7 +72,8 @@ def _native_forced(name, net, x, seeds, cases):
     the workspace, (emb, feats))."""
     from crfr_b200 import _lib as L
     from crfr_b200 import ops
-    num_layers, se = VARIANTS[name]
+    num_layers, se = net._variant
+    assert name not in VARIANTS or VARIANTS[name] == net._variant
     b = x.shape[0]
     xg = x.cuda().contiguous()
     ws = torch.empty(L.lib().crfr_irnet_grad_workspace_bytes(num_layers, se, b, 112), dtype=torch.uint8, device="cuda")

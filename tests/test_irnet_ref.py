@@ -185,6 +185,70 @@ def test_irnet_tape_lists_the_se_units():
                 assert e.stats_off >= 0 and e.has_res == 1 and e.n == 2
 
 
+def _grad_tape(lib, L, num_layers, se, b, mask):
+    n = lib.crfr_irnet_grad_tape(num_layers, se, b, 112, mask, None, 0)
+    assert n > 0, (num_layers, se, b, mask)
+    arr = (L.TapeEntry * n)()
+    assert lib.crfr_irnet_grad_tape(num_layers, se, b, 112, mask, arr, n) == n
+    return list(arr)
+
+
+@pytest.mark.parametrize("name", ["IR_50"] + sorted(VARIANTS))
+def test_irnet_grad_tape_layout(name):
+    """crfr_irnet_grad_tape: one entry per stored gradient of the IR backward, each inside the grad workspace past the
+    forward arena, no two overlapping (except a unit's output gradient that is the very buffer of the gradient flowing
+    into it), each naming the stored forward tensor it differentiates."""
+    import crfr_b200
+    crfr_b200.build()
+    from crfr_b200 import _lib as L
+    lib = L.lib()
+    num_layers, se = (50, 0) if name == "IR_50" else VARIANTS[name][:2]
+    units = {50: (3, 4, 14, 3), 100: (3, 13, 30, 3), 152: (3, 8, 36, 3)}[num_layers]
+    per_unit = 4 if se else 3
+    for b in (2, 5):
+        fwd_end = lib.crfr_irnet_workspace_bytes(num_layers, se, b, 112) - 65536   # the forward arena's end
+        grad_bytes = lib.crfr_irnet_grad_workspace_bytes(num_layers, se, b, 112)
+        nf = lib.crfr_irnet_tape(num_layers, se, b, 112, None, 0)
+        ftape = (L.TapeEntry * nf)()
+        lib.crfr_irnet_tape(num_layers, se, b, 112, ftape, nf)
+        fwd = {e.out_off: e for e in ftape}
+        for mask in (1, 2, 4, 8, 16, 17, 30, 31):
+            tape = _grad_tape(lib, L, num_layers, se, b, mask)
+            # the units up to the deepest seeded output have a gradient
+            last_stage = 3 if mask & 1 else max(l for l in range(4) if mask >> (l + 1) & 1)
+            n_units = sum(units[:last_stage + 1])
+            assert len(tape) == (mask & 1) + n_units * per_unit + 1, (name, mask)
+            kinds = [e.kind for e in tape]
+            assert kinds[-1] == 16 and (kinds[0] == 11) == bool(mask & 1)
+            body = kinds[(mask & 1):-1]
+            assert body == ([12, 13, 14, 15] if se else [12, 14, 15]) * n_units, (name, mask)
+            assert [e.w_idx for e in tape[(mask & 1):-1]] == [u for u in reversed(range(n_units)) for _ in range(per_unit)]
+            spans = []
+            for i, e in enumerate(tape):
+                f = fwd.get(e.in_off)
+                assert f is not None, (name, mask, i, e.kind)   # every gradient is of a stored forward tensor
+                assert (e.n, e.h, e.w, e.c) == (f.n, f.h, f.w, f.c) and e.ld >= e.c, (name, mask, i)
+                if e.kind == 13:
+                    assert f.kind == 0                               # dr is paired with y, res_layer.3's output
+                    spans.append((e.stats_off, e.stats_off + 4 * e.n * e.c, i))
+                else:
+                    assert e.stats_off == -1
+                if e.kind == 14:
+                    assert f.kind == 0                               # res_layer.1's output
+                spans.append((e.out_off, e.out_off + 2 * e.n * e.h * e.w * e.ld, i))
+            for lo, hi, i in spans:
+                assert fwd_end <= lo < hi <= grad_bytes, (name, mask, i, lo, hi, fwd_end, grad_bytes)
+            spans.sort()
+            for (lo0, hi0, i0), (lo1, hi1, i1) in zip(spans, spans[1:]):
+                if lo1 < hi0:   # only a unit's summed output gradient may alias, and only the buffer that produced it
+                    a, c = sorted((i0, i1))
+                    assert (lo0, hi0) == (lo1, hi1) and tape[c].kind == 12, (name, mask, i0, i1)
+                    assert tape[a].kind in (11, 15) and tape[a].in_off == tape[c].in_off, (name, mask, i0, i1)
+    for args in ((num_layers, se, 0, 112, 1), (num_layers, se, 4, 96, 1), (num_layers, se, 4, 112, 0),
+                 (num_layers, se, 4, 112, 32), (num_layers, se, 4, 112, -1), (34, 0, 4, 112, 1), (50, 2, 4, 112, 1)):
+        assert lib.crfr_irnet_grad_tape(*args, None, 0) == -1, args
+
+
 def test_irnet_grad_reference_forward_is_the_oracle():
     """The bf16 gradient reference of tests/test_irnet_gpu.py adds gradient roundings to irnet_forward; its forward must
     stay irnet_forward's, for an SE and a plain variant."""
