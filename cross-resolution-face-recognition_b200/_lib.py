@@ -24,6 +24,11 @@ class FsrnetIO(C.Structure):
                 ("hr", vp), ("heatmap", vp), ("labels", vp), ("loss_div", cf), ("w_pix", cf), ("bucket_events", vp * 3)]
 
 
+class FsrnetIdIO(C.Structure):
+    _fields_ = [("teacher_layers", ci), ("teacher_se", ci), ("teacher_params", vp), ("teacher_buffers", vp), ("w_id", cf),
+                ("terms", ci), ("id_scale", cf)]
+
+
 class TapeEntry(C.Structure):
     _fields_ = [("kind", ci), ("n", ci), ("h", ci), ("w", ci), ("c", ci), ("ld", ci), ("out_off", cll),
                 ("in_off", cll), ("stats_off", cll), ("w_idx", ci), ("has_res", ci)]
@@ -111,6 +116,8 @@ SIGNATURES = {
     "crfr_fsrnet_section_forward": (ci, [ci, vp, C.POINTER(FsrnetSectionIO), ci, vp, csz, vp]),
     "crfr_fsrnet_section_backward": (ci, [ci, vp, vp, C.POINTER(FsrnetSectionIO), vp, vp, vp, csz, vp]),
     "crfr_fsrnet_train_step": (ci, [ci, vp, vp, C.POINTER(FsrnetIO), vp, vp, csz, vp]),
+    "crfr_fsrnet_id_workspace_bytes": (csz, [ci, ci, ci, ci]),
+    "crfr_fsrnet_id_train_step": (ci, [ci, vp, vp, C.POINTER(FsrnetIO), C.POINTER(FsrnetIdIO), vp, vp, csz, vp]),
     "crfr_bn_update_running": (ci, [vp, vp, vp, vp, ci, cll, cf, cf, vp]),
     "crfr_bn_running_to_stats": (ci, [vp, vp, ci, cf, vp, vp]),
     "crfr_resnet34_workspace_bytes": (csz, [ci, ci, ci]),

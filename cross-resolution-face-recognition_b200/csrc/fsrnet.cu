@@ -791,9 +791,9 @@ void alloc_out_grads(Net& net, bool coarse, bool out, bool heads) {
 // Dry run of the program over the real arena: collects the weight-pack jobs of the forward (and backward) pass and
 // issues them as one batch.  The arena is a deterministic bump allocator, so the real run finds every packed weight at
 // the offset the dry run gave it.
-int pack_all(int engine, const float* const* params, const crfr_fsrnet_io* io, void* ws, size_t ws_bytes, cudaStream_t st,
-             bool training, bool backward, bool og_coarse, bool og_out, bool og_heads) {
-  std::vector<crfr_pack_job> jobs;
+int collect_packs(std::vector<crfr_pack_job>& jobs, int engine, const float* const* params, const crfr_fsrnet_io* io,
+                  void* ws, size_t ws_bytes, cudaStream_t st, bool training, bool backward, bool og_coarse, bool og_out,
+                  bool og_heads) {
   Net dry;
   init_net(dry, engine, params, nullptr, io, ws, ws_bytes, st, false, training);
   dry.collect = &jobs;
@@ -802,7 +802,12 @@ int pack_all(int engine, const float* const* params, const crfr_fsrnet_io* io, v
     alloc_out_grads(dry, og_coarse, og_out, og_heads);
     dry.backward();
   }
-  if (!dry.ok()) return dry.err;
+  return dry.err;
+}
+int pack_all(int engine, const float* const* params, const crfr_fsrnet_io* io, void* ws, size_t ws_bytes, cudaStream_t st,
+             bool training, bool backward, bool og_coarse, bool og_out, bool og_heads) {
+  std::vector<crfr_pack_job> jobs;
+  CRFR_TRY(collect_packs(jobs, engine, params, io, ws, ws_bytes, st, training, backward, og_coarse, og_out, og_heads));
   return crfr_pack_weight_batch(jobs.data(), (int)jobs.size(), st);
 }
 
@@ -1031,16 +1036,44 @@ extern "C" int crfr_fsrnet_section_backward(int engine, const float* const* host
   return net.err;
 }
 
-extern "C" int crfr_fsrnet_train_step(int engine, const float* const* host_params, float* const* host_grads,
-                                      const crfr_fsrnet_io* io, float* losses, void* ws, size_t ws_bytes,
-                                      void* stream) {
-  CRFR_TRY(check_io(io, "fsrnet_train_step"));
-  CRFR_CHECK_ARG(host_params && host_grads && ws && losses, "fsrnet_train_step: null pointer");
-  CRFR_CHECK_ARG(io->hr && io->heatmap && io->labels && io->loss_div > 0.f, "fsrnet_train_step: missing targets");
-  cudaStream_t st = (cudaStream_t)stream;
-  CRFR_TRY(pack_all(engine, host_params, io, ws, ws_bytes, st, true, true, true, true, true));
+namespace {
+
+constexpr int kIdCrop = 8;   // crop(t) = t[:, :, 8:120, 8:120] of the 128 x 128 output
+
+size_t fsr_arena_bytes(int batch, int size) {
+  return (crfr_fsrnet_workspace_bytes(batch, size, 1) + 4095) & ~(size_t)4095;
+}
+
+crfr_ir_identity_args id_args(int engine, const crfr_fsrnet_io* io, const crfr_fsrnet_id_io* id, float* losses,
+                              void* ws, size_t ws_bytes, cudaStream_t st) {
+  crfr_ir_identity_args a;
+  a.engine = engine; a.layers = id->teacher_layers; a.se = id->teacher_se; a.batch = io->batch;
+  a.params = id->teacher_params; a.buffers = id->teacher_buffers;
+  a.hr = io->hr; a.sr = io->out; a.src_size = io->size; a.crop = kIdCrop; a.terms = id->terms;
+  a.gscale = id->w_id * id->id_scale; a.w_id = id->w_id; a.id_scale = id->id_scale;
+  a.losses = losses; a.ws = ws; a.ws_bytes = ws_bytes; a.st = st;
+  return a;
+}
+
+// forward + losses + backward of crfr_fsrnet_train_step; id != NULL adds the identity term of crfr_fsrnet_id_train_step,
+// whose teacher programs use the workspace after the FSRNet arena
+int train_step(int engine, const float* const* host_params, float* const* host_grads, const crfr_fsrnet_io* io,
+               const crfr_fsrnet_id_io* id, float* losses, void* ws, size_t ws_bytes, cudaStream_t st) {
+  const size_t fsr_bytes = id ? fsr_arena_bytes(io->batch, io->size) : ws_bytes;
+  if (fsr_bytes > ws_bytes) {
+    crfr_set_error("fsrnet_id_train_step: workspace too small (%zu given, crfr_fsrnet_id_workspace_bytes)", ws_bytes);
+    return CRFR_EWORKSPACE;
+  }
+  crfr_ir_identity_args ia{};
+  if (id) ia = id_args(engine, io, id, losses, (uint8_t*)ws + fsr_bytes, ws_bytes - fsr_bytes, st);
+  {   // every weight pack of the step - FSRNet both directions, the teacher's two forwards - in one batched launch
+    std::vector<crfr_pack_job> jobs;
+    CRFR_TRY(collect_packs(jobs, engine, host_params, io, ws, fsr_bytes, st, true, true, true, true, true));
+    if (id) CRFR_TRY(crfr_ir_identity(ia, false, &jobs, nullptr, nullptr));
+    CRFR_TRY(crfr_pack_weight_batch(jobs.data(), (int)jobs.size(), st));
+  }
   Net net;
-  init_net(net, engine, host_params, host_grads, io, ws, ws_bytes, st, true, true);
+  init_net(net, engine, host_params, host_grads, io, ws, fsr_bytes, st, true, true);
   net.packs_done = true;
   net.forward();
   if (!net.ok()) return net.err;
@@ -1055,12 +1088,67 @@ extern "C" int crfr_fsrnet_train_step(int engine, const float* const* host_param
                                 host_grads[C_CONV_MID_B], net.scratch, net.scratch_bytes, st));
   CRFR_CUDA(cudaMemsetAsync(net.d_heads, 0, (size_t)B * Q * Q * kHeadsPad * sizeof(bf16), st));
   CRFR_TRY(crfr_loss_landmark(io->landmark, io->heatmap, B, 97, Q * Q, inv, losses + 3, net.d_heads, kHeadsPad, 11,
-                              net.scratch, net.scratch_bytes, stream));
+                              net.scratch, net.scratch_bytes, st));
   CRFR_TRY(crfr_loss_ce2d(io->parsing, io->labels, B, 11, Q * Q, inv, losses + 4, net.d_heads, kHeadsPad, 0, net.scratch,
-                          net.scratch_bytes, stream));
+                          net.scratch_bytes, st));
   total_loss_kernel<<<1, 1, 0, st>>>(losses, io->w_pix, inv);
   CRFR_COUNT_LAUNCH();
   CRFR_LAUNCH_CHECK();
+  if (id) {
+    // the teacher's forwards on crop(hr) and crop(sr), the feature terms and its input gradient, which joins the pixel
+    // loss's gradient at the output image (and the output convolution's bias gradient) before the FSRNet backward
+    const void* dx4 = nullptr;
+    CRFR_TRY(crfr_ir_identity(ia, true, nullptr, nullptr, &dx4));
+    CRFR_TRY(crfr_mse97_add_window_grad(io->out, io->hr, B, 3, S, S, io->w_pix * inv, dx4, kIdSize, kIdSize, 4, kIdCrop,
+                                        kIdCrop, net.d_out4, 4, host_grads[D_CONV_OUT_B], net.scratch, net.scratch_bytes,
+                                        st));
+  }
   net.backward();
   return net.err;
+}
+
+}  // namespace
+
+extern "C" int crfr_fsrnet_train_step(int engine, const float* const* host_params, float* const* host_grads,
+                                      const crfr_fsrnet_io* io, float* losses, void* ws, size_t ws_bytes,
+                                      void* stream) {
+  CRFR_TRY(check_io(io, "fsrnet_train_step"));
+  CRFR_CHECK_ARG(host_params && host_grads && ws && losses, "fsrnet_train_step: null pointer");
+  CRFR_CHECK_ARG(io->hr && io->heatmap && io->labels && io->loss_div > 0.f, "fsrnet_train_step: missing targets");
+  return train_step(engine, host_params, host_grads, io, nullptr, losses, ws, ws_bytes, (cudaStream_t)stream);
+}
+
+extern "C" size_t crfr_fsrnet_id_workspace_bytes(int teacher_layers, int teacher_se, int batch, int size) {
+  if (batch <= 0 || size != kIdSize + 2 * kIdCrop) return 0;
+  crfr_fsrnet_io io = {};
+  io.batch = batch; io.size = size;
+  crfr_fsrnet_id_io id = {};
+  id.teacher_layers = teacher_layers; id.teacher_se = teacher_se; id.terms = 31;
+  crfr_ir_identity_args a = id_args(CRFR_ENGINE_AUTO, &io, &id, nullptr, nullptr, ~(size_t)0 >> 2, nullptr);
+  size_t ir_bytes = 0;
+  if (crfr_ir_identity(a, false, nullptr, &ir_bytes, nullptr) != CRFR_OK) return 0;
+  return fsr_arena_bytes(batch, size) + ir_bytes;
+}
+
+extern "C" int crfr_fsrnet_id_train_step(int engine, const float* const* host_params, float* const* host_grads,
+                                         const crfr_fsrnet_io* io, const crfr_fsrnet_id_io* id, float* losses, void* ws,
+                                         size_t ws_bytes, void* stream) {
+  CRFR_TRY(check_io(io, "fsrnet_id_train_step"));
+  CRFR_CHECK_ARG(io->size == kIdSize + 2 * kIdCrop,
+                 "fsrnet_id_train_step: size %d unsupported (the identity term takes the 112 x 112 centre of a 128 x 128 "
+                 "output)", io->size);
+  CRFR_CHECK_ARG(host_params && host_grads && ws && losses && id && id->teacher_params && id->teacher_buffers,
+                 "fsrnet_id_train_step: null pointer");
+  CRFR_CHECK_ARG(io->hr && io->heatmap && io->labels && io->loss_div > 0.f, "fsrnet_id_train_step: missing targets");
+  CRFR_CHECK_ARG(id->terms > 0 && id->terms < 32, "fsrnet_id_train_step: terms 0x%x must select 1 to 5 of the outputs "
+                 "(embedding, x1, x2, x3, x4)", id->terms);
+  CRFR_CHECK_ARG(id->id_scale > 0.f && id->id_scale <= 1.f, "fsrnet_id_train_step: id_scale %g not in (0, 1]",
+                 (double)id->id_scale);
+  CRFR_TRY(crfr_irnet_sizes(id->teacher_layers, id->teacher_se, nullptr, nullptr));   // the variant is supported
+  const size_t need = crfr_fsrnet_id_workspace_bytes(id->teacher_layers, id->teacher_se, io->batch, io->size);
+  if (ws_bytes < need) {
+    crfr_set_error("fsrnet_id_train_step: workspace %zu < %zu (crfr_fsrnet_id_workspace_bytes)", ws_bytes, need);
+    return CRFR_EWORKSPACE;
+  }
+  return train_step(engine, host_params, host_grads, io, id, losses, ws, ws_bytes, (cudaStream_t)stream);
 }

@@ -97,6 +97,41 @@ int crfr_norm_fwd_stream(const void* y, int y_ld, const float* stats, const floa
 int crfr_loss_mse97_chan(const float* x, const float* t, int n, int c, int hw, float gscale, float* loss, void* dx,
                          int dx_ld, float* dchan, void* ws, size_t ws_bytes, cudaStream_t st);
 int crfr_nchw_chansum(const float* g, int n, int c, int hw, float* out, void* ws, size_t ws_bytes, cudaStream_t st);
+// The identity gradient of crfr_fsrnet_id_train_step at the output image: dx (bf16 NHWC [n][h][w][dx_ld], written by
+// crfr_loss_mse97_chan(x, t, n, c, h * w, gscale, ...)) gets, on the gh x gw window at (oy, ox), the pixel-loss gradient
+// recomputed in fp32 from x and t plus g (bf16 NHWC [n][gh][gw][g_ld]), rounded once; dchan[ch] += the sum of g over the
+// window (a fixed-order reduction: per-block partials in ws, then one block per channel).
+int crfr_mse97_add_window_grad(const float* x, const float* t, int n, int c, int h, int w, float gscale, const void* g,
+                               int gh, int gw, int g_ld, int oy, int ox, void* dx, int dx_ld, float* dchan, void* ws,
+                               size_t ws_bytes, cudaStream_t st);
+
+// resnet.cu: the IR teacher half of crfr_fsrnet_id_train_step.  Two eval-mode IR forwards on the kIdSize window at
+// (crop, crop) of the fp32 NCHW images hr and sr [batch][3][src_size][src_size], read in place: the first over the arena of
+// crfr_irnet_workspace_bytes at the start of ws, the second after it.  Then the MSE terms selected by terms (bit k: output
+// k of (embedding, x1, x2, x3, x4)), each with gradient scale gscale, on the stored bf16 features; losses[5] = w_id * their
+// sum and losses[0] += id_scale * losses[5]; then the input gradient of the second forward.
+// exec false: a dry run that appends the forward weight packs of both programs to jobs; with ws NULL and ws_bytes huge, a
+// sizing run.  *bytes (optional): the arena used; *dx4 (optional): where the bf16 NHWC [batch][112][112][4] input gradient
+// is left.
+constexpr int kIdSize = 112;
+struct crfr_ir_identity_args {
+  int engine, layers, se, batch;
+  const float* const* params;
+  void* const* buffers;
+  const float* hr;
+  const float* sr;
+  int src_size, crop, terms;
+  float gscale, w_id, id_scale;
+  float* losses;
+  void* ws;
+  size_t ws_bytes;
+  cudaStream_t st;
+};
+#ifdef __cplusplus
+#include <vector>
+int crfr_ir_identity(const crfr_ir_identity_args& a, bool exec, std::vector<crfr_pack_job>* jobs, size_t* bytes,
+                     const void** dx4);
+#endif
 
 // direct_conv.cu
 int crfr_direct_gather(int down, int n, int bh, int bw, int sh, int sw, int k, int stride, int pad, const void* src,

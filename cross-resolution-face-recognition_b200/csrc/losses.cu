@@ -80,6 +80,34 @@ __global__ void chan_finalize_kernel(const float* __restrict__ partial, int nblo
   if (threadIdx.x == 0) dchan[blockIdx.x] += (float)(sm[0] * scale);
 }
 
+// One thread per window pixel: dx at the pixel = bf16(gcoef * (x - t) + g), the first term computed exactly as
+// mse97_kernel does (so that g = 0 reproduces its bits); partial[ch][block] = the block's sum of g (c <= 4)
+__global__ void __launch_bounds__(kT)
+mse97_window_kernel(const float* __restrict__ x, const float* __restrict__ t, int c, int h, int w, float gcoef,
+                    const bf16* __restrict__ g, int gh, int gw, int g_ld, int oy, int ox, bf16* __restrict__ dx, int dx_ld,
+                    long long npix, float* __restrict__ partial) {
+  const long long i = (long long)blockIdx.x * kT + threadIdx.x;
+  float gsum[4] = {0.f, 0.f, 0.f, 0.f};
+  if (i < npix) {
+    const long long n = i / ((long long)gh * gw);
+    const int p = (int)(i - n * gh * gw), y = p / gw, xx = p - (p / gw) * gw;
+    const long long q = (n * h + oy + y) * w + ox + xx;     // pixel of the full image
+    const long long hw = (long long)h * w;
+    for (int ch = 0; ch < c; ++ch) {
+      const long long e = (n * c + ch) * hw + (q - n * hw);
+      const float d = x[e] - t[e];
+      const float gi = __bfloat162float(g[i * g_ld + ch]);
+      gsum[ch] = gi;
+      dx[q * dx_ld + ch] = __float2bfloat16_rn(__fmaf_rn(gcoef, d, gi));
+    }
+  }
+  if (partial)
+    for (int ch = 0; ch < c; ++ch) {
+      if (ch) __syncthreads();
+      block_partial(gsum[ch], partial + (size_t)ch * gridDim.x);
+    }
+}
+
 // per-(block, channel) partial sums of an fp32 NCHW tensor: grid (chunks, c), partial[c][chunks]
 __global__ void __launch_bounds__(kT)
 nchw_chansum_kernel(const float* __restrict__ g, int n, int c, int hw, float* __restrict__ partial) {
@@ -219,6 +247,27 @@ int crfr_loss_mse97_chan(const float* x, const float* t, int n, int c, int hw, f
 extern "C" int crfr_loss_mse97(const float* x, const float* t, int n, int c, int hw, float gscale, float* loss,
                                void* dx, int dx_ld, void* ws, size_t ws_bytes, void* stream) {
   return crfr_loss_mse97_chan(x, t, n, c, hw, gscale, loss, dx, dx_ld, nullptr, ws, ws_bytes, (cudaStream_t)stream);
+}
+
+int crfr_mse97_add_window_grad(const float* x, const float* t, int n, int c, int h, int w, float gscale, const void* g,
+                               int gh, int gw, int g_ld, int oy, int ox, void* dx, int dx_ld, float* dchan, void* ws,
+                               size_t ws_bytes, cudaStream_t st) {
+  CRFR_CHECK_ARG(x && t && g && dx && n > 0 && c > 0 && c <= 4 && g_ld >= c && dx_ld >= c && oy >= 0 && ox >= 0 &&
+                     oy + gh <= h && ox + gw <= w && gh > 0 && gw > 0,
+                 "mse97_add_window_grad: bad argument");
+  const long long npix = (long long)n * gh * gw;
+  const int blocks = crfr_cdiv(npix, kT);
+  if (dchan) CRFR_TRY(check_ws("mse97_add_window_grad", ws, ws_bytes, blocks * c));
+  const double gcoef = gscale * 2.0 * 97.0 / ((double)n * h * w * c);   // as crfr_loss_mse97_chan
+  mse97_window_kernel<<<blocks, kT, 0, st>>>(x, t, c, h, w, (float)gcoef, (const bf16*)g, gh, gw, g_ld, oy, ox, (bf16*)dx,
+                                             dx_ld, npix, dchan ? (float*)ws : nullptr);
+  CRFR_COUNT_LAUNCH();
+  if (dchan) {
+    chan_finalize_kernel<<<c, kT, 0, st>>>((const float*)ws, blocks, 1.0, dchan);
+    CRFR_COUNT_LAUNCH();
+  }
+  CRFR_LAUNCH_CHECK();
+  return CRFR_OK;
 }
 
 // out[ch] += sum over (n, h, w) of g[n][ch][h][w]  (fp32 NCHW), deterministic two-stage reduction

@@ -113,6 +113,28 @@ __global__ void identity_stats_kernel(float* __restrict__ stats, int c) {
   }
 }
 
+// The s x s window at (off, off) of an fp32 NCHW image batch src [n][3][pitch][pitch] -> bf16 NHWC [n][s][s][4] (channel 3
+// zero): the same values as crfr_nchw_f32_to_nhwc_bf16 of a copy of the window, read in place
+__global__ void crop_to_nhwc4_kernel(const float* __restrict__ src, int pitch, int off, bf16* __restrict__ dst, int s,
+                                     long long npix) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= npix) return;
+  const long long n = i / ((long long)s * s);
+  const int p = (int)(i - n * s * s), y = p / s, x = p - (p / s) * s;
+  const float* sp = src + n * 3 * pitch * pitch + (long long)(off + y) * pitch + off + x;
+  const long long plane = (long long)pitch * pitch;
+  bf16* d = dst + i * 4;
+  d[0] = __float2bfloat16_rn(sp[0]);
+  d[1] = __float2bfloat16_rn(sp[plane]);
+  d[2] = __float2bfloat16_rn(sp[2 * plane]);
+  d[3] = __float2bfloat16_rn(0.f);
+}
+
+__global__ void id_loss_kernel(const float* __restrict__ parts, float w_id, float id_scale, float* __restrict__ losses) {
+  losses[5] = w_id * (((parts[0] + parts[1]) + (parts[2] + parts[3])) + parts[4]);
+  losses[0] += id_scale * losses[5];
+}
+
 // s[c] = gamma[c] * rstd[c]: the scale of an eval-mode BatchNorm (stats [c][2] = (mean, rstd))
 __global__ void bn_scale_kernel(const float* __restrict__ stats, const float* __restrict__ gamma, int c,
                                 float* __restrict__ s) {
@@ -374,6 +396,11 @@ struct Net {
   int ir_stem_conv = -1, ir_stem_bn = -1, ir_head_bn0 = -1, ir_head_lin = -1, ir_head_bn1 = -1;
   int ir_layers = 50, ir_se = 0;              // IR program variant: 50 / 100 / 152 layers, bottleneck_IR(_SE)
   std::vector<crfr_tape_entry>* grad_tape = nullptr;   // set: backward_ir lists its stored gradients here (kinds 11-16)
+  // forward_ir input: set, the io->size window at (crop_off, crop_off) of the fp32 NCHW [B,3,crop_pitch,crop_pitch] images
+  // crop_src instead of io->x
+  const float* crop_src = nullptr;
+  int crop_pitch = 0, crop_off = 0;
+  bf16* dx4 = nullptr;   // backward_ir: the bf16 NHWC [B,S,S,4] input gradient it leaves in the arena
 
   void* alloc(size_t bytes) {
     size_t a = (off + 1023) & ~(size_t)1023;
@@ -651,7 +678,14 @@ struct Net {
       CRFR_COUNT_LAUNCH();
     }
     Tensor x4 = new_tensor(B, S, S, 3);
-    if (run()) check(crfr_nchw_f32_to_nhwc_bf16(io->x, x4.p, B, 3, S, S, 4, 4, st));
+    if (run() && crop_src) {
+      const long long npix = (long long)B * S * S;
+      crop_to_nhwc4_kernel<<<crfr_cdiv(npix, 256), 256, 0, st>>>(crop_src, crop_pitch, crop_off, x4.p, S, npix);
+      CRFR_COUNT_LAUNCH();
+      check_cuda(cudaGetLastError());
+    } else if (run()) {
+      check(crfr_nchw_f32_to_nhwc_bf16(io->x, x4.p, B, 3, S, S, 4, 4, st));
+    }
     Tensor a = bn(conv(x4, 0, 64, 3, 1, 1, false), 1, 0, nullptr, 3, 0);     // input_layer: conv, BN, PReLU
     ir_stem_conv = last() - 1; ir_stem_bn = last();
     ir_units.clear();
@@ -811,8 +845,11 @@ struct Net {
   // BatchNorm1d's into the transposed linear weights; what remains element-wise (PReLU masks, the stem's BatchNorm +
   // PReLU, the gradient sum at each unit's input) is ir50_bwd_ew_kernel.  In an SE unit the per-(image, channel)
   // excitation cannot be folded: se_grad turns g into the residual branch's gradient first.
+  // Upstream gradients are the fp32 d_emb / d_feat, or bf16 slots the caller already added to emb / feat[k].  dx (may be
+  // NULL) receives the input gradient in fp32 NCHW; its bf16 NHWC form stays in the arena at dx4.
   void backward_ir(const float* d_emb, const float* const* d_feat, float* dx) {
     const int B = io->batch;
+    const bool head = d_emb || has_grad(emb);
     size_t need = crfr_lowered_dgrad_cin3_ws_bytes(&tape[ir_stem_conv].cd);
     for (const Op& op : tape)
       if (op.kind == OP_CONV) {
@@ -837,7 +874,7 @@ struct Net {
     const Tensor& a4 = tape[ir_head_bn0].a;
     const int K = a4.h * a4.w * a4.c;
     bf16* wlt = nullptr;
-    if (d_emb) {
+    if (head) {
       const float* s_o0 = bn_scale(tape[ir_head_bn0]);
       const float* s_emb = bn_scale(tape[ir_head_bn1]);
       wlt = (bf16*)alloc((size_t)kEmb * K * sizeof(bf16));
@@ -852,7 +889,7 @@ struct Net {
     if (run()) check(crfr_pack_weight_batch(jobs.data(), (int)jobs.size(), st));
 
     // head: d a4 = s_o0 * W^T (s_emb * d_emb)
-    if (d_emb) {
+    if (head) {
       seed_grad(emb, d_emb);
       const Slot de = slots[emb.id][0];
       Tensor da = map_like(a4);
@@ -903,7 +940,7 @@ struct Net {
     const Op& sb = tape[ir_stem_bn];
     const Op& s0 = tape[ir_stem_conv];
     if (!has_grad(sb.out)) {
-      if (run()) check_cuda(cudaMemsetAsync(dx, 0, sizeof(float) * (size_t)B * 3 * io->size * io->size, st));
+      if (run() && dx) check_cuda(cudaMemsetAsync(dx, 0, sizeof(float) * (size_t)B * 3 * io->size * io->size, st));
       return;
     }
     squash(sb.out, 1);
@@ -912,7 +949,8 @@ struct Net {
     record_grad(16, -1, sb.a, dy0.p, dy0.ld);
     Tensor dx4 = map_like(s0.a);
     dgrad(s0, Slot{dy0.p, dy0.ld}, w0, dx4, true);
-    if (run()) check(crfr_nhwc_bf16_to_nchw_f32(dx4.p, dx, B, 3, dx4.h, dx4.w, dx4.ld, st));
+    this->dx4 = dx4.p;
+    if (run() && dx) check(crfr_nhwc_bf16_to_nchw_f32(dx4.p, dx, B, 3, dx4.h, dx4.w, dx4.ld, st));
   }
 
   // ---- backward ----
@@ -1369,6 +1407,58 @@ extern "C" int crfr_ir50_backward(int engine, const float* const* host_params, v
                                   const crfr_resnet_io* io, const float* d_emb, const float* const* d_feat, float* dx,
                                   void* ws, size_t ws_bytes, void* stream) {
   return crfr_irnet_backward(engine, 50, 0, host_params, host_buffers, io, d_emb, d_feat, dx, ws, ws_bytes, stream);
+}
+
+// The identity term of crfr_fsrnet_id_train_step (fsrnet.cu), see internal.h.  The feature gradients are seeded as bf16
+// slots of the stored features, as crfr_kd_train_step does: no fp32 NCHW round trip.
+int crfr_ir_identity(const crfr_ir_identity_args& a, bool exec, std::vector<crfr_pack_job>* jobs, size_t* bytes,
+                     const void** dx4) {
+  CRFR_TRY(check_ir_variant(a.layers, a.se, "fsrnet_id_train_step"));
+  const size_t hr_bytes = (crfr_irnet_workspace_bytes(a.layers, a.se, a.batch, kIdSize) + 4095) & ~(size_t)4095;
+  if (a.ws_bytes < hr_bytes) {
+    crfr_set_error("fsrnet_id_train_step: workspace too small for the teacher (%zu given)", a.ws_bytes);
+    return CRFR_EWORKSPACE;
+  }
+  crfr_resnet_io io = {};
+  io.batch = a.batch; io.size = kIdSize; io.training = 0; io.momentum = 0.1f; io.eps = 1e-5f;
+  uint8_t* base = (uint8_t*)a.ws;
+  Net H, S;
+  init_net(H, a.engine, a.params, nullptr, a.buffers, &io, base, hr_bytes, a.st, exec);
+  init_net(S, a.engine, a.params, nullptr, a.buffers, &io, base + hr_bytes, a.ws_bytes - hr_bytes, a.st, exec);
+  for (Net* n : {&H, &S}) {
+    n->ir_layers = a.layers; n->ir_se = a.se;
+    n->crop_pitch = a.src_size; n->crop_off = a.crop;
+    n->collect = jobs;
+    n->packs_done = exec;
+  }
+  H.crop_src = a.hr;
+  S.crop_src = a.sr;
+  H.forward_ir();
+  if (!H.ok()) return H.err;
+  S.forward_ir();
+  float* parts = (float*)S.alloc(8 * sizeof(float));
+  if (S.run()) S.check_cuda(cudaMemsetAsync(parts, 0, 8 * sizeof(float), a.st));
+  for (int k = 0; k < 5 && S.ok(); ++k) {
+    if (!((a.terms >> k) & 1)) continue;
+    const Tensor& ts = k == 0 ? S.emb : S.feat[k - 1];
+    const Tensor& th = k == 0 ? H.emb : H.feat[k - 1];
+    const long long numel = (long long)ts.n * ts.h * ts.w * ts.c;   // ld == c: contiguous
+    bf16* d = (bf16*)S.alloc((size_t)numel * sizeof(bf16));
+    S.add_slot(ts, d, ts.ld);
+    if (S.run())
+      S.check(crfr_loss_kd(ts.p, nullptr, th.p, numel, 0, a.gscale, parts + k, d, nullptr, nullptr, S.scratch,
+                           S.scratch_bytes, a.st));
+  }
+  if (S.run()) {
+    id_loss_kernel<<<1, 1, 0, a.st>>>(parts, a.w_id, a.id_scale, a.losses);
+    CRFR_COUNT_LAUNCH();
+    S.check_cuda(cudaGetLastError());
+  }
+  if (!S.ok()) return S.err;
+  S.backward_ir(nullptr, nullptr, nullptr);
+  if (bytes) *bytes = hr_bytes + S.off + 65536;
+  if (dx4) *dx4 = S.dx4;
+  return S.err;
 }
 
 extern "C" int crfr_resnet34_backward(int engine, const float* const* host_params, float* const* host_grads,

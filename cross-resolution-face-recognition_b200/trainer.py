@@ -26,6 +26,12 @@ replayed from static input buffers; only the all-reduce and the optimiser step s
 Loss scaling: FSR_main.py:234 divides by 2*train_batch.  With G = global batch (all ranks) and chunk size c, the
 chunk's share of the batch-mean losses is c/G, so each chunk is run with loss_div = 2*G*G/c and gradients are
 SUM-reduced across ranks: the result equals the single-GPU gradient of the concatenated batch.
+
+Identity term (``identity_net``, a frozen 112 x 112 IR / IR-SE ``Backbone`` in eval mode): every chunk runs
+crfr_fsrnet_id_train_step instead, which adds w_id * sum_k MSE(f(sr)[k], f(hr)[k]) over the selected outputs of
+f = identity_net.forward_features on the 112 x 112 centres (SUPER_RESOLUTION/train_FHN.py:255-265).  Each MSE is a mean
+over the chunk, run with id_scale = c/G, so the summed chunk gradients, SUM-reduced across ranks, are again those of
+the global-batch mean.  The losses then have a sixth entry, the identity term.
 """
 import ctypes as C
 
@@ -89,8 +95,8 @@ class _Lane:
         params = trainer.model.ordered_parameters()
         self.grad_views = [self.flat_g[o:o + p.numel()].view(p.shape) for p, o in zip(params, trainer.offs)]
         self.gtable = M._ParamTable(self.grad_views)
-        self.losses = torch.zeros((5,), dtype=torch.float32, device=dev)
-        self.loss_acc = torch.zeros((5,), dtype=torch.float32, device=dev)
+        self.losses = torch.zeros((trainer.n_losses,), dtype=torch.float32, device=dev)
+        self.loss_acc = torch.zeros((trainer.n_losses,), dtype=torch.float32, device=dev)
         self.events = [torch.cuda.Event() for _ in trainer.buckets]
         for e in self.events:
             e.record()
@@ -99,11 +105,34 @@ class _Lane:
         self.outs = None
 
 
+def _identity_tables(net, terms):
+    """Checks the identity teacher and the selected outputs -> (parameter table, buffer table, terms bit mask)."""
+    from .model import model_irse as IR
+    if not isinstance(net, IR.Backbone):
+        raise TypeError("identity_net must be an IR / IR-SE Backbone (model_irse), got %s" % type(net).__name__)
+    if not net._native:
+        raise NotImplementedError("only the 112 x 112 IR / IR_SE backbones have a native network program")
+    if net.training:
+        raise RuntimeError("identity_net is the frozen teacher: call .eval() first (train-mode Dropout is stochastic and "
+                           "has no parity definition)")
+    terms = tuple(terms)
+    if not terms or any(k not in range(5) for k in terms) or len(set(terms)) != len(terms):
+        raise ValueError("id_terms must be distinct indices into (embedding, x1, x2, x3, x4), got %s" % (terms,))
+    n_params, n_bn = L.irnet_sizes(*net._variant)
+    params = [p.detach() for _, p in net.named_parameters()]
+    buffers = [t for _, t in net.named_buffers()]
+    return IR._Table(params, n_params), IR._Table(buffers, 3 * n_bn), sum(1 << k for k in terms)
+
+
 class FSRNetTrainer:
     def __init__(self, model, lr=1e-3, alpha=0.99, eps=1e-8, weight_decay=1e-5, chunk=16, w_pix=5.0,
-                 engine=L.ENGINE_AUTO, process_group=None, world_size=None, lanes=1, use_graph=False):
+                 engine=L.ENGINE_AUTO, process_group=None, world_size=None, lanes=1, use_graph=False, identity_net=None,
+                 w_id=1.0, id_terms=(0, 1, 2, 3, 4)):
         import torch.distributed as dist
         self.model = model
+        self.identity_net, self.w_id = identity_net, float(w_id)
+        self._id_tabs = None if identity_net is None else _identity_tables(identity_net, id_terms)
+        self.n_losses = 5 if identity_net is None else 6
         self.lr, self.alpha, self.eps, self.wd = lr, alpha, eps, weight_decay
         self.chunk, self.w_pix, self.engine = chunk, w_pix, engine
         self.dist = dist if (dist.is_available() and dist.is_initialized()) else None
@@ -127,8 +156,8 @@ class FSRNetTrainer:
         self.live_ranges = live_ranges(offs, tot, M._DEAD_PARAMS)
         self.ptable = M._ParamTable([p.data for p in params])
         self.gtable = M._ParamTable(self.grad_views)
-        self.losses = torch.zeros((5,), dtype=torch.float32, device=dev)
-        self.loss_acc = torch.zeros((5,), dtype=torch.float32, device=dev)
+        self.losses = torch.zeros((self.n_losses,), dtype=torch.float32, device=dev)
+        self.loss_acc = torch.zeros((self.n_losses,), dtype=torch.float32, device=dev)
         self.ws = None
         self.outs = None
         if dev.type == "cuda":
@@ -160,6 +189,39 @@ class FSRNetTrainer:
         L.call("crfr_fsrnet_train_step", self.engine, self.ptable.arr, self.gtable.arr, C.byref(io),
                self.losses.data_ptr(), self.ws.data_ptr(), self.ws.numel(), ops.stream())
 
+    def _ws_need(self, b, s):
+        if self.identity_net is None:
+            return L.lib().crfr_fsrnet_workspace_bytes(b, s, 1)
+        return L.lib().crfr_fsrnet_id_workspace_bytes(*self.identity_net._variant, b, s)
+
+    def _id_call(self, io, gtable, losses, ws, id_scale):
+        """crfr_fsrnet_id_train_step of one chunk (io: its crfr_fsrnet_io) into gtable / losses over ws."""
+        ptab, btab, mask = self._id_tabs
+        idio = L.FsrnetIdIO()
+        idio.teacher_layers, idio.teacher_se = self.identity_net._variant
+        idio.teacher_params = C.cast(ptab.arr, C.c_void_p)
+        idio.teacher_buffers = C.cast(btab.arr, C.c_void_p)
+        idio.w_id, idio.terms, idio.id_scale = self.w_id, mask, id_scale
+        L.call("crfr_fsrnet_id_train_step", self.engine, self.ptable.arr, gtable.arr, C.byref(io), C.byref(idio),
+               losses.data_ptr(), ws.data_ptr(), ws.numel(), ops.stream())
+
+    # -- one native chunk with the identity term (id_scale = chunk / global batch): overridable like _native_chunk --
+    def _native_id_chunk(self, x, hr, heatmap, labels, outs, loss_div, id_scale, events):
+        b, s = x.shape[0], x.shape[2]
+        need = self._ws_need(b, s)
+        if self.ws is None or self.ws.numel() < need:
+            self.ws = torch.empty(need, dtype=torch.uint8, device=x.device)
+        io = M._io(x, outs, (hr, heatmap, labels), loss_div=loss_div, w_pix=self.w_pix)
+        for i, e in enumerate(events or ()):
+            io.bucket_events[i] = e.cuda_event
+        self._id_call(io, self.gtable, self.losses, self.ws, id_scale)
+
+    def _chunk(self, x, hr, heatmap, labels, outs, c, G, events):
+        if self.identity_net is None:
+            self._native_chunk(x, hr, heatmap, labels, outs, chunk_loss_div(G, c), events)
+        else:
+            self._native_id_chunk(x, hr, heatmap, labels, outs, chunk_loss_div(G, c), c / G, events)
+
     def _allreduce_bucket(self, k):
         lo, hi = self.buckets[k]
         return self.dist.all_reduce(self.flat_g[lo:hi], op=self.dist.ReduceOp.SUM, group=self.pg, async_op=True)
@@ -168,7 +230,7 @@ class FSRNetTrainer:
         """total adds up over chunks; the parts are chunk means -> weight by c/B (cached device constants)."""
         key = (c, B)
         if key not in self._w_cache:
-            self._w_cache[key] = torch.tensor([1.0] + [c / B] * 4, device=self.device)
+            self._w_cache[key] = torch.tensor([1.0] + [c / B] * (self.n_losses - 1), device=self.device)
         return self._w_cache[key]
 
     def _step_lanes(self, x, hr, heatmap, labels, lr, events_for_dp=True, finish=True):
@@ -194,7 +256,7 @@ class FSRNetTrainer:
             with torch.cuda.stream(ln.stream):
                 if ln.outs is None or ln.outs[0].shape[0] != c or ln.outs[0].shape[2] != x.shape[2]:
                     ln.outs = M.alloc_outputs(x[s0:s1])
-                need = L.lib().crfr_fsrnet_workspace_bytes(c, x.shape[2], 1)
+                need = self._ws_need(c, x.shape[2])
                 if ln.ws is None or ln.ws.numel() < need:
                     ln.ws = torch.empty(need, dtype=torch.uint8, device=x.device)
                 io = M._io(x[s0:s1], ln.outs, (hr[s0:s1], heatmap[s0:s1], labels[s0:s1]),
@@ -202,8 +264,11 @@ class FSRNetTrainer:
                 if dp and last_of_lane:
                     for i, e in enumerate(ln.events):
                         io.bucket_events[i] = e.cuda_event
-                L.call("crfr_fsrnet_train_step", self.engine, self.ptable.arr, ln.gtable.arr, C.byref(io),
-                       ln.losses.data_ptr(), ln.ws.data_ptr(), ln.ws.numel(), ops.stream())
+                if self.identity_net is None:
+                    L.call("crfr_fsrnet_train_step", self.engine, self.ptable.arr, ln.gtable.arr, C.byref(io),
+                           ln.losses.data_ptr(), ln.ws.data_ptr(), ln.ws.numel(), ops.stream())
+                else:
+                    self._id_call(io, ln.gtable, ln.losses, ln.ws, c / G)
                 ln.loss_acc.add_(ln.losses * self._loss_weights(c, B))
                 if last_of_lane:
                     ln.done.record(ln.stream)
@@ -246,7 +311,7 @@ class FSRNetTrainer:
             c = s1 - s0
             if self.outs is None or self.outs[0].shape[0] != c or self.outs[0].shape[2] != x.shape[2]:
                 self.outs = M.alloc_outputs(x[s0:s1])
-            self._native_chunk(x[s0:s1], hr[s0:s1], heatmap[s0:s1], labels[s0:s1], self.outs, chunk_loss_div(G, c), None)
+            self._chunk(x[s0:s1], hr[s0:s1], heatmap[s0:s1], labels[s0:s1], self.outs, c, G, None)
             self.loss_acc.add_(self.losses * self._loss_weights(c, B))
 
     def _step_graph(self, x, hr, heatmap, labels, lr):
@@ -278,7 +343,10 @@ class FSRNetTrainer:
     def step(self, x, hr, heatmap, labels, lr=None):
         """x [B,3,S,S] fp32 (already upsampled + normalised), hr [B,3,S,S], heatmap [B,S/4,S/4], labels int64
         [B,1,S/4,S/4]; all on this rank's device.  Returns the device tensor (total, L_sr, L_coarse, L_lm, L_ce) of
-        this rank's share of the global-batch loss (parts are rank-local batch means)."""
+        this rank's share of the global-batch loss (parts are rank-local batch means); with ``identity_net`` a sixth
+        entry, the identity term's rank-local batch mean, whose share is part of the total."""
+        if self.identity_net is not None and self.identity_net.training:
+            raise RuntimeError("identity_net is the frozen teacher: call .eval() first")
         if x.is_cuda:
             M.check_input(x)
             # the native program reads raw pointers: coerce dtype / contiguity here (slices of a bigger batch are fine)
@@ -302,8 +370,8 @@ class FSRNetTrainer:
             outs = self.outs if c == self.outs[0].shape[0] else M.alloc_outputs(x[s0:s1])
             last = ci == len(starts) - 1
             use_events = last and self.dist is not None and self.world > 1 and self.events
-            self._native_chunk(x[s0:s1], hr[s0:s1], heatmap[s0:s1], labels[s0:s1], outs, chunk_loss_div(G, c),
-                               self.events if use_events else None)
+            self._chunk(x[s0:s1], hr[s0:s1], heatmap[s0:s1], labels[s0:s1], outs, c, G,
+                        self.events if use_events else None)
             self.loss_acc.add_(self.losses * self._loss_weights(c, B))
             if use_events:
                 main = torch.cuda.current_stream()

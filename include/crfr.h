@@ -315,6 +315,28 @@ int crfr_fsrnet_section_backward(int engine, const float* const* host_params, fl
 int crfr_fsrnet_train_step(int engine, const float* const* host_params, float* const* host_grads,
                            const crfr_fsrnet_io* io, float* losses, void* ws, size_t ws_bytes, void* stream);
 
+/* ref: the identity / perceptual loss through a frozen face-recognition network, SUPER_RESOLUTION/train_FHN.py:255-265.
+ * crfr_fsrnet_train_step plus an identity term on the 112 x 112 centre of the super-resolved output (size 128 only):
+ *   L = L_FSR + w_id * sum_{k in terms} MSE(f(sr)[k], f(hr)[k]),  f(t) = Backbone.forward_features(t[:, :, 8:120, 8:120])
+ * with f an IR / IR-SE teacher (crfr_irnet_*, eval mode, frozen: no parameter gradient, buffers unchanged).  Each MSE is
+ * the mean over the chunk; id_scale = chunk / global batch makes the summed chunk gradients, SUM-reduced across ranks, the
+ * gradient of the global-batch mean (as loss_div does for L_FSR).  losses: device fp32[6] = (total, L_sr, L_coarse,
+ * L_landmark, L_ce, w_id * sum_k MSE_k), total = the L_FSR share + id_scale * losses[5].  io as for crfr_fsrnet_train_step;
+ * the same three bucket events are recorded.  No host synchronisation or allocation (graph-capturable). */
+typedef struct crfr_fsrnet_id_io {
+  int teacher_layers, teacher_se;       /* the IR variant: 50 / 100 / 152 layers, se 1 = IR-SE */
+  const float* const* teacher_params;   /* device pointers, named_parameters() order (crfr_irnet_sizes) */
+  void* const* teacher_buffers;         /* 3 per BatchNorm, named_buffers() order */
+  float w_id;                           /* weight of the identity term (1.0) */
+  int terms;                            /* bit k selects output k of (embedding, x1, x2, x3, x4); 31 = all five */
+  float id_scale;                       /* this chunk's share of the global batch: chunk / global batch */
+} crfr_fsrnet_id_io;
+/* the FSRNet training arena, the teacher's forward arena for hr and its gradient arena for sr; 0 when unsupported */
+size_t crfr_fsrnet_id_workspace_bytes(int teacher_layers, int teacher_se, int batch, int size);
+int crfr_fsrnet_id_train_step(int engine, const float* const* host_params, float* const* host_grads,
+                              const crfr_fsrnet_io* io, const crfr_fsrnet_id_io* id, float* losses, void* ws,
+                              size_t ws_bytes, void* stream);
+
 /* ---------------------------------------------------------------- ResNet_34 embedding network program ------ */
 #define CRFR_RESNET34_NPARAMS 114 /* named_parameters() order of model/resnet.py:ResNet_34 */
 #define CRFR_RESNET34_NBN 38      /* BatchNorm layers in module order */
