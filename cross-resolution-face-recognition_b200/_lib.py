@@ -110,6 +110,7 @@ SIGNATURES = {
     "crfr_linear_bwd": (ci, [vp, vp, ci, ci, ci, vp, ci, vp, vp, vp, vp, csz, vp]),
     "crfr_fsrnet_workspace_bytes": (csz, [ci, ci, ci]),
     "crfr_fsrnet_tape": (ci, [ci, ci, ci, C.POINTER(TapeEntry), ci]),
+    "crfr_fsrnet_id_tape": (ci, [ci, ci, ci, ci, ci, C.POINTER(TapeEntry), ci]),
     "crfr_fsrnet_forward": (ci, [ci, vp, C.POINTER(FsrnetIO), ci, vp, csz, vp]),
     "crfr_fsrnet_backward": (ci, [ci, vp, vp, C.POINTER(FsrnetIO), vp, vp, vp, vp, vp, csz, vp]),
     "crfr_fsrnet_section_workspace_bytes": (csz, [ci, ci, ci, ci]),

@@ -833,15 +833,9 @@ extern "C" size_t crfr_fsrnet_workspace_bytes(int batch, int size, int training)
   return need + 65536;
 }
 
-// Layout of the saved forward tensors in the workspace (a dry run: nothing is launched).  Parity tests read the stored
-// bf16 activations through this table and replay them into the CPU oracle (teacher-forced forward / backward checks).
-extern "C" int crfr_fsrnet_tape(int batch, int size, int training, crfr_tape_entry* entries, int max_entries) {
-  if (batch <= 0 || size < 32 || size % 16) return -1;
-  crfr_fsrnet_io io = {};
-  io.batch = batch; io.size = size;
-  Net net;
-  init_net(net, CRFR_ENGINE_AUTO, nullptr, nullptr, &io, nullptr, ~(size_t)0 >> 2, nullptr, false, training != 0);
-  net.forward();
+namespace {
+// the stored forward tensors of a program run (dry or not) whose workspace base is the null pointer
+int fill_tape(const Net& net, crfr_tape_entry* entries, int max_entries) {
   const int count = (int)net.tape.size();
   for (int i = 0; i < count && i < max_entries && entries; ++i) {
     const Op& op = net.tape[i];
@@ -856,6 +850,19 @@ extern "C" int crfr_fsrnet_tape(int batch, int size, int training, crfr_tape_ent
     e.has_res = op.has_res ? 1 : 0;
   }
   return count;
+}
+}  // namespace
+
+// Layout of the saved forward tensors in the workspace (a dry run: nothing is launched).  Parity tests read the stored
+// bf16 activations through this table and replay them into the CPU oracle (teacher-forced forward / backward checks).
+extern "C" int crfr_fsrnet_tape(int batch, int size, int training, crfr_tape_entry* entries, int max_entries) {
+  if (batch <= 0 || size < 32 || size % 16) return -1;
+  crfr_fsrnet_io io = {};
+  io.batch = batch; io.size = size;
+  Net net;
+  init_net(net, CRFR_ENGINE_AUTO, nullptr, nullptr, &io, nullptr, ~(size_t)0 >> 2, nullptr, false, training != 0);
+  net.forward();
+  return fill_tape(net, entries, max_entries);
 }
 
 extern "C" int crfr_fsrnet_forward(int engine, const float* const* host_params, const crfr_fsrnet_io* io,
@@ -1128,6 +1135,39 @@ extern "C" size_t crfr_fsrnet_id_workspace_bytes(int teacher_layers, int teacher
   size_t ir_bytes = 0;
   if (crfr_ir_identity(a, false, nullptr, &ir_bytes, nullptr) != CRFR_OK) return 0;
   return fsr_arena_bytes(batch, size) + ir_bytes;
+}
+
+// Where crfr_fsrnet_id_train_step leaves its tensors (include/crfr.h): the dry runs of train_step's two halves over the
+// step's own layout - the FSRNet forward and its output gradients in the arena at 0, then crfr_ir_identity recording from
+// inside, with its arena at fsr_arena_bytes
+extern "C" int crfr_fsrnet_id_tape(int teacher_layers, int teacher_se, int batch, int size, int terms,
+                                   crfr_tape_entry* entries, int max_entries) {
+  if (crfr_fsrnet_id_workspace_bytes(teacher_layers, teacher_se, batch, size) == 0 || terms < 1 || terms > 31) return -1;
+  crfr_fsrnet_io io = {};
+  io.batch = batch; io.size = size;
+  crfr_fsrnet_id_io id = {};
+  id.teacher_layers = teacher_layers; id.teacher_se = teacher_se; id.terms = terms;
+  const size_t fsr_bytes = fsr_arena_bytes(batch, size);
+  Net net;
+  init_net(net, CRFR_ENGINE_AUTO, nullptr, nullptr, &io, nullptr, fsr_bytes, nullptr, false, true);
+  net.forward();
+  alloc_out_grads(net, true, true, true);
+  if (!net.ok()) return -1;
+  std::vector<crfr_tape_entry> tape(net.tape.size());
+  fill_tape(net, tape.data(), (int)tape.size());
+  crfr_tape_entry d{};
+  d.kind = 19;
+  d.n = batch; d.h = size; d.w = size; d.c = 3; d.ld = 4;
+  d.out_off = (long long)((uint8_t*)net.d_out4 - (uint8_t*)nullptr);
+  d.in_off = d.stats_off = -1;
+  d.w_idx = -1;
+  tape.push_back(d);
+  const crfr_ir_identity_args a = id_args(CRFR_ENGINE_AUTO, &io, &id, nullptr, (uint8_t*)nullptr + fsr_bytes,
+                                          ~(size_t)0 >> 2, nullptr);
+  if (crfr_ir_identity(a, false, nullptr, nullptr, nullptr, &tape) != CRFR_OK) return -1;
+  const int count = (int)tape.size();
+  for (int i = 0; i < count && i < max_entries && entries; ++i) entries[i] = tape[i];
+  return count;
 }
 
 extern "C" int crfr_fsrnet_id_train_step(int engine, const float* const* host_params, float* const* host_grads,

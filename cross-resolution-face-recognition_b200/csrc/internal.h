@@ -112,7 +112,8 @@ int crfr_mse97_add_window_grad(const float* x, const float* t, int n, int c, int
 // sum and losses[0] += id_scale * losses[5]; then the input gradient of the second forward.
 // exec false: a dry run that appends the forward weight packs of both programs to jobs; with ws NULL and ws_bytes huge, a
 // sizing run.  *bytes (optional): the arena used; *dx4 (optional): where the bf16 NHWC [batch][112][112][4] input gradient
-// is left.
+// is left; tape (optional, a dry run with ws = the null base + the arena's offset in the step's workspace): appends
+// sections 3-7 of crfr_fsrnet_id_tape.
 constexpr int kIdSize = 112;
 struct crfr_ir_identity_args {
   int engine, layers, se, batch;
@@ -130,7 +131,7 @@ struct crfr_ir_identity_args {
 #ifdef __cplusplus
 #include <vector>
 int crfr_ir_identity(const crfr_ir_identity_args& a, bool exec, std::vector<crfr_pack_job>* jobs, size_t* bytes,
-                     const void** dx4);
+                     const void** dx4, std::vector<crfr_tape_entry>* tape = nullptr);
 #endif
 
 // direct_conv.cu

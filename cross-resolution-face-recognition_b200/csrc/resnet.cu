@@ -1412,7 +1412,7 @@ extern "C" int crfr_ir50_backward(int engine, const float* const* host_params, v
 // The identity term of crfr_fsrnet_id_train_step (fsrnet.cu), see internal.h.  The feature gradients are seeded as bf16
 // slots of the stored features, as crfr_kd_train_step does: no fp32 NCHW round trip.
 int crfr_ir_identity(const crfr_ir_identity_args& a, bool exec, std::vector<crfr_pack_job>* jobs, size_t* bytes,
-                     const void** dx4) {
+                     const void** dx4, std::vector<crfr_tape_entry>* tape) {
   CRFR_TRY(check_ir_variant(a.layers, a.se, "fsrnet_id_train_step"));
   const size_t hr_bytes = (crfr_irnet_workspace_bytes(a.layers, a.se, a.batch, kIdSize) + 4095) & ~(size_t)4095;
   if (a.ws_bytes < hr_bytes) {
@@ -1433,9 +1433,23 @@ int crfr_ir_identity(const crfr_ir_identity_args& a, bool exec, std::vector<crfr
   }
   H.crop_src = a.hr;
   S.crop_src = a.sr;
+  // tape: the forward tapes of both programs (fill_tape: offsets from the null base, i.e. from the step's workspace when
+  // a.ws is the arena's offset in it), then S's gradient tape - the seed slots (kind 17), backward_ir's kinds 11-16 and
+  // dx4 (kind 18) - recorded relative to S's arena and shifted by its offset
+  std::vector<crfr_tape_entry> grads;
+  auto append_tape = [tape](const Net& n) {
+    const size_t at = tape->size();
+    tape->resize(at + n.tape.size());
+    fill_tape(n, tape->data() + at, (int)n.tape.size());
+  };
   H.forward_ir();
   if (!H.ok()) return H.err;
   S.forward_ir();
+  if (tape) {
+    append_tape(H);
+    append_tape(S);
+    S.grad_tape = &grads;
+  }
   float* parts = (float*)S.alloc(8 * sizeof(float));
   if (S.run()) S.check_cuda(cudaMemsetAsync(parts, 0, 8 * sizeof(float), a.st));
   for (int k = 0; k < 5 && S.ok(); ++k) {
@@ -1445,6 +1459,7 @@ int crfr_ir_identity(const crfr_ir_identity_args& a, bool exec, std::vector<crfr
     const long long numel = (long long)ts.n * ts.h * ts.w * ts.c;   // ld == c: contiguous
     bf16* d = (bf16*)S.alloc((size_t)numel * sizeof(bf16));
     S.add_slot(ts, d, ts.ld);
+    S.record_grad(17, k, ts, d, ts.ld);
     if (S.run())
       S.check(crfr_loss_kd(ts.p, nullptr, th.p, numel, 0, a.gscale, parts + k, d, nullptr, nullptr, S.scratch,
                            S.scratch_bytes, a.st));
@@ -1456,6 +1471,17 @@ int crfr_ir_identity(const crfr_ir_identity_args& a, bool exec, std::vector<crfr
   }
   if (!S.ok()) return S.err;
   S.backward_ir(nullptr, nullptr, nullptr);
+  if (tape && S.ok() && S.dx4) {
+    const Op& s0 = S.tape[S.ir_stem_conv];
+    S.record_grad(18, -1, s0.a, S.dx4, s0.a.ld);
+    const long long shift = (long long)(S.ws - (uint8_t*)nullptr);
+    for (crfr_tape_entry e : grads) {
+      e.out_off += shift;
+      e.in_off += shift;
+      if (e.stats_off >= 0) e.stats_off += shift;
+      tape->push_back(e);
+    }
+  }
   if (bytes) *bytes = hr_bytes + S.off + 65536;
   if (dx4) *dx4 = S.dx4;
   return S.err;

@@ -280,6 +280,21 @@ typedef struct crfr_tape_entry {
 } crfr_tape_entry;
 /* fills up to max_entries entries (entries may be NULL) and returns the number of recorded ops, < 0 on bad arguments */
 int crfr_fsrnet_tape(int batch, int size, int training, crfr_tape_entry* entries, int max_entries);
+/* Where crfr_fsrnet_id_train_step leaves its tensors (test aid, from the dry run of the step itself).  Offsets are bytes
+ * from the base of the step's workspace; the entries, in order:
+ *   1. those of crfr_fsrnet_tape(batch, size, 1): the FSRNet arena starts at 0;
+ *   2. kind 19: the output-image gradient d_out4, bf16 NHWC [batch][size][size], c = 3, ld 4;
+ *   3. crfr_irnet_tape of the crop(hr) program, shifted by the base of its arena;
+ *   4. the same for the crop(sr) program;
+ *   5. kind 17, one per selected term k in increasing k: the bf16 seed slot of the feature gradient (w_idx = k, in_off =
+ *      out_off of the crop(sr) tensor it is the gradient of);
+ *   6. the crop(sr) backward's gradient tape (kinds 11-16, as crfr_irnet_grad_tape);
+ *   7. kind 18: dx4, the bf16 NHWC [batch][112][112] (c = 3, ld 4) input gradient the window kernel adds to d_out4.
+ * A kind-12 entry shares its buffer with the kind-15 entry of the next unit, the head's kind 11 or a kind-17 seed when
+ * that is the unit output's only gradient.  Fills up to max_entries entries (entries may be NULL) and returns the count;
+ * -1 where crfr_fsrnet_id_workspace_bytes is 0 or terms is outside 1..31. */
+int crfr_fsrnet_id_tape(int teacher_layers, int teacher_se, int batch, int size, int terms, crfr_tape_entry* entries,
+                        int max_entries);
 
 /* ref: OverallNetwork.forward model/FSRnet.py:497-508 with the runnable wiring of :538-541.
  * params: 202 fp32 device pointers in state_dict order.  engine selects the conv engine for eligible layers. */

@@ -475,12 +475,18 @@ def ce2d(logits, target):
     return F.nll_loss(F.log_softmax(logits, 1), torch.squeeze(target))
 
 
-def fsrnet_loss(outputs, hr, heatmap, labels, train_batch=None, w_pix=5.0, pr=FP32):
+def fsrnet_loss(outputs, hr, heatmap, labels, train_batch=None, w_pix=5.0, pr=FP32, out_grad=None):
+    """``out_grad`` (optional, fp32 like ``out``): a further gradient at the output image, as another loss term adds it
+    (the identity term of crfr_fsrnet_id_train_step): total gains sum(out * out_grad), not counted in ``parts``, and the
+    output's gradient is stored once, with the pixel term's."""
     coarse, out, landmark, parsing = outputs
     b = hr.shape[0] if train_batch is None else train_batch
-    parts = (mse97(pr.qg(out), hr), mse97(pr.qg(coarse), hr), landmark_loss(pr.qg(landmark), heatmap),
+    out = pr.qg(out)
+    parts = (mse97(out, hr), mse97(pr.qg(coarse), hr), landmark_loss(pr.qg(landmark), heatmap),
              ce2d(pr.qg(parsing), labels))
     total = (w_pix * parts[0] + w_pix * parts[1] + parts[2] + parts[3]) / (2.0 * b)
+    if out_grad is not None:
+        total = total + (out * out_grad).sum()
     return total, parts
 
 
@@ -494,13 +500,14 @@ def synthetic_batch(batch, size=128, seed=4321):
     return x, hr, lbl, hm
 
 
-def fsrnet_loss_and_grads(sd, x, hr, hm, lbl, train_batch=None, precision="fp32"):
+def fsrnet_loss_and_grads(sd, x, hr, hm, lbl, train_batch=None, precision="fp32", out_grad=None):
     """One forward+backward; returns (outputs, total, parts, {name: grad}) - used as the parity oracle.
-    ``precision``: "fp32", "bf16" or a ``Precision`` instance (e.g. ``ForcedPrecision``)."""
+    ``precision``: "fp32", "bf16" or a ``Precision`` instance (e.g. ``ForcedPrecision``); ``out_grad``: see
+    ``fsrnet_loss``."""
     pr = precision if isinstance(precision, Precision) else Precision(precision)
     leaves = OrderedDict((k, v.detach().clone().requires_grad_(True)) for k, v in sd.items())
     outs = fsrnet_forward(leaves, x, pr)
-    total, parts = fsrnet_loss(outs, hr, hm, lbl, train_batch, pr=pr)
+    total, parts = fsrnet_loss(outs, hr, hm, lbl, train_batch, pr=pr, out_grad=out_grad)
     names = [k for k in leaves if not fsrnet_dead_param(k)]
     grads = torch.autograd.grad(total, [leaves[k] for k in names], allow_unused=True)
     gd = OrderedDict((k, None) for k in leaves)

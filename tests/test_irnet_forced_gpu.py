@@ -9,7 +9,7 @@ downstream.  Where the native kernel rounds to bf16 the reference rounds at the 
 the order of fp32 sums.  Every bound is also checked to reject a reference with one known error planted (``_Report.mutant``): the SE shift
 left out of dr, the last pixel of each reduction chunk dropped, e in place of e(1 - e), the hidden ReLU mask inverted, the
 PReLU slope of channel c + 1 used for channel c, the odd pixel in the stride-2 gather, res_layer.0's folded scale left
-out."""
+out, the seed of a stage output dropped from or doubled in that unit's output gradient."""
 import pytest
 import torch
 import torch.nn.functional as F
@@ -262,10 +262,18 @@ def _se_shift(P, p, y, g, e, mutate=None):
     return ((u @ w2) * mask) @ w1 / hw
 
 
+def _stage_ends(units):
+    """{index of a stage's last unit: the stage (0..3, the outputs x1..x4)}"""
+    stage = {64: 0, 128: 1, 256: 2, 512: 3}
+    return {i: stage[u["d"]] for i, u in enumerate(units) if i + 1 == len(units) or units[i + 1]["d"] != u["d"]}
+
+
 def _check_backward(run, P, x, seeds, dx, stem, units, head, gtape, mask, rep):
-    """Every stored gradient of the IR backward from the native gradient one step downstream."""
+    """Every stored gradient of the IR backward from the native gradient one step downstream.  seeds: the upstream
+    gradients by output (embedding [B, 512], x1..x4 NCHW) as given, for all images; those not in mask are not read."""
     by = {(e.kind, e.w_idx): e for e in gtape}
     assert len(by) == len(gtape)
+    ends = _stage_ends(units)
     if mask & 1:   # head: da = s_o0 * W^T (s_emb * d_emb), the scales folded into the bf16 pack
         e = by[(11, -1)]
         assert e.in_off == head["bn0"].in_off
@@ -281,6 +289,21 @@ def _check_backward(run, P, x, seeds, dx, stem, units, head, gtape, mask, rep):
         eg, ed2, ein = by[(12, i)], by[(14, i)], by[(15, i)]
         assert eg.in_off == u["bn4"].out_off and ed2.in_off == u["conv1"].out_off and ein.in_off == u["bn0"].in_off
         g = run.t(eg)
+        # g itself: the gradient arriving from downstream (the next unit's d_in, or the head's da), plus at a stage end
+        # the seed of that stage output, summed in fp32 and rounded once (crfr_add_n); a single gradient is used in place
+        nxt = by.get((15, i + 1) if i + 1 < len(units) else (11, -1))
+        if i in ends and mask >> (ends[i] + 1) & 1:
+            seed = q(seeds[ends[i] + 1][list(run.idx)].cuda().double())
+            down = run.t(nxt) if nxt is not None else torch.zeros_like(seed)
+            frac = lambda a, s: (_ulps(a, q(down + s)) > 1).double().mean().item()
+            rep.err("bwd stage end >1ulp", frac(g, seed), TIE_FRAC, p)
+            # required where the planted error moves the reference itself past the bound: a seed below half an ulp of
+            # the downstream gradient almost everywhere cannot show in g
+            for m, f in (("dropped", 0), ("doubled", 2)):
+                rep.mutant("stage-end seed " + m, frac(g, f * seed), TIE_FRAC, p,
+                           required=frac(q(down + seed), f * seed) > TIE_FRAC)
+        else:
+            assert nxt is not None and eg.out_off == nxt.out_off, p
         dz = g
         if u["bn4"].kind == 10:   # res_layer.5: the squeeze gradient, then dr = e * g + shift
             edr = by[(13, i)]
