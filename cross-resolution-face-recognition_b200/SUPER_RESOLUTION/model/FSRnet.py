@@ -6,9 +6,10 @@ image heads.
 Same class names, constructor arguments, ``nn.Sequential`` indices and parameter names (identical ``state_dict`` keys;
 the parameter-free layers - ReflectionPad2d, InstanceNorm2d, ReLU, Tanh - are kept as containers so the indices match),
 same ``forward`` signatures.  ``forward`` never calls the torch layers: every op is a native kernel through
-``crfr_b200.functional`` (tcgen05 implicit GEMM for the 3x3 stride-1 convolutions, the lowered / CUDA-core engines for
-the stride-2, 7x7, 1x1 and transposed ones, fused InstanceNorm + ReLU / PReLU / residual passes, reflection-pad gathers,
-hourglass pooling).  Activations are NHWC bf16 between ops; module inputs and outputs are fp32 NCHW.
+``crfr_b200.functional`` (tcgen05 implicit GEMM for the 3x3 stride-1 convolutions, padding 0 or 1; the lowered tcgen05
+recipes for the stride-2, 7x7, 1x1, transposed and 3-channel ones; CUDA cores only for the 13- and 68-channel 1x1 prior heads
+and the 3x3 stem's input gradient; fused InstanceNorm + ReLU / PReLU / residual passes, reflection-pad gathers, hourglass
+pooling).  Activations are NHWC bf16 between ops; module inputs and outputs are fp32 NCHW.
 
 The reference's ``OverallNetwork`` of this file cannot be constructed (it names a class ``Course_SR_Network`` that the
 file does not define, :449; SURVEY Appendix C); ``SRNetwork`` below is that wiring with the classes that do exist

@@ -145,7 +145,7 @@ int crfr_colsum(const void* t, int ld, int c, long long npix, float* out, void* 
 
 // tc_conv.cu: generic tcgen05 launchers used by the lowered (im2col) edge layers
 struct TcGemm {           // out[pixel][n] = bias[n] + sum_{tap,k} src[pixel + sign*(tap - pad)][k] * w[tap][n][k]
-  const void* src; int n, h, w, k_total, src_ld;
+  const void* src; int n, h, w, k_total, src_ld;   // h, w: the output grid (the pixel tiles)
   const void* wt;         // bf16 [ksize*ksize][n_total][k_total]
   int ksize, pad, sign;
   int n_total, tile_n;    // tile_n = 0: pick automatically
@@ -157,10 +157,12 @@ struct TcGemm {           // out[pixel][n] = bias[n] + sum_{tap,k} src[pixel + s
   // stat_batch: ONE statistic group over the whole batch (BatchNorm): partial sums [1][tiles x 4][2][n_total], any tiling (rows
   // of a tile that lie outside the tensor are masked out); needs bias == nullptr
   int stat_batch = 0;
+  // spatial size of src when it differs from the output grid (3x3 stride-1 pad-0 convolutions and their dgrad); 0 = h, w
+  int src_h = 0, src_w = 0;
 };
 int crfr_tc_gemm(const TcGemm& g, cudaStream_t st);
-struct TcWgrad {          // G[tap][ci][co] = sum_pixel x[pixel + tap - 1][ci] * dy[pixel][co]   (fp32, G is overwritten)
-  const void* x; int n, h, w, cin, x_ld;
+struct TcWgrad {          // G[tap][ci][co] = sum_pixel x[pixel + tap - pad][ci] * dy[pixel][co]   (fp32, G is overwritten)
+  const void* x; int n, h, w, cin, x_ld;   // h, w: the grid of dy (the pixels summed over)
   const void* dy; int cout, dy_ld;
   int taps3x3;            // 1: 3x3 pad 1 (9 taps), 0: single tap
   float* G;
@@ -168,6 +170,8 @@ struct TcWgrad {          // G[tap][ci][co] = sum_pixel x[pixel + tap - 1][ci] *
   // as this buffer holds; crfr_tc_wgrad_part_bytes() bytes always suffice for the full split
   float* part = nullptr;
   size_t part_bytes = 0;
+  int pad = 1;            // taps3x3: 1 (same-size) or 0 (valid: x is (h + 2) x (w + 2))
+  int x_h = 0, x_w = 0;   // spatial size of x when it differs from the grid of dy; 0 = h, w
 };
 int crfr_tc_wgrad_raw(const TcWgrad& g, cudaStream_t st);
 size_t crfr_tc_wgrad_part_bytes();

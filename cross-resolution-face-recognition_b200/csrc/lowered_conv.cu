@@ -13,9 +13,19 @@
 //       64 -> 16*64 channels with a block-sparse weight (49 of 144 blocks non-zero), run on the implicit-GEMM kernel,
 //       followed by a pixel shuffle; dgrad / wgrad are that convolution's dgrad / wgrad on the un-shuffled dOut.
 //       (The earlier x . W -> 1.6 GB fp32 -> col2im formulation moved 12x more bytes.)
-//   R5  Conv2d 3x3 s2 p1 / 1x1 s2 p0, channels % 64 == 0 (ResNet stage transitions and downsample branches,
-//       model/resnet.py:9-16, 193-200)                                 fwd, wgrad : im2col(T*cin) . W
+//   R5  Conv2d 3x3 s2 p1|p0 / 1x1 s2 p0, channels % 64 == 0 (ResNet stage transitions and downsample branches,
+//       model/resnet.py:9-16, 193-200; p0: the reflection-padded stride-2 stages of SUPER_RESOLUTION/model/FSRnet.py)
+//                                                                     fwd, wgrad : im2col(T*cin) . W
 //                                                                     dgrad : dY . W (T*cin cols, fp32) then col2im
+//   R6  Conv2d 1x1 s1 p0, channels % 64 == 0 (the pre-activation Bottlenecks of SUPER_RESOLUTION/model/FSRnet.py:75-114)
+//                                                                     fwd, dgrad : one GEMM;  wgrad : X^T . dY
+//   R7  ConvTranspose2d 3x3 s2 p1 op1, channels % 64 == 0 (the up stages of SUPER_RESOLUTION/model/FSRnet.py): the
+//       transpose of R5's convolution, so R5's three forms with the roles exchanged
+//                                                                     fwd : X . W (9*cout cols, fp32) then col2im
+//                                                                     dgrad : im2col(dY) . W
+//                                                                     wgrad : im2col(dY)^T . X
+// R1 - R3 also take the padding-0 ("valid") 3x3 / 7x7 stride-1 forms of the variant's reflection-padded stems and heads
+// (R2 with 64 or 128 input channels).
 // Partial products that are summed by a col2im kernel stay fp32 until the single final rounding, so the arithmetic
 // contract is the same as the direct kernels': fp32 accumulation over all taps and channels, one bf16 rounding.
 #include "common.cuh"
@@ -387,9 +397,10 @@ __global__ void im2col_vec_kernel(const bf16* __restrict__ x, int x_ld, int C, i
   *reinterpret_cast<uint4*>(P + o * ((long long)T * C) + (long long)tap * C + g * 8) = v;
 }
 
-// Its transpose: dx[p][c] = sum over the taps that reach input pixel p of dP[o][tap*C + c] (fp32 in, one rounding)
+// Its transpose: dx[p][c] = bias[c] + sum over the taps that reach input pixel p of dP[o][tap*C + c] (fp32 in, one
+// rounding; bias may be NULL)
 __global__ void col2im_vec_kernel(const float* __restrict__ dP, int C, int oh, int ow, int h, int w, int ks, int stride,
-                                  int pad, bf16* __restrict__ dx, int dx_ld, long long total) {
+                                  int pad, const float* __restrict__ bias, bf16* __restrict__ dx, int dx_ld, long long total) {
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= total) return;
   const int groups = C >> 3;
@@ -401,6 +412,9 @@ __global__ void col2im_vec_kernel(const float* __restrict__ dP, int C, int oh, i
   const long long n = q / h;
   const long long ld = (long long)ks * ks * C;
   float acc[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+  if (bias)
+#pragma unroll
+    for (int j = 0; j < 8; ++j) acc[j] = bias[g * 8 + j];
   for (int ky = 0; ky < ks; ++ky) {
     const int ty = Y + pad - ky;
     if (ty < 0 || ty % stride) continue;
@@ -484,6 +498,15 @@ struct Arena {
 
 inline int kpad_of(const crfr_conv_desc* d) { return ((d->k * d->k * 3 + 63) / 64) * 64; }   // 27 -> 64, 147 -> 192
 
+// Recipe 2's GEMMs are per-pixel products (no taps): at pad 0 they run over the n * h * w input pixels as one flat row of
+// the tile engine, which keeps every 128-pixel tile full at the variant's 130-wide padded maps (as images, the second
+// column tile of each 130-pixel row would hold 2 pixels).
+struct PixGrid { int n, h, w; };
+inline PixGrid valid_flat(const crfr_conv_desc* d) {
+  if (d->pad == 1) return {d->n, d->h, d->w};
+  return {1, 1, d->n * d->h * d->w};
+}
+
 int tcgen05_spatial_ok(int h, int w) { return crfr_tc_supported(2, h, w, 64, 64, 3, 1, 1); }
 
 }  // namespace
@@ -492,24 +515,31 @@ int tcgen05_spatial_ok(int h, int w) { return crfr_tc_supported(2, h, w, 64, 64,
 // recipe selection
 // ---------------------------------------------------------------------------------------------------------
 int crfr_lowered_recipe(const crfr_conv_desc* d) {
+  const bool ld8 = (d->in_ld & 7) == 0 && (d->out_ld & 7) == 0, c64 = d->cin % 64 == 0 && d->cout % 64 == 0;
   if (!d->transposed) {
-    if (d->k == 3 && d->stride == 1 && d->pad == 1 && d->cin == 3 && d->in_ld == 4 && d->cout % 64 == 0 && d->cout <= 256 &&
-        tcgen05_spatial_ok(d->h, d->w))
+    if (d->k == 3 && d->stride == 1 && (d->pad == 1 || d->pad == 0) && d->cin == 3 && d->in_ld == 4 && d->cout % 64 == 0 &&
+        d->cout <= 256 && tcgen05_spatial_ok(d->oh, d->ow))
       return 1;
-    if (d->k == 3 && d->stride == 1 && d->pad == 1 && d->cout == 3 && d->cin == 64 && d->out_ld == 4 &&
-        tcgen05_spatial_ok(d->h, d->w))
+    // pad 1 keeps its image-shaped GEMMs (tiled over h x w); pad 0 runs them over the flat pixel list (valid_flat below)
+    if (d->k == 3 && d->stride == 1 && d->cout == 3 && d->out_ld == 4 &&
+        ((d->pad == 1 && d->cin == 64 && tcgen05_spatial_ok(d->h, d->w)) ||
+         (d->pad == 0 && (d->cin == 64 || d->cin == 128) && (d->in_ld & 7) == 0 && d->h > 2 && d->w > 2)))
       return 2;
-    if (d->k == 7 && (d->stride == 4 || d->stride == 2) && d->pad == 3 && d->cin == 3 && d->in_ld == 4 &&
-        (d->cout == 64 || d->cout == 128) && tcgen05_spatial_ok(d->oh, d->ow))
+    if (d->k == 7 && (((d->stride == 4 || d->stride == 2) && d->pad == 3) || (d->stride == 1 && d->pad == 0)) && d->cin == 3 &&
+        d->in_ld == 4 && (d->cout == 64 || d->cout == 128) && tcgen05_spatial_ok(d->oh, d->ow))
       return 3;
-    if (d->stride == 2 && ((d->k == 3 && d->pad == 1) || (d->k == 1 && d->pad == 0)) && d->cin % 64 == 0 &&
-        d->cout % 64 == 0 && (d->in_ld & 7) == 0 && (d->out_ld & 7) == 0 && tcgen05_spatial_ok(d->oh, d->ow))
+    if (d->stride == 2 && ((d->k == 3 && (d->pad == 1 || d->pad == 0)) || (d->k == 1 && d->pad == 0)) && c64 && ld8 &&
+        tcgen05_spatial_ok(d->oh, d->ow))
       return 5;
+    if (d->k == 1 && d->stride == 1 && d->pad == 0 && c64 && ld8 && tcgen05_spatial_ok(d->h, d->w)) return 6;
     return 0;
   }
   if (d->k == 7 && d->stride == 4 && d->pad == 2 && d->cin == 64 && d->cout == 64 && d->oh == 4 * d->h && d->ow == 4 * d->w &&
       tcgen05_spatial_ok(d->h, d->w))
     return 4;
+  if (d->k == 3 && d->stride == 2 && d->pad == 1 && d->oh == 2 * d->h && d->ow == 2 * d->w && c64 && ld8 &&
+      tcgen05_spatial_ok(d->h, d->w))
+    return 7;
   return 0;
 }
 
@@ -534,9 +564,16 @@ size_t crfr_lowered_ws_bytes(const crfr_conv_desc* d) {
       b = small * kc * 2 + small * kc * 4 + (size_t)d->cout * kc * 2 + kc * d->cout * 4;
       break;
     }
+    case 6: b = (size_t)d->cin * d->cout * 4; break;
+    case 7: {   // big = the input grid here: [ipix][9 * cout] fp32 (forward) or bf16 (dgrad / wgrad) + weights / G
+      const size_t kc = (size_t)9 * d->cout;
+      b = big * kc * 4 + (size_t)d->cin * kc * 4 + 1024;
+      break;
+    }
     default: return 0;
   }
-  if (r == 1 || r == 3 || r == 5) b += stat_partial_bytes(d) + 1024;
+  if (r == 2 && d->pad == 0) b += (size_t)d->cin * 64 * 2 * 2 + (size_t)d->cin * 64 * 4;   // up to 128 input channels
+  if (r == 1 || r == 3 || r == 5 || r == 6) b += stat_partial_bytes(d) + 1024;
   return b + 16 * 1024 + crfr_tc_wgrad_part_bytes() + 1024;   // + the wgrad's per-split partial sums
 }
 
@@ -604,15 +641,44 @@ int crfr_lowered_fwd(const crfr_conv_desc* d, const void* x, const void* w_packe
     TcGemm g{P, d->n, d->oh, d->ow, kc, kc, wg, 1, 0, 1, d->cout, 0, y, d->out_ld, 0, bias};
     return gemm_with_stats(g, d, A, stats, eps, stats_done, st);
   }
+  if (recipe == 6 || recipe == 7) {
+    if (!y || y_nchw) {
+      crfr_set_error("lowered conv: recipe %d produces the bf16 NHWC output only", recipe);
+      return CRFR_EUNSUPPORTED;
+    }
+    CRFR_CHECK_ARG(cin_pad == d->cin, "lowered conv: cin_pad %d != cin %d", cin_pad, d->cin);
+    if (recipe == 6) {   // [1][cout][cin] is the GEMM weight
+      TcGemm g{x, d->n, d->h, d->w, d->cin, d->in_ld, w_packed, 1, 0, 1, d->cout, 0, y, d->out_ld, 0, bias};
+      return gemm_with_stats(g, d, A, stats, eps, stats_done, st);
+    }
+    // R7: dP[i][tap*cout + co] = sum_ci X[i][ci] W[ci][co][tap] (fp32; w_packed [tap][cout][cin] is that GEMM weight), then
+    // y[P][co] = bias + sum over the (input pixel, tap) pairs that reach P, exactly R5's dgrad col2im
+    const int kc = 9 * d->cout;
+    const long long ipix = (long long)d->n * d->h * d->w, opix = (long long)d->n * d->oh * d->ow;
+    TAKE(dP, float, A, (size_t)ipix * kc * 4);
+    TcGemm g{x, d->n, d->h, d->w, d->cin, d->in_ld, w_packed, 1, 0, 1, kc, 0, dP, kc, 1, nullptr};
+    CRFR_TRY(crfr_tc_gemm(g, st));
+    LAUNCH(col2im_vec_kernel, opix * (d->cout / 8), st, dP, d->cout, d->h, d->w, d->oh, d->ow, 3, 2, 1, bias, (bf16*)y,
+           d->out_ld, opix * (d->cout / 8));
+    return CRFR_OK;
+  }
   if (recipe == 2) {
+    CRFR_CHECK_ARG(cin_pad == d->cin, "lowered conv: cin_pad %d != cin %d", cin_pad, d->cin);
     const long long pix = (long long)d->n * d->h * d->w;
+    const PixGrid pg = valid_flat(d);
     TAKE(Q, float, A, (size_t)pix * 32 * 4);
-    TAKE(Wq, bf16, A, (size_t)32 * 64 * 2);
-    CRFR_CUDA(cudaMemsetAsync(Wq, 0, (size_t)32 * 64 * 2, st));
-    CRFR_CUDA(cudaMemcpyAsync(Wq, w_packed, (size_t)27 * 64 * 2, cudaMemcpyDeviceToDevice, st));   // rows (tap, co)
-    TcGemm g{x, d->n, d->h, d->w, 64, d->in_ld, Wq, 1, 0, 1, 32, 32, Q, 32, 1, nullptr};
+    TAKE(Wq, bf16, A, (size_t)32 * d->cin * 2);
+    CRFR_CUDA(cudaMemsetAsync(Wq, 0, (size_t)32 * d->cin * 2, st));
+    CRFR_CUDA(cudaMemcpyAsync(Wq, w_packed, (size_t)27 * d->cin * 2, cudaMemcpyDeviceToDevice, st));   // rows (tap, co)
+    TcGemm g{x, pg.n, pg.h, pg.w, d->cin, d->in_ld, Wq, 1, 0, 1, 32, 32, Q, 32, 1, nullptr};
     CRFR_TRY(crfr_tc_gemm(g, st));
     // y[p] = bias + sum_tap Q[p + (tap - pad)][tap*3 + co]
+    if (d->pad == 0) {
+      const long long opix = (long long)d->n * d->oh * d->ow;
+      LAUNCH(col2im_small_kernel, opix, st, Q, 32, 3, d->h, d->w, d->oh, d->ow, 3, 1, 0, -1, bias, y_nchw, (bf16*)y,
+             y ? d->out_ld : 0, opix);
+      return CRFR_OK;
+    }
     if (d->h % 8 == 0 && d->w % 32 == 0) {
       col2im3_s1_kernel<<<(unsigned)(d->n * (d->h / 8) * (d->w / 32)), 256, 0, st>>>(Q, d->h, d->w, -1, bias, y_nchw, (bf16*)y,
                                                                                    y ? d->out_ld : 0);
@@ -656,11 +722,31 @@ int crfr_lowered_dgrad(const crfr_conv_desc* d, const void* dy, const void* w_pa
   if (recipe == 2) {
     // dX[q][ci] = sum_k R[q][k] Wd[ci][k],  R[q][tap*3+co] = dY[q - (tap - pad)][co],  Wd[ci][tap*3+co] = W[co][ci][tap]
     const long long pix = (long long)d->n * d->h * d->w;
+    const PixGrid pg = valid_flat(d);
     TAKE(R, bf16, A, (size_t)pix * 64 * 2);
-    TAKE(Wd, bf16, A, (size_t)64 * 64 * 2);
-    CRFR_TRY(launch_im2col_small((const bf16*)dy, d->n, d->h, d->w, d->h, d->w, 3, 1, 1, -1, R, 64, st));
-    LAUNCH(repack_tapmajor_kernel, 64 * 64, st, (const bf16*)w_packed_t, T, 64, 3, cout_pad, Wd, 64, 64);
-    TcGemm g{R, d->n, d->h, d->w, 64, 64, Wd, 1, 0, 1, 64, 64, dx, d->in_ld, 0, nullptr};
+    TAKE(Wd, bf16, A, (size_t)d->cin * 64 * 2);
+    CRFR_TRY(launch_im2col_small((const bf16*)dy, d->n, d->oh, d->ow, d->h, d->w, 3, 1, d->pad, -1, R, 64, st));
+    LAUNCH(repack_tapmajor_kernel, d->cin * 64, st, (const bf16*)w_packed_t, T, d->cin, 3, cout_pad, Wd, d->cin, 64);
+    TcGemm g{R, pg.n, pg.h, pg.w, 64, 64, Wd, 1, 0, 1, d->cin, d->cin, dx, d->in_ld, 0, nullptr};
+    return crfr_tc_gemm(g, st);
+  }
+  if (recipe == 6) {   // dX = dY . W, w_packed_t [1][cin][cout]
+    CRFR_CHECK_ARG(cout_pad == d->cout, "lowered dgrad: cout_pad %d != cout %d", cout_pad, d->cout);
+    TcGemm g{dy, d->n, d->h, d->w, d->cout, d->out_ld, w_packed_t, 1, 0, 1, d->cin, 0, dx, d->in_ld, 0, nullptr};
+    return crfr_tc_gemm(g, st);
+  }
+  if (recipe == 7) {
+    // dX[i][ci] = sum_{tap, co} P[i][tap*cout + co] Wd[ci][tap*cout + co],  P = im2col(dY) with R5's geometry (3x3 s2 p1 from
+    // the output grid to the input grid),  Wd[ci][tap*cout + co] = W[ci][co][tap] (w_packed_t [tap][cin][cout])
+    CRFR_CHECK_ARG(cout_pad == d->cout, "lowered dgrad: cout_pad %d != cout %d", cout_pad, d->cout);
+    const int kc = 9 * d->cout;
+    const long long ipix = (long long)d->n * d->h * d->w;
+    TAKE(P, bf16, A, (size_t)ipix * kc * 2);
+    TAKE(Wd, bf16, A, (size_t)d->cin * kc * 2);
+    LAUNCH(im2col_vec_kernel, ipix * 9 * (d->cout / 8), st, (const bf16*)dy, d->out_ld, d->cout, d->oh, d->ow, d->h, d->w, 3,
+           2, 1, P, ipix * 9 * (d->cout / 8));
+    LAUNCH(repack_tapmajor_kernel, d->cin * kc, st, (const bf16*)w_packed_t, T, d->cin, d->cout, cout_pad, Wd, d->cin, kc);
+    TcGemm g{P, d->n, d->h, d->w, kc, kc, Wd, 1, 0, 1, d->cin, 0, dx, d->in_ld, 0, nullptr};
     return crfr_tc_gemm(g, st);
   }
   if (recipe == 3) {
@@ -688,7 +774,7 @@ int crfr_lowered_dgrad(const crfr_conv_desc* d, const void* dy, const void* w_pa
     TcGemm g{dy, d->n, d->oh, d->ow, d->cout, d->out_ld, w_packed_t, 1, 0, 1, kc, 0, dP, kc, 1, nullptr};
     CRFR_TRY(crfr_tc_gemm(g, st));
     LAUNCH(col2im_vec_kernel, ipix * (d->cin / 8), st, dP, d->cin, d->oh, d->ow, d->h, d->w, d->k, d->stride, d->pad,
-           (bf16*)dx, d->in_ld, ipix * (d->cin / 8));
+           nullptr, (bf16*)dx, d->in_ld, ipix * (d->cin / 8));
     return CRFR_OK;
   }
   if (recipe == 4) {
@@ -772,14 +858,39 @@ int crfr_lowered_wgrad(const crfr_conv_desc* d, const void* x, const void* dy, f
   }
   if (recipe == 2) {
     const long long pix = (long long)d->n * d->h * d->w;
+    const PixGrid pg = valid_flat(d);
     TAKE(R, bf16, A, (size_t)pix * 64 * 2);
-    TAKE(G, float, A, (size_t)64 * 64 * 4);
-    CRFR_TRY(launch_im2col_small((const bf16*)dy, d->n, d->h, d->w, d->h, d->w, 3, 1, 1, -1, R, 64, st));
-    CRFR_CUDA(cudaMemsetAsync(G, 0, (size_t)64 * 64 * 4, st));
-    TcWgrad g{x, d->n, d->h, d->w, 64, d->in_ld, R, 64, 64, 0, G};
+    TAKE(G, float, A, (size_t)d->cin * 64 * 4);
+    CRFR_TRY(launch_im2col_small((const bf16*)dy, d->n, d->oh, d->ow, d->h, d->w, 3, 1, d->pad, -1, R, 64, st));
+    CRFR_CUDA(cudaMemsetAsync(G, 0, (size_t)d->cin * 64 * 4, st));
+    TcWgrad g{x, pg.n, pg.h, pg.w, d->cin, d->in_ld, R, 64, 64, 0, G};
     A.rest(&g.part, &g.part_bytes);
     CRFR_TRY(crfr_tc_wgrad_raw(g, st));
-    LAUNCH(unpack_lowered_kernel, (long long)3 * 64 * T, st, G, 64, dw, 3, 64, T, 1);
+    LAUNCH(unpack_lowered_kernel, (long long)3 * d->cin * T, st, G, 64, dw, 3, d->cin, T, 1);
+    return CRFR_OK;
+  }
+  if (recipe == 6) {   // G[ci][co] = X^T dY
+    TAKE(G, float, A, (size_t)d->cin * d->cout * 4);
+    CRFR_CUDA(cudaMemsetAsync(G, 0, (size_t)d->cin * d->cout * 4, st));
+    TcWgrad g{x, d->n, d->h, d->w, d->cin, d->in_ld, dy, d->cout, d->out_ld, 0, G};
+    A.rest(&g.part, &g.part_bytes);
+    CRFR_TRY(crfr_tc_wgrad_raw(g, st));
+    LAUNCH(unpack_lowered_kernel, (long long)d->cout * d->cin, st, G, d->cout, dw, d->cout, d->cin, 1, 0);
+    return CRFR_OK;
+  }
+  if (recipe == 7) {
+    // G[tap*cout + co][ci] = sum_i P[i][tap*cout + co] X[i][ci] with P = im2col(dY) as in the dgrad; dW[ci][co][tap] += G
+    const int kc = 9 * d->cout;
+    const long long ipix = (long long)d->n * d->h * d->w;
+    TAKE(P, bf16, A, (size_t)ipix * kc * 2);
+    TAKE(G, float, A, (size_t)kc * d->cin * 4);
+    CRFR_CUDA(cudaMemsetAsync(G, 0, (size_t)kc * d->cin * 4, st));
+    LAUNCH(im2col_vec_kernel, ipix * 9 * (d->cout / 8), st, (const bf16*)dy, d->out_ld, d->cout, d->oh, d->ow, d->h, d->w, 3,
+           2, 1, P, ipix * 9 * (d->cout / 8));
+    TcWgrad g{P, d->n, d->h, d->w, kc, kc, x, d->cin, d->in_ld, 0, G};
+    A.rest(&g.part, &g.part_bytes);
+    CRFR_TRY(crfr_tc_wgrad_raw(g, st));
+    LAUNCH(unpack_lowered_kernel, (long long)d->cin * d->cout * 9, st, G, d->cin, dw, d->cin, d->cout, 9, 0);
     return CRFR_OK;
   }
   if (recipe == 4) {

@@ -1,9 +1,11 @@
 // tcgen05 / TMEM implicit-GEMM convolution engine for sm_100a, fed by TMA.
 //
-// Forward / dgrad (3x3, stride 1, pad 1, channels in multiples of 64), NHWC bf16:
+// Forward / dgrad (3x3, stride 1, pad 1 or 0, channels in multiples of 64), NHWC bf16:
 //   one CTA computes a tile of 128 output pixels x N output channels.  The 128 pixels are a TMA box
 //   (64 channels x bw x bh x bn) of the NHWC activation tensor, so the im2col gather of tap (ky,kx) is just the
-//   same box shifted by (kx-1, ky-1); out-of-bounds elements are zero-filled by the TMA unit (= the padding).
+//   same box shifted by (kx-pad, ky-pad); out-of-bounds elements are zero-filled by the TMA unit (= the padding).  With
+//   pad 0 the pixel tiles cover the smaller output grid and the source map keeps its own size (forward: x is
+//   (oh + 2) x (ow + 2); dgrad: the tiles cover dx and the shifted dY boxes fall off dY's edges into the zero fill).
 //   K loop = taps x (Cin/64): per step one 16 KB activation tile (A, K-major, SWIZZLE_128B) and one N x 64 weight
 //   tile (B, K-major) land in a 3-4 stage smem ring (mbarrier full/empty), one elected thread issues 4
 //   tcgen05.mma (M=128, N, K=16) per step into a TMEM accumulator, and 4 epilogue warps drain TMEM with
@@ -412,6 +414,7 @@ struct WgradParams {
   int bw, bh, bn, tiles_x, tiles_y, total_tiles;
   int cin, cout;   // cout = all dY channels; a CTA handles columns [ntile * N, +N)
   int rows;        // pixels per tile (bw*bh*bn <= 128); rows beyond it are kept zero in shared memory
+  int pad;         // TAPS = 3: tap (ky, kx) reads X at (y + ky - pad, x + kx - pad); X is (h + 2 - 2 pad) x (w + 2 - 2 pad)
   float* G;        // [gridDim.x][taps][cin][cout] fp32: one slice per split, every element stored once
 };
 
@@ -496,11 +499,11 @@ tc_wgrad_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
       if (leader) {
         mbar_expect_tx(&full[s], stage_tx);
         if (H) {   // `ky` is this CTA's kx: the box of rows y0 - 1 .. y0 + bh at its x shift
-          tma_load_4d(sb, &tmX, &full[s], kc * 64, x0 + ky - 1, y0 - 1, n0);
+          tma_load_4d(sb, &tmX, &full[s], kc * 64, x0 + ky - p.pad, y0 - p.pad, n0);
         } else if (TAPS == 3) {
 #pragma unroll
           for (int kx = 0; kx < 3; ++kx)
-            tma_load_4d(sb + kx * kTile16K, &tmX, &full[s], kc * 64, x0 + kx - 1, y0 + ky - 1, n0);
+            tma_load_4d(sb + kx * kTile16K, &tmX, &full[s], kc * 64, x0 + kx - p.pad, y0 + ky - p.pad, n0);
         } else {
           tma_load_4d(sb, &tmX, &full[s], kc * 64, x0, y0, n0);
         }
@@ -668,8 +671,9 @@ int crfr_tc_gemm(const TcGemm& g, cudaStream_t st) {
     crfr_set_error("tc_gemm: unsupported spatial size %dx%d", g.h, g.w);
     return CRFR_EUNSUPPORTED;
   }
+  const int src_h = g.src_h ? g.src_h : g.h, src_w = g.src_w ? g.src_w : g.w;
   CUtensorMap tmA, tmB, tmY;
-  CRFR_TRY(make_act_map(&tmA, g.src, g.n, g.h, g.w, g.k_total, g.src_ld, t.bw, t.bh, t.bn));
+  CRFR_TRY(make_act_map(&tmA, g.src, g.n, src_h, src_w, g.k_total, g.src_ld, t.bw, t.bh, t.bn));
   if (!g.out_f32) {
     CRFR_CHECK_ARG(tile_n % 64 == 0 && (g.out_ld & 7) == 0, "tc_gemm: bf16 output needs a tile width multiple of 64");
     CRFR_TRY(make_act_map(&tmY, g.out, g.n, g.h, g.w, g.n_total, g.out_ld, t.bw, t.bh, t.bn));
@@ -715,7 +719,7 @@ int crfr_tc_gemm(const TcGemm& g, cudaStream_t st) {
     case 64:
       if (p.ksize == 3 && p.pad == 1 && p.kchunks == 1 && p.bn == 1 && (p.bw & 7) == 0 && (p.bh + 2) * p.bw <= 256) {
         CUtensorMap tmA2;   // the box with its two halo rows
-        CRFR_TRY(make_act_map(&tmA2, g.src, g.n, g.h, g.w, g.k_total, g.src_ld, t.bw, t.bh + 2, 1));
+        CRFR_TRY(make_act_map(&tmA2, g.src, g.n, src_h, src_w, g.k_total, g.src_ld, t.bw, t.bh + 2, 1));
         return launch_conv<64, 1>(tmA2, tmB, tmY, p, tiles, st);
       }
       return launch_conv<64>(tmA, tmB, tmY, p, tiles, st);
@@ -737,7 +741,7 @@ int launch_wgrad_any(const TcWgrad& g, const Tiling& t, const CUtensorMap& tmX, 
   if (g.taps3x3) {
     if (t.bn == 1 && (t.bh + 2) * t.bw <= 256 && (g.cout == 64 || g.cout % 128 == 0)) {
       CUtensorMap tmXh;   // the X box with its two halo rows
-      CRFR_TRY(make_act_map(&tmXh, g.x, g.n, g.h, g.w, g.cin, g.x_ld, t.bw, t.bh + 2, 1));
+      CRFR_TRY(make_act_map(&tmXh, g.x, g.n, g.x_h ? g.x_h : g.h, g.x_w ? g.x_w : g.w, g.cin, g.x_ld, t.bw, t.bh + 2, 1));
       if (g.cout == 64) return launch_wgrad<64, 3, true>(tmXh, tmDY, p, splits, st);
       return launch_wgrad<128, 3, true>(tmXh, tmDY, p, splits, st);
     }
@@ -760,8 +764,9 @@ int crfr_tc_wgrad_raw(const TcWgrad& g, cudaStream_t st) {
     crfr_set_error("tc_wgrad: unsupported spatial size %dx%d", g.h, g.w);
     return CRFR_EUNSUPPORTED;
   }
+  CRFR_CHECK_ARG(g.pad == 0 || g.pad == 1, "tc_wgrad: pad %d", g.pad);
   CUtensorMap tmX, tmDY;
-  CRFR_TRY(make_act_map(&tmX, g.x, g.n, g.h, g.w, g.cin, g.x_ld, t.bw, t.bh, t.bn));
+  CRFR_TRY(make_act_map(&tmX, g.x, g.n, g.x_h ? g.x_h : g.h, g.x_w ? g.x_w : g.w, g.cin, g.x_ld, t.bw, t.bh, t.bn));
   CRFR_TRY(make_act_map(&tmDY, g.dy, g.n, g.h, g.w, g.cout, g.dy_ld, t.bw, t.bh, t.bn));
   WgradParams p;
   p.n = g.n; p.h = g.h; p.w = g.w;
@@ -769,6 +774,7 @@ int crfr_tc_wgrad_raw(const TcWgrad& g, cudaStream_t st) {
   p.total_tiles = t.tiles_x * t.tiles_y * t.tiles_n;
   p.cin = g.cin; p.cout = g.cout;
   p.rows = t.rows;
+  p.pad = g.pad;
   const int tile_n = (g.cout % 128 == 0) ? 128 : 64;
   const int ctas_per_split = (g.taps3x3 ? 3 : 1) * (g.cout / tile_n) * (g.cin / 64);
   // One CTA per SM at a time (160-192 KB of shared memory): the grid runs in waves of `sms` CTAs, so it must not exceed a whole
@@ -799,15 +805,19 @@ size_t crfr_tc_wgrad_part_bytes() {
 }
 
 int crfr_tc_supported(int op, int h, int w, int cin, int cout, int k, int stride, int pad) {
-  if (k != 3 || stride != 1 || pad != 1) return 0;
+  // pad 1: same-size; pad 0: the "valid" form (reflection-padded maps of the SUPER_RESOLUTION variant), whose output grid
+  // is (h - 2) x (w - 2): the forward and the weight gradient tile that grid, the dgrad tiles the input grid
+  if (k != 3 || stride != 1 || (pad != 1 && pad != 0)) return 0;
   if (cin % 64 || cout % 64) return 0;
+  const int oh = h + 2 * pad - 2, ow = w + 2 * pad - 2;
+  if (oh < 1 || ow < 1) return 0;
   const int nout = (op == 1) ? cin : cout;  // GEMM N
   if (op == 2) {
     if (cout != 64 && cout % 128 != 0) return 0;
-    return spatial_ok(h, w, true) ? 1 : 0;
+    return spatial_ok(oh, ow, true) ? 1 : 0;
   }
   if (pick_tile_n(nout) == 0) return 0;
-  return spatial_ok(h, w, false) ? 1 : 0;
+  return (op == 1 ? spatial_ok(h, w, false) : spatial_ok(oh, ow, false)) ? 1 : 0;
 }
 
 size_t crfr_tc_workspace_bytes(const crfr_conv_desc* d) {
@@ -836,7 +846,9 @@ int crfr_tc_conv(const crfr_conv_desc* d, int dgrad, const void* src, const void
                         dgrad ? d->in_ld : d->out_ld, dgrad ? nullptr : stats, eps, ws, ws_bytes, st);
   }
   TcGemm g;
-  g.src = src; g.n = d->n; g.h = d->h; g.w = d->w;
+  // the pixel tiles cover the output grid: forward (oh, ow), dgrad (h, w); src is the other one
+  g.src = src; g.n = d->n; g.h = dgrad ? d->h : d->oh; g.w = dgrad ? d->w : d->ow;
+  g.src_h = dgrad ? d->oh : d->h; g.src_w = dgrad ? d->ow : d->w;
   g.k_total = dgrad ? d->cout : d->cin;
   g.src_ld = dgrad ? d->out_ld : d->in_ld;
   g.wt = w_packed; g.ksize = d->k; g.pad = d->pad; g.sign = dgrad ? -1 : 1;
@@ -874,7 +886,8 @@ int crfr_tc_wgrad(const crfr_conv_desc* d, const void* x, const void* dy, float*
   }
   CRFR_CUDA(cudaMemsetAsync(ws, 0, need, st));
   TcWgrad g;
-  g.x = x; g.n = d->n; g.h = d->h; g.w = d->w; g.cin = d->cin; g.x_ld = d->in_ld;
+  g.x = x; g.n = d->n; g.h = d->oh; g.w = d->ow; g.cin = d->cin; g.x_ld = d->in_ld;
+  g.x_h = d->h; g.x_w = d->w; g.pad = d->pad;
   g.dy = dy; g.cout = d->cout; g.dy_ld = d->out_ld; g.taps3x3 = 1; g.G = (float*)ws;
   const size_t part_off = (need + 255) & ~(size_t)255;
   g.part = ws_bytes > part_off ? (float*)((uint8_t*)ws + part_off) : nullptr;

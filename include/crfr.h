@@ -69,7 +69,16 @@ typedef struct crfr_conv_desc {
 } crfr_conv_desc;
 
 /* ref: nn.Conv2d / nn.ConvTranspose2d forward at model/FSRnet.py:79,85,110,114,312,318,345,351,384,391,392,432,436,439
- *      and model/resnet.py:23-26,158,196.
+ *      and model/resnet.py:23-26,158,196; the SUPER_RESOLUTION variant's layers (SUPER_RESOLUTION/model/FSRnet.py:251-416).
+ * Shapes on the tcgen05 engine (ENGINE_AUTO picks them, ENGINE_TCGEN05 rejects the others with CRFR_EUNSUPPORTED; the
+ * same for crfr_conv_dgrad / crfr_conv_wgrad unless noted; ENGINE_DIRECT runs every shape on CUDA cores):
+ *   3x3 s1 pad 1 or 0, cin / cout multiples of 64 (wgrad: cout 64 or a multiple of 128);
+ *   3x3 s2 pad 1 or 0 and 1x1 s2 / 1x1 s1 pad 0, channels multiples of 64;
+ *   ConvTranspose2d 3x3 s2 pad 1 output_padding 1 and 7x7 s4 pad 2 output_padding 1 (64 -> 64), channels multiples of 64;
+ *   3-channel input: 3x3 s1 pad 1 or 0 (cout a multiple of 64 up to 256; dgrad on CUDA cores), 7x7 s4 / s2 pad 3 and
+ *   7x7 s1 pad 0 (cout 64 or 128);  3-channel output: 3x3 s1 pad 1 (cin 64) or pad 0 (cin 64 or 128).
+ * A 1x1 layer with an output channel count that is not a multiple of 64 (the 11 / 13 / 68-channel heads) runs on CUDA
+ * cores.  crfr_conv_engine_supported reports the Conv2d shapes (it has no transposed flag).
  * x: NHWC bf16.  w_packed: bf16 [k*k][cout][cin_pad] made by crfr_pack_weight.  bias: fp32 [cout] or NULL.
  * y: NHWC bf16 or NULL.  y_nchw: fp32 NCHW [n][cout][oh][ow] or NULL.
  * stats: fp32 [n][cout][2] = (mean, rstd) of y over (oh,ow) per (n, channel) - the InstanceNorm statistics
@@ -80,9 +89,11 @@ int crfr_conv_fwd(int engine, const crfr_conv_desc* d, const void* x, const void
 /* dx = gradient w.r.t. x.  w_packed_t: bf16 [k*k][cin][cout_pad].  dx: NHWC bf16 with stride d->in_ld. */
 int crfr_conv_dgrad(int engine, const crfr_conv_desc* d, const void* dy, const void* w_packed_t, int cout_pad,
                     void* dx, void* ws, size_t ws_bytes, void* stream);
-/* dw (fp32, reference layout: Conv2d [cout][cin][k][k], ConvTranspose2d [cin][cout][k][k]) += ...; dbias += sum dy */
+/* dw (fp32, reference layout: Conv2d [cout][cin][k][k], ConvTranspose2d [cin][cout][k][k]) += ...; dbias += sum dy.
+ * Both are reduced in a fixed order (no float atomics): two calls give the same bits. */
 int crfr_conv_wgrad(int engine, const crfr_conv_desc* d, const void* x, const void* dy, float* dw, float* dbias,
                     void* ws, size_t ws_bytes, void* stream);
+/* scratch for any of the three calls on d; a smaller workspace is CRFR_EWORKSPACE where the path needs one */
 size_t crfr_conv_workspace_bytes(const crfr_conv_desc* d);
 
 /* ---------------------------------------------------------------- normalisation + activation -------------- */
