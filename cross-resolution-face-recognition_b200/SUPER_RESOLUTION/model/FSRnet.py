@@ -5,27 +5,151 @@ image heads.
 
 Same class names, constructor arguments, ``nn.Sequential`` indices and parameter names (identical ``state_dict`` keys;
 the parameter-free layers - ReflectionPad2d, InstanceNorm2d, ReLU, Tanh - are kept as containers so the indices match),
-same ``forward`` signatures.  ``forward`` never calls the torch layers: every op is a native kernel through
-``crfr_b200.functional`` (tcgen05 implicit GEMM for the 3x3 stride-1 convolutions, padding 0 or 1; the lowered tcgen05
-recipes for the stride-2, 7x7, 1x1, transposed and 3-channel ones; CUDA cores only for the 13- and 68-channel 1x1 prior heads
-and the 3x3 stem's input gradient; fused InstanceNorm + ReLU / PReLU / residual passes, reflection-pad gathers, hourglass
-pooling).  Activations are NHWC bf16 between ops; module inputs and outputs are fp32 NCHW.
+same ``forward`` signatures.  ``forward`` never calls the torch layers: ``SRNetwork`` and each sub-network run as one
+native network program (crfr_srnet_forward, csrc/srnet.cu) with one autograd node (crfr_srnet_backward).  Inside it
+every layer keeps the routing of the single-op entry points (tcgen05 implicit GEMM for the 3x3 stride-1 convolutions;
+the lowered tcgen05 recipes for the stride-2, 7x7, 1x1, transposed and 3-channel ones; the 3x3 stem's input gradient on
+CUDA cores), the two 1x1 prior heads run as one tensor-core GEMM, and activations stay NHWC bf16 in the program's
+workspace.  Module inputs and outputs are fp32 NCHW.
 
 The reference's ``OverallNetwork`` of this file cannot be constructed (it names a class ``Course_SR_Network`` that the
 file does not define, :449; SURVEY Appendix C); ``SRNetwork`` below is that wiring with the classes that do exist
 (coarse image -> encoder and prior network -> concatenation -> decoder), the one ``train_FHN.py`` drives by hand.
 """
+import ctypes as C
+
 import torch
 import torch.nn as nn
 
-from ... import functional as Fn
+from ... import _lib as L
+from ... import ops
 
 
-def _check(x, channels):
+def _check(x, channels, section):
     if not x.is_cuda:
         raise RuntimeError("crfr_b200 SUPER_RESOLUTION networks need CUDA tensors: the hot path has no CPU fallback")
     if x.dim() != 4 or x.shape[1] != channels:
         raise ValueError("expected [B,%d,H,W], got %s" % (channels, tuple(x.shape)))
+    if L.lib().crfr_srnet_workspace_bytes(section, x.shape[0], x.shape[2], x.shape[3], 0) == 0:
+        raise ValueError("input %s not supported: H and W must be >= 5 (multiples of 16 for the prior network and "
+                         "SRNetwork; include/crfr.h, crfr_srnet_io)" % (tuple(x.shape),))
+
+
+def _out_shapes(section, b, h, w):
+    big_h, big_w = 4 * -(-h // 4), 4 * -(-w // 4)
+    if section == L.SRNET_NETWORK:
+        return [(b, 3, h, w), (b, 3, h, w), (b, 68, h, w), (b, 13, h, w)]
+    if section == L.SRNET_PRIOR:
+        return [(b, 64, h, w), (b, 68, h, w), (b, 13, h, w)]
+    return [(b, 64 if section == L.SRNET_ENCODER else 3, big_h, big_w)]
+
+
+def _unreached(section, given):
+    """Parameter indices no given output gradient reaches (they keep grad None, as under autograd through the layers):
+    the heads without their output's gradient; in SRNetwork also the encoder and decoder without the image gradient,
+    and the prior trunk when neither the image nor a head has one."""
+    if section == L.SRNET_PRIOR:
+        return set(([0, 1] if not given[2] else []) + ([2] if not given[1] else []))
+    if section != L.SRNET_NETWORK:
+        return set()
+    dead = set(([52, 53] if not given[3] else []) + ([54] if not given[2] else []))
+    if not given[1]:
+        dead |= set(range(1006, 1108))
+        if not (given[2] or given[3]):
+            dead |= set(range(55, 1006))
+    return dead
+
+
+def _table(tensors):
+    return (C.c_void_p * len(tensors))(*[None if t is None else t.data_ptr() for t in tensors])
+
+
+def _flat_grads(params, dev):
+    """One zeroed flat fp32 buffer with a 16-byte aligned view per parameter (the native backward accumulates)."""
+    offs, tot = [], 0
+    for p in params:
+        offs.append(tot)
+        tot += (p.numel() + 3) // 4 * 4
+    flat = torch.zeros(tot, dtype=torch.float32, device=dev)
+    return flat, [flat[o:o + p.numel()].view(p.shape) for o, p in zip(offs, params)]
+
+
+class _SRProgram(torch.autograd.Function):
+    """One section as a native program (crfr_srnet_forward) with its own autograd node (crfr_srnet_backward)."""
+
+    @staticmethod
+    def forward(ctx, x, engine, section, need_grad, *params):
+        x = x.contiguous().float()
+        b, _, h, w = x.shape
+        outs = [torch.empty(s, dtype=torch.float32, device=x.device) for s in _out_shapes(section, b, h, w)]
+        nbytes = L.lib().crfr_srnet_workspace_bytes(section, b, h, w, 1 if need_grad else 0)
+        # a private workspace per call when a backward may follow: it holds the saved activations
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=x.device) if need_grad else ops.workspace(nbytes)
+        io = L.SrnetIO()
+        io.section, io.batch, io.h, io.w = section, b, h, w
+        io.x = x.data_ptr()
+        for i, o in enumerate(outs):
+            io.out[i] = o.data_ptr()
+        L.call("crfr_srnet_forward", engine, _table([p.detach() for p in params]), C.byref(io), 1 if need_grad else 0,
+               ws.data_ptr(), ws.numel(), ops.stream())
+        # only shapes are kept: outputs on ctx would close the cycle output -> grad_fn -> ctx -> output
+        ctx.engine, ctx.section, ctx.xshape, ctx.dev = engine, section, tuple(x.shape), x.device
+        ctx.ws = ws if need_grad else None
+        ctx.set_materialize_grads(False)
+        ctx.save_for_backward(*params)
+        return tuple(outs)
+
+    @staticmethod
+    def backward(ctx, *d_outs):
+        params = ctx.saved_tensors
+        _, grads = _flat_grads(params, ctx.dev)
+        b, _, h, w = ctx.xshape
+        io = L.SrnetIO()                       # the backward reads neither x nor the outputs
+        io.section, io.batch, io.h, io.w = ctx.section, b, h, w
+        keep = [None if d is None else d.contiguous().float() for d in d_outs]
+        darr = (C.c_void_p * 4)(*[None if d is None else d.data_ptr() for d in keep] + [None] * (4 - len(keep)))
+        dx = torch.empty(ctx.xshape, dtype=torch.float32, device=ctx.dev) if ctx.needs_input_grad[0] else None
+        L.call("crfr_srnet_backward", ctx.engine, _table([p.detach() for p in params]), _table(grads), C.byref(io), darr,
+               ops.ptr(dx), ctx.ws.data_ptr(), ctx.ws.numel(), ops.stream())
+        ctx.ws = None
+        dead = _unreached(ctx.section, [d is not None for d in keep] + [False] * (4 - len(keep)))
+        return (dx, None, None, None) + tuple(None if i in dead else g for i, g in enumerate(grads))
+
+
+_TABLES = {}
+
+
+def check_parameter_table(module, params):
+    """The program's channel counts are those of the reference's default constructor arguments: every parameter must
+    have the shape the default-constructed module gives it (checked on the host, before any launch)."""
+    cls = type(module)
+    if cls not in _TABLES:
+        ref = cls()
+        _TABLES[cls] = [tuple(t.shape) for t in ref.state_dict().values()]
+    want = _TABLES[cls]
+    got = [tuple(p.shape) for p in params]
+    if got != want:
+        bad = next(i for i in range(min(len(got), len(want)) + 1) if i >= len(got) or i >= len(want) or got[i] != want[i])
+        raise NotImplementedError(
+            "%s: the native program runs the reference's default configuration only; parameter %d has shape %s, the "
+            "program expects %s (%d parameters, %d expected)" % (cls.__name__, bad, got[bad] if bad < len(got) else None,
+                                                                  want[bad] if bad < len(want) else None, len(got),
+                                                                  len(want)))
+
+
+class _Program(nn.Module):
+    """forward(x) of a whole section: its parameters in state_dict order are the program's parameter table."""
+    _section = None
+    _in_channels = 3
+    engine = L.ENGINE_AUTO
+
+    def _run(self, x):
+        sd = dict(self.named_parameters())
+        params = [sd[k] for k in self.state_dict().keys()]
+        check_parameter_table(self, params)
+        _check(x, self._in_channels, self._section)
+        need_grad = torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in params))
+        return _SRProgram.apply(x, self.engine, self._section, need_grad, *params)
 
 
 class _Residual_Block(nn.Module):
@@ -39,12 +163,6 @@ class _Residual_Block(nn.Module):
         self.relu = nn.PReLU(out_channels)
         self.conv2 = nn.Conv2d(out_channels, out_channels, 3, 1, 1, bias=False)
         self.in2 = nn.InstanceNorm2d(out_channels, affine=True)
-
-    def run(self, x):
-        y = Fn.conv2d(x, self.conv1.weight, None, 1, 1)
-        a, _ = Fn.norm_act(y, self.in1.weight, self.in1.bias, alpha=self.relu.weight)
-        y = Fn.conv2d(a, self.conv2.weight, None, 1, 1)
-        return Fn.norm_act(y, self.in2.weight, self.in2.bias, res=x)[0]
 
 
 class Bottleneck(nn.Module):
@@ -63,15 +181,6 @@ class Bottleneck(nn.Module):
         self.downsample = downsample
         self.stride = stride
 
-    def run(self, x):
-        a, _ = Fn.norm_act(x, relu=True)
-        y = Fn.conv2d(a, self.conv1.weight, self.conv1.bias, 1, 0)
-        a, _ = Fn.norm_act(y, relu=True)
-        y = Fn.conv2d(a, self.conv2.weight, self.conv2.bias, self.stride, 1)
-        a, _ = Fn.norm_act(y, relu=True)
-        y = Fn.conv2d(a, self.conv3.weight, self.conv3.bias, 1, 0)
-        return Fn.add(y, x)
-
 
 class Hourglass(nn.Module):
     """ref: :117-156 (same recursion as model/FSRnet.py:176-215)."""
@@ -84,46 +193,6 @@ class Hourglass(nn.Module):
             nn.ModuleList(nn.Sequential(*[block(planes * block.expansion, planes) for _ in range(num_blocks)])
                           for _ in range(4 if d == 0 else 3))
             for d in range(depth))
-
-    @staticmethod
-    def _seq(seq, x):
-        for blk in seq:
-            x = blk.run(x)
-        return x
-
-    def _forward(self, n, x):
-        up1 = self._seq(self.hg[n - 1][0], x)
-        low1 = self._seq(self.hg[n - 1][1], Fn.max_pool2(x))
-        low2 = self._forward(n - 1, low1) if n > 1 else self._seq(self.hg[n - 1][3], low1)
-        low3 = self._seq(self.hg[n - 1][2], low2)
-        return Fn.up2_add(up1, low3)
-
-    def run(self, x):
-        return self._forward(self.depth, x)
-
-
-def _pad_conv(x, conv, pad, stride=1, c=None):
-    return Fn.conv2d(Fn.reflect_pad(x, pad, c), conv.weight, None, stride, 0)
-
-
-def _down_stage(seq, i, x):
-    """ReflectionPad(1) conv3x3 s2, ReflectionPad(1) conv3x3 s1, InstanceNorm, ReLU  (six Sequential entries from i)."""
-    y = _pad_conv(x, seq[i + 1], 1, 2)
-    y = _pad_conv(y, seq[i + 3], 1, 1)
-    return Fn.norm_act(y, relu=True)[0]
-
-
-def _up_stage(seq, i, x):
-    """ConvTranspose2d(3, 2, 1, 1), ReflectionPad(1) conv3x3, InstanceNorm, ReLU  (five Sequential entries from i)."""
-    y = Fn.conv_transpose2d(x, seq[i].weight, 2, 1, 1)
-    y = _pad_conv(y, seq[i + 2], 1, 1)
-    return Fn.norm_act(y, relu=True)[0]
-
-
-def _image_head(seq, x):
-    """ReflectionPad(1), conv3x3 -> 3 channels, Tanh; returns fp32 NCHW."""
-    y = Fn.conv2d(Fn.reflect_pad(x, 1), seq[1].weight, None, 1, 0)
-    return Fn.tanh(Fn.to_nchw(y, 3))
 
 
 def _trunk(ngf, n_blocks, stem):
@@ -141,19 +210,9 @@ def _trunk(ngf, n_blocks, stem):
     return m
 
 
-def _run_trunk(seq, i, x, n_blocks):
-    """Runs the body built by _trunk starting at Sequential index i."""
-    x = _down_stage(seq, i, x)
-    x = _down_stage(seq, i + 6, x)
-    for b in range(n_blocks):
-        x = seq[i + 12 + b].run(x)
-    j = i + 12 + n_blocks
-    x = _up_stage(seq, j, x)
-    return _up_stage(seq, j + 5, x)
-
-
-class Coarse_SR_Network(nn.Module):
+class Coarse_SR_Network(_Program):
     """ref: :251-301; forward(x) -> coarse image [B,3,H,W]."""
+    _section = L.SRNET_COARSE
 
     def __init__(self, ngf=64, n_blocks=6):
         super().__init__()
@@ -162,18 +221,13 @@ class Coarse_SR_Network(nn.Module):
         self.out = nn.Sequential(nn.ReflectionPad2d(1), nn.Conv2d(ngf, 3, 3, 1, 0, bias=False), nn.Tanh())
         self.n_blocks = n_blocks
 
-    def features(self, x4):
-        y = _pad_conv(x4, self.model[1], 3, 1, c=3)
-        a, _ = Fn.norm_act(y, relu=True)
-        return _run_trunk(self.model, 4, a, self.n_blocks)
-
     def forward(self, x):
-        _check(x, 3)
-        return _image_head(self.out, self.features(Fn.to_nhwc(x.float())))
+        return self._run(x)[0]
 
 
-class Fine_SR_Encoder(nn.Module):
+class Fine_SR_Encoder(_Program):
     """ref: :304-346; forward(x) -> features [B,ngf,H,W]."""
+    _section = L.SRNET_ENCODER
 
     def __init__(self, ngf=64, n_blocks=6):
         super().__init__()
@@ -181,17 +235,13 @@ class Fine_SR_Encoder(nn.Module):
         self.model = nn.Sequential(*_trunk(ngf, n_blocks, stem))
         self.n_blocks, self.ngf = n_blocks, ngf
 
-    def features(self, x4):
-        y = _pad_conv(x4, self.model[1], 1, 1, c=3)          # no norm / activation behind the first conv (:315-316)
-        return _run_trunk(self.model, 2, y, self.n_blocks)
-
     def forward(self, x):
-        _check(x, 3)
-        return Fn.to_nchw(self.features(Fn.to_nhwc(x.float())))
+        return self._run(x)[0]
 
 
-class Prior_Estimation_Network(nn.Module):
+class Prior_Estimation_Network(_Program):
     """ref: :349-376; forward(x) -> (features, landmark_out, parsing_out)."""
+    _section = L.SRNET_PRIOR
 
     def __init__(self, n_hourglass=4, n_blocks=2, ngf=64, parsing_classes=13, num_landmark=68):
         super().__init__()
@@ -202,42 +252,31 @@ class Prior_Estimation_Network(nn.Module):
         model += [Hourglass(planes=ngf, depth=4, block=Bottleneck, num_blocks=3) for _ in range(n_hourglass)]
         self.model = nn.Sequential(*model)
 
-    def features(self, x4):
-        y = _pad_conv(x4, self.model[1], 3, 1, c=3)
-        a, _ = Fn.norm_act(y, relu=True)
-        for m in list(self.model)[4:]:
-            a = m.run(a)
-        return a
-
     def forward(self, x):
-        _check(x, 3)
-        f = self.features(Fn.to_nhwc(x.float()))
-        parsing = Fn.to_nchw(Fn.conv2d(f, self.fc.weight, self.fc.bias, 1, 0), self.fc.out_channels)
-        landmark = Fn.to_nchw(Fn.conv2d(f, self.fc_landmark.weight, None, 1, 0), self.fc_landmark.out_channels)
-        return Fn.to_nchw(f), landmark, parsing
+        return self._run(x)
 
 
-class Fine_SR_Decoder(nn.Module):
+class Fine_SR_Decoder(_Program):
     """ref: :379-416; forward(x [B,ngf,H,W]) -> image [B,3,H,W]."""
+    _section = L.SRNET_DECODER
 
     def __init__(self, ngf=128, n_blocks=6):
         super().__init__()
         self.model = nn.Sequential(*_trunk(ngf, n_blocks, []))
         self.out = nn.Sequential(nn.ReflectionPad2d(1), nn.Conv2d(ngf, 3, 3, 1, 0, bias=False), nn.Tanh())
         self.n_blocks, self.ngf = n_blocks, ngf
-
-    def run(self, x):
-        return _image_head(self.out, _run_trunk(self.model, 0, x, self.n_blocks))
+        self._in_channels = ngf
 
     def forward(self, x):
-        _check(x, self.ngf)
-        return self.run(Fn.to_nhwc(x.float()))
+        return self._run(x)[0]
 
 
-class SRNetwork(nn.Module):
+class SRNetwork(_Program):
     """The wiring the reference's (unconstructible, :449) ``OverallNetwork`` of this file describes, with the classes that
     exist: coarse image -> encoder and prior network -> cat(prior, encoder) -> decoder;
-    forward(x) -> (coarse_out, out, landmark_out, parsing_out).  All activations stay NHWC bf16 between the sub-networks."""
+    forward(x) -> (coarse_out, out, landmark_out, parsing_out).  One native program: the prior and encoder features are
+    written straight into the two channel halves of the decoder's 128-channel input."""
+    _section = L.SRNET_NETWORK
 
     def __init__(self):
         super().__init__()
@@ -247,13 +286,4 @@ class SRNetwork(nn.Module):
         self._fine_sr_decoder = Fine_SR_Decoder()
 
     def forward(self, x):
-        coarse = self._coarse_sr_network(x)
-        c4 = Fn.to_nhwc(coarse)
-        enc = self._fine_sr_encoder.features(c4)
-        p = self._prior_estimation_network
-        pe = p.features(c4)
-        parsing = Fn.to_nchw(Fn.conv2d(pe, p.fc.weight, p.fc.bias, 1, 0), p.fc.out_channels)
-        landmark = Fn.to_nchw(Fn.conv2d(pe, p.fc_landmark.weight, None, 1, 0), p.fc_landmark.out_channels)
-        cat = torch.cat((pe, enc), 3)                    # channel concat = last NHWC axis
-        out = self._fine_sr_decoder.run(cat)
-        return coarse, out, landmark, parsing
+        return self._run(x)

@@ -41,6 +41,15 @@ class FsrnetSectionIO(C.Structure):
 FSRNET_COARSE, FSRNET_ENCODER, FSRNET_PRIOR, FSRNET_DECODER = 0, 1, 2, 3
 
 
+class SrnetIO(C.Structure):
+    _fields_ = [("section", ci), ("batch", ci), ("h", ci), ("w", ci), ("x", vp), ("out", vp * 4)]
+
+
+# SUPER_RESOLUTION FSRNet variant program (crfr_srnet_*): sections and their state_dict lengths
+SRNET_COARSE, SRNET_ENCODER, SRNET_PRIOR, SRNET_DECODER, SRNET_NETWORK = 0, 1, 2, 3, 4
+SRNET_NPARAMS = {SRNET_COARSE: 52, SRNET_ENCODER: 51, SRNET_PRIOR: 954, SRNET_DECODER: 51, SRNET_NETWORK: 1108}
+
+
 class ResnetIO(C.Structure):
     _fields_ = [("batch", ci), ("size", ci), ("x", vp), ("emb", vp), ("feat", vp * 4), ("training", ci),
                 ("momentum", cf), ("eps", cf)]
@@ -119,6 +128,11 @@ SIGNATURES = {
     "crfr_fsrnet_train_step": (ci, [ci, vp, vp, C.POINTER(FsrnetIO), vp, vp, csz, vp]),
     "crfr_fsrnet_id_workspace_bytes": (csz, [ci, ci, ci, ci]),
     "crfr_fsrnet_id_train_step": (ci, [ci, vp, vp, C.POINTER(FsrnetIO), C.POINTER(FsrnetIdIO), vp, vp, csz, vp]),
+    "crfr_srnet_workspace_bytes": (csz, [ci, ci, ci, ci, ci]),
+    "crfr_srnet_tape": (ci, [ci, ci, ci, ci, ci, C.POINTER(TapeEntry), ci]),
+    "crfr_srnet_grad_tape": (ci, [ci, ci, ci, ci, ci, ci, C.POINTER(TapeEntry), ci]),
+    "crfr_srnet_forward": (ci, [ci, vp, C.POINTER(SrnetIO), ci, vp, csz, vp]),
+    "crfr_srnet_backward": (ci, [ci, vp, vp, C.POINTER(SrnetIO), vp, vp, vp, csz, vp]),
     "crfr_bn_update_running": (ci, [vp, vp, vp, vp, ci, cll, cf, cf, vp]),
     "crfr_bn_running_to_stats": (ci, [vp, vp, ci, cf, vp, vp]),
     "crfr_resnet34_workspace_bytes": (csz, [ci, ci, ci]),

@@ -363,6 +363,67 @@ int crfr_fsrnet_id_train_step(int engine, const float* const* host_params, float
                               const crfr_fsrnet_io* io, const crfr_fsrnet_id_io* id, float* losses, void* ws,
                               size_t ws_bytes, void* stream);
 
+/* ----------------------------------------------------------- SUPER_RESOLUTION FSRNet variant program ---- */
+/* ref: SUPER_RESOLUTION/model/FSRnet.py:251-416 (Coarse_SR_Network, Fine_SR_Encoder, Prior_Estimation_Network,
+ * Fine_SR_Decoder) and the SRNetwork wiring of its unconstructible OverallNetwork (:449): coarse image -> encoder and
+ * prior network -> cat(prior, encoder) -> decoder.  One call per forward and per backward over a caller-provided arena;
+ * every layer keeps the routing of crfr_conv_fwd / _dgrad / _wgrad, the two 1x1 prior heads (fc 13 channels with bias,
+ * fc_landmark 68 without) run as one tensor-core GEMM 64 -> 128.
+ * params / grads: device pointers in the section's state_dict order - CRFR_SRNET_NPARAMS for SRNetwork
+ * (_coarse_sr_network, _prior_estimation_network, _fine_sr_encoder, _fine_sr_decoder), 52 / 51 / 954 / 51 for the
+ * coarse network / encoder / prior network / decoder alone.
+ * Shapes (h and w separately; what the composed modules compute without a size mismatch):
+ *   coarse, encoder, decoder: h, w >= 5 (the second stride-2 stage's reflection pad needs 2 rows); their outputs are
+ *     4 * ceil(h / 4) x 4 * ceil(w / 4) (two stride-2 stages, two exact 2x transposed stages);
+ *   prior, SRNetwork: h, w multiples of 16 (the hourglass pools four times and adds the up-sampled map back);
+ *   batch * (4 * ceil(h / 4) + 6) * (4 * ceil(w / 4) + 6) * 128 < 2^31 (element indices of the widest padded map).
+ * Anything else is CRFR_EINVAL before any launch; the size query returns 0 and the tape -1.  The tables must come from
+ * modules built with the reference's default constructor arguments (the program's channel counts are fixed). */
+#define CRFR_SRNET_NPARAMS 1108
+enum { CRFR_SRNET_COARSE = 0, CRFR_SRNET_ENCODER = 1, CRFR_SRNET_PRIOR = 2, CRFR_SRNET_DECODER = 3,
+       CRFR_SRNET_NETWORK = 4 };
+typedef struct crfr_srnet_io {
+  int section, batch, h, w;
+  const float* x;   /* fp32 NCHW [B,3,h,w]; decoder: [B,128,h,w] */
+  float* out[4];    /* fp32 NCHW, (H, W) = the output size above:
+                       SRNetwork {coarse [B,3,h,w], out [B,3,h,w], landmark [B,68,h,w], parsing [B,13,h,w]};
+                       coarse {[B,3,H,W]}; encoder {[B,64,H,W]}; prior {feat [B,64,h,w], landmark, parsing};
+                       decoder {[B,3,H,W]} */
+} crfr_srnet_io;
+/* ref: SUPER_RESOLUTION/model/FSRnet.py:251-416.  The arena of one call; training != 0 also holds what the backward
+ * needs (a backward follows a training forward over the same arena).  0 for an unsupported shape. */
+size_t crfr_srnet_workspace_bytes(int section, int batch, int h, int w, int training);
+/* ref: SUPER_RESOLUTION/model/FSRnet.py:251-416.  Layout of the stored forward tensors (a dry run, as crfr_fsrnet_tape):
+ * one entry per op in program order, offsets from the workspace base.  Kinds: 0 convolution (w_idx: its weight; the
+ * input is the stored padded map), 1 InstanceNorm (+ affine) (+ ReLU / PReLU) (+ residual), 2 max-pool, 3 nearest-up + add
+ * (stats_off: the low-resolution input), 4 concat view (out: the decoder's 128-channel input, in_off / stats_off: its prior
+ * / encoder halves), 5 the combined prior heads (w_idx: fc.weight; in_off: the features; out_off -1, the outputs go to
+ * the caller), 20 reflection pad (w_idx: the padding), 21 Bottleneck add (in_off: conv3's output, stats_off: the block
+ * input), 22 Tanh image head (in_off: the 3-channel bf16 NHWC4 convolution output; out_off: the bf16 NHWC4 copy of the
+ * coarse image inside SRNetwork, else -1). */
+int crfr_srnet_tape(int section, int batch, int h, int w, int training, crfr_tape_entry* entries, int max_entries);
+/* ref: SUPER_RESOLUTION/model/FSRnet.py:251-416.  Where crfr_srnet_backward leaves its bf16 gradients in the workspace (a
+ * dry run of that call, in backward order; offsets from the workspace base).  grad_mask: bit i set = d_out[i] given (at
+ * least one, only the section's outputs); input_grad: dx requested.  Kind 30: a gradient the op at forward-tape index
+ * w_idx consumes for its output (one entry per summed slot; n, h, w, c the tensor's, ld the buffer's; in_off the
+ * crfr_srnet_tape offset of the tensor, -1 for the prior heads' gathered [pixel][128] output gradient).  Kind 31: a
+ * gradient that op produces for an input (has_res: 0 first input, 1 second - residual, Bottleneck input, low-resolution
+ * map, encoder half; in_off: that input's offset).  A tensor's producer consumes the sum of the kind-31 gradients of its
+ * consumers.  Gradients that only pass through (add, concat, up-add's first input) share the consumed buffer.  Returns the
+ * count, -1 on bad arguments. */
+int crfr_srnet_grad_tape(int section, int batch, int h, int w, int grad_mask, int input_grad, crfr_tape_entry* entries,
+                         int max_entries);
+/* ref: SUPER_RESOLUTION/model/FSRnet.py:251-416, forward of the section io->section.  ws_bytes below
+ * crfr_srnet_workspace_bytes is CRFR_EWORKSPACE with nothing written. */
+int crfr_srnet_forward(int engine, const float* const* host_params, const crfr_srnet_io* io, int training, void* ws,
+                       size_t ws_bytes, void* stream);
+/* ref: autograd through SUPER_RESOLUTION/model/FSRnet.py:251-416.  ws holds a training forward of the same section and
+ * shape (x and out are not read).  d_out[i]: fp32 gradient of io->out[i], NULL = none.  Parameter gradients are
+ * accumulated into host_grads (NULL entries skipped); dx (optional, the shape of x) is overwritten with the input
+ * gradient.  The saved forward is not modified: repeated calls give the same bits. */
+int crfr_srnet_backward(int engine, const float* const* host_params, float* const* host_grads, const crfr_srnet_io* io,
+                        const float* const* d_out, float* dx, void* ws, size_t ws_bytes, void* stream);
+
 /* ---------------------------------------------------------------- ResNet_34 embedding network program ------ */
 #define CRFR_RESNET34_NPARAMS 114 /* named_parameters() order of model/resnet.py:ResNet_34 */
 #define CRFR_RESNET34_NBN 38      /* BatchNorm layers in module order */

@@ -1,5 +1,5 @@
 """Convolution shape classes of the SUPER_RESOLUTION FSRNet variant: CUDA-core direct kernels against the tensor-core paths,
-and SRNetwork forward + backward with and without them.
+and SRNetwork forward + backward as the network program against the op-by-op composition.
 
 Usage: python tools/bench_sr_variant.py [--batch 32] [--iters 20] [--warmup 3] [--skip-layers] [--skip-net]
        python tools/bench_sr_variant.py --profile      (its own run: the kernels of one shipped forward + backward)
@@ -8,15 +8,16 @@ Usage: python tools/bench_sr_variant.py [--batch 32] [--iters 20] [--warmup 3] [
    on ENGINE_AUTO (the tensor-core paths), CUDA events around 10 launches after 3 warm-up launches.  The inputs rotate
    over as many copies as exceed 256 MB, twice the 126 MB L2, so the operands come from HBM.  FLOP/s are 2 x the
    algorithm's MACs over the measured time.
-2. SRNetwork forward + backward at 128 x 128 (loss = sum of the four outputs times fixed random gradients), two arms
-   alternating iteration by iteration, --iters timed after --warmup, medians:
-     shipped - crfr_b200.functional as it is;
-     old     - crfr_b200.functional.conv2d / conv_transpose2d pinned to ENGINE_DIRECT for the shapes that the tensor-core
-               paths of this change cover (3x3 / 7x7 padding 0, 1x1 stride 1, 3x3 stride-2 transposed): the routing before
-               them, in the same process.  The other layers (3x3 padding 1) stay on ENGINE_AUTO in both arms.
-3. --profile: torch.profiler over one shipped forward + backward after a warm-up; every kernel with its count and total
-   time, and the CUDA-core convolution kernels (gather_down_kernel, gather_up_kernel, wgrad_kernel) with the layer
-   shapes that still call them.
+2. SRNetwork forward + backward at 128 x 128 (loss = sum of the four outputs times fixed random gradients), three arms
+   alternating step by step, --iters timed after --warmup, CUDA events, medians.  The inputs rotate over as many batches
+   as exceed 256 MB:
+     program  - the module (crfr_srnet_forward / crfr_srnet_backward, one autograd node), eagerly;
+     graph    - the same two calls captured once into a CUDA graph over a fixed workspace, replayed;
+     composed - the op-by-op composition the module ran before (oracle/sr_composed.py).
+   Also launches per forward + backward (crfr_launch_count) for each arm and the workspace bytes per image.
+3. --profile: torch.profiler over one program forward + backward after a warm-up; every kernel with its count and total
+   time, the CUDA-core convolution kernels (gather_down_kernel, gather_up_kernel, wgrad_kernel), and the prior heads'
+   own kernels (sr_heads_*) and their GEMM (the one tc_gemm launch of 64 -> 128 channels, timed with CUDA events).
 Prints the device name and power limit, then one JSON line.  Writes nothing.
 """
 import argparse
@@ -53,13 +54,6 @@ def out_size(k, stride, pad, transposed, size):
 def macs(batch, cin, cout, k, stride, pad, transposed, size):
     o = out_size(k, stride, pad, transposed, size)
     return batch * (size * size if transposed else o * o) * cin * cout * k * k
-
-
-def is_new_class(cin, cout, k, stride, pad, transposed):
-    """The shapes whose tensor-core paths this benchmark measures (the rest were on the tensor cores before)."""
-    if transposed:
-        return k == 3 and stride == 2
-    return (k == 1 and stride == 1) or (pad == 0 and k in (3, 7))
 
 
 def time_layers(batch, gpu):
@@ -111,20 +105,70 @@ def time_layers(batch, gpu):
     return rows
 
 
-def pin_old_routing(Fn, L):
-    """crfr_b200.functional.conv2d / conv_transpose2d with the new shape classes pinned to ENGINE_DIRECT."""
-    conv2d, convT = Fn.conv2d, Fn.conv_transpose2d
+def graph_step(net, xs, grads, L):
+    """crfr_srnet_forward + crfr_srnet_backward on a fixed workspace, captured into one CUDA graph; returns replay(i)
+    for input batch i (the batches are copied into the captured input buffer first)."""
+    import ctypes as C
+    import torch
+    from crfr_b200 import ops
+    b, _, h, w = xs[0].shape
+    sd = dict(net.named_parameters())
+    params = [sd[k].detach() for k in net.state_dict().keys()]
+    pgrads = [torch.zeros_like(p) for p in params]
+    table = lambda ts: (C.c_void_p * len(ts))(*[t.data_ptr() for t in ts])
+    ws = torch.empty(L.lib().crfr_srnet_workspace_bytes(L.SRNET_NETWORK, b, h, w, 1), dtype=torch.uint8, device=xs[0].device)
+    x = xs[0].clone()
+    outs = [torch.empty(g.shape, device=x.device) for g in grads]
+    io = L.SrnetIO()
+    io.section, io.batch, io.h, io.w, io.x = L.SRNET_NETWORK, b, h, w, x.data_ptr()
+    for i, o in enumerate(outs):
+        io.out[i] = o.data_ptr()
+    pt, gt, dt = table(params), table(pgrads), table(grads)
 
-    def conv2d_old(x, weight, bias=None, stride=1, pad=0, engine=L.ENGINE_AUTO):
-        cout, cin, k = weight.shape[0], weight.shape[1], weight.shape[2]
-        if is_new_class(cin, cout, k, stride, pad, False):
-            engine = L.ENGINE_DIRECT
-        return conv2d(x, weight, bias, stride, pad, engine)
+    def calls():
+        for t in pgrads:
+            t.zero_()
+        L.call("crfr_srnet_forward", L.ENGINE_AUTO, pt, C.byref(io), 1, ws.data_ptr(), ws.numel(), ops.stream())
+        L.call("crfr_srnet_backward", L.ENGINE_AUTO, pt, gt, C.byref(io), dt, None, ws.data_ptr(), ws.numel(), ops.stream())
 
-    def convT_old(x, weight, stride, pad, out_pad, engine=L.ENGINE_AUTO):
-        return convT(x, weight, stride, pad, out_pad, L.ENGINE_DIRECT)
+    side = torch.cuda.Stream()
+    side.wait_stream(torch.cuda.current_stream())
+    with torch.cuda.stream(side):
+        calls()
+    torch.cuda.current_stream().wait_stream(side)
+    graph = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(graph):
+        calls()
 
-    return (conv2d, convT), (conv2d_old, convT_old)
+    def replay(i):
+        x.copy_(xs[i])
+        graph.replay()
+    return replay, ws.numel()
+
+
+def time_heads_gemm(B, S, dev):
+    """The prior heads' 1x1 GEMMs at the program's shapes (recipe 6 stands in: 64 -> 128 forward, 128 -> 64 dgrad,
+    X^T dY wgrad), CUDA events around 10 launches after 3 warm-up launches."""
+    import torch
+    from crfr_b200 import ops
+    x = torch.randn(B, S, S, 64, device=dev).bfloat16()
+    dy = torch.randn(B, S, S, 128, device=dev).bfloat16()
+    w = torch.randn(128, 64, 1, 1, device=dev) / 8
+    wp, wt = ops.pack_conv_weight(w), ops.pack_conv_weight(w, for_dgrad=True)
+    fns = [lambda: ops.conv_fwd(x, wp, 64, 128, 1, 1, 0), lambda: ops.conv_dgrad(dy, wt, tuple(x.shape), 64, 128, 1, 1, 0),
+           lambda: ops.conv_wgrad(x, dy, 64, 128, 1, 1, 0)]
+    out = []
+    for fn in fns:
+        for _ in range(3):
+            fn()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        for _ in range(10):
+            fn()
+        e1.record()
+        torch.cuda.synchronize()
+        out.append(e0.elapsed_time(e1) * 100.0)
+    return out
 
 
 def main():
@@ -141,7 +185,6 @@ def main():
     crfr_b200.build()
     from bench_ir50_grad import gpu_info
     from crfr_b200 import _lib as L
-    from crfr_b200 import functional as Fn
     from crfr_b200.SUPER_RESOLUTION.model.FSRnet import SRNetwork
     assert torch.cuda.is_available(), "this benchmark needs a CUDA device"
     gpu = gpu_info()
@@ -153,23 +196,21 @@ def main():
     net = SRNetwork().to(dev).train() if (args.profile or not args.skip_net) else None
     B, S = args.batch, 128
     g = torch.Generator(device=dev).manual_seed(11)
-    x = torch.randn(B, 3, S, S, device=dev, generator=g)
-    grads = None
+    copies = max(2, -(-(256 << 20) // (B * 3 * S * S * 4)))
+    xs = [torch.randn(B, 3, S, S, device=dev, generator=g) for _ in range(copies)]
+    grads = [torch.randn(s, device=dev, generator=g) for s in [(B, 3, S, S), (B, 3, S, S), (B, 68, S, S), (B, 13, S, S)]]
 
-    def step():
-        nonlocal grads
+    def step(i, fwd=None):
         net.zero_grad(set_to_none=True)
-        outs = net(x)
-        if grads is None:
-            grads = [torch.randn(o.shape, device=dev, generator=g) for o in outs]
+        outs = (fwd or net)(xs[i % copies])
         torch.autograd.backward(outs, grads)
 
     if args.profile:
         from torch.profiler import ProfilerActivity, profile
-        step()
+        step(0)
         torch.cuda.synchronize()
         with profile(activities=[ProfilerActivity.CUDA]) as prof:
-            step()
+            step(1)
             torch.cuda.synchronize()
         kern = {}
         for ev in prof.events():
@@ -182,39 +223,50 @@ def main():
             print("  %9.1f us %5d x  %s" % (t, c, name[:150]))
         cuda_core = re.compile(r"(^|[^a-z_])(gather_down_kernel|gather_up_kernel|wgrad_kernel)\b")
         direct = {n: v for n, v in kern.items() if cuda_core.search(n)}
-        # the layers that still reach the CUDA-core kernels: the 13- and 68-channel 1x1 prior heads, the 3x3 stem's dgrad
         direct_us = sum(t for _, t in direct.values())
+        heads = {n: v for n, v in kern.items() if "sr_heads" in n}
+        heads_us = sum(t for _, t in heads.values())
         print("CUDA-core convolution kernels: %s, %.1f us of %.1f us (%.2f %%)" % (
             {n[:60]: c for n, (c, _) in direct.items()}, direct_us, total, 100.0 * direct_us / max(total, 1e-9)))
+        gemm_us = time_heads_gemm(B, S, dev)
+        print("prior heads: sr_heads_* kernels %.1f us (%s), 64 -> 128 GEMM forward %.1f us, dgrad %.1f us, wgrad %.1f us"
+              % (heads_us, {n[:40]: c for n, (c, _) in heads.items()}, *gemm_us))
         result["profile"] = {"total_kernel_us": total, "direct_conv_us": direct_us,
-                             "direct_conv_kernels": {n[:80]: c for n, (c, _) in direct.items()}}
+                             "direct_conv_kernels": {n[:80]: c for n, (c, _) in direct.items()},
+                             "heads_kernels_us": heads_us, "heads_gemm_fwd_dgrad_wgrad_us": gemm_us}
         print(json.dumps(result))
         return
 
     if not args.skip_layers:
         result["layers"] = time_layers(args.batch, gpu)
     if not args.skip_net:
-        (c2, ct), (c2_old, ct_old) = pin_old_routing(Fn, L)
-        arms = {"shipped": (c2, ct), "old_routing": (c2_old, ct_old)}
+        from oracle import sr_composed as SC
+        replay, ws_bytes = graph_step(net, xs, grads, L)
+        arms = {"program": lambda i: step(i), "graph": replay, "composed": lambda i: step(i, lambda t: SC.network(net, t))}
         times = {a: [] for a in arms}
-        try:
-            for it in range(args.warmup + args.iters):
-                for arm, (a, b) in arms.items():
-                    Fn.conv2d, Fn.conv_transpose2d = a, b
-                    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                    e0.record()
-                    step()
-                    e1.record()
-                    torch.cuda.synchronize()
-                    if it >= args.warmup:
-                        times[arm].append(e0.elapsed_time(e1))
-        finally:
-            Fn.conv2d, Fn.conv_transpose2d = c2, ct
+        launches = {}
+        for it in range(args.warmup + args.iters):
+            for arm, fn in arms.items():
+                torch.cuda.synchronize()
+                n0 = L.lib().crfr_launch_count()
+                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                e0.record()
+                fn(it)
+                e1.record()
+                torch.cuda.synchronize()
+                launches[arm] = L.lib().crfr_launch_count() - n0
+                if it >= args.warmup:
+                    times[arm].append(e0.elapsed_time(e1))
         med = {a: statistics.median(v) for a, v in times.items()}
         for a, v in times.items():
-            print("SRNetwork fwd+bwd batch %d, %-11s median %.2f ms  min %.2f  max %.2f" % (B, a, med[a], min(v), max(v)))
-        print("speed-up of the shipped routing: %.2fx" % (med["old_routing"] / med["shipped"]))
+            print("SRNetwork fwd+bwd batch %d, %-8s median %.2f ms  min %.2f  max %.2f  (%d native launches per step)"
+                  % (B, a, med[a], min(v), max(v), launches[a]))
+        print("program speed-up over the composed path: %.2fx eager, %.2fx graph"
+              % (med["composed"] / med["program"], med["composed"] / med["graph"]))
+        print("workspace: %.1f MB per image (training arena %.2f GB at batch %d)" % (ws_bytes / B / 2 ** 20, ws_bytes / 2 ** 30, B))
         result["net_median_ms"] = med
+        result["launches_per_step"] = launches
+        result["workspace_bytes_per_image"] = ws_bytes / B
     print(json.dumps(result))
 
 
